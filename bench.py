@@ -5,6 +5,7 @@
                     [--scaling weak|strong]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the reference's own ctc_best_path on the host cores
+    python bench.py --dump-outputs DIR ...    # also write the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one pass of the hot path over one batch of synthetic lattices.  The default
 workload is BASELINE config 2 (10 000 silence-split segments of 1-10 s: T_b ~ U{86..861},
@@ -30,8 +31,10 @@ import contextlib
 import io
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -315,8 +318,6 @@ def sub_record(name, seed, steps, dev, peak, files_dir=None):
         del d_lp
     if files_dir:   # files -> files: run_example.py:247-254's loop over *.logits.npz / *.voca.txt
         from kokoro_align_b200 import encoder
-        import shutil
-        os.makedirs(files_dir, exist_ok=True)
         tokens = list(encoder.VOCAB[1:])
         rng = np.random.default_rng(seed + 2)
         lf, vf, bf = [], [], []
@@ -340,9 +341,28 @@ def sub_record(name, seed, steps, dev, peak, files_dir=None):
             walls[mode] = time.perf_counter() - t0
             assert len(written) == len(T)
         rec["files_to_files_s"] = {"log_softmax_numpy_host": walls["host_numpy"], "log_softmax_device": walls["device"],
-                                   "what": f"{len(T)} *.logits.npz + *.voca.txt -> *.best_path.npz (align.best_path_files, /dev/shm)"}
-        shutil.rmtree(files_dir, ignore_errors=True)
+                                   "what": f"{len(T)} *.logits.npz + *.voca.txt -> *.best_path.npz (align.best_path_files, {os.path.dirname(files_dir)})"}
     return rec
+
+
+DUMP_BYTES = 64_000_000 - 4096     # --dump-outputs: 64 MB in all, .npy headers included
+
+
+def dump_outputs(dirname, outs, t_off, budget, suffix=""):
+    """--dump-outputs: what AlignPlan.run_torch returned (best_path, best_labels, best_scores per frame;
+    final_score, status per lattice) as DIR/<name><suffix>.npy in float32, exact for these integers
+    (all below 2^24).  When the batch's outputs exceed `budget` bytes, a fixed seeded sample of whole
+    lattices is kept; lattice_index.npy names them, their frames stay in batch order."""
+    path, labs, scores, final, status = (x.cpu().numpy() for x in outs)
+    T = np.diff(t_off)
+    order = np.random.default_rng(0).permutation(len(T))
+    keep = np.zeros(len(T), bool)
+    keep[order[np.cumsum(12 * T[order] + 12) <= budget]] = True    # 3 float32 per frame, 3 per lattice
+    rows = np.repeat(keep, T)
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in (("best_path", path[rows]), ("best_labels", labs[rows]), ("best_scores", scores[rows]),
+                    ("final_score", final[keep]), ("status", status[keep]), ("lattice_index", np.flatnonzero(keep))):
+        np.save(os.path.join(dirname, f"{name}{suffix}.npy"), a.astype(np.float32))
 
 
 def main():
@@ -358,7 +378,10 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the gon / book / hand-off sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -499,7 +522,7 @@ def main():
         def with_plan():
             with align.AlignPlan(t_off, labels, l_off, 39, device=local_rank) as p2:
                 p2.run_host(h_lp.numpy(), out=h_out_np)
-        wp_s = timed_host(with_plan, reps=max(3, args.steps // 2))
+        wp_s = timed_host(with_plan)
         extras["e2e_with_plan"] = {"value": cells_all / wp_s, "unit": UNIT, "ms_per_step": wp_s * 1e3,
                                    "note": "kab_plan_create + kab_plan_run_host + kab_plan_destroy per step"}
 
@@ -572,8 +595,16 @@ def main():
         plan.close()
         del d_lp, h_lp
         align.trim_pool()
-        subs["gon"] = sub_record("gon", 1000, max(5, args.steps // 2), dev, peak)
-        subs["book"] = sub_record("chapters", args.seed, max(5, args.steps // 2), dev, peak, files_dir="/dev/shm/kab_bench_book")
+        subs["gon"] = sub_record("gon", 1000, args.steps, dev, peak)
+        # the book's files go to a fresh directory, in /dev/shm when writable (no disk I/O in the wall time)
+        book_dir = tempfile.mkdtemp(prefix="kab_bench_book_", dir="/dev/shm" if os.access("/dev/shm", os.W_OK) else None)
+        try:
+            subs["book"] = sub_record("chapters", args.seed, args.steps, dev, peak, files_dir=book_dir)
+        finally:
+            shutil.rmtree(book_dir, ignore_errors=True)
+
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs, t_off, DUMP_BYTES // world, f"_rank{rank}" if world > 1 else "")
 
     if rank == 0:
         achieved = int(info.algorithmic_bytes) / (kernel_ms * 1e-3) / 1e9
