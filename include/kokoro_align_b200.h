@@ -91,6 +91,21 @@ int kab_device_count(int *count);
 int kab_plan_create(kab_plan **plan, int device, int64_t n_lattices, const int64_t *t_off,
                     const int32_t *labels, const int64_t *l_off, int32_t vocab_size,
                     int32_t beam_size, int32_t max_move);
+/*
+ * A plan in CTC forced-alignment mode: the recurrence of torchaudio.functional.forced_align (three
+ * moves, +2 forbidden into a blank and between equal labels, select on the previous frame's scores
+ * with its tie rule, the better of the last two states at the end; DESIGN.md 3.9), for a batch.
+ * `blank` in [0, vocab_size) is the blank id; labels are token ids in [0, vocab_size) other than it.
+ * Every kab_plan_run_* entry takes such a plan: best_path = extended-state index, best_labels =
+ * token id per frame (`blank` on even states), best_scores = log_probs[t, best_labels[t]],
+ * final_score = DP score of the chosen end state.  Statuses: KAB_ST_DEAD_BAND when T_b < L_b + R_b
+ * (R_b = adjacent equal labels; decided here), KAB_ST_BAD_LABEL for a label outside [0, V) or equal
+ * to the blank, KAB_ST_NONFINITE for a NaN or +inf log-prob (-inf is accepted: masking).
+ * kab_plan_segment_stats_device and kab_plan_run_host_segments return KAB_E_UNSUPPORTED.
+ * KAB_E_BAD_ARG for a blank outside [0, vocab_size).
+ */
+int kab_plan_create_ctc(kab_plan **plan, int device, int64_t n_lattices, const int64_t *t_off,
+                        const int32_t *labels, const int64_t *l_off, int32_t vocab_size, int32_t blank);
 int kab_plan_get_info(const kab_plan *plan, kab_plan_info *info);
 int kab_plan_destroy(kab_plan *plan);
 

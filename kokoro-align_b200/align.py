@@ -60,6 +60,20 @@ class AlignPlan:
     """
 
     def __init__(self, t_off, labels, l_off, vocab_size, beam_size=1000, max_move=4, device=0):
+        self._setup(t_off, labels, l_off, vocab_size, device)
+        self._create(_lib.lib().kab_plan_create, int(beam_size), int(max_move))
+
+    @classmethod
+    def ctc(cls, t_off, labels, l_off, vocab_size, blank=0, device=0):
+        """A plan in CTC forced-alignment mode (kab_plan_create_ctc): torchaudio's forced_align
+        recurrence for every lattice of the batch; labels are token ids in [0, vocab_size) other
+        than ``blank``.  best_labels are then token ids per frame (``blank`` on even states)."""
+        plan = cls.__new__(cls)
+        plan._setup(t_off, labels, l_off, vocab_size, device)
+        plan._create(_lib.lib().kab_plan_create_ctc, int(blank))
+        return plan
+
+    def _setup(self, t_off, labels, l_off, vocab_size, device):
         self.t_off = np.ascontiguousarray(t_off, dtype=np.int64)
         self.l_off = np.ascontiguousarray(l_off, dtype=np.int64)
         self.labels = np.ascontiguousarray(labels).astype(np.int32, copy=False)
@@ -69,10 +83,11 @@ class AlignPlan:
         self.total_T = int(self.t_off[-1]) if self.B else 0
         self.device = int(device)
         self._h = ctypes.c_void_p(0)
+
+    def _create(self, create, *mode_args):
         L = _lib.lib()
-        _lib.check(L.kab_plan_create(ctypes.byref(self._h), self.device, self.B, _ptr(self.t_off),
-                                     _ptr(self.labels), _ptr(self.l_off), self.V, int(beam_size),
-                                     int(max_move)))
+        _lib.check(create(ctypes.byref(self._h), self.device, self.B, _ptr(self.t_off), _ptr(self.labels),
+                          _ptr(self.l_off), self.V, *mode_args))
         info = PlanInfo()
         _lib.check(L.kab_plan_get_info(self._h, ctypes.byref(info)))
         self.info = info
@@ -225,6 +240,143 @@ def ctc_best_path(log_probs, labels, beam_size=1000, max_move=4, return_final_sc
     if return_final_score:
         return path, labs, scores, final[0]
     return path, labs, scores
+
+
+# ---------------------------------------------------------------- CTC forced alignment
+# torchaudio.functional.forced_align's recurrence (three moves, its tie rule, the better of the last
+# two states at the end; DESIGN.md 3.9) on the CTC plans of the C ABI (kab_plan_create_ctc).
+
+def _ctc_item_checks(tg, V, blank, where=""):
+    """torchaudio's checks of one item, in its order and with its exception types.  tg: int64
+    numpy [L].  Returns R, the number of adjacent equal targets."""
+    if (tg == blank).any():
+        raise ValueError(f"{where}targets Tensor shouldn't contain blank index. Found {tg}.")
+    if tg.size == 0:
+        raise RuntimeError(f"{where}targets must not be empty")
+    if tg.max() >= V:
+        raise ValueError(f"{where}targets values must be less than the CTC dimension")
+    if tg.min() < 0:
+        raise ValueError(f"{where}targets values must be non-negative")
+    return int((tg[1:] == tg[:-1]).sum())
+
+
+def _ctc_tensor_checks(log_probs, targets, blank):
+    import torch
+    if log_probs.dim() != 3:
+        raise RuntimeError("log_probs must be 3-D (batch_size, input length, num classes)")
+    if targets.dim() != 2:
+        raise RuntimeError("targets must be 2-D (batch_size, target length,)")
+    if log_probs.dtype != torch.float32:
+        raise RuntimeError(f"log_probs must be float32 (the kernels align in fp32), got {log_probs.dtype}")
+    if targets.dtype not in (torch.int32, torch.int64):
+        raise RuntimeError(f"targets must be int32 or int64, got {targets.dtype}")
+    if targets.device != log_probs.device:
+        raise RuntimeError("log_probs and targets must be on the same device")
+    if not 0 <= blank < log_probs.shape[-1]:
+        raise RuntimeError("blank must be within [0, num classes)")
+
+
+def _ctc_lengths(lengths, B, full, what):
+    """input_lengths / target_lengths -> int64 numpy [B] (None: every item is `full` long)."""
+    if lengths is None:
+        return np.full(B, full, np.int64)
+    n = np.asarray(lengths.cpu() if hasattr(lengths, "cpu") else lengths, dtype=np.int64)
+    if n.ndim != 1 or n.shape[0] != B:
+        raise RuntimeError(f"{what} must be 1-D (batch_size,)")
+    if B and (n.min() < 0 or n.max() > full):
+        raise RuntimeError(f"{what} must lie in [0, {full}]")
+    return n
+
+
+def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, blank=0):
+    """Drop-in for torchaudio.functional.forced_align (same arguments, output shapes and dtypes,
+    exception types): log_probs float32 [1, T, V], targets int32 / int64 [1, L] on the same device
+    (CPU or CUDA).  Returns (paths [1, T] of the targets' dtype: the token id of every frame,
+    scores float32 [1, T]: log_probs[0, t, paths[0, t]]) on the input's device; the output is what
+    torchaudio.functional.merge_tokens takes.  Bit-exact with torchaudio's CPU implementation
+    whenever the chosen end state has a finite score (where both end states are -inf, torchaudio's
+    traceback is undefined; this one follows the recurrence, DESIGN.md 3.9).  NaN or +inf
+    log-probs raise ValueError (-inf, for masking, is accepted)."""
+    import torch
+    _ctc_tensor_checks(log_probs, targets, blank)
+    if log_probs.size(0) != 1 or targets.size(0) != 1:
+        raise RuntimeError("The batch dimension for log_probs and targets must be 1 (forced_align_batch takes batches)")
+    T, V = int(log_probs.shape[1]), int(log_probs.shape[2])
+    if int(_ctc_lengths(input_lengths, 1, T, "input_lengths").max()) != T:
+        raise RuntimeError("input length mismatch")
+    L = int(targets.shape[1])
+    if target_lengths is not None and int(_ctc_lengths(target_lengths, 1, L, "target_lengths").max()) != L:
+        raise RuntimeError("target length mismatch")
+    tg = targets[0].cpu().numpy().astype(np.int64)
+    R = _ctc_item_checks(tg, V, blank)
+    if T < L + R:
+        raise RuntimeError(f"targets length is too long for CTC. Found log_probs length: {T}, targets length: {L}, "
+                           f"and number of repeats: {R}")
+    dev = log_probs.device
+    with AlignPlan.ctc([0, T], tg, [0, L], V, blank,
+                       device=dev.index if dev.type == "cuda" else _current_device()) as plan:
+        if dev.type == "cuda":
+            with torch.cuda.device(dev):
+                _, labs, scores, _, status = plan.run_torch(log_probs[0].contiguous())
+                status = int(status[0])   # (synchronises: the plan is destroyed below)
+        else:
+            _, labs, scores, _, st = plan.run_host(log_probs[0].contiguous().numpy())
+            labs, scores, status = torch.from_numpy(labs), torch.from_numpy(scores), int(st[0])
+    if status == ST_NONFINITE:
+        raise ValueError("log_probs must not contain NaN or +inf")
+    raise_for_status(status, V)
+    return labs.to(targets.dtype).view(1, T), scores.view(1, T)
+
+
+def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=None, blank=0):
+    """forced_align for a padded batch, in one plan: log_probs float32 [B, T_max, V], targets
+    int32 / int64 [B, L_max], input_lengths / target_lengths [B] (None: all full length).  Item b
+    is aligned over its first input_lengths[b] frames and target_lengths[b] targets.  Returns
+    (paths [B, T_max] of the targets' dtype, scores float32 [B, T_max]) on the input's device;
+    frames past an item's length hold the blank and score 0.  Raises, like forced_align, for the
+    first item that fails, naming its index.  On CUDA the valid rows are packed on the device."""
+    import torch
+    _ctc_tensor_checks(log_probs, targets, blank)
+    B, T_max, V = (int(x) for x in log_probs.shape)
+    if targets.size(0) != B:
+        raise RuntimeError(f"log_probs and targets hold {B} and {targets.size(0)} items")
+    L_max = int(targets.shape[1])
+    tl = _ctc_lengths(input_lengths, B, T_max, "input_lengths")
+    ll = _ctc_lengths(target_lengths, B, L_max, "target_lengths")
+    tg_all = targets.cpu().numpy().astype(np.int64)
+    for b in range(B):
+        where = f"item {b}: "
+        R = _ctc_item_checks(tg_all[b, :ll[b]], V, blank, where)
+        if tl[b] < 1:
+            raise RuntimeError(f"{where}input length must be >= 1")
+        if tl[b] < ll[b] + R:
+            raise RuntimeError(f"{where}targets length is too long for CTC. Found log_probs length: {tl[b]}, "
+                               f"targets length: {ll[b]}, and number of repeats: {R}")
+    t_off = np.concatenate([[0], np.cumsum(tl)]).astype(np.int64)
+    l_off = np.concatenate([[0], np.cumsum(ll)]).astype(np.int64)
+    labels = (np.concatenate([tg_all[b, :ll[b]] for b in range(B)]) if B else np.zeros(0, np.int64)).astype(np.int32)
+    dev = log_probs.device
+    valid = torch.arange(T_max, device=dev)[None, :] < torch.from_numpy(tl).to(dev)[:, None]   # [B, T_max]
+    paths = torch.full((B, T_max), blank, dtype=targets.dtype, device=dev)
+    scores = torch.zeros((B, T_max), dtype=torch.float32, device=dev)
+    if B == 0:
+        return paths, scores
+    with AlignPlan.ctc(t_off, labels, l_off, V, blank,
+                       device=dev.index if dev.type == "cuda" else _current_device()) as plan:
+        if dev.type == "cuda":
+            with torch.cuda.device(dev):
+                _, labs, sc, _, status = plan.run_torch(log_probs[valid].contiguous())   # rows packed on the device
+                status = status.cpu().numpy()
+        else:
+            _, labs, sc, _, status = plan.run_host(log_probs[valid].numpy())
+            labs, sc = torch.from_numpy(labs), torch.from_numpy(sc)
+    for b in np.flatnonzero(status != ST_OK):
+        if status[b] == ST_NONFINITE:
+            raise ValueError(f"item {b}: log_probs must not contain NaN or +inf")
+        raise_for_status(int(status[b]), V)
+    paths[valid] = labs.to(targets.dtype)
+    scores[valid] = sc
+    return paths, scores
 
 
 def trim_pool():

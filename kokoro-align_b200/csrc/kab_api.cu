@@ -157,7 +157,9 @@ struct kab_plan {
   int32_t band_cw = 0;  // compute warps per CTA of that kernel (ring of 40 * band_cw * band_nc slots)
   kab_plan_info info{};
   std::vector<KabLattice> lists[N_QUEUES];
-  bool any_bad_label = false;
+  bool any_bad_label = false;  // some lattices have a status decided here (bad label; CTC: T < L + R too)
+  bool ctc = false;            // CTC forced-alignment plan (kab_plan_create_ctc)
+  int32_t blank = 0;           // ... and its blank id
   // device memory
   KabLattice *d_lists[N_QUEUES] = {};
   uint16_t *d_col16 = nullptr;
@@ -320,19 +322,32 @@ int kab_device_count(int *count) {
 
 namespace {
 // mask: only the lattices with mask[b] != 0 belong to this plan (nullptr: all); band_mode: -1 the
-// plan chooses (and may go hybrid), 0 the single-CTA band kernel, 1 kab_bandr.cuh
+// plan chooses (and may go hybrid), 0 the single-CTA band kernel, 1 kab_bandr.cuh; ctc: a CTC
+// forced-alignment plan with blank id `blank` (W and M as kab_plan_create_ctc sets them)
 int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
-                     const int64_t *l_off, int32_t V, int32_t W, int32_t M, const uint8_t *mask, int band_mode);
+                     const int64_t *l_off, int32_t V, int32_t W, int32_t M, const uint8_t *mask, int band_mode,
+                     bool ctc, int32_t blank);
+// CTC plans: every lattice is unbanded -- a window this wide is [0, S) in every frame of the band
+// kernel (S <= 3296 there) -- and has three moves
+constexpr int32_t CTC_W = 0x3fffffff, CTC_M = 3;
 }  // namespace
 
 int kab_plan_create(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
                     const int64_t *l_off, int32_t V, int32_t W, int32_t M) {
-  return plan_create_impl(out, device, B, t_off, labels, l_off, V, W, M, nullptr, -1);
+  return plan_create_impl(out, device, B, t_off, labels, l_off, V, W, M, nullptr, -1, false, 0);
+}
+
+int kab_plan_create_ctc(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
+                        const int64_t *l_off, int32_t V, int32_t blank) {
+  if (blank < 0 || blank >= V) return KAB_E_BAD_ARG;
+  // (only the single-CTA band kernel has a CTC mode)
+  return plan_create_impl(out, device, B, t_off, labels, l_off, V, CTC_W, CTC_M, nullptr, 0, true, blank);
 }
 
 namespace {
 int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
-                     const int64_t *l_off, int32_t V, int32_t W, int32_t M, const uint8_t *mask, int band_mode) {
+                     const int64_t *l_off, int32_t V, int32_t W, int32_t M, const uint8_t *mask, int band_mode,
+                     bool ctc, int32_t blank) {
   if (!out || B < 0 || !t_off || !l_off || V < 1 || V > 65535 || W < 0 || M < 1 || M > 255) return KAB_E_BAD_ARG;
   if (B > 0 && (t_off[0] < 0 || l_off[0] < 0)) return KAB_E_BAD_ARG;
   if (B > 0 && l_off[B] > l_off[0] && !labels) return KAB_E_BAD_ARG;
@@ -345,6 +360,7 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
   kab_plan *pl = new (std::nothrow) kab_plan();
   if (!pl) return KAB_E_NOMEM;
   pl->device = device; pl->B = B; pl->V = V; pl->W = W; pl->M = M;
+  pl->ctc = ctc; pl->blank = blank;
   pl->total_T = B ? t_off[B] : 0;  // offsets are absolute rows / entries of the caller's arrays
   pl->total_L = B ? l_off[B] : 0;
   if (B > 0) {
@@ -370,7 +386,7 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
   };
   {
     const char *ge = getenv("KAB_BAND_GATHER");
-    bool ok = V > MAX_STAGE_V && M <= 4 && !(ge && atoi(ge) == 0) && kab_bandr_geom(64).smem_bytes <= 227 * 1024, any_band = false;
+    bool ok = !ctc && V > MAX_STAGE_V && M <= 4 && !(ge && atoi(ge) == 0) && kab_bandr_geom(64).smem_bytes <= 227 * 1024, any_band = false;
     for (int64_t b = 0; b < B && ok; ++b) {
       if (mask && !mask[b]) continue;
       const int64_t T = t_off[b + 1] - t_off[b], S = 2 * (l_off[b + 1] - l_off[b]) + 1;
@@ -378,7 +394,7 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
     }
     pl->band_ga = ok && any_band;
   }
-  if (V > MAX_STAGE_V && M <= 4) {
+  if (!ctc && V > MAX_STAGE_V && M <= 4) {
     std::vector<uint8_t> seen((size_t)V, 0);
     int64_t dmax = 0;
     bool any = false;
@@ -459,8 +475,8 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
     LatFacts f{};
     std::fill(distinct_mask, distinct_mask + n_mask, (int64_t)0);
     for (int64_t l = 0; l < L; ++l) {
-      if (lab[l] < -V || lab[l] >= V) { f.bad = 1; break; }
-      if (lab[l] <= 0) f.special = 1;
+      if (ctc ? (lab[l] < 0 || lab[l] >= V || lab[l] == blank) : (lab[l] < -V || lab[l] >= V)) { f.bad = 1; break; }
+      if (!ctc && lab[l] <= 0) f.special = 1;  // (CTC: the blank test is the state's parity, any label is fast)
       const int32_t c = lab[l] < 0 ? lab[l] + V : lab[l];
       if (!(distinct_mask[c >> 6] >> (c & 63) & 1)) { distinct_mask[c >> 6] |= (int64_t)1 << (c & 63); ++f.distinct; }
     }
@@ -508,6 +524,16 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
       pl->any_bad_label = true;
       continue;
     }
+    if (ctc) {  // CTC: no path fits when T < L + R (R = adjacent equal labels, which need a blank between)
+      const int32_t *lab = labels + l_off[b];
+      int64_t R = 0;
+      for (int64_t l = 1; l < L; ++l) R += lab[l] == lab[l - 1];
+      if (T < L + R) {
+        status_init[(size_t)b] = KAB_ST_DEAD_BAND;
+        pl->any_bad_label = true;
+        continue;
+      }
+    }
     KabLattice d{};
     d.t_off = t_off[b];
     d.lab_off = l_off[b];
@@ -519,7 +545,7 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
     // candidates into -inf); more than four moves only exist in the generic kernel
     const bool fast = M <= 4 && !special && (ga || (Veff <= MAX_STAGE_V && (!pl->Vc || distinct + 1 <= pl->Vc)));
     const bool full = W >= S && (S * (T - 1)) / T <= W / 2;
-    const int64_t weff = std::min<int64_t>(W, S);
+    const int64_t weff = ctc ? S : std::min<int64_t>(W, S);
     int q;
     if (fast && !ga && full && S <= 248) {
       q = Q_WARP;
@@ -549,7 +575,7 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
     pl->lists[q].push_back(d);
     pl->max_T[q] = std::max(pl->max_T[q], (int)T);
     info.n_class[q == Q_WARP ? KAB_CLASS_WARP : (q == Q_GENERIC ? KAB_CLASS_GENERIC : (q == Q_WIDE ? KAB_CLASS_WIDE : KAB_CLASS_BAND))]++;
-    const int64_t cells = cells_eval_of(T, S, W);
+    const int64_t cells = ctc ? T * S : cells_eval_of(T, S, W);
     info.cells_eval += cells;
     info.cells_nominal += T * S;
     int bbits = 0;
@@ -757,7 +783,8 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
     // ---- launch geometry
     if (!pl->lists[Q_WARP].empty()) {
       const size_t smem = 128 + (size_t)KAB_WARPS_PER_CTA * (KAB_WARP_STAGES * pl->stage_bytes + 256);  // + label tables
-      const void *fn = M == 4 ? (Veff == 39 ? (const void *)kab_warp_kernel<39, false> : (const void *)kab_warp_kernel<0, false>)
+      const void *fn = ctc ? (const void *)kab_warp_ctc_kernel
+                     : M == 4 ? (Veff == 39 ? (const void *)kab_warp_kernel<39, false> : (const void *)kab_warp_kernel<0, false>)
                               : (Veff == 39 ? (const void *)kab_warp_kernel<39, true> : (const void *)kab_warp_kernel<0, true>);
       if ((e = ensure_dyn_smem(fn, device, smem)) != cudaSuccess) { rc = cuda_fail(e, "cudaFuncSetAttribute(warp)"); break; }
       int occ = 0;
@@ -801,7 +828,8 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
       pl->grid[Q_BAND] = ncl * pl->band_nc;
     } else if (!pl->lists[Q_BAND].empty()) {
       const KabBandGeom geo = kab_band_geom(pl->band_nw, pl->stage_bytes);
-      const void *fn = M == 4 ? (pl->band_nw <= 16 ? (const void *)kab_band_kernel<512, false> : (const void *)kab_band_kernel<1024, false>)
+      const void *fn = ctc ? (pl->band_nw <= 16 ? (const void *)kab_band_ctc_kernel<512> : (const void *)kab_band_ctc_kernel<1024>)
+                     : M == 4 ? (pl->band_nw <= 16 ? (const void *)kab_band_kernel<512, false> : (const void *)kab_band_kernel<1024, false>)
                               : (pl->band_nw <= 16 ? (const void *)kab_band_kernel<512, true> : (const void *)kab_band_kernel<1024, true>);
       if ((e = ensure_dyn_smem(fn, device, geo.smem_bytes)) != cudaSuccess) { rc = cuda_fail(e, "cudaFuncSetAttribute(band)"); break; }
       int occ = 0;
@@ -834,7 +862,7 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
   if (pl->Vc)                                          // kab_compact_kernel, kab_expand_labels_kernel
     for (int q : {Q_WARP, Q_BAND, Q_WIDE}) info.kernel_launches += pl->lists[q].empty() ? 0 : 2;
   if (hyb_k > 0) {  // the sub-plan of a hybrid band plan: same arrays, its own lattices, workspaces and stream
-    int rcs = plan_create_impl(&pl->sub, device, B, t_off, labels, l_off, V, W, M, hyb_mask.data(), 1);
+    int rcs = plan_create_impl(&pl->sub, device, B, t_off, labels, l_off, V, W, M, hyb_mask.data(), 1, pl->ctc, pl->blank);
     if (rcs == KAB_OK) {
       pl->sub->is_child = true;
       pl->sub->grid[Q_BAND] = std::min(pl->sub->grid[Q_BAND], hyb_k * pl->sub->band_nc);
@@ -925,7 +953,9 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
     KabParams pw = pf; pw.queue = pl->d_queue + Q_WARP;
     const int nwl = (int)pl->lists[Q_WARP].size();
     const dim3 wg((unsigned)pl->grid[Q_WARP]), wb(KAB_WARPS_PER_CTA * 32);
-    if (pl->M == 4) {
+    if (pl->ctc) {
+      kab_warp_ctc_kernel<<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw, pl->blank);
+    } else if (pl->M == 4) {
       if (pf.V == 39) kab_warp_kernel<39, false><<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw);
       else kab_warp_kernel<0, false><<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw);
     } else {
@@ -992,7 +1022,10 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
     } else {
       const int nbl = (int)pl->lists[Q_BAND].size();
       const dim3 bg((unsigned)pl->grid[Q_BAND]), bb((unsigned)(pl->band_nw * 32));
-      if (pl->band_nw <= 16) {
+      if (pl->ctc) {
+        if (pl->band_nw <= 16) kab_band_ctc_kernel<512><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb, pl->blank);
+        else kab_band_ctc_kernel<1024><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb, pl->blank);
+      } else if (pl->band_nw <= 16) {
         if (pl->M == 4) kab_band_kernel<512, false><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb);
         else kab_band_kernel<512, true><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb);
       } else {
@@ -1022,8 +1055,12 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
       }
   if (!pl->lists[Q_GENERIC].empty()) {
     KabParams pg = p; pg.queue = pl->d_queue + Q_GENERIC;
-    kab_generic_kernel<GENERIC_NT><<<pl->grid[Q_GENERIC], GENERIC_NT, 0, stream>>>(
-        pl->d_lists[Q_GENERIC], (int)pl->lists[Q_GENERIC].size(), pg);
+    if (pl->ctc)
+      kab_generic_ctc_kernel<GENERIC_NT><<<pl->grid[Q_GENERIC], GENERIC_NT, 0, stream>>>(
+          pl->d_lists[Q_GENERIC], (int)pl->lists[Q_GENERIC].size(), pg, pl->blank);
+    else
+      kab_generic_kernel<GENERIC_NT><<<pl->grid[Q_GENERIC], GENERIC_NT, 0, stream>>>(
+          pl->d_lists[Q_GENERIC], (int)pl->lists[Q_GENERIC].size(), pg);
   }
   KAB_CUDA(cudaGetLastError());
   if (pl->sub) KAB_CUDA(cudaStreamWaitEvent(stream, pl->ev_join, 0));
@@ -1124,6 +1161,7 @@ int kab_plan_segment_stats_device(kab_plan *pl, const int32_t *d_best_path, cons
                                   const int64_t *d_seg_lat_off, const int64_t *d_seg_end,
                                   kab_segment_record *d_records, uint8_t *d_labels_u8, void *stream_) {
   if (!pl || n_segments < 0) return KAB_E_BAD_ARG;
+  if (pl->ctc) return KAB_E_UNSUPPORTED;  // (the records are those of Kokoro-Align's align())
   if (pl->B == 0) return n_segments == 0 ? KAB_OK : KAB_E_BAD_ARG;
   if (!d_best_path || !d_best_labels || !d_best_scores || !d_status) return KAB_E_BAD_ARG;
   if (n_segments > 0 && (!d_seg_lat_off || !d_seg_end || !d_records)) return KAB_E_BAD_ARG;
@@ -1205,7 +1243,8 @@ int host_setup(kab_plan *pl) {
         for (auto &x : lo) x -= l0;
         const int32_t *lab = pl->h_labels.empty() ? nullptr : pl->h_labels.data() + l0;
         child_rc[k] = (inject && atoi(inject) == (int)k) ? KAB_E_NOMEM
-                                                        : kab_plan_create(&child[k], pl->device, b1 - b0, to.data(), lab, lo.data(), pl->V, pl->W, pl->M);
+                                                        : plan_create_impl(&child[k], pl->device, b1 - b0, to.data(), lab, lo.data(), pl->V, pl->W, pl->M,
+                                                                           nullptr, pl->ctc ? 0 : -1, pl->ctc, pl->blank);
       };
       if (std::thread::hardware_concurrency() >= 4 && !getenv("KAB_SERIAL_SETUP")) {
         std::vector<std::thread> th;
@@ -1271,7 +1310,7 @@ int host_setup(kab_plan *pl) {
       auto make = [&](int k) {
         if (k + 1 < NP && cnt[k] == 0) return;
         rcs[k] = plan_create_impl(&pl->pipe[k], pl->device, (int64_t)B, pl->h_t_off.data(), lab, pl->h_l_off.data(), pl->V, pl->W, pl->M,
-                                  m[k].data(), k + 1 < NP ? 1 : -1);
+                                  m[k].data(), k + 1 < NP ? 1 : -1, pl->ctc, pl->blank);
       };
       {
         std::vector<std::thread> th;
@@ -1460,6 +1499,7 @@ int kab_plan_run_host_segments(kab_plan *pl, const float *h_in, int32_t is_logit
                                kab_segment_record *h_records, uint8_t *h_labels_u8, int32_t *h_best_path,
                                int32_t *h_best_labels, float *h_best_scores, float *h_final_score,
                                int32_t *h_status) {
+  if (pl && pl->ctc) return KAB_E_UNSUPPORTED;  // (the records are those of Kokoro-Align's align())
   HostRun r;
   r.h_in = h_in; r.logits = is_logits != 0;
   r.n_seg = n_segments; r.h_seg_lat_off = h_seg_lat_off; r.h_seg_end = h_seg_end; r.h_rec = h_records;

@@ -68,10 +68,12 @@ __device__ __forceinline__ void kab_bulk_wait_read0() {
 }
 __device__ __forceinline__ void kab_bulk_wait0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
-// MAXT: upper bound of the block size (512 -> up to 128 registers per thread, 1024 -> 64).
-template <int MAXT, bool MM>
-__global__ void __launch_bounds__(MAXT, 1) kab_band_kernel(const KabLattice *__restrict__ lats, int n_lat,
-                                                           KabParams p) {
+// CTC: the CTC forced-alignment recurrence (kab_common.cuh) over the whole lattice: the host sets W so
+// that the window is [0, S) in every frame, and S + 32 <= R, so no chunk is ever recycled.  Junk from
+// lane 0 climbs at most two states per frame there (16 in a group), so the 24 ghost states still cover it.
+template <int MAXT, bool MM, bool CTC>
+__device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lats, int n_lat, const KabParams &p,
+                                              const int blank) {
   constexpr int G = KAB_BAND_G, GH = KAB_BAND_GHOST, OW = KAB_BAND_OW;
   const KabBandGeom geo = kab_band_geom(p.band_nw, p.stage_bytes);
   const int NW = geo.nw, NT = NW * 32, R = OW * NW, NBP = geo.nbp, FB = geo.fb;
@@ -86,6 +88,7 @@ __global__ void __launch_bounds__(MAXT, 1) kab_band_kernel(const KabLattice *__r
   __shared__ unsigned int s_item;
   __shared__ int s_vmax;
   __shared__ float s_final;
+  __shared__ float s_end[2];  // CTC: scores of states S-1, S-2 of the last frame
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const bool owned = lane >= GH;
@@ -164,8 +167,16 @@ __global__ void __launch_bounds__(MAXT, 1) kab_band_kernel(const KabLattice *__r
     load_cols(vb, c1, c3);
     load_cols(vb + R, nc1, nc3);
     const int half = W / 2;
+    const uint32_t boff = CTC ? 4u * (uint32_t)blank : 0u;  // byte offset of the blank's column
+    // CTC: bit 0 / 1 = move 2 forbidden into label state vb+1 / vb+3 (state 1, or a repeated label)
+    uint32_t rep = 0;
+    if (CTC) {
+      const int l1 = vb >> 1;  // label index of state vb+1
+      if (vb + 1 < 3 || vb + 1 >= S || col16[l1] == col16[l1 - 1]) rep |= 1u;
+      if (vb + 3 >= S || col16[l1 + 1] == col16[l1]) rep |= 2u;
+    }
 
-    float poison = 0.0f;  // NaN once a non-finite log-prob was staged (kab_poison)
+    float poison = kab_poison_init<CTC>();  // NaN once a rejected log-prob was staged (kab_poison_t)
     if (tid == 0) {
       kab_mbar_wait(&ebars[st], ph);
       if (F < 2 * G && n_chunks > 1) {  // F == G: chunk 1 opens at group 1, before the look-ahead wait
@@ -180,10 +191,10 @@ __global__ void __launch_bounds__(MAXT, 1) kab_band_kernel(const KabLattice *__r
     auto check_chunk = [&](int c) {  // finiteness of chunk c's words (all threads, strided)
       const float *w = stage_base + st * stage_words + skew;
       const int nw = min(F, T - c * F) * V;
-      for (int j = tid; j < nw; j += NT) poison = kab_poison(poison, w[j]);
+      for (int j = tid; j < nw; j += NT) poison = kab_poison_t<CTC>(poison, w[j]);
     };
     check_chunk(0);
-    float eb = *reinterpret_cast<const float *>(rowc);
+    float eb = *reinterpret_cast<const float *>(rowc + boff);
     float e1 = *reinterpret_cast<const float *>(rowc + c1);
     float e3 = *reinterpret_cast<const float *>(rowc + c3);
 
@@ -226,6 +237,13 @@ __global__ void __launch_bounds__(MAXT, 1) kab_band_kernel(const KabLattice *__r
       float n1 = kab_label_sel(a0, kab_mm<MM>(a1, p.mm1), kab_mm<MM>(a2, p.mm2), kab_mm<MM>(a3, p.mm3), m, 1u << 2, 2u << 2, one);
       float n2 = kab_blank_sel(t2, kab_mm<MM>(t1, p.mm1), kab_mm<MM>(th1, p.mm3), m, 1u << 4, 2u << 4, one);
       float n3 = kab_label_sel(b0, kab_mm<MM>(b1, p.mm1), kab_mm<MM>(b2, p.mm2), kab_mm<MM>(b3, p.mm3), m, 1u << 6, 2u << 6, one);
+      if (CTC) {  // (replaces all of the above but h1, which is the one state below the lane's chunk)
+        m = 0;
+        n0 = __fadd_rn(kab_ctc_blank_sel(s0, h1, m, 0), eb);
+        n1 = __fadd_rn(kab_ctc_label_sel(s1, s0, rep & 1u ? ninf : h1, m, 2), e1);
+        n2 = __fadd_rn(kab_ctc_blank_sel(s2, s1, m, 4), eb);
+        n3 = __fadd_rn(kab_ctc_label_sel(s3, s2, rep & 2u ? ninf : s1, m, 6), e3);
+      }
       if (SLOW) {  // cells outside [lo, hi) are inactive: state vb+k is inside iff 0 <= vb+k-lo < hi-lo
         const unsigned a = (unsigned)(vb - lo), wd = (unsigned)(hi - lo);
         n0 = (a + 0u < wd) ? n0 : ninf;
@@ -237,7 +255,7 @@ __global__ void __launch_bounds__(MAXT, 1) kab_band_kernel(const KabLattice *__r
       if (owned) *bpdst = (unsigned char)m;
       if (has_next) {  // emissions of frame i+1 (its chunk was published by an earlier barrier)
         rowc = rownext;
-        eb = *reinterpret_cast<const float *>(rownext);
+        eb = *reinterpret_cast<const float *>(rownext + boff);
         e1 = *reinterpret_cast<const float *>(rownext + c1);
         e3 = *reinterpret_cast<const float *>(rownext + c3);
       }
@@ -360,8 +378,18 @@ __global__ void __launch_bounds__(MAXT, 1) kab_band_kernel(const KabLattice *__r
 #endif
     echunks = ec0 + n_chunks;
 
-    // ---- forced end state: highest active state of frame T-1 (align.py:99-101)
-    {
+    if (CTC) {  // CTC end rule: the better of the last two states, S-2 on a tie (kab_common.cuh)
+      if (owned) {
+        if (vb + 0 == S - 1) s_end[0] = s0;
+        if (vb + 1 == S - 1) s_end[0] = s1;
+        if (vb + 2 == S - 1) s_end[0] = s2;
+        if (vb + 3 == S - 1) s_end[0] = s3;
+        if (vb + 0 == S - 2) s_end[1] = s0;
+        if (vb + 1 == S - 2) s_end[1] = s1;
+        if (vb + 2 == S - 2) s_end[1] = s2;
+        if (vb + 3 == S - 2) s_end[1] = s3;
+      }
+    } else {  // ---- forced end state: highest active state of frame T-1 (align.py:99-101)
       int cand = -1;
       if (owned) {
         if (vb + 0 < S && s0 > ninf) cand = vb + 0;
@@ -375,6 +403,7 @@ __global__ void __launch_bounds__(MAXT, 1) kab_band_kernel(const KabLattice *__r
     if (tid == 0) kab_bulk_wait0();  // all backpointer blocks are in global memory
     const int any_bad = __syncthreads_or(poison != poison ? 1 : 0);
     int v = s_vmax;
+    if (CTC) v = (S >= 2 && !(s_end[0] > s_end[1])) ? S - 2 : S - 1;
     const int status = any_bad ? 3 : (v < 0 ? 1 : 0);
     if (owned && status == 0) {
       if (vb + 0 == v) s_final = s0;
@@ -410,7 +439,7 @@ __global__ void __launch_bounds__(MAXT, 1) kab_band_kernel(const KabLattice *__r
         const int *pbuf = pathbuf + (blk & 1) * FB;
         for (int i = i0 + (tid - first_thread); i < i1; i += n_threads) {
           const int pv = pbuf[i - i0];
-          const int lab = (pv & 1) ? (int)col16[(pv - 1) >> 1] : 0;
+          const int lab = (pv & 1) ? (int)col16[(pv - 1) >> 1] : (CTC ? blank : 0);
           out_path[i] = pv;
           out_lab[i] = lab;                              // align.py:106
           out_sc[i] = __ldg(&lp[(int64_t)i * V + lab]);  // align.py:107
@@ -448,4 +477,18 @@ __global__ void __launch_bounds__(MAXT, 1) kab_band_kernel(const KabLattice *__r
     }
     __syncthreads();
   }
+}
+
+// MAXT: upper bound of the block size (512 -> up to 128 registers per thread, 1024 -> 64).
+template <int MAXT, bool MM>
+__global__ void __launch_bounds__(MAXT, 1) kab_band_kernel(const KabLattice *__restrict__ lats, int n_lat,
+                                                           KabParams p) {
+  kab_band_body<MAXT, MM, false>(lats, n_lat, p, 0);
+}
+
+// CTC forced alignment (whole-lattice window; blank column: see kab_warp_ctc_kernel)
+template <int MAXT>
+__global__ void __launch_bounds__(MAXT, 1) kab_band_ctc_kernel(const KabLattice *__restrict__ lats, int n_lat,
+                                                               KabParams p, int blank) {
+  kab_band_body<MAXT, false, true>(lats, n_lat, p, blank);
 }

@@ -79,6 +79,35 @@ __device__ __forceinline__ bool kab_finite(float x) { return fabsf(x) < __int_as
 // and NaN for +-inf / NaN, so `acc` turns NaN, and stays NaN, once a non-finite value was seen.
 __device__ __forceinline__ float kab_poison(float acc, float x) { return fmaf(x, 0.0f, acc); }
 
+// ---------------------------------------------------------------- CTC forced alignment (the CTC
+// instantiations; torchaudio.functional.forced_align's recurrence, DESIGN.md 3.9)
+//   x0 = a[v], x1 = a[v-1], x2 = a[v-2] (label states only, -inf into a repeated label and for v == 1);
+//   j = 2 if x2 > x1 and x2 > x0, else 1 if x1 > x0 and x1 > x2, else 0 -- so x1 == x2 > x0 keeps x0;
+//   a'[v] = fl32(x_j + lp[t, ext[v]]): the select is on the previous scores, then ONE add.
+// The 2-bit backpointer code is the move, as in the Kokoro kernels, so their walks apply unchanged.
+// -inf log-probs are accepted (masking); only NaN and +inf are rejected.  Accumulator that starts at
+// -inf: acc + x stays -inf for a finite or -inf x and turns NaN, for good, at the first NaN or +inf.
+__device__ __forceinline__ float kab_poison_ctc(float acc, float x) { return __fadd_rn(acc, x); }
+template <bool CTC>
+__device__ __forceinline__ float kab_poison_t(float acc, float x) {
+  return CTC ? kab_poison_ctc(acc, x) : kab_poison(acc, x);
+}
+template <bool CTC>
+__device__ __forceinline__ float kab_poison_init() { return CTC ? kab_neg_inf() : 0.0f; }
+// Blank state: moves 0, 1.  The code's bits are OR-ed into w at bit pos.
+__device__ __forceinline__ float kab_ctc_blank_sel(float x0, float x1, uint32_t &w, const int pos) {
+  const bool p1 = x1 > x0;
+  w |= (uint32_t)p1 << pos;
+  return p1 ? x1 : x0;
+}
+// Label state: moves 0, 1, 2 (x2 already -inf where move 2 is forbidden).
+__device__ __forceinline__ float kab_ctc_label_sel(float x0, float x1, float x2, uint32_t &w, const int pos) {
+  const bool p2 = x2 > x1 && x2 > x0;
+  const bool p1 = x1 > x0 && x1 > x2;  // (excludes p2)
+  w |= ((uint32_t)p2 << 1 | (uint32_t)p1) << pos;
+  return p2 ? x2 : (p1 ? x1 : x0);
+}
+
 // ---------------------------------------------------------------- mbarrier + 1-D bulk copy (TMA)
 __device__ __forceinline__ uint32_t kab_smem_u32(const void *p) {
   return (uint32_t)__cvta_generic_to_shared(p);

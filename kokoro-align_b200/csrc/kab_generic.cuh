@@ -7,9 +7,11 @@
 #pragma once
 #include "kab_common.cuh"
 
-template <int NT>
-__global__ void __launch_bounds__(NT) kab_generic_kernel(const KabLattice *__restrict__ lats, int n_lat,
-                                                         KabParams p) {
+// CTC: the CTC forced-alignment recurrence (kab_common.cuh) over the whole lattice (no window,
+// value-independent blank test: the state's parity), blank column `blank`.
+template <int NT, bool CTC>
+__device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ lats, int n_lat, const KabParams &p,
+                                                 const int blank) {
   __shared__ unsigned int s_item;
   __shared__ long long s_vmax;
   const int tid = threadIdx.x;
@@ -24,7 +26,7 @@ __global__ void __launch_bounds__(NT) kab_generic_kernel(const KabLattice *__res
     if (item >= (unsigned int)n_lat) break;
     const KabLattice lat = lats[item];
     const int64_t T = lat.T, S = 2 * (int64_t)lat.L + 1, W = p.W, M = p.M, V = p.V;
-    const int64_t Wc = max((int64_t)1, min(W, S));
+    const int64_t Wc = CTC ? S : max((int64_t)1, min(W, S));
     const int32_t *raw = p.raw + lat.lab_off;
     const float *lp = p.lp + lat.t_off * V;
     uint8_t *bp = p.bp + lat.bp_off;
@@ -38,11 +40,28 @@ __global__ void __launch_bounds__(NT) kab_generic_kernel(const KabLattice *__res
     bool bad = false;
     for (int64_t i = 0; i < T; ++i) {
       int64_t lo = (S * i) / T - W / 2;  // align.py:64 (64-bit: S*i reaches 1e11)
-      if (lo < 0) lo = 0;
-      int64_t hi = min(lo + W, S);       // align.py:65
+      if (lo < 0 || CTC) lo = 0;
+      int64_t hi = CTC ? S : min(lo + W, S);  // align.py:65
       if (hi < lo) hi = lo;
       const float *row = lp + i * V;
-      for (int64_t c = tid; c < V; c += NT) bad |= !kab_finite(__ldg(&row[c]));
+      for (int64_t c = tid; c < V; c += NT) {
+        const float x = __ldg(&row[c]);
+        bad |= CTC ? !(x < __int_as_float(0x7f800000)) : !kab_finite(x);  // CTC: -inf is accepted
+      }
+      if (CTC) {
+        for (int64_t v = tid; v < S; v += NT) {
+          const bool lab = (v & 1) != 0;
+          const int32_t ext = lab ? raw[(v - 1) >> 1] : blank;
+          const float e = __ldg(&row[ext]);
+          const float x0 = v < phi ? __ldcg(&prev[v]) : kab_neg_inf();
+          const float x1 = v >= 1 && v - 1 < phi ? __ldcg(&prev[v - 1]) : kab_neg_inf();
+          const float x2 = lab && v >= 3 && v - 2 < phi && ext != raw[(v - 3) >> 1] ? __ldcg(&prev[v - 2]) : kab_neg_inf();
+          uint32_t code = 0;
+          const float best = lab ? kab_ctc_label_sel(x0, x1, x2, code, 0) : kab_ctc_blank_sel(x0, x1, code, 0);
+          __stcg(&cur[v], __fadd_rn(best, e));
+          bp[i * Wc + v] = (uint8_t)code;
+        }
+      } else
       for (int64_t v = lo + tid; v < hi; v += NT) {
         const int32_t ext = (v & 1) ? raw[(v - 1) >> 1] : 0;
         const int32_t col = ext < 0 ? ext + (int32_t)V : ext;
@@ -66,11 +85,14 @@ __global__ void __launch_bounds__(NT) kab_generic_kernel(const KabLattice *__res
 
     // forced end state: highest active state of the last frame, align.py:99-101
     long long vmax = -1;
-    for (int64_t v = plo + tid; v < phi; v += NT)
-      if (__ldcg(&prev[v]) > kab_neg_inf()) vmax = v;
+    if (!CTC)
+      for (int64_t v = plo + tid; v < phi; v += NT)
+        if (__ldcg(&prev[v]) > kab_neg_inf()) vmax = v;
     if (vmax >= 0) atomicMax(&s_vmax, vmax);
     const int any_bad = __syncthreads_or(bad ? 1 : 0);
     int64_t v = s_vmax;
+    // CTC end rule: the better of the last two states, S-2 on a tie
+    if (CTC) v = (S >= 2 && !(__ldcg(&prev[S - 1]) > __ldcg(&prev[S - 2]))) ? S - 2 : S - 1;
 
     if (tid == 0) {
       int st = 0;
@@ -84,8 +106,8 @@ __global__ void __launch_bounds__(NT) kab_generic_kernel(const KabLattice *__res
         float *out_sc = p.best_scores + lat.t_off;
         for (int64_t i = T - 1; i >= 0; --i) {  // == flush_determined_path, align.py:21-40
           int64_t lo = (S * i) / T - W / 2;
-          if (lo < 0) lo = 0;
-          const int32_t ext = (v & 1) ? raw[(v - 1) >> 1] : 0;
+          if (lo < 0 || CTC) lo = 0;
+          const int32_t ext = (v & 1) ? raw[(v - 1) >> 1] : (CTC ? blank : 0);
           const int32_t col = ext < 0 ? ext + (int32_t)V : ext;
           out_path[i] = (int32_t)v;
           out_lab[i] = ext;                      // align.py:106
@@ -96,4 +118,16 @@ __global__ void __launch_bounds__(NT) kab_generic_kernel(const KabLattice *__res
     }
     __syncthreads();
   }
+}
+
+template <int NT>
+__global__ void __launch_bounds__(NT) kab_generic_kernel(const KabLattice *__restrict__ lats, int n_lat,
+                                                         KabParams p) {
+  kab_generic_body<NT, false>(lats, n_lat, p, 0);
+}
+
+template <int NT>
+__global__ void __launch_bounds__(NT) kab_generic_ctc_kernel(const KabLattice *__restrict__ lats, int n_lat,
+                                                             KabParams p, int blank) {
+  kab_generic_body<NT, true>(lats, n_lat, p, blank);
 }

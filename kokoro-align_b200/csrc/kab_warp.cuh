@@ -78,10 +78,30 @@ __device__ __forceinline__ void kab_warp_frame(float (&s)[K], const float eb, co
   for (int k = 0; k < K; ++k) s[k] = n[k];
 }
 
-// VCT: compile-time vocabulary (39) or 0 = runtime p.V.
-template <int K, int VCT, bool MM>
+// CTC forced alignment (kab_common.cuh): lane l >= 1 owns the same K states; the only halo is state
+// K*(l-1)-1 (moves reach two states down, and state v-2 of a label state v is inside the lane for
+// v >= 3 of the lane).  rep bit q = move 2 is forbidden into the lane's label state 2q+1.
+template <int K>
+__device__ __forceinline__ void kab_warp_frame_ctc(float (&s)[K], const float eb, const float (&el)[K / 2],
+                                                   const uint32_t rep, uint32_t &w, const int shift) {
+  const float h1 = __shfl_up_sync(KAB_FULL_MASK, s[K - 1], 1);
+  float n[K];
+#pragma unroll
+  for (int q = 0; q < K / 2; ++q) {
+    const int kb = 2 * q, kl = 2 * q + 1;
+    n[kb] = __fadd_rn(kab_ctc_blank_sel(s[kb], kb >= 1 ? s[kb >= 1 ? kb - 1 : 0] : h1, w, shift + 2 * kb), eb);
+    const float x2 = (rep >> q) & 1u ? kab_neg_inf() : (kl >= 3 ? s[kl >= 3 ? kl - 2 : 0] : h1);
+    n[kl] = __fadd_rn(kab_ctc_label_sel(s[kl], s[kl - 1], x2, w, shift + 2 * kl), el[q]);
+  }
+#pragma unroll
+  for (int k = 0; k < K; ++k) s[k] = n[k];
+}
+
+// VCT: compile-time vocabulary (39) or 0 = runtime p.V.  CTC: the CTC forced-alignment recurrence.
+template <int K, int VCT, bool MM, bool CTC>
 __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float *stage_base, uint64_t *bars,
-                               uint16_t *labtab, const uint64_t policy, uint32_t &chunk_counter, const int lane) {
+                               uint16_t *labtab, const uint64_t policy, uint32_t &chunk_counter, const int lane,
+                               const int blank) {
   using Cfg = KabWarpCfg<K>;
   constexpr int BPF = Cfg::BPF, FPW = Cfg::FPW;
   const int T = lat.T, S = 2 * lat.L + 1;
@@ -98,13 +118,16 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
 
   // byte offsets (col * 4) of this lane's K/2 label states inside an emission row
   uint32_t coff[K / 2];
+  uint32_t rep = 0;  // CTC: bit q = move 2 forbidden into label state sbase + 2q + 1 (v == 1, or a repeated label)
 #pragma unroll
   for (int q = 0; q < K / 2; ++q) {
     const int v = sbase + 2 * q + 1;
     const uint32_t col = (v > 0 && v < S) ? col16[(v - 1) >> 1] : 0u;
     coff[q] = 4u * col;
     if (v > 0 && v < S) labtab[(v - 1) >> 1] = (uint16_t)col;  // per-warp copy for the backtrack's output rows
+    if (CTC && (v < 3 || v >= S || col == col16[(v - 3) >> 1])) rep |= 1u << q;
   }
+  const uint32_t boff = CTC ? 4u * (uint32_t)blank : 0u;  // byte offset of the blank's column
 
   float s[K];
 #pragma unroll
@@ -143,7 +166,7 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
   const int pre = min(n_chunks, KAB_WARP_STAGES - 1);
   for (int c = 0; c < pre; ++c) issue(c);
 
-  float poison = 0.0f;  // NaN once a non-finite log-prob was staged (kab_poison)
+  float poison = kab_poison_init<CTC>();  // NaN once a rejected log-prob was staged (kab_poison_t)
   uint32_t *bprow = bpw + lane;  // this lane's slot in the current word-row
   uint32_t st = cc0 % KAB_WARP_STAGES, ph = (cc0 / KAB_WARP_STAGES) & 1u;  // stage / phase of the chunk being read
   for (int c = 0; c < n_chunks; ++c) {
@@ -163,10 +186,10 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
       const float4 *s4 = reinterpret_cast<const float4 *>(stage);
       for (int j = v0 + lane; j < v1; j += 32) {
         const float4 x = s4[j];
-        poison = kab_poison(kab_poison(kab_poison(kab_poison(poison, x.x), x.y), x.z), x.w);
+        poison = kab_poison_t<CTC>(kab_poison_t<CTC>(kab_poison_t<CTC>(kab_poison_t<CTC>(poison, x.x), x.y), x.z), x.w);
       }
-      if (lane < 4 * v0 - w0 && w0 + lane < w1) poison = kab_poison(poison, stage[w0 + lane]);
-      if (4 * v1 >= w0 && lane < w1 - 4 * v1) poison = kab_poison(poison, stage[4 * v1 + lane]);
+      if (lane < 4 * v0 - w0 && w0 + lane < w1) poison = kab_poison_t<CTC>(poison, stage[w0 + lane]);
+      if (4 * v1 >= w0 && lane < w1 - 4 * v1) poison = kab_poison_t<CTC>(poison, stage[4 * v1 + lane]);
     }
     const char *rowb = reinterpret_cast<const char *>(stage + w0);
     const int n_groups = nf / FPW;
@@ -175,11 +198,12 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
 #pragma unroll
       for (int f = 0; f < FPW; ++f) {
         const char *rb = rowb + f * V * 4;
-        const float eb = *reinterpret_cast<const float *>(rb);
+        const float eb = *reinterpret_cast<const float *>(rb + boff);
         float el[K / 2];
 #pragma unroll
         for (int q = 0; q < K / 2; ++q) el[q] = *reinterpret_cast<const float *>(rb + coff[q]);
-        kab_warp_frame<K, MM>(s, eb, el, lane1, word, f * BPF, one, mm1, mm2, mm3);
+        if (CTC) kab_warp_frame_ctc<K>(s, eb, el, rep, word, f * BPF);
+        else kab_warp_frame<K, MM>(s, eb, el, lane1, word, f * BPF, one, mm1, mm2, mm3);
       }
       *bprow = word;
       bprow += 32;
@@ -189,12 +213,13 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
       uint32_t word = 0;
 #pragma unroll 1
       for (int f = 0; f < rem; ++f, rowb += V * 4) {
-        const float eb = *reinterpret_cast<const float *>(rowb);
+        const float eb = *reinterpret_cast<const float *>(rowb + boff);
         float el[K / 2];
 #pragma unroll
         for (int q = 0; q < K / 2; ++q) el[q] = *reinterpret_cast<const float *>(rowb + coff[q]);
         uint32_t fw = 0;
-        kab_warp_frame<K, MM>(s, eb, el, lane1, fw, 0, one, mm1, mm2, mm3);
+        if (CTC) kab_warp_frame_ctc<K>(s, eb, el, rep, fw, 0);
+        else kab_warp_frame<K, MM>(s, eb, el, lane1, fw, 0, one, mm1, mm2, mm3);
         word |= fw << (f * BPF);
       }
       *bprow = word;
@@ -203,14 +228,29 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
   chunk_counter = cc0 + n_chunks;
   __syncwarp();
 
-  // -- forced end state: highest active state of frame T-1 (align.py:99-101)
-  int cand = -1;
+  // score of state u of frame T-1 (from its owner lane)
+  auto score_of = [&](int u) {
+    float mine = s[0];
 #pragma unroll
-  for (int k = 0; k < K; ++k) {
-    const int v = sbase + k;
-    if (v >= 0 && v < S && s[k] > kab_neg_inf()) cand = v;
+    for (int k = 1; k < K; ++k) if (k == u % K) mine = s[k];
+    return __shfl_sync(KAB_FULL_MASK, mine, u / K + 1);
+  };
+  int v;
+  if (CTC) {  // CTC end rule: the better of the last two states, S-2 on a tie (kab_common.cuh)
+    v = S - 1;
+    if (S >= 2) {
+      const float a1 = score_of(S - 1), a2 = score_of(S - 2);
+      if (!(a1 > a2)) v = S - 2;
+    }
+  } else {  // -- forced end state: highest active state of frame T-1 (align.py:99-101)
+    int cand = -1;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+      const int v = sbase + k;
+      if (v >= 0 && v < S && s[k] > kab_neg_inf()) cand = v;
+    }
+    v = __reduce_max_sync(KAB_FULL_MASK, cand);
   }
-  int v = __reduce_max_sync(KAB_FULL_MASK, cand);
   const bool any_bad = __any_sync(KAB_FULL_MASK, poison != poison);
   const int status = any_bad ? 3 : (v < 0 ? 1 : 0);
   {
@@ -275,7 +315,7 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
       const int t = fb + lane;
       pend_t = -1;
       if (t < T) {
-        const int lab = (myv & 1) ? (int)labtab[(myv - 1) >> 1] : 0;
+        const int lab = (myv & 1) ? (int)labtab[(myv - 1) >> 1] : (CTC ? blank : 0);
         out_path[t] = myv;
         out_lab[t] = lab;                           // align.py:106
         pend_s = __ldg(&lp[(int64_t)t * V + lab]);  // align.py:107
@@ -288,9 +328,9 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
   if (pend_t >= 0) out_sc[pend_t] = pend_s;
 }
 
-template <int VCT, bool MM>
-__global__ void __launch_bounds__(KAB_WARPS_PER_CTA * 32, KAB_WARP_MINBLOCKS)
-    kab_warp_kernel(const KabLattice *__restrict__ lats, int n_lat, KabParams p) {
+template <int VCT, bool MM, bool CTC>
+__device__ __forceinline__ void kab_warp_body(const KabLattice *__restrict__ lats, int n_lat, const KabParams &p,
+                                              const int blank) {
   extern __shared__ __align__(128) unsigned char kab_smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   uint64_t *bars = reinterpret_cast<uint64_t *>(kab_smem) + warp * KAB_WARP_STAGES;
@@ -318,11 +358,24 @@ __global__ void __launch_bounds__(KAB_WARPS_PER_CTA * 32, KAB_WARP_MINBLOCKS)
     if (item >= (unsigned int)n_lat) break;
     const KabLattice lat = lats[item];
     switch (lat.k) {
-      case 2: kab_warp_align<2, VCT, MM>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane); break;
-      case 4: kab_warp_align<4, VCT, MM>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane); break;
-      case 6: kab_warp_align<6, VCT, MM>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane); break;
-      default: kab_warp_align<8, VCT, MM>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane); break;
+      case 2: kab_warp_align<2, VCT, MM, CTC>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
+      case 4: kab_warp_align<4, VCT, MM, CTC>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
+      case 6: kab_warp_align<6, VCT, MM, CTC>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
+      default: kab_warp_align<8, VCT, MM, CTC>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
     }
     __syncwarp();
   }
+}
+
+template <int VCT, bool MM>
+__global__ void __launch_bounds__(KAB_WARPS_PER_CTA * 32, KAB_WARP_MINBLOCKS)
+    kab_warp_kernel(const KabLattice *__restrict__ lats, int n_lat, KabParams p) {
+  kab_warp_body<VCT, MM, false>(lats, n_lat, p, 0);
+}
+
+// CTC forced alignment (runtime vocabulary; `blank` = the blank's column -- a kernel argument, not a
+// KabParams field, whose growth would move the parameters of every kernel that takes more after it)
+__global__ void __launch_bounds__(KAB_WARPS_PER_CTA * 32, KAB_WARP_MINBLOCKS)
+    kab_warp_ctc_kernel(const KabLattice *__restrict__ lats, int n_lat, KabParams p, int blank) {
+  kab_warp_body<0, false, true>(lats, n_lat, p, blank);
 }
