@@ -62,7 +62,9 @@ typedef struct kab_plan_info {
   int64_t cells_eval;       /* sum_b sum_i (hi_i - lo_i): cells the recurrence evaluates */
   int64_t cells_nominal;    /* sum_b T_b * S_b */
   int64_t workspace_bytes;  /* device memory held by the plan (backpointers, labels, queues) */
-  int64_t backptr_bytes;    /* of which packed backpointers */
+  int64_t backptr_bytes;    /* of which packed backpointers; for KAB_CLASS_WARP lattices of a best-path
+                               plan with more than 124 states: the score checkpoint rows that replace them
+                               (one row per 8 frames) */
   int64_t algorithmic_bytes;/* SURVEY.md 8(d): 4*min(V,D+1)*T + cells*b/8 + T*b/8 + 12*T, summed */
   int32_t kernel_launches;  /* kernels launched by one kab_plan_run_* */
   int32_t device;

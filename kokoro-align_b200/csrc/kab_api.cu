@@ -550,9 +550,13 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
     if (fast && !ga && full && S <= 248) {
       q = Q_WARP;
       d.k = S <= 62 ? 2 : (S <= 124 ? 4 : (S <= 186 ? 6 : 8));  // 31 lanes x K states
-      const int fpw = d.k <= 2 ? 8 : (d.k <= 4 ? 4 : 2);
       d.bp_off = bp_bytes;
-      bp_bytes += align_up((T + fpw - 1) / fpw * 128, 256);
+      if (ctc || d.k <= 4) {  // backpointer word-rows (kab_warp_align: the BP scheme)
+        const int fpw = d.k <= 2 ? 8 : (d.k <= 4 ? 4 : 2);
+        bp_bytes += align_up((T + fpw - 1) / fpw * 128, 256);
+      } else {  // score checkpoint rows, one per KAB_CKPT_C frames
+        bp_bytes += align_up((T + KAB_CKPT_C - 1) / KAB_CKPT_C * kab_ckpt_stride((int)S, d.k) * 4, 256);
+      }
     } else if (fast && W >= 1 && S <= 3 * T && weff + 32 <= KAB_BAND_OW * BAND_MAX_WARPS) {
       q = Q_BAND;  // backpointer offsets are assigned below, once the ring size is known
       max_band_weff = std::max(max_band_weff, weff);

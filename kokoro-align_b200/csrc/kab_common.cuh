@@ -244,6 +244,18 @@ __device__ __forceinline__ void kab_add2v(float lo, float hi, float elo, float e
       : "=f"(olo), "=f"(ohi)
       : "f"(lo), "f"(hi), "f"(elo), "f"(ehi));
 }
+// max.f32 of two / three values (FMNMX / FMNMX3).  The values-only warp forward pass takes the
+// maximum BEFORE the add: rounding is monotone, so max_j fl(x_j + e) == fl(max_j x_j + e).
+__device__ __forceinline__ float kab_max2(float a, float b) {
+  float m;
+  asm("max.f32 %0, %1, %2;" : "=f"(m) : "f"(a), "f"(b));
+  return m;
+}
+__device__ __forceinline__ float kab_max3(float a, float b, float c) {
+  float m;
+  asm("max.f32 %0, %1, %2, %3;" : "=f"(m) : "f"(a), "f"(b), "f"(c));
+  return m;
+}
 // Blank state: candidates a0 (move 0), a1 (move 1), a3 (move 3); ascending strict-'>' scan.
 // The predicated "OR" is issued as mad.lo (w = one * bit + w, `one` is a register holding 1 that
 // ptxas cannot fold): IMAD runs on the FMA pipe, the compares/max/selects on the ALU pipe, and
