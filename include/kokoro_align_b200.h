@@ -206,6 +206,39 @@ int kab_plan_run_host_segments(kab_plan *plan, const float *h_log_probs_or_logit
                                int32_t *h_status);
 
 /*
+ * Token spans of per-frame token sequences (torchaudio.functional.merge_tokens), on the device, for a
+ * flat batch: item b = frames d_t_off[b] .. d_t_off[b+1] of d_tokens int32 / d_scores float32
+ * (d_t_off int64 [n_items + 1], T_b < 2^31).  A run is a maximal stretch of equal tokens (frame 0
+ * always starts one); every run whose token is not `blank` is a span {token, start, end (exclusive),
+ * score} in item-relative frames.  score = the mean of scores[start:end]: the values converted to
+ * double and added in frame order from the first, divided by end - start in double, rounded once to
+ * float32 (DESIGN.md 3.10; -inf and NaN propagate).  Any token values are accepted.
+ * The spans of item b go to d_spans[d_t_off[b] .. d_t_off[b] + d_n_spans[b]) (capacity sum T: an
+ * item has at most as many spans as frames).  Device pointers on the caller's current device;
+ * asynchronous on `stream` (a cudaStream_t, NULL = default stream): the call only launches
+ * kab_merge_tokens_kernel.  KAB_E_BAD_ARG for a NULL pointer or n_items < 0.
+ */
+typedef struct kab_token_span { int32_t token, start, end; float score; } kab_token_span;      /* 16 B */
+typedef struct kab_word_span  { int32_t start, end, first_token; float score; } kab_word_span;  /* 16 B */
+
+int kab_merge_tokens_device(int64_t n_items, const int64_t *d_t_off, const int32_t *d_tokens,
+                            const float *d_scores, int32_t blank, kab_token_span *d_spans,
+                            int32_t *d_n_spans, void *stream);
+/*
+ * Word spans of those token spans (the word grouping of torchaudio's forced-alignment tutorial):
+ * word w of item b groups d_word_len[d_word_off[b] + w] consecutive spans (d_word_off int64
+ * [n_items + 1]) and goes to d_words[d_word_off[b] + w]: start = its first span's start, end = its
+ * last span's end, first_token = the item-relative index of its first span, score =
+ * float32(sum_j double(score_j) * len_j / sum_j len_j), the numerator summed in span order from 0.
+ * d_spans / d_n_spans / d_t_off as kab_merge_tokens_device left them.  d_word_status[b] = 1 when
+ * the item's word lengths do not sum to d_n_spans[b] or one is < 1 (its words are then not
+ * written), else 0.  Asynchronous like kab_merge_tokens_device (kab_word_spans_kernel).
+ */
+int kab_word_spans_device(int64_t n_items, const int64_t *d_t_off, const kab_token_span *d_spans,
+                          const int32_t *d_n_spans, const int64_t *d_word_off, const int32_t *d_word_len,
+                          kab_word_span *d_words, int32_t *d_word_status, void *stream);
+
+/*
  * One-shot single lattice with host buffers == kokoro_align/align.py:43
  * ctc_best_path(log_probs[T,V], labels[L], beam_size, max_move) -> (best_path, best_labels,
  * best_scores); *status receives KAB_ST_*; final_score may be NULL.

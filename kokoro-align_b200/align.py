@@ -10,6 +10,9 @@ form (``AlignPlan``) is what a B200 pipeline uses: many independent chapter / se
 lattices per launch, inputs optionally already resident in HBM.
 """
 import ctypes
+import itertools
+from dataclasses import dataclass
+from typing import NamedTuple
 
 import numpy as np
 
@@ -377,6 +380,199 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
     paths[valid] = labs.to(targets.dtype)
     scores[valid] = sc
     return paths, scores
+
+
+# ---------------------------------------------------------------- token and word spans
+# torchaudio.functional.merge_tokens and the word grouping of torchaudio's forced-alignment tutorial,
+# batched on the device (kab_merge_tokens_device / kab_word_spans_device, DESIGN.md 3.10).
+
+@dataclass
+class TokenSpan:
+    """A span of one token (torchaudio.functional.TokenSpan's fields): frames [start, end)."""
+    token: int
+    start: int
+    end: int
+    score: float
+
+    def __len__(self):
+        return self.end - self.start
+
+
+class TokenSpans(NamedTuple):
+    """Padded token spans of a batch: [B, N_max] tensors (token: the tokens' dtype, start / end:
+    int64, score: float32; padding -1 / -1 / -1 / 0) and count int64 [B]."""
+    token: "torch.Tensor"
+    start: "torch.Tensor"
+    end: "torch.Tensor"
+    score: "torch.Tensor"
+    count: "torch.Tensor"
+
+
+class WordSpans(NamedTuple):
+    """Padded word spans of a batch: [B, W_max] tensors (start / end / first_token: int64, score:
+    float32; padding -1 and 0) and count int64 [B] (words per item)."""
+    start: "torch.Tensor"
+    end: "torch.Tensor"
+    score: "torch.Tensor"
+    first_token: "torch.Tensor"
+    count: "torch.Tensor"
+
+
+def _span_device(t):
+    """The CUDA device the span kernels run on for tensor t (CPU tensors: the current one)."""
+    import torch
+    if t.is_cuda:
+        return t.device
+    if not torch.cuda.is_available():
+        raise KabError("no CUDA device: the span kernels have no CPU fallback")
+    return torch.device("cuda", torch.cuda.current_device())
+
+
+def _vp(t):
+    return ctypes.c_void_p(t.data_ptr())
+
+
+def _unpad(flat, off, count, n_max, fill):
+    """Rows off[b] + j (j < count[b]) of a flat [n, 4] int32 record tensor -> [B, n_max, 4], padded
+    with the row `fill`."""
+    import torch
+    j = torch.arange(n_max, device=flat.device)
+    rows = off[:, None] + j[None, :]
+    valid = j[None, :] < count[:, None]
+    out = flat[rows.clamp_(max=max(flat.shape[0] - 1, 0))] if flat.shape[0] else flat.new_zeros(rows.shape + (4,))
+    return torch.where(valid[..., None], out, torch.tensor(fill, dtype=torch.int32, device=flat.device))
+
+
+def merge_tokens_batch(tokens, scores, lengths=None, blank=0):
+    """torchaudio.functional.merge_tokens for a padded batch, on the device: tokens int32 / int64
+    [B, T_max] (e.g. forced_align_batch's paths, or greedy CTC decodes), scores float32 [B, T_max]
+    (what a span's score averages: forced_align's log-probs or their exp()), lengths [B] (None: every
+    item is T_max frames long).  Returns TokenSpans of padded [B, N_max] tensors, N_max =
+    count.max(), on the input's device (CPU tensors run on the current CUDA device).  Span scores are
+    float32 means computed in double in frame order (DESIGN.md 3.10), within 2.4e-7 relative of
+    torchaudio's float32 mean().  ValueError for negative tokens, non-float32 scores or mismatched
+    shapes."""
+    import torch
+    if tokens.dim() != 2 or scores.dim() != 2 or tuple(tokens.shape) != tuple(scores.shape):
+        raise ValueError(f"tokens and scores must both be [B, T_max], got {tuple(tokens.shape)} and {tuple(scores.shape)}")
+    if tokens.dtype not in (torch.int32, torch.int64):
+        raise ValueError(f"tokens must be int32 or int64, got {tokens.dtype}")
+    if scores.dtype != torch.float32:
+        raise ValueError(f"scores must be float32, got {scores.dtype}")
+    B, T_max = (int(x) for x in tokens.shape)
+    if lengths is None:
+        tl = np.full(B, T_max, np.int64)
+    else:
+        tl = np.asarray(lengths.cpu() if hasattr(lengths, "cpu") else lengths, dtype=np.int64)
+        if tl.ndim != 1 or tl.shape[0] != B:
+            raise ValueError(f"lengths must be [B] = [{B}], got shape {tl.shape}")
+        if B and (tl.min() < 0 or tl.max() > T_max):
+            raise ValueError(f"lengths must lie in [0, {T_max}]")
+    if lengths is None:
+        tok_f, sc_f = tokens.reshape(-1), scores.reshape(-1)
+    else:   # the valid frames, packed on the input's device
+        valid = torch.arange(T_max, device=tokens.device)[None, :] < torch.from_numpy(tl).to(tokens.device)[:, None]
+        tok_f, sc_f = tokens[valid], scores[valid]
+    if tok_f.numel():
+        lo, hi = torch.stack(list(torch.aminmax(tok_f))).tolist()
+        if lo < 0:
+            raise ValueError("tokens must be non-negative")
+        if hi > 0x7fffffff:
+            raise ValueError("tokens must fit in int32")
+    out_dev = tokens.device
+    dev = _span_device(tokens)
+    with torch.cuda.device(dev):
+        tok_f = tok_f.to(dev, torch.int32).contiguous()
+        sc_f = sc_f.to(dev).contiguous()
+        n = int(tl.sum())
+        t_off_h = np.concatenate([[0], np.cumsum(tl)]).astype(np.int64)
+        t_off = torch.from_numpy(t_off_h).to(dev)
+        recs = torch.empty((max(n, 1), 4), dtype=torch.int32, device=dev)
+        cnt = torch.empty(max(B, 1), dtype=torch.int32, device=dev)
+        if n == 0:   # (C entry points take no NULL buffers)
+            tok_f = torch.zeros(1, dtype=torch.int32, device=dev)
+            sc_f = torch.zeros(1, dtype=torch.float32, device=dev)
+        s = torch.cuda.current_stream(dev)
+        _lib.check(_lib.lib().kab_merge_tokens_device(B, _vp(t_off), _vp(tok_f), _vp(sc_f), int(blank), _vp(recs),
+                                                      _vp(cnt), ctypes.c_void_p(s.cuda_stream)))
+        count = cnt[:B].to(torch.int64)
+        n_max = int(count.max()) if B else 0
+        pad = _unpad(recs, t_off[:-1], count, n_max, [-1, -1, -1, 0])
+        res = TokenSpans(pad[..., 0].to(tokens.dtype), pad[..., 1].to(torch.int64), pad[..., 2].to(torch.int64),
+                         pad[..., 3].contiguous().view(torch.float32), count)
+    if out_dev != dev:
+        res = TokenSpans(*(x.to(out_dev) for x in res))
+    return res
+
+
+def merge_tokens(tokens, scores, blank=0):
+    """Drop-in for torchaudio.functional.merge_tokens (one item): tokens int32 / int64 [T], scores
+    float32 [T] -> List[TokenSpan], computed on the device (merge_tokens_batch)."""
+    if tokens.ndim != 1 or scores.ndim != 1:
+        raise ValueError("`tokens` and `scores` must be 1D Tensor.")
+    if len(tokens) != len(scores):
+        raise ValueError("`tokens` and `scores` must be the same length.")
+    r = merge_tokens_batch(tokens[None], scores[None], None, blank)
+    n = int(r.count[0])
+    tok, st, en = (x[0, :n].tolist() for x in r[:3])
+    sc = r.score[0, :n].tolist()
+    return [TokenSpan(token=a, start=b, end=c, score=d) for a, b, c, d in zip(tok, st, en, sc)]
+
+
+def word_spans(token_spans, word_lengths):
+    """Word spans from the TokenSpans of merge_tokens_batch, on their device: word_lengths[b] lists
+    the number of tokens (spans) of each word of item b (each >= 1, summing to the item's span
+    count).  Returns WordSpans: start = the first span's start, end = the last span's end,
+    first_token = the index of the first span, score = float32(sum(score * len) / sum(len)) over
+    the word's spans -- the tutorial's `_score`, bit for bit.  ValueError naming the first item
+    whose lengths do not fit."""
+    import torch
+    token, start, end, score, count = token_spans
+    B = int(count.shape[0])
+    if len(word_lengths) != B:
+        raise ValueError(f"word_lengths must hold one sequence per item ({B}), got {len(word_lengths)}")
+    cnt_h = count.cpu().numpy().astype(np.int64)
+    n_words = np.fromiter((len(w) for w in word_lengths), np.int64, B)
+    w_off_h = np.concatenate([[0], np.cumsum(n_words)]).astype(np.int64)
+    flat = np.fromiter(itertools.chain.from_iterable(word_lengths), np.int64, int(w_off_h[-1]))
+    csum = np.concatenate([[0], np.cumsum(flat)])
+    zero = np.searchsorted(w_off_h, np.flatnonzero(flat < 1), "right") - 1   # items with a word of length < 1
+    short = np.flatnonzero(csum[w_off_h[1:]] - csum[w_off_h[:-1]] != cnt_h)
+    if zero.size or short.size:
+        b = int(min(zero.min() if zero.size else B, short.min() if short.size else B))
+        if zero.size and b == zero.min():
+            raise ValueError(f"item {b}: every word must have at least one token")
+        total = int(csum[w_off_h[b + 1]] - csum[w_off_h[b]])
+        raise ValueError(f"item {b}: word lengths sum to {total}, the item has {int(cnt_h[b])} token spans")
+    out_dev = count.device
+    dev = _span_device(count)
+    with torch.cuda.device(dev):
+        n_max = int(token.shape[1]) if token.dim() == 2 else 0
+        valid = torch.arange(n_max, device=dev)[None, :] < count.to(dev)[:, None]
+        recs = torch.stack([token.to(dev).to(torch.int32), start.to(dev).to(torch.int32), end.to(dev).to(torch.int32),
+                            score.to(dev).to(torch.float32).view(torch.int32)], -1)[valid].contiguous()
+        s_off = torch.from_numpy(np.concatenate([[0], np.cumsum(cnt_h)]).astype(np.int64)).to(dev)
+        n_w = int(w_off_h[-1])
+        w_off = torch.from_numpy(w_off_h).to(dev)
+        w_len = torch.from_numpy(flat.astype(np.int32)).to(dev)
+        words = torch.empty((max(n_w, 1), 4), dtype=torch.int32, device=dev)
+        status = torch.empty(max(B, 1), dtype=torch.int32, device=dev)
+        if recs.shape[0] == 0:
+            recs = torch.zeros((1, 4), dtype=torch.int32, device=dev)
+        if w_len.numel() == 0:
+            w_len = torch.zeros(1, dtype=torch.int32, device=dev)
+        cnt32 = count.to(dev).to(torch.int32)
+        s = torch.cuda.current_stream(dev)
+        _lib.check(_lib.lib().kab_word_spans_device(B, _vp(s_off), _vp(recs), _vp(cnt32),
+                                                    _vp(w_off), _vp(w_len), _vp(words), _vp(status),
+                                                    ctypes.c_void_p(s.cuda_stream)))
+        wc = torch.from_numpy(n_words).to(dev)
+        pad = _unpad(words, w_off[:-1], wc, int(n_words.max()) if B else 0, [-1, -1, -1, 0])
+        res = WordSpans(pad[..., 0].to(torch.int64), pad[..., 1].to(torch.int64), pad[..., 3].contiguous().view(torch.float32),
+                        pad[..., 2].to(torch.int64), wc)
+    if out_dev != dev:
+        res = WordSpans(*(x.to(out_dev) for x in res))
+    return res
 
 
 def trim_pool():

@@ -30,6 +30,7 @@
 #include "kab_generic.cuh"
 #include "kab_softmax.cuh"
 #include "kab_segstats.cuh"
+#include "kab_spans.cuh"
 #include "kab_warp.cuh"
 #include "kab_pool.h"  // pool_malloc / pool_free / pool_trim_device
 
@@ -1112,6 +1113,44 @@ int kab_log_softmax_device(const float *d_logits, float *d_log_probs, int64_t n_
     const unsigned grid = (unsigned)std::min<int64_t>((n_rows + 7) / 8, (int64_t)sms * 8);
     kab_log_softmax_wide_kernel<<<grid, 256, 0, stream>>>(d_logits, d_log_probs, n_rows, V);
   }
+  KAB_CUDA(cudaGetLastError());
+  return KAB_OK;
+}
+
+namespace {
+// one CTA per item, at most this many CTAs per SM in the grid (the kernels grid-stride over the rest)
+int span_grid(int64_t n_items, int *grid) {
+  int dev = 0, sms = 0;
+  KAB_CUDA(cudaGetDevice(&dev));
+  KAB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  *grid = (int)std::min<int64_t>(n_items, (int64_t)sms * 32);
+  return KAB_OK;
+}
+}  // namespace
+
+int kab_merge_tokens_device(int64_t n_items, const int64_t *d_t_off, const int32_t *d_tokens, const float *d_scores,
+                            int32_t blank, kab_token_span *d_spans, int32_t *d_n_spans, void *stream) {
+  if (n_items < 0 || !d_t_off || !d_tokens || !d_scores || !d_spans || !d_n_spans) return KAB_E_BAD_ARG;
+  int grid = 0, rc;
+  if ((rc = span_grid(n_items, &grid)) != KAB_OK || n_items == 0) return rc;
+  const int vec = (uintptr_t)d_spans % 16 == 0;
+  kab_merge_tokens_kernel<<<grid, KAB_SPAN_THREADS, 0, (cudaStream_t)stream>>>(
+      n_items, d_t_off, d_tokens, d_scores, blank, reinterpret_cast<KabTokenSpan *>(d_spans), d_n_spans, vec);
+  KAB_CUDA(cudaGetLastError());
+  return KAB_OK;
+}
+
+int kab_word_spans_device(int64_t n_items, const int64_t *d_t_off, const kab_token_span *d_spans,
+                          const int32_t *d_n_spans, const int64_t *d_word_off, const int32_t *d_word_len,
+                          kab_word_span *d_words, int32_t *d_word_status, void *stream) {
+  if (n_items < 0 || !d_t_off || !d_spans || !d_n_spans || !d_word_off || !d_word_len || !d_words || !d_word_status)
+    return KAB_E_BAD_ARG;
+  int grid = 0, rc;
+  if ((rc = span_grid(n_items, &grid)) != KAB_OK || n_items == 0) return rc;
+  const int vec = ((uintptr_t)d_spans % 16 == 0 ? 1 : 0) | ((uintptr_t)d_words % 16 == 0 ? 2 : 0);
+  kab_word_spans_kernel<<<grid, KAB_WORD_THREADS, 0, (cudaStream_t)stream>>>(
+      n_items, d_t_off, reinterpret_cast<const KabTokenSpan *>(d_spans), d_n_spans, d_word_off, d_word_len,
+      reinterpret_cast<KabWordSpan *>(d_words), d_word_status, vec);
   KAB_CUDA(cudaGetLastError());
   return KAB_OK;
 }
