@@ -108,6 +108,19 @@ int kab_plan_create(kab_plan **plan, int device, int64_t n_lattices, const int64
  */
 int kab_plan_create_ctc(kab_plan **plan, int device, int64_t n_lattices, const int64_t *t_off,
                         const int32_t *labels, const int64_t *l_off, int32_t vocab_size, int32_t blank);
+/*
+ * kab_plan_create_ctc for long-form alignment (a chapter or any long recording against its text in
+ * one lattice): the same arguments, outputs, statuses and errors, but lattices with more than 3296
+ * states go to KAB_CLASS_WIDE (a chain of warps over the whole GPU, 2 bits of backpointer per cell)
+ * instead of KAB_CLASS_GENERIC (1 byte per cell) where they fit -- vocab_size <= 338 (the wide
+ * kernel's emission stages) and ceil(S/104)/4 + 1 CTAs resident at once -- and where a makespan
+ * estimate says so: wide lattices run one after another, each on the whole GPU, generic ones side by
+ * side, so a batch of many shorter lattices may stay generic (DESIGN.md 3.9).  Warp and band
+ * lattices are routed as by kab_plan_create_ctc.
+ */
+int kab_plan_create_ctc_long(kab_plan **plan, int device, int64_t n_lattices, const int64_t *t_off,
+                             const int32_t *labels, const int64_t *l_off, int32_t vocab_size,
+                             int32_t blank);
 int kab_plan_get_info(const kab_plan *plan, kab_plan_info *info);
 int kab_plan_destroy(kab_plan *plan);
 

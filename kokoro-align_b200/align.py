@@ -67,13 +67,17 @@ class AlignPlan:
         self._create(_lib.lib().kab_plan_create, int(beam_size), int(max_move))
 
     @classmethod
-    def ctc(cls, t_off, labels, l_off, vocab_size, blank=0, device=0):
+    def ctc(cls, t_off, labels, l_off, vocab_size, blank=0, device=0, long_form=False):
         """A plan in CTC forced-alignment mode (kab_plan_create_ctc): torchaudio's forced_align
         recurrence for every lattice of the batch; labels are token ids in [0, vocab_size) other
-        than ``blank``.  best_labels are then token ids per frame (``blank`` on even states)."""
+        than ``blank``.  best_labels are then token ids per frame (``blank`` on even states).
+        long_form=True (kab_plan_create_ctc_long): lattices with more than 3296 states run on the
+        wide kernel where it fits and is estimated faster (a whole chapter in one lattice), with the
+        same outputs."""
         plan = cls.__new__(cls)
         plan._setup(t_off, labels, l_off, vocab_size, device)
-        plan._create(_lib.lib().kab_plan_create_ctc, int(blank))
+        L = _lib.lib()
+        plan._create(L.kab_plan_create_ctc_long if long_form else L.kab_plan_create_ctc, int(blank))
         return plan
 
     def _setup(self, t_off, labels, l_off, vocab_size, device):
@@ -291,7 +295,7 @@ def _ctc_lengths(lengths, B, full, what):
     return n
 
 
-def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, blank=0):
+def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, blank=0, *, long_form=False):
     """Drop-in for torchaudio.functional.forced_align (same arguments, output shapes and dtypes,
     exception types): log_probs float32 [1, T, V], targets int32 / int64 [1, L] on the same device
     (CPU or CUDA).  Returns (paths [1, T] of the targets' dtype: the token id of every frame,
@@ -299,7 +303,8 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
     torchaudio.functional.merge_tokens takes.  Bit-exact with torchaudio's CPU implementation
     whenever the chosen end state has a finite score (where both end states are -inf, torchaudio's
     traceback is undefined; this one follows the recurrence, DESIGN.md 3.9).  NaN or +inf
-    log-probs raise ValueError (-inf, for masking, is accepted)."""
+    log-probs raise ValueError (-inf, for masking, is accepted).  long_form=True: a lattice of more
+    than 3296 states (2 L + 1) runs on the wide kernel, with the same outputs (AlignPlan.ctc)."""
     import torch
     _ctc_tensor_checks(log_probs, targets, blank)
     if log_probs.size(0) != 1 or targets.size(0) != 1:
@@ -316,8 +321,8 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
         raise RuntimeError(f"targets length is too long for CTC. Found log_probs length: {T}, targets length: {L}, "
                            f"and number of repeats: {R}")
     dev = log_probs.device
-    with AlignPlan.ctc([0, T], tg, [0, L], V, blank,
-                       device=dev.index if dev.type == "cuda" else _current_device()) as plan:
+    with AlignPlan.ctc([0, T], tg, [0, L], V, blank, device=dev.index if dev.type == "cuda" else _current_device(),
+                       long_form=long_form) as plan:
         if dev.type == "cuda":
             with torch.cuda.device(dev):
                 _, labs, scores, _, status = plan.run_torch(log_probs[0].contiguous())
@@ -331,13 +336,14 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
     return labs.to(targets.dtype).view(1, T), scores.view(1, T)
 
 
-def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=None, blank=0):
+def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=None, blank=0, *, long_form=False):
     """forced_align for a padded batch, in one plan: log_probs float32 [B, T_max, V], targets
     int32 / int64 [B, L_max], input_lengths / target_lengths [B] (None: all full length).  Item b
     is aligned over its first input_lengths[b] frames and target_lengths[b] targets.  Returns
     (paths [B, T_max] of the targets' dtype, scores float32 [B, T_max]) on the input's device;
     frames past an item's length hold the blank and score 0.  Raises, like forced_align, for the
-    first item that fails, naming its index.  On CUDA the valid rows are packed on the device."""
+    first item that fails, naming its index.  On CUDA the valid rows are packed on the device.
+    long_form: as in forced_align."""
     import torch
     _ctc_tensor_checks(log_probs, targets, blank)
     B, T_max, V = (int(x) for x in log_probs.shape)
@@ -364,8 +370,8 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
     scores = torch.zeros((B, T_max), dtype=torch.float32, device=dev)
     if B == 0:
         return paths, scores
-    with AlignPlan.ctc(t_off, labels, l_off, V, blank,
-                       device=dev.index if dev.type == "cuda" else _current_device()) as plan:
+    with AlignPlan.ctc(t_off, labels, l_off, V, blank, device=dev.index if dev.type == "cuda" else _current_device(),
+                       long_form=long_form) as plan:
         if dev.type == "cuda":
             with torch.cuda.device(dev):
                 _, labs, sc, _, status = plan.run_torch(log_probs[valid].contiguous())   # rows packed on the device

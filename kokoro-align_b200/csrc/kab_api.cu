@@ -161,6 +161,7 @@ struct kab_plan {
   bool any_bad_label = false;  // some lattices have a status decided here (bad label; CTC: T < L + R too)
   bool ctc = false;            // CTC forced-alignment plan (kab_plan_create_ctc)
   int32_t blank = 0;           // ... and its blank id
+  bool ctc_long = false;       // ... whose lattices too wide for the band kernel go to the wide kernel (kab_plan_create_ctc_long)
   // device memory
   KabLattice *d_lists[N_QUEUES] = {};
   uint16_t *d_col16 = nullptr;
@@ -324,10 +325,11 @@ int kab_device_count(int *count) {
 namespace {
 // mask: only the lattices with mask[b] != 0 belong to this plan (nullptr: all); band_mode: -1 the
 // plan chooses (and may go hybrid), 0 the single-CTA band kernel, 1 kab_bandr.cuh; ctc: a CTC
-// forced-alignment plan with blank id `blank` (W and M as kab_plan_create_ctc sets them)
+// forced-alignment plan with blank id `blank` (W and M as kab_plan_create_ctc sets them); ctc_long: its
+// lattices with S > 3296 go to the wide kernel where they fit (kab_plan_create_ctc_long)
 int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
                      const int64_t *l_off, int32_t V, int32_t W, int32_t M, const uint8_t *mask, int band_mode,
-                     bool ctc, int32_t blank);
+                     bool ctc, int32_t blank, bool ctc_long);
 // CTC plans: every lattice is unbanded -- a window this wide is [0, S) in every frame of the band
 // kernel (S <= 3296 there) -- and has three moves
 constexpr int32_t CTC_W = 0x3fffffff, CTC_M = 3;
@@ -335,20 +337,27 @@ constexpr int32_t CTC_W = 0x3fffffff, CTC_M = 3;
 
 int kab_plan_create(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
                     const int64_t *l_off, int32_t V, int32_t W, int32_t M) {
-  return plan_create_impl(out, device, B, t_off, labels, l_off, V, W, M, nullptr, -1, false, 0);
+  return plan_create_impl(out, device, B, t_off, labels, l_off, V, W, M, nullptr, -1, false, 0, false);
 }
 
 int kab_plan_create_ctc(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
                         const int64_t *l_off, int32_t V, int32_t blank) {
   if (blank < 0 || blank >= V) return KAB_E_BAD_ARG;
   // (only the single-CTA band kernel has a CTC mode)
-  return plan_create_impl(out, device, B, t_off, labels, l_off, V, CTC_W, CTC_M, nullptr, 0, true, blank);
+  return plan_create_impl(out, device, B, t_off, labels, l_off, V, CTC_W, CTC_M, nullptr, 0, true, blank, false);
+}
+
+int kab_plan_create_ctc_long(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
+                             const int64_t *l_off, int32_t V, int32_t blank) {
+  if (blank < 0 || blank >= V) return KAB_E_BAD_ARG;
+  // (the single-CTA band kernel below S = 3297, the wide kernel above it where it fits)
+  return plan_create_impl(out, device, B, t_off, labels, l_off, V, CTC_W, CTC_M, nullptr, 0, true, blank, true);
 }
 
 namespace {
 int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
                      const int64_t *l_off, int32_t V, int32_t W, int32_t M, const uint8_t *mask, int band_mode,
-                     bool ctc, int32_t blank) {
+                     bool ctc, int32_t blank, bool ctc_long) {
   if (!out || B < 0 || !t_off || !l_off || V < 1 || V > 65535 || W < 0 || M < 1 || M > 255) return KAB_E_BAD_ARG;
   if (B > 0 && (t_off[0] < 0 || l_off[0] < 0)) return KAB_E_BAD_ARG;
   if (B > 0 && l_off[B] > l_off[0] && !labels) return KAB_E_BAD_ARG;
@@ -361,7 +370,7 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
   kab_plan *pl = new (std::nothrow) kab_plan();
   if (!pl) return KAB_E_NOMEM;
   pl->device = device; pl->B = B; pl->V = V; pl->W = W; pl->M = M;
-  pl->ctc = ctc; pl->blank = blank;
+  pl->ctc = ctc; pl->blank = blank; pl->ctc_long = ctc_long;
   pl->total_T = B ? t_off[B] : 0;  // offsets are absolute rows / entries of the caller's arrays
   pl->total_L = B ? l_off[B] : 0;
   if (B > 0) {
@@ -433,10 +442,10 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
   int wide_capacity = 0;
   {
     const KabWideGeom wgeo = kab_wide_geom(pl->stage_bytes);
+    const void *wfn = ctc ? (const void *)kab_wide_ctc_kernel : (const void *)kab_wide_kernel;
     int occ = 0;
-    if (wgeo.smem_bytes <= 227 * 1024 &&
-        ensure_dyn_smem((const void *)kab_wide_kernel, device, wgeo.smem_bytes) == cudaSuccess &&
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kab_wide_kernel, KAB_WD_THREADS, wgeo.smem_bytes) == cudaSuccess)
+    if (wgeo.smem_bytes <= 227 * 1024 && ensure_dyn_smem(wfn, device, wgeo.smem_bytes) == cudaSuccess &&
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, wfn, KAB_WD_THREADS, wgeo.smem_bytes) == cudaSuccess)
       wide_capacity = occ * pl->sm_count;
     (void)cudaGetLastError();
   }
@@ -515,6 +524,26 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
       for (int64_t l = 0; l < L; ++l) c[l] = (uint16_t)(lab[l] < 0 ? lab[l] + V : lab[l]);
     }
   });
+  // CTC long-form plans: the wide kernel runs its lattices one after another, each on the whole GPU; the
+  // generic kernel runs them side by side, one CTA each.  A makespan estimate from measured costs (B200, V = 32,
+  // tools/forced_align_long_bench.py, DESIGN.md 3.9) gives all lattices that both kernels could take to one of
+  // them: wide ~102 ns per frame of a sequence of lattices; generic 0.68 Gcells/s for a lone lattice (its
+  // longest one bounds it) and 79 Gcells/s for 256 lattices side by side.  256 utterances of 2-5 minutes:
+  // 276 ms wide, 230 ms generic; one 10-minute utterance: 5.2 ms wide, 796 ms generic.
+  bool ctc_wide = false;
+  if (ctc && ctc_long) {
+    double frames = 0.0, cells = 0.0, max_cells = 0.0;
+    for (int64_t b = 0; b < B; ++b) {
+      if ((mask && !mask[b]) || facts[(size_t)b].bad) continue;
+      const int64_t T = t_off[b + 1] - t_off[b], S = 2 * (l_off[b + 1] - l_off[b]) + 1;
+      if (S + 32 <= KAB_BAND_OW * BAND_MAX_WARPS) continue;  // warp or band class
+      if (((S + KAB_BAND_OW - 1) / KAB_BAND_OW + KAB_WD_CW - 1) / KAB_WD_CW + 1 > wide_capacity) continue;
+      frames += (double)T;
+      cells += (double)T * (double)S;
+      max_cells = std::max(max_cells, (double)T * (double)S);
+    }
+    ctc_wide = frames * 102.0 <= std::max(max_cells / 0.68, cells / 79.0);  // (ns)
+  }
   for (int64_t b = 0; b < B; ++b) {
     if (mask && !mask[b]) continue;
     const int64_t T = t_off[b + 1] - t_off[b], L = l_off[b + 1] - l_off[b], S = 2 * L + 1;
@@ -561,7 +590,7 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
     } else if (fast && W >= 1 && S <= 3 * T && weff + 32 <= KAB_BAND_OW * BAND_MAX_WARPS) {
       q = Q_BAND;  // backpointer offsets are assigned below, once the ring size is known
       max_band_weff = std::max(max_band_weff, weff);
-    } else if (fast && !ga && M == 4 && full && ((S + KAB_BAND_OW - 1) / KAB_BAND_OW + KAB_WD_CW - 1) / KAB_WD_CW + 1 <= wide_capacity) {
+    } else if (fast && !ga && (ctc ? ctc_wide : M == 4) && full && ((S + KAB_BAND_OW - 1) / KAB_BAND_OW + KAB_WD_CW - 1) / KAB_WD_CW + 1 <= wide_capacity) {
       q = Q_WIDE;  // unbanded and wider than a CTA: a chain of warps over the whole GPU
       const int nww = (int)((S + KAB_BAND_OW - 1) / KAB_BAND_OW);
       d.k = nww;
@@ -867,7 +896,7 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
   if (pl->Vc)                                          // kab_compact_kernel, kab_expand_labels_kernel
     for (int q : {Q_WARP, Q_BAND, Q_WIDE}) info.kernel_launches += pl->lists[q].empty() ? 0 : 2;
   if (hyb_k > 0) {  // the sub-plan of a hybrid band plan: same arrays, its own lattices, workspaces and stream
-    int rcs = plan_create_impl(&pl->sub, device, B, t_off, labels, l_off, V, W, M, hyb_mask.data(), 1, pl->ctc, pl->blank);
+    int rcs = plan_create_impl(&pl->sub, device, B, t_off, labels, l_off, V, W, M, hyb_mask.data(), 1, pl->ctc, pl->blank, pl->ctc_long);
     if (rcs == KAB_OK) {
       pl->sub->is_child = true;
       pl->sub->grid[Q_BAND] = std::min(pl->sub->grid[Q_BAND], hyb_k * pl->sub->band_nc);
@@ -1047,9 +1076,11 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
     const KabLattice *wl = pl->d_lists[Q_WIDE];
     int wn = (int)pl->lists[Q_WIDE].size();
     unsigned char *wws = pl->d_wide_ws;
-    void *wargs[] = {(void *)&wl, (void *)&wn, (void *)&pf, (void *)&wws};
-    KAB_CUDA(cudaLaunchCooperativeKernel((const void *)kab_wide_kernel, dim3((unsigned)pl->grid[Q_WIDE]),
-                                         dim3(KAB_WD_THREADS), wargs, pl->smem[Q_WIDE], stream));
+    int wblank = pl->blank;
+    void *wargs[] = {(void *)&wl, (void *)&wn, (void *)&pf, (void *)&wws, (void *)&wblank};
+    const void *wfn = pl->ctc ? (const void *)kab_wide_ctc_kernel : (const void *)kab_wide_kernel;
+    KAB_CUDA(cudaLaunchCooperativeKernel(wfn, dim3((unsigned)pl->grid[Q_WIDE]), dim3(KAB_WD_THREADS), wargs,
+                                         pl->smem[Q_WIDE], stream));
   }
   if (pl->Vc)  // best_labels of the staged kernels: compact index -> label value
     for (int q : fast_lists)
@@ -1287,7 +1318,7 @@ int host_setup(kab_plan *pl) {
         const int32_t *lab = pl->h_labels.empty() ? nullptr : pl->h_labels.data() + l0;
         child_rc[k] = (inject && atoi(inject) == (int)k) ? KAB_E_NOMEM
                                                         : plan_create_impl(&child[k], pl->device, b1 - b0, to.data(), lab, lo.data(), pl->V, pl->W, pl->M,
-                                                                           nullptr, pl->ctc ? 0 : -1, pl->ctc, pl->blank);
+                                                                           nullptr, pl->ctc ? 0 : -1, pl->ctc, pl->blank, pl->ctc_long);
       };
       if (std::thread::hardware_concurrency() >= 4 && !getenv("KAB_SERIAL_SETUP")) {
         std::vector<std::thread> th;
@@ -1353,7 +1384,7 @@ int host_setup(kab_plan *pl) {
       auto make = [&](int k) {
         if (k + 1 < NP && cnt[k] == 0) return;
         rcs[k] = plan_create_impl(&pl->pipe[k], pl->device, (int64_t)B, pl->h_t_off.data(), lab, pl->h_l_off.data(), pl->V, pl->W, pl->M,
-                                  m[k].data(), k + 1 < NP ? 1 : -1, pl->ctc, pl->blank);
+                                  m[k].data(), k + 1 < NP ? 1 : -1, pl->ctc, pl->blank, pl->ctc_long);
       };
       {
         std::vector<std::thread> th;

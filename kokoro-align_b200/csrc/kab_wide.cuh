@@ -55,6 +55,7 @@
 
 // Global scratch of one wide lattice (zeroed before every run), at wide_ws + lat.scr_off * 4:
 //   [0] vmax + 1 (0 = no active state)   [1] non-finite flag   [2] warps finished   [3] unused
+//   (CTC: [0] score bits of state S-2, [3] score bits of state S-1)
 //   then cand[nww] (state, score bits), cons[nww] (messages consumed by warp w), fifo[nww][D][192 B]
 __host__ __device__ inline size_t kab_wide_cand_off() { return 16; }
 __host__ __device__ inline size_t kab_wide_cons_off(int nww) { return 16 + (size_t)nww * 8; }
@@ -68,7 +69,9 @@ struct KabWideGeom {
 };
 __host__ __device__ inline KabWideGeom kab_wide_geom(int stage_bytes) {
   KabWideGeom g;
-  g.bpst_off = 256;  // after the mbarriers
+  // after the mbarriers efull[NS], eempty[NS], btbar[2] (272 bytes at NS = 16; an offset of 256 put warp 0's
+  // staged backpointers of states 0..7, frames 0..7 on btbar)
+  g.bpst_off = ((size_t)(2 * KAB_WD_NS + 2) * 8 + 127) & ~(size_t)127;
   g.bt_off = g.bpst_off + (size_t)KAB_WD_CW * 2 * KAB_WD_FBW * 32;
   g.path_off = g.bt_off + (size_t)2 * KAB_WD_NREG * KAB_WD_FBK * 32;
   g.stage_off = g.path_off + (size_t)2 * KAB_WD_FBK * 4;
@@ -78,8 +81,15 @@ __host__ __device__ inline KabWideGeom kab_wide_geom(int stage_bytes) {
 
 // Grid: n_fwd forward CTAs + 1 backtrack CTA (the last one), all resident.  Every CTA runs over the
 // wide lattices in the same order.
-__global__ void __launch_bounds__(KAB_WD_THREADS, 1)
-    kab_wide_kernel(const KabLattice *__restrict__ lats, int n_lat, KabParams p, unsigned char *wide_ws) {
+// CTC: the CTC forced-alignment recurrence (kab_common.cuh, DESIGN.md 3.9) over the whole lattice, blank
+// column `blank`.  Junk enters lane 0 of a warp only through h1 (state vb by move 1, vb+1 by move 2) and
+// climbs at most two states per frame, so at most 16 states in a group of 8 frames: the 24 ghost states
+// still absorb it.  The end states S-1 and S-2 may sit in different warps (S = 1 mod 104: S-1 is the
+// first state of the top warp), so their owners publish both scores to the lattice's scratch and the
+// backtrack CTA applies the end rule.
+template <bool CTC>
+__device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lats, int n_lat, const KabParams &p,
+                                              unsigned char *wide_ws, const int blank) {
   constexpr int G = KAB_BAND_G, GH = KAB_BAND_GHOST, OW = KAB_BAND_OW;
   constexpr int CW = KAB_WD_CW, NS = KAB_WD_NS, D = KAB_WD_D, FBW = KAB_WD_FBW, FBK = KAB_WD_FBK, NREG = KAB_WD_NREG;
   static_assert(G == 8, "a group of 8 frames is one 64-bit backpointer word per lane");
@@ -134,13 +144,13 @@ __global__ void __launch_bounds__(KAB_WD_THREADS, 1)
         const char *lp_base = reinterpret_cast<const char *>(p.lp) + ((lat.t_off * (int64_t)V * 4) & ~(int64_t)15);
         const uint32_t chunk_stride = (uint32_t)(F * V * 4);
         const uint32_t full_bytes = (chunk_stride + skew * 4 + 15) & ~15u;
-        float poison = 0.0f;
+        float poison = kab_poison_init<CTC>();  // NaN once a rejected log-prob was staged (kab_poison_t)
         auto check_chunk = [&](int c) {
           const uint32_t gc = ec0 + (uint32_t)c, stg = gc % NS;
           kab_mbar_wait(&efull[stg], (gc / NS) & 1u);
           const float *w = stage_base + stg * stage_words + skew;
           const int nw = min(F, T - c * F) * V;
-          for (int j = lane; j < nw; j += 32) poison = kab_poison(poison, w[j]);
+          for (int j = lane; j < nw; j += 32) poison = kab_poison_t<CTC>(poison, w[j]);
         };
         for (int c = 0; c < n_chunks; ++c) {
           const uint32_t gc = ec0 + (uint32_t)c, stg = gc % NS, use = gc / NS;
@@ -184,13 +194,22 @@ __global__ void __launch_bounds__(KAB_WD_THREADS, 1)
         float s0 = (vb == 0) ? 0.0f : ninf, s1 = ninf, s2 = ninf, s3 = ninf;  // start state 0 (align.py:57-58)
         const uint32_t c1 = (vb + 1 > 0 && vb + 1 < S) ? 4u * col16[vb >> 1] : 0u;
         const uint32_t c3 = (vb + 3 > 0 && vb + 3 < S) ? 4u * col16[(vb >> 1) + 1] : 0u;
+        const uint32_t boff = CTC ? 4u * (uint32_t)blank : 0u;  // byte offset of the blank's column
+        // CTC: bit 0 / 1 = move 2 forbidden into label state vb+1 / vb+3 (state 1, outside the lattice
+        // -- the ghost lanes of warp 0 hold states below 0 --, or a repeated label)
+        uint32_t rep = 0;
+        if (CTC) {
+          const int l1 = vb >> 1;  // label index of state vb+1
+          if (vb + 1 < 3 || vb + 1 >= S || col16[l1] == col16[l1 - 1]) rep |= 1u;
+          if (vb + 3 < 3 || vb + 3 >= S || col16[l1 + 1] == col16[l1]) rep |= 2u;
+        }
         uint32_t st = ec0 % NS, ph = (ec0 / NS) & 1u;
         auto chunk_ptr = [&](uint32_t stg) { return reinterpret_cast<const char *>(stage_base + stg * stage_words + skew); };
         float eb[G], e1[G], e3[G], nb[G], n1[G], n3[G];
         auto load_group = [&](const char *row, float (&xb)[G], float (&x1)[G], float (&x3)[G]) {
 #pragma unroll
           for (int f = 0; f < G; ++f) {
-            xb[f] = *reinterpret_cast<const float *>(row + f * VB);
+            xb[f] = *reinterpret_cast<const float *>(row + f * VB + boff);
             x1[f] = *reinterpret_cast<const float *>(row + f * VB + c1);
             x3[f] = *reinterpret_cast<const float *>(row + f * VB + c3);
           }
@@ -230,6 +249,15 @@ __global__ void __launch_bounds__(KAB_WD_THREADS, 1)
           const float m2 = kab_blank_sel(t2, t1, th1, w, 1u << (sh + 4), 2u << (sh + 4), one);
           const float m3 = kab_label_sel(b0, b1, b2, b3, w, 1u << (sh + 6), 2u << (sh + 6), one);
           s0 = n0; s1 = m1; s2 = m2; s3 = m3;
+        };
+        // CTC: select on the previous scores, then one add; only h1 comes from the lane below
+        auto frame_ctc = [&](const float xb, const float x1, const float x3, uint32_t &w, const int sh) {
+          const float h1 = __shfl_up_sync(KAB_FULL_MASK, s3, 1);
+          const float n0 = __fadd_rn(kab_ctc_blank_sel(s0, h1, w, sh + 0), xb);
+          const float n1 = __fadd_rn(kab_ctc_label_sel(s1, s0, rep & 1u ? ninf : h1, w, sh + 2), x1);
+          const float n2 = __fadd_rn(kab_ctc_blank_sel(s2, s1, w, sh + 4), xb);
+          const float n3 = __fadd_rn(kab_ctc_label_sel(s3, s2, rep & 2u ? ninf : s1, w, sh + 6), x3);
+          s0 = n0; s1 = n1; s2 = n2; s3 = n3;
         };
 
         // ---- build the wavefront: wait until the warp below is KAB_WD_LAG groups ahead (its message
@@ -288,11 +316,17 @@ __global__ void __launch_bounds__(KAB_WD_THREADS, 1)
           uint32_t wlo = 0, whi = 0;
           if (nfr == G) {
 #pragma unroll
-            for (int f = 0; f < G; ++f) frame(eb[f], e1[f], e3[f], f < 4 ? wlo : whi, 8 * (f & 3));
+            for (int f = 0; f < G; ++f) {
+              if (CTC) frame_ctc(eb[f], e1[f], e3[f], f < 4 ? wlo : whi, 8 * (f & 3));
+              else frame(eb[f], e1[f], e3[f], f < 4 ? wlo : whi, 8 * (f & 3));
+            }
           } else {
 #pragma unroll
             for (int f = 0; f < G; ++f)
-              if (f < nfr) frame(eb[f], e1[f], e3[f], f < 4 ? wlo : whi, 8 * (f & 3));
+              if (f < nfr) {
+                if (CTC) frame_ctc(eb[f], e1[f], e3[f], f < 4 ? wlo : whi, 8 * (f & 3));
+                else frame(eb[f], e1[f], e3[f], f < 4 ? wlo : whi, 8 * (f & 3));
+              }
           }
           KAB_TM(td);
           // ---- message g for the warp above: (score, seq) pairs, one 8-byte store each
@@ -354,13 +388,20 @@ __global__ void __launch_bounds__(KAB_WD_THREADS, 1)
         // ---- this warp's highest active state and its score (align.py:99-101), then "finished"
         int cand = -1;
         float cs = 0.0f;
-        if (owned) {
+        if (CTC) {  // the scores of the two end states S-1 -> ctl[3], S-2 -> ctl[0] (end rule: backtrack CTA)
+          if (owned) {
+            if (vb + 0 == S - 1) ctl[3] = __float_as_uint(s0);
+            if (vb + 2 == S - 1) ctl[3] = __float_as_uint(s2);
+            if (vb + 1 == S - 2) ctl[0] = __float_as_uint(s1);
+            if (vb + 3 == S - 2) ctl[0] = __float_as_uint(s3);
+          }
+        } else if (owned) {
           if (vb + 0 < S && s0 > ninf) { cand = vb + 0; cs = s0; }
           if (vb + 1 < S && s1 > ninf) { cand = vb + 1; cs = s1; }
           if (vb + 2 < S && s2 > ninf) { cand = vb + 2; cs = s2; }
           if (vb + 3 < S && s3 > ninf) { cand = vb + 3; cs = s3; }
         }
-        const int wcand = __reduce_max_sync(KAB_FULL_MASK, cand);
+        const int wcand = __reduce_max_sync(KAB_FULL_MASK, cand);  // (CTC: -1)
         if (cand >= 0 && cand == wcand) {
           int2 *cp = reinterpret_cast<int2 *>(ws + kab_wide_cand_off()) + gw;
           *cp = make_int2(cand, __float_as_int(cs));
@@ -394,15 +435,26 @@ __global__ void __launch_bounds__(KAB_WD_THREADS, 1)
         if (done >= (unsigned int)nww) break;
         __nanosleep(500);
       }
-      const int v = (int)kab_ld_volatile_u32(&ctl[0]) - 1;
-      const int status = kab_ld_volatile_u32(&ctl[1]) ? 3 : (v < 0 ? 1 : 0);
-      s_v = v;
-      s_status = status;
-      p.status[lat.index] = status;
-      if (p.final_score) {
-        float fs = __int_as_float(0x7fc00000);
-        if (status == 0) fs = __int_as_float(reinterpret_cast<const int2 *>(ws + kab_wide_cand_off())[v / OW].y);
-        p.final_score[lat.index] = fs;
+      if (CTC) {  // end rule: S-1 if a[S-1] > a[S-2], else S-2 (a tie, and two -inf, pick S-2)
+        const int S = 2 * lat.L + 1;
+        const float a1 = __uint_as_float(kab_ld_volatile_u32(&ctl[3])), a2 = __uint_as_float(kab_ld_volatile_u32(&ctl[0]));
+        const int v = a1 > a2 ? S - 1 : S - 2;
+        const int status = kab_ld_volatile_u32(&ctl[1]) ? 3 : 0;
+        s_v = v;
+        s_status = status;
+        p.status[lat.index] = status;
+        if (p.final_score) p.final_score[lat.index] = status == 0 ? (a1 > a2 ? a1 : a2) : __int_as_float(0x7fc00000);
+      } else {
+        const int v = (int)kab_ld_volatile_u32(&ctl[0]) - 1;
+        const int status = kab_ld_volatile_u32(&ctl[1]) ? 3 : (v < 0 ? 1 : 0);
+        s_v = v;
+        s_status = status;
+        p.status[lat.index] = status;
+        if (p.final_score) {
+          float fs = __int_as_float(0x7fc00000);
+          if (status == 0) fs = __int_as_float(reinterpret_cast<const int2 *>(ws + kab_wide_cand_off())[v / OW].y);
+          p.final_score[lat.index] = fs;
+        }
       }
     }
     __syncthreads();
@@ -433,7 +485,7 @@ __global__ void __launch_bounds__(KAB_WD_THREADS, 1)
         const int *pbuf = pathbuf + (b & 1) * FBK;
         for (int i = i0 + (tid - first_thread); i < i1; i += n_threads) {
           const int pv = pbuf[i - i0];
-          const int lab = (pv & 1) ? (int)col16[(pv - 1) >> 1] : 0;
+          const int lab = (pv & 1) ? (int)col16[(pv - 1) >> 1] : (CTC ? blank : 0);
           out_path[i] = pv;
           out_lab[i] = lab;                              // align.py:106
           out_sc[i] = __ldg(&lp[(int64_t)i * V + lab]);  // align.py:107
@@ -522,4 +574,15 @@ __global__ void __launch_bounds__(KAB_WD_THREADS, 1)
     }
     __syncthreads();
   }
+}
+
+__global__ void __launch_bounds__(KAB_WD_THREADS, 1)
+    kab_wide_kernel(const KabLattice *__restrict__ lats, int n_lat, KabParams p, unsigned char *wide_ws) {
+  kab_wide_body<false>(lats, n_lat, p, wide_ws, 0);
+}
+
+// CTC forced alignment (blank column: see kab_warp_ctc_kernel)
+__global__ void __launch_bounds__(KAB_WD_THREADS, 1)
+    kab_wide_ctc_kernel(const KabLattice *__restrict__ lats, int n_lat, KabParams p, unsigned char *wide_ws, int blank) {
+  kab_wide_body<true>(lats, n_lat, p, wide_ws, blank);
 }
