@@ -105,6 +105,10 @@ int kab_plan_create(kab_plan **plan, int device, int64_t n_lattices, const int64
  * to the blank, KAB_ST_NONFINITE for a NaN or +inf log-prob (-inf is accepted: masking).
  * kab_plan_segment_stats_device and kab_plan_run_host_segments return KAB_E_UNSUPPORTED.
  * KAB_E_BAD_ARG for a blank outside [0, vocab_size).
+ * Classes: S <= 248 KAB_CLASS_WARP, S <= 3296 KAB_CLASS_BAND, longer lattices KAB_CLASS_GENERIC.  A
+ * vocabulary above 512 reaches the warp and band classes through a compact copy of each lattice's own
+ * columns (the blank first, then its distinct labels; DESIGN.md 3.9c); a lattice with more than 511
+ * distinct labels goes to KAB_CLASS_GENERIC on its own.  The outputs are the same on every class.
  */
 int kab_plan_create_ctc(kab_plan **plan, int device, int64_t n_lattices, const int64_t *t_off,
                         const int32_t *labels, const int64_t *l_off, int32_t vocab_size, int32_t blank);
@@ -113,7 +117,8 @@ int kab_plan_create_ctc(kab_plan **plan, int device, int64_t n_lattices, const i
  * one lattice): the same arguments, outputs, statuses and errors, but lattices with more than 3296
  * states go to KAB_CLASS_WIDE (a chain of warps over the whole GPU, 2 bits of backpointer per cell)
  * instead of KAB_CLASS_GENERIC (1 byte per cell) where they fit -- vocab_size <= 338 (the wide
- * kernel's emission stages) and ceil(S/104)/4 + 1 CTAs resident at once -- and where a makespan
+ * kernel's emission stages; above 512, the compact width Vc <= 336, i.e. at most 335 distinct labels
+ * in the plan's largest compact lattice) and ceil(S/104)/4 + 1 CTAs resident at once -- and where a makespan
  * estimate says so: wide lattices run one after another, each on the whole GPU, generic ones side by
  * side, so a batch of many shorter lattices may stay generic (DESIGN.md 3.9).  Warp and band
  * lattices are routed as by kab_plan_create_ctc.

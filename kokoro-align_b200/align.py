@@ -73,7 +73,10 @@ class AlignPlan:
         than ``blank``.  best_labels are then token ids per frame (``blank`` on even states).
         long_form=True (kab_plan_create_ctc_long): lattices with more than 3296 states run on the
         wide kernel where it fits and is estimated faster (a whole chapter in one lattice), with the
-        same outputs."""
+        same outputs.  Wide vocabularies (vocab_size > 512, e.g. NeMo's 1025) reach the warp, band
+        and wide kernels through a compact copy of every lattice's own columns; a lattice with more
+        than 511 distinct labels runs on the generic kernel on its own, and the wide kernel takes
+        long lattices while no compact lattice of the plan has more than 335 distinct labels."""
         plan = cls.__new__(cls)
         plan._setup(t_off, labels, l_off, vocab_size, device)
         L = _lib.lib()
@@ -303,8 +306,10 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
     torchaudio.functional.merge_tokens takes.  Bit-exact with torchaudio's CPU implementation
     whenever the chosen end state has a finite score (where both end states are -inf, torchaudio's
     traceback is undefined; this one follows the recurrence, DESIGN.md 3.9).  NaN or +inf
-    log-probs raise ValueError (-inf, for masking, is accepted).  long_form=True: a lattice of more
-    than 3296 states (2 L + 1) runs on the wide kernel, with the same outputs (AlignPlan.ctc)."""
+    log-probs raise ValueError (-inf, for masking, is accepted), in any column of the row.
+    long_form=True: a lattice of more than 3296 states (2 L + 1) runs on the wide kernel, with the
+    same outputs.  Any vocabulary size up to 65535 reaches the staged kernels while the target has at
+    most 511 distinct ids (AlignPlan.ctc)."""
     import torch
     _ctc_tensor_checks(log_probs, targets, blank)
     if log_probs.size(0) != 1 or targets.size(0) != 1:
@@ -343,7 +348,8 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
     (paths [B, T_max] of the targets' dtype, scores float32 [B, T_max]) on the input's device;
     frames past an item's length hold the blank and score 0.  Raises, like forced_align, for the
     first item that fails, naming its index.  On CUDA the valid rows are packed on the device.
-    long_form: as in forced_align."""
+    long_form: as in forced_align.  With more than 512 classes, the items with at most 511 distinct
+    target ids run on the staged kernels and the others on the generic kernel (AlignPlan.ctc)."""
     import torch
     _ctc_tensor_checks(log_probs, targets, blank)
     B, T_max, V = (int(x) for x in log_probs.shape)

@@ -404,10 +404,16 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
     }
     pl->band_ga = ok && any_band;
   }
-  if (!ctc && V > MAX_STAGE_V && M <= 4) {
+  // CTC plans: the compact copy with the blank as compact column 0 (kab_compact_ctc_kernel).  Vc is sized
+  // by the lattices that fit it; one with more than MAX_STAGE_V - 1 distinct labels goes to the generic
+  // kernel on its own instead of taking the whole plan there.  KAB_CTC_COMPACT=0 (development, the
+  // reference arm of the tests and tools/forced_align_vocab_bench.py) sends every lattice there.
+  const bool ctc_compact = ctc && V > MAX_STAGE_V && [] { const char *ce = getenv("KAB_CTC_COMPACT"); return !(ce && atoi(ce) == 0); }();
+  if ((!ctc && V > MAX_STAGE_V && M <= 4) || ctc_compact) {
     std::vector<uint8_t> seen((size_t)V, 0);
     int64_t dmax = 0;
     bool any = false;
+    auto in_range = [&](int32_t x) { return ctc ? (x >= 0 && x < V && x != blank) : (x > 0 && x < V); };
     for (int64_t b = 0; b < B; ++b) {
       if (mask && !mask[b]) continue;
       const int64_t L = l_off[b + 1] - l_off[b];
@@ -416,12 +422,12 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
       bool usable = true;
       int64_t dist = 0;
       for (int64_t l = 0; l < L && usable; ++l) {
-        if (lab[l] <= 0 || lab[l] >= V) usable = false;
+        if (!in_range(lab[l])) usable = false;
         else if (!seen[(size_t)lab[l]]) { seen[(size_t)lab[l]] = 1; ++dist; }
       }
       for (int64_t l = 0; l < L; ++l)
-        if (lab[l] > 0 && lab[l] < V) seen[(size_t)lab[l]] = 0;
-      if (usable) { dmax = std::max(dmax, dist); any = true; }
+        if (in_range(lab[l])) seen[(size_t)lab[l]] = 0;
+      if (usable && (!ctc || dist + 1 <= MAX_STAGE_V)) { dmax = std::max(dmax, dist); any = true; }
     }
     if (any && dmax + 1 <= MAX_STAGE_V) {
       pl->Vc = (int32_t)std::max<int64_t>(8, align_up(dmax + 1, 4));
@@ -492,9 +498,11 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
     }
     const bool ga = pl->band_ga && !f.special && band_shaped(T, S);
     if (!f.bad && pl->Vc && !f.special && !ga && f.distinct + 1 <= pl->Vc) {
-      // compact numbering: blank 0, then the lattice's distinct label columns in ascending order
+      // compact numbering: the blank's column (0, or the CTC blank id), then the lattice's distinct label
+      // columns in ascending order
       f.compact = 1;
       int32_t *g = h_gather.data() + (size_t)b * pl->Vc;
+      g[0] = ctc ? blank : 0;
       int32_t n = 1;
       for (int w = 0; w < n_mask; ++w)
         for (int64_t m = distinct_mask[w]; m; m &= m - 1) g[n++] = w * 64 + __builtin_ctzll((unsigned long long)m);
@@ -529,12 +537,15 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
   // tools/forced_align_long_bench.py, DESIGN.md 3.9) gives all lattices that both kernels could take to one of
   // them: wide ~102 ns per frame of a sequence of lattices; generic 0.68 Gcells/s for a lone lattice (its
   // longest one bounds it) and 79 Gcells/s for 256 lattices side by side.  256 utterances of 2-5 minutes:
-  // 276 ms wide, 230 ms generic; one 10-minute utterance: 5.2 ms wide, 796 ms generic.
+  // 276 ms wide, 230 ms generic; one 10-minute utterance: 5.2 ms wide, 796 ms generic.  (Compact plans, V > 512:
+  // 177 ns per frame wide at Vc = 272 and 0.58 Gcells/s for a lone generic lattice at V = 1025; the constants
+  // stay, DESIGN.md 3.9c.)
   bool ctc_wide = false;
   if (ctc && ctc_long) {
     double frames = 0.0, cells = 0.0, max_cells = 0.0;
     for (int64_t b = 0; b < B; ++b) {
       if ((mask && !mask[b]) || facts[(size_t)b].bad) continue;
+      if (pl->Vc && !facts[(size_t)b].compact) continue;  // (too many distinct labels for the compact copy: generic)
       const int64_t T = t_off[b + 1] - t_off[b], S = 2 * (l_off[b + 1] - l_off[b]) + 1;
       if (S + 32 <= KAB_BAND_OW * BAND_MAX_WARPS) continue;  // warp or band class
       if (((S + KAB_BAND_OW - 1) / KAB_BAND_OW + KAB_WD_CW - 1) / KAB_WD_CW + 1 > wide_capacity) continue;
@@ -893,7 +904,7 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
   }
   if (!pl->bt_meta.empty()) info.kernel_launches += 3;  // kab_bt_maps_kernel, kab_bt_stitch_kernel, kab_bt_gather_kernel
   if (pl->band_r) info.kernel_launches += 1;            // kab_finite_rows_kernel
-  if (pl->Vc)                                          // kab_compact_kernel, kab_expand_labels_kernel
+  if (pl->Vc)                                          // kab_compact_kernel (CTC: _ctc_), kab_expand_labels_kernel
     for (int q : {Q_WARP, Q_BAND, Q_WIDE}) info.kernel_launches += pl->lists[q].empty() ? 0 : 2;
   if (hyb_k > 0) {  // the sub-plan of a hybrid band plan: same arrays, its own lattices, workspaces and stream
     int rcs = plan_create_impl(&pl->sub, device, B, t_off, labels, l_off, V, W, M, hyb_mask.data(), 1, pl->ctc, pl->blank, pl->ctc_long);
@@ -960,13 +971,20 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
     for (int q : fast_lists)
       if (!pl->lists[q].empty() && !(q == Q_BAND && pl->band_ga)) {
         const dim3 grid((unsigned)pl->lists[q].size(), (unsigned)((pl->max_T[q] + KAB_COMPACT_FRAMES - 1) / KAB_COMPACT_FRAMES));
-        kab_compact_kernel<<<grid, 256, 0, stream>>>(pl->d_lists[q], d_log_probs, pl->d_lpc, pl->d_gather, pl->V, pl->Vc,
-                                                     pl->d_nonfinite);
+        if (pl->ctc)
+          kab_compact_ctc_kernel<<<grid, 256, 0, stream>>>(pl->d_lists[q], d_log_probs, pl->d_lpc, pl->d_gather, pl->V, pl->Vc,
+                                                           pl->d_nonfinite);
+        else
+          kab_compact_kernel<<<grid, 256, 0, stream>>>(pl->d_lists[q], d_log_probs, pl->d_lpc, pl->d_gather, pl->V, pl->Vc,
+                                                       pl->d_nonfinite);
       }
     pf.lp = pl->d_lpc;
     pf.V = pl->Vc;
     pf.lp_bytes = pl->total_T * (int64_t)pl->Vc * 4;
   }
+  // CTC: the blank's column in the staged kernels' view (compact column 0 of the copy); the generic kernel
+  // reads the caller's array and keeps the blank id
+  const int32_t sblank = pl->Vc ? 0 : pl->blank;
 
   if (pl->sub) {  // hybrid band plan: the long lattices first (their clusters need whole SMs), on the side stream
     KAB_CUDA(cudaEventRecord(pl->ev_fork, stream));
@@ -988,7 +1006,7 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
     const int nwl = (int)pl->lists[Q_WARP].size();
     const dim3 wg((unsigned)pl->grid[Q_WARP]), wb(KAB_WARPS_PER_CTA * 32);
     if (pl->ctc) {
-      kab_warp_ctc_kernel<<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw, pl->blank);
+      kab_warp_ctc_kernel<<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw, sblank);
     } else if (pl->M == 4) {
       if (pf.V == 39) kab_warp_kernel<39, false><<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw);
       else kab_warp_kernel<0, false><<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw);
@@ -1057,8 +1075,8 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
       const int nbl = (int)pl->lists[Q_BAND].size();
       const dim3 bg((unsigned)pl->grid[Q_BAND]), bb((unsigned)(pl->band_nw * 32));
       if (pl->ctc) {
-        if (pl->band_nw <= 16) kab_band_ctc_kernel<512><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb, pl->blank);
-        else kab_band_ctc_kernel<1024><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb, pl->blank);
+        if (pl->band_nw <= 16) kab_band_ctc_kernel<512><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb, sblank);
+        else kab_band_ctc_kernel<1024><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb, sblank);
       } else if (pl->band_nw <= 16) {
         if (pl->M == 4) kab_band_kernel<512, false><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb);
         else kab_band_kernel<512, true><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb);
@@ -1076,7 +1094,7 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
     const KabLattice *wl = pl->d_lists[Q_WIDE];
     int wn = (int)pl->lists[Q_WIDE].size();
     unsigned char *wws = pl->d_wide_ws;
-    int wblank = pl->blank;
+    int wblank = sblank;
     void *wargs[] = {(void *)&wl, (void *)&wn, (void *)&pf, (void *)&wws, (void *)&wblank};
     const void *wfn = pl->ctc ? (const void *)kab_wide_ctc_kernel : (const void *)kab_wide_kernel;
     KAB_CUDA(cudaLaunchCooperativeKernel(wfn, dim3((unsigned)pl->grid[Q_WIDE]), dim3(KAB_WD_THREADS), wargs,

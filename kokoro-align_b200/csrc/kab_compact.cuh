@@ -10,29 +10,48 @@
 // as every other kernel has it): the gather kernel streams the whole rows once
 // (coalesced; 4 V bytes per frame, a fraction of what the recurrence moves) and flags the lattice,
 // and the label expansion that runs after the staged kernels turns the flag into the status.
+// CTC forced-alignment plans (kab_plan_create_ctc, V > 512) use the same copy with gather[b][0] = the
+// plan's blank id; their staged kernels then take blank column 0, and a lattice with more than 511
+// distinct labels goes to the generic kernel on its own (not the whole plan).  The whole-row check is the CTC one
+// there (kab_poison_t<true>): NaN and +inf flag the lattice, -inf (masking) does not -- what
+// kab_generic_ctc_kernel checks over the same rows.
 #pragma once
 #include "kab_common.cuh"
 
 #define KAB_COMPACT_FRAMES 64  // frames per CTA of the two helper kernels
 
 // grid (lattices of one work list, frame chunks); block 256 = 8 warps, a warp per frame
-__global__ void kab_compact_kernel(const KabLattice *__restrict__ lats, const float *__restrict__ lp,
-                                   float *__restrict__ lpc, const int32_t *__restrict__ gather, int V, int Vc,
-                                   int32_t *__restrict__ nonfinite) {
+template <bool CTC>
+__device__ __forceinline__ void kab_compact_body(const KabLattice *__restrict__ lats, const float *__restrict__ lp,
+                                                 float *__restrict__ lpc, const int32_t *__restrict__ gather, int V,
+                                                 int Vc, int32_t *__restrict__ nonfinite) {
   const KabLattice lat = lats[blockIdx.x];
   const int f0 = blockIdx.y * KAB_COMPACT_FRAMES;
   if (f0 >= lat.T) return;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int32_t *g = gather + (size_t)lat.index * Vc;
   const int f1 = min(lat.T, f0 + KAB_COMPACT_FRAMES);
-  float poison = 0.0f;
+  float poison = kab_poison_init<CTC>();
   for (int f = f0 + warp; f < f1; f += 8) {
     const float *src = lp + (size_t)(lat.t_off + f) * V;
     float *dst = lpc + (size_t)(lat.t_off + f) * Vc;
-    for (int j = lane; j < V; j += 32) poison = kab_poison(poison, __ldg(src + j));  // the whole row, once
-    for (int j = lane; j < Vc; j += 32) dst[j] = __ldg(src + g[j]);                  // (now L1 / L2 hits)
+    for (int j = lane; j < V; j += 32) poison = kab_poison_t<CTC>(poison, __ldg(src + j));  // the whole row, once
+    for (int j = lane; j < Vc; j += 32) dst[j] = __ldg(src + g[j]);                         // (now L1 / L2 hits)
   }
   if (__any_sync(KAB_FULL_MASK, poison != poison) && lane == 0) nonfinite[lat.index] = 1;
+}
+
+__global__ void kab_compact_kernel(const KabLattice *__restrict__ lats, const float *__restrict__ lp,
+                                   float *__restrict__ lpc, const int32_t *__restrict__ gather, int V, int Vc,
+                                   int32_t *__restrict__ nonfinite) {
+  kab_compact_body<false>(lats, lp, lpc, gather, V, Vc, nonfinite);
+}
+
+// CTC forced alignment: gather[b][0] is the blank's column; NaN / +inf anywhere in the rows flag the lattice
+__global__ void kab_compact_ctc_kernel(const KabLattice *__restrict__ lats, const float *__restrict__ lp,
+                                       float *__restrict__ lpc, const int32_t *__restrict__ gather, int V, int Vc,
+                                       int32_t *__restrict__ nonfinite) {
+  kab_compact_body<true>(lats, lp, lpc, gather, V, Vc, nonfinite);
 }
 
 // best_labels: compact index -> label value, for the lattices that were aligned (status 0)
