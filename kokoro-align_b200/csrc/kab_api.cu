@@ -15,8 +15,10 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <limits>
 #include <new>
+#include <optional>
 #include <vector>
 
 #include "kab_band.cuh"
@@ -115,9 +117,21 @@ constexpr int MAX_STAGE_V = 512;  // widest vocabulary the staged (warp / band) 
 
 inline int64_t align_up(int64_t x, int64_t a) { return (x + a - 1) / a * a; }
 
+// the window of align.py:64-65 never clips: every frame sees the whole lattice
+inline bool unbanded(int64_t T, int64_t S, int64_t W) { return W >= S && (S * (T - 1)) / T <= W / 2; }
+
+// a lattice the band kernels take (not the warp class, and its window fits a CTA's ring)
+inline bool band_shaped(int64_t T, int64_t S, int64_t W) {
+  if (unbanded(T, S, W) && S <= 248) return false;  // warp class
+  return W >= 1 && S <= 3 * T && std::min<int64_t>(W, S) + 32 <= (int64_t)KAB_BAND_OW * BAND_MAX_WARPS;
+}
+
+// forward CTAs of the wide kernel's chain of warps over S states (the backtrack CTA comes on top)
+inline int64_t wide_ctas(int64_t S) { return ((S + KAB_BAND_OW - 1) / KAB_BAND_OW + KAB_WD_CW - 1) / KAB_WD_CW; }
+
 int64_t cells_eval_of(int64_t T, int64_t S, int64_t W) {
   // sum_i (hi_i - lo_i), align.py:64-65.  Closed form when the window never clips.
-  if (W >= S && (S * (T - 1)) / T <= W / 2) return T * S;
+  if (unbanded(T, S, W)) return T * S;
   int64_t cells = 0;
   for (int64_t i = 0; i < T; ++i) {
     int64_t lo = std::max<int64_t>(0, (S * i) / T - W / 2);
@@ -129,10 +143,34 @@ int64_t cells_eval_of(int64_t T, int64_t S, int64_t W) {
 
 }  // namespace
 
+// What a plan computes.  Child plans (segments, book pipes, the hybrid sub-plan) take their parent's.
+struct PlanSpec {
+  int32_t V = 0, W = 0, M = 0;
+  bool ctc = false;       // CTC forced-alignment plan (kab_plan_create_ctc)
+  int32_t blank = 0;      // ... and its blank id
+  bool ctc_long = false;  // ... whose lattices too wide for the band kernel go to the wide kernel (kab_plan_create_ctc_long)
+};
+
+// The kernel of a plan's band list.  CTA: kab_band.cuh (two lattices per SM).  The cluster kernels: P kab_bandp.cuh
+// (KabBtLayoutP, has its own backtrack walker), Q kab_bandq.cuh (two states per lane, KabBtLayoutQ), R kab_bandr.cuh
+// (Q's lanes, warp-specialised: prep warps, shared-memory mailboxes), R_GATHER kab_bandr.cuh in its gather mode
+// (V > 512: emissions straight from the caller's log-probs, any number of distinct labels, no compact copy).
+enum class BandKernel { CTA, P, Q, R, R_GATHER };
+
+// How a warp, band or wide list is launched; resolved once at plan creation
+struct Launch {
+  const void *fn = nullptr;
+  dim3 grid, block;
+  size_t smem = 0;
+  unsigned cluster = 0;                       // > 0: cluster dimension (cluster band kernels)
+  bool cooperative = false;                   // the whole grid must be resident (wide kernel)
+  int32_t stage_frames = 0, stage_bytes = 0;  // band list: the emission staging of its KabParams
+};
+
 struct kab_plan {
   int device = 0;
   int64_t B = 0, total_T = 0, total_L = 0;
-  int32_t V = 0, W = 0, M = 0;
+  PlanSpec spec;
   int32_t Vc = 0;              // > 0: the staged kernels work on compact log-probs of Vc columns (kab_compact.cuh)
   int32_t *d_gather = nullptr;  // [B][Vc] compact column -> column of log_probs (= label value)
   float *d_lpc = nullptr;       // [sum T][Vc] compact log-probs
@@ -141,9 +179,8 @@ struct kab_plan {
   int sm_count = 0;
   int32_t stage_frames = 0, stage_bytes = 0;
   int32_t band_nw = 0;  // warps per CTA of the band kernel (ring of 104 * band_nw states)
-  int32_t band_nc = 0;  // > 0: a cluster band kernel (kab_bandp.cuh / kab_bandq.cuh) with clusters of band_nc CTAs
-  bool band_q = false;  // the cluster kernel is kab_bandq_kernel / kab_bandr_kernel (two states per lane, KabBtLayoutQ)
-  bool band_r = false;  // ... kab_bandr_kernel (warp-specialised: prep warps, shared-memory mailboxes)
+  BandKernel band_kernel = BandKernel::CTA;
+  int32_t band_nc = 0, band_cw = 0;  // cluster band kernels: CTAs per cluster, compute warps per CTA
   // Hybrid band plan: the longest band lattices run in a sub-plan (kab_bandr.cuh, whole clusters: the
   // shortest frame) on a side stream while this plan's single-CTA kernel (kab_band.cuh: the highest
   // throughput) takes the others on the SMs that are left.
@@ -153,15 +190,9 @@ struct kab_plan {
   int32_t band_sm_reserved = 0;  // SMs left to the sub-plan's clusters
   unsigned int *d_started = nullptr;  // sub-plan: CTAs of kab_bandr_kernel that have started, over all runs
   unsigned int gate_target = 0;       // ... and the count the current run will bring it to
-  bool band_ga = false;  // the band lattices run kab_bandr_kernel in its gather mode (V > 512: emissions straight from the
-                         // caller's log-probs, any number of distinct labels, no compact copy)
-  int32_t band_cw = 0;  // compute warps per CTA of that kernel (ring of 40 * band_cw * band_nc slots)
   kab_plan_info info{};
   std::vector<KabLattice> lists[N_QUEUES];
   bool any_bad_label = false;  // some lattices have a status decided here (bad label; CTC: T < L + R too)
-  bool ctc = false;            // CTC forced-alignment plan (kab_plan_create_ctc)
-  int32_t blank = 0;           // ... and its blank id
-  bool ctc_long = false;       // ... whose lattices too wide for the band kernel go to the wide kernel (kab_plan_create_ctc_long)
   // device memory
   KabLattice *d_lists[N_QUEUES] = {};
   uint16_t *d_col16 = nullptr;
@@ -180,9 +211,7 @@ struct kab_plan {
   int32_t bt_blocks = 0, bt_max_wl = 0;
   unsigned char *d_band_fifo = nullptr;  // cluster band kernel: per-lattice progress counters and FIFOs
   int64_t band_fifo_bytes = 0;
-  // launch geometry
-  int grid[N_QUEUES] = {};
-  size_t smem[N_QUEUES] = {};
+  Launch launch[N_QUEUES];  // (the generic list: its grid only)
   // host copies (used to build the pipelined segments of kab_plan_run_host)
   std::vector<int64_t> h_t_off, h_l_off;
   std::vector<int32_t> h_labels;
@@ -324,12 +353,9 @@ int kab_device_count(int *count) {
 
 namespace {
 // mask: only the lattices with mask[b] != 0 belong to this plan (nullptr: all); band_mode: -1 the
-// plan chooses (and may go hybrid), 0 the single-CTA band kernel, 1 kab_bandr.cuh; ctc: a CTC
-// forced-alignment plan with blank id `blank` (W and M as kab_plan_create_ctc sets them); ctc_long: its
-// lattices with S > 3296 go to the wide kernel where they fit (kab_plan_create_ctc_long)
-int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
-                     const int64_t *l_off, int32_t V, int32_t W, int32_t M, const uint8_t *mask, int band_mode,
-                     bool ctc, int32_t blank, bool ctc_long);
+// plan chooses (and may go hybrid), 0 the single-CTA band kernel, 1 kab_bandr.cuh
+int plan_create_impl(kab_plan **out, int device, const PlanSpec &s, int64_t B, const int64_t *t_off,
+                     const int32_t *labels, const int64_t *l_off, const uint8_t *mask, int band_mode);
 // CTC plans: every lattice is unbanded -- a window this wide is [0, S) in every frame of the band
 // kernel (S <= 3296 there) -- and has three moves
 constexpr int32_t CTC_W = 0x3fffffff, CTC_M = 3;
@@ -337,201 +363,187 @@ constexpr int32_t CTC_W = 0x3fffffff, CTC_M = 3;
 
 int kab_plan_create(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
                     const int64_t *l_off, int32_t V, int32_t W, int32_t M) {
-  return plan_create_impl(out, device, B, t_off, labels, l_off, V, W, M, nullptr, -1, false, 0, false);
+  return plan_create_impl(out, device, PlanSpec{V, W, M}, B, t_off, labels, l_off, nullptr, -1);
 }
 
 int kab_plan_create_ctc(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
                         const int64_t *l_off, int32_t V, int32_t blank) {
   if (blank < 0 || blank >= V) return KAB_E_BAD_ARG;
   // (only the single-CTA band kernel has a CTC mode)
-  return plan_create_impl(out, device, B, t_off, labels, l_off, V, CTC_W, CTC_M, nullptr, 0, true, blank, false);
+  return plan_create_impl(out, device, PlanSpec{V, CTC_W, CTC_M, true, blank}, B, t_off, labels, l_off, nullptr, 0);
 }
 
 int kab_plan_create_ctc_long(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
                              const int64_t *l_off, int32_t V, int32_t blank) {
   if (blank < 0 || blank >= V) return KAB_E_BAD_ARG;
   // (the single-CTA band kernel below S = 3297, the wide kernel above it where it fits)
-  return plan_create_impl(out, device, B, t_off, labels, l_off, V, CTC_W, CTC_M, nullptr, 0, true, blank, true);
+  return plan_create_impl(out, device, PlanSpec{V, CTC_W, CTC_M, true, blank, true}, B, t_off, labels, l_off, nullptr, 0);
 }
 
 namespace {
-int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
-                     const int64_t *l_off, int32_t V, int32_t W, int32_t M, const uint8_t *mask, int band_mode,
-                     bool ctc, int32_t blank, bool ctc_long) {
-  if (!out || B < 0 || !t_off || !l_off || V < 1 || V > 65535 || W < 0 || M < 1 || M > 255) return KAB_E_BAD_ARG;
-  if (B > 0 && (t_off[0] < 0 || l_off[0] < 0)) return KAB_E_BAD_ARG;
-  if (B > 0 && l_off[B] > l_off[0] && !labels) return KAB_E_BAD_ARG;
-  for (int64_t b = 0; b < B; ++b) {
-    const int64_t T = t_off[b + 1] - t_off[b], L = l_off[b + 1] - l_off[b];
-    if (T < 1 || T > 0x3fffffff || L < 0 || L > 0x3ffffff0) return KAB_E_BAD_ARG;
-  }
-  DeviceGuard guard;
-  KAB_CUDA(guard.enter(device));
-  kab_plan *pl = new (std::nothrow) kab_plan();
-  if (!pl) return KAB_E_NOMEM;
-  pl->device = device; pl->B = B; pl->V = V; pl->W = W; pl->M = M;
-  pl->ctc = ctc; pl->blank = blank; pl->ctc_long = ctc_long;
-  pl->total_T = B ? t_off[B] : 0;  // offsets are absolute rows / entries of the caller's arrays
-  pl->total_L = B ? l_off[B] : 0;
-  if (B > 0) {
-    pl->h_t_off.assign(t_off, t_off + B + 1);
-    pl->h_l_off.assign(l_off, l_off + B + 1);
-    if (pl->total_L > 0) pl->h_labels.assign(labels, labels + pl->total_L);
-  }
-  Trace tr("kab_plan_create");
-  if (int rcs = sm_count_of(device, &pl->sm_count)) { delete pl; return rcs; }
 
-  // ---- wide vocabularies: can the staged kernels work on a compact copy of the log-probs?
-  // (every lattice they would take uses at most MAX_STAGE_V - 1 distinct label columns)
-  std::vector<int32_t> h_gather;
+// The development / test knobs KAB_<NAME> of INTEGRATION.md section 6 (-1: not set), read at every plan
+// creation: tests change them between plans.  serial_bt: KAB_BAND_SERIAL_BT != 0.
+struct Knobs {
+  int stage_frames, band_cluster, band_q, band_r, band_hybrid, serial_bt, warp_ctas_per_sm;
+  bool band_gather, ctc_compact, serial_setup;
+  static int get(const char *name) { const char *v = getenv(name); return v ? atoi(v) : -1; }
+  static Knobs read() {
+    const char *sb = getenv("KAB_BAND_SERIAL_BT");
+    return Knobs{get("KAB_STAGE_FRAMES"), get("KAB_BAND_CLUSTER"), get("KAB_BAND_Q"), get("KAB_BAND_R"), get("KAB_BAND_HYBRID"),
+                 sb ? (atoi(sb) != 0) : -1, get("KAB_WARP_CTAS_PER_SM"), get("KAB_BAND_GATHER") != 0, get("KAB_CTC_COMPACT") != 0,
+                 getenv("KAB_SERIAL_SETUP") != nullptr};
+  }
+};
+
+// what the label scan finds out about one lattice (repeats: adjacent equal labels)
+struct LatFacts { uint8_t bad, special, compact; int32_t distinct, repeats; int64_t col_off; };
+
+// The working state of one plan creation, handed from stage to stage
+struct Setup {
+  kab_plan *pl;
+  const PlanSpec &s;
+  const Knobs knob;
+  int64_t B;
+  const int64_t *t_off, *l_off;
+  const int32_t *labels;
+  const uint8_t *mask;
+  bool gather = false;  // band-shaped lattices run kab_bandr.cuh's gather mode (BandKernel::R_GATHER)
+  int32_t Veff = 0;     // vocabulary the staged kernels see
+  std::vector<LatFacts> facts;
+  std::vector<int32_t> gather_rows;  // [B][Vc] compact column -> column of log_probs
+  std::vector<uint16_t> col16;
+  std::vector<int32_t> status_init;
+  int64_t bp_bytes = 0, scr_floats = 0, max_band_weff = 0;
+  int wide_capacity = 0, wide_max_ctas = 0;
+  std::vector<uint8_t> hyb_mask;  // hybrid band plan: the lattices of the sub-plan
+  int hyb_k = 0;                  // ... and its clusters
+  bool in(int64_t b) const { return !mask || mask[b]; }
+  int64_t frames(int64_t b) const { return t_off[b + 1] - t_off[b]; }
+  int64_t len(int64_t b) const { return l_off[b + 1] - l_off[b]; }
+  void for_lattices(const std::function<void(int64_t, int64_t *)> &fn) const;
+  void scan_labels(), compact_vocabulary(), classify(), choose_band_kernel(int band_mode), lay_out_band();
+  int allocate(), finish();
+};
+
+// The label scans (range check, distinct labels, column table) are independent per lattice and are
+// most of plan creation for a batch of 10 000 segments (4.5 of 5 ms): several host threads do them
+// ahead of the (cheap, sequential) classification.  fn(b, scratch bit words) over the plan's lattices.
+void Setup::for_lattices(const std::function<void(int64_t, int64_t *)> &fn) const {
+  const int n_mask = (s.V + 63) / 64;
+  const unsigned hw = std::thread::hardware_concurrency();
+  const int nt = (B >= 2048 && pl->total_L >= 65536 && hw >= 4 && !knob.serial_setup) ? (int)std::min<unsigned>(8, hw / 2) : 1;
+  auto work = [&](int t) {
+    std::vector<int64_t> words((size_t)std::max(n_mask, 1), 0);
+    const int64_t b0 = B * t / nt, b1 = B * (t + 1) / nt;
+    for (int64_t b = b0; b < b1; ++b)
+      if (in(b)) fn(b, words.data());
+  };
+  std::vector<std::thread> th;
+  for (int t = 1; t < nt; ++t) th.emplace_back(work, t);
+  work(0);
+  for (auto &w : th) w.join();
+}
+
+void Setup::scan_labels() {
+  const int n_mask = (s.V + 63) / 64;
+  facts.assign((size_t)B, LatFacts{});
+  for_lattices([&](int64_t b, int64_t *seen) {
+    const int64_t L = len(b);
+    const int32_t *lab = labels + l_off[b];
+    LatFacts f{};
+    std::fill(seen, seen + n_mask, (int64_t)0);
+    for (int64_t l = 0; l < L; ++l) {
+      if (s.ctc ? (lab[l] < 0 || lab[l] >= s.V || lab[l] == s.blank) : (lab[l] < -s.V || lab[l] >= s.V)) { f.bad = 1; break; }
+      if (!s.ctc && lab[l] <= 0) f.special = 1;  // (CTC: the blank test is the state's parity, any label is fast)
+      if (l > 0 && lab[l] == lab[l - 1]) ++f.repeats;
+      const int32_t c = lab[l] < 0 ? lab[l] + s.V : lab[l];
+      if (!(seen[c >> 6] >> (c & 63) & 1)) { seen[c >> 6] |= (int64_t)1 << (c & 63); ++f.distinct; }
+    }
+    facts[(size_t)b] = f;
+  });
+}
+
+// ---- stage 2: wide vocabularies -- can the staged kernels work on a compact copy of the log-probs?  Then
+// the emission staging and the padded column table (numpy-style wrap of negative labels).
+void Setup::compact_vocabulary() {
   // Band-shaped lattices of a wide vocabulary do not need the compact copy at all: kab_bandr.cuh's
   // gather mode reads log_probs[t, label] itself (VERDICT round 1, item 8: a chapter with more than
   // 511 distinct BPE tokens sent the whole plan to the generic kernel).  It is used when every
   // band-shaped lattice of the plan fits that kernel's ring (beam + 32 <= 1280 states).
   const int64_t ga_max_weff = (int64_t)KAB_BQ_OW * KAB_BR_CW * 8 - 32;
-  auto band_shaped = [&](int64_t T, int64_t S) {
-    const bool full = W >= S && T > 0 && (S * (T - 1)) / T <= W / 2;
-    if (full && S <= 248) return false;  // warp class
-    return W >= 1 && S <= 3 * T && std::min<int64_t>(W, S) + 32 <= (int64_t)KAB_BAND_OW * BAND_MAX_WARPS;
-  };
-  {
-    const char *ge = getenv("KAB_BAND_GATHER");
-    bool ok = !ctc && V > MAX_STAGE_V && M <= 4 && !(ge && atoi(ge) == 0) && kab_bandr_geom(64).smem_bytes <= 227 * 1024, any_band = false;
-    for (int64_t b = 0; b < B && ok; ++b) {
-      if (mask && !mask[b]) continue;
-      const int64_t T = t_off[b + 1] - t_off[b], S = 2 * (l_off[b + 1] - l_off[b]) + 1;
-      if (band_shaped(T, S)) { any_band = true; ok = std::min<int64_t>(W, S) <= ga_max_weff; }
-    }
-    pl->band_ga = ok && any_band;
+  bool ok = !s.ctc && s.V > MAX_STAGE_V && s.M <= 4 && knob.band_gather && kab_bandr_geom(64).smem_bytes <= 227 * 1024, any_band = false;
+  for (int64_t b = 0; b < B && ok; ++b) {
+    const int64_t S = 2 * len(b) + 1;
+    if (in(b) && band_shaped(frames(b), S, s.W)) { any_band = true; ok = std::min<int64_t>(s.W, S) <= ga_max_weff; }
   }
-  // CTC plans: the compact copy with the blank as compact column 0 (kab_compact_ctc_kernel).  Vc is sized
-  // by the lattices that fit it; one with more than MAX_STAGE_V - 1 distinct labels goes to the generic
-  // kernel on its own instead of taking the whole plan there.  KAB_CTC_COMPACT=0 (development, the
-  // reference arm of the tests and tools/forced_align_vocab_bench.py) sends every lattice there.
-  const bool ctc_compact = ctc && V > MAX_STAGE_V && [] { const char *ce = getenv("KAB_CTC_COMPACT"); return !(ce && atoi(ce) == 0); }();
-  if ((!ctc && V > MAX_STAGE_V && M <= 4) || ctc_compact) {
-    std::vector<uint8_t> seen((size_t)V, 0);
-    int64_t dmax = 0;
-    bool any = false;
-    auto in_range = [&](int32_t x) { return ctc ? (x >= 0 && x < V && x != blank) : (x > 0 && x < V); };
-    for (int64_t b = 0; b < B; ++b) {
-      if (mask && !mask[b]) continue;
-      const int64_t L = l_off[b + 1] - l_off[b];
-      const int32_t *lab = labels + l_off[b];
-      if (pl->band_ga && band_shaped(t_off[b + 1] - t_off[b], 2 * L + 1)) continue;  // (not through the compact copy)
-      bool usable = true;
-      int64_t dist = 0;
-      for (int64_t l = 0; l < L && usable; ++l) {
-        if (!in_range(lab[l])) usable = false;
-        else if (!seen[(size_t)lab[l]]) { seen[(size_t)lab[l]] = 1; ++dist; }
-      }
-      for (int64_t l = 0; l < L; ++l)
-        if (in_range(lab[l])) seen[(size_t)lab[l]] = 0;
-      if (usable && (!ctc || dist + 1 <= MAX_STAGE_V)) { dmax = std::max(dmax, dist); any = true; }
-    }
-    if (any && dmax + 1 <= MAX_STAGE_V) {
-      pl->Vc = (int32_t)std::max<int64_t>(8, align_up(dmax + 1, 4));
-      h_gather.assign((size_t)B * pl->Vc, 0);
-    }
+  gather = ok && any_band;
+  // Vc: the blank's column and the most distinct labels of a lattice that goes through the copy.  CTC plans
+  // (kab_compact_ctc_kernel): one with more than MAX_STAGE_V - 1 distinct labels goes to the generic kernel on
+  // its own instead of taking the whole plan there; KAB_CTC_COMPACT=0 (the reference arm of the tests and
+  // tools/forced_align_vocab_bench.py) sends every lattice there.
+  int64_t dmax = -1, off = 0;
+  for (int64_t b = 0; b < B; ++b) {
+    if (!in(b)) continue;
+    LatFacts &f = facts[(size_t)b];
+    f.col_off = off;  // in the padded column table (a bad-label lattice has no columns)
+    if (f.bad) continue;
+    off += align_up(len(b), 8) + 8;
+    if (f.special || (gather && band_shaped(frames(b), 2 * len(b) + 1, s.W))) continue;
+    if (!s.ctc || f.distinct + 1 <= MAX_STAGE_V) dmax = std::max<int64_t>(dmax, f.distinct);
   }
-  const int32_t Veff = pl->Vc ? pl->Vc : V;  // vocabulary the staged kernels see
+  if (s.V > MAX_STAGE_V && (s.ctc ? knob.ctc_compact : s.M <= 4) && dmax >= 0 && dmax + 1 <= MAX_STAGE_V) {
+    pl->Vc = (int32_t)std::max<int64_t>(8, align_up(dmax + 1, 4));
+    gather_rows.assign((size_t)B * pl->Vc, 0);
+  }
+  Veff = pl->Vc ? pl->Vc : s.V;
 
   // emission staging geometry: ~4 KB stages, at most 16 frames each
   pl->stage_frames = Veff <= 64 ? 16 : 8;  // multiple of 8: frame groups never straddle stages
-  if (const char *sf = getenv("KAB_STAGE_FRAMES")) {  // development knob: 8 or 16
-    const int v = atoi(sf);
-    if (v == 8 || v == 16 || v == 32) pl->stage_frames = v;
-  }
+  if (knob.stage_frames == 8 || knob.stage_frames == 16 || knob.stage_frames == 32) pl->stage_frames = knob.stage_frames;
   pl->stage_bytes = (int32_t)align_up((int64_t)pl->stage_frames * Veff * 4 + 24, 16);
 
-  // resident CTAs of the wide kernel (its warps spin on each other: the whole grid must be resident)
-  int wide_capacity = 0;
-  {
-    const KabWideGeom wgeo = kab_wide_geom(pl->stage_bytes);
-    const void *wfn = ctc ? (const void *)kab_wide_ctc_kernel : (const void *)kab_wide_kernel;
-    int occ = 0;
-    if (wgeo.smem_bytes <= 227 * 1024 && ensure_dyn_smem(wfn, device, wgeo.smem_bytes) == cudaSuccess &&
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, wfn, KAB_WD_THREADS, wgeo.smem_bytes) == cudaSuccess)
-      wide_capacity = occ * pl->sm_count;
-    (void)cudaGetLastError();
-  }
-  int wide_max_ctas = 0;
-
-  // ---- classify, build the padded column table (numpy-style wrap of negative labels)
-  std::vector<uint16_t> col16;
-  std::vector<int32_t> status_init((size_t)B, 0);
-  int64_t bp_bytes = 0, scr_floats = 0, max_band_weff = 0;
-  std::vector<uint8_t> hyb_mask;  // hybrid band plan: the lattices of the sub-plan
-  int hyb_k = 0;                  // ... and its clusters
-  kab_plan_info &info = pl->info;
-  info.n_lattices = B; info.device = device; info.total_frames = pl->total_T;
-  const int n_mask = (V + 63) / 64;
-  // The label scans (range check, distinct labels, column table) are independent per lattice and are
-  // most of this function for a batch of 10 000 segments (4.5 of 5 ms): several host threads do them
-  // ahead of the (cheap, sequential) classification below.
-  struct LatFacts { uint8_t bad, special, compact; int32_t distinct; int64_t col_off; };
-  std::vector<LatFacts> facts((size_t)B);
-  auto for_lattices = [&](auto &&fn) {  // fn(b, scratch words) over the plan's lattices
-    const unsigned hw = std::thread::hardware_concurrency();
-    const int nt = (B >= 2048 && pl->total_L >= 65536 && hw >= 4 && !getenv("KAB_SERIAL_SETUP")) ? (int)std::min<unsigned>(8, hw / 2) : 1;
-    auto work = [&](int t) {
-      std::vector<int64_t> words((size_t)std::max(n_mask, 1), 0);
-      const int64_t b0 = B * t / nt, b1 = B * (t + 1) / nt;
-      for (int64_t b = b0; b < b1; ++b)
-        if (!mask || mask[b]) fn(b, words.data());
-    };
-    std::vector<std::thread> th;
-    for (int t = 1; t < nt; ++t) th.emplace_back(work, t);
-    work(0);
-    for (auto &x : th) x.join();
-  };
-  for_lattices([&](int64_t b, int64_t *distinct_mask) {  // pass A: facts (and the compact numbering's gather row)
-    const int64_t T = t_off[b + 1] - t_off[b], L = l_off[b + 1] - l_off[b], S = 2 * L + 1;
+  col16.assign((size_t)off, 0);
+  const int n_mask = (s.V + 63) / 64;
+  for_lattices([&](int64_t b, int64_t *seen) {  // the compact numbering's gather rows, the column table
+    LatFacts &f = facts[(size_t)b];
+    if (f.bad) return;
+    const int64_t L = len(b);
     const int32_t *lab = labels + l_off[b];
-    LatFacts f{};
-    std::fill(distinct_mask, distinct_mask + n_mask, (int64_t)0);
-    for (int64_t l = 0; l < L; ++l) {
-      if (ctc ? (lab[l] < 0 || lab[l] >= V || lab[l] == blank) : (lab[l] < -V || lab[l] >= V)) { f.bad = 1; break; }
-      if (!ctc && lab[l] <= 0) f.special = 1;  // (CTC: the blank test is the state's parity, any label is fast)
-      const int32_t c = lab[l] < 0 ? lab[l] + V : lab[l];
-      if (!(distinct_mask[c >> 6] >> (c & 63) & 1)) { distinct_mask[c >> 6] |= (int64_t)1 << (c & 63); ++f.distinct; }
-    }
-    const bool ga = pl->band_ga && !f.special && band_shaped(T, S);
-    if (!f.bad && pl->Vc && !f.special && !ga && f.distinct + 1 <= pl->Vc) {
+    uint16_t *c = col16.data() + f.col_off;
+    const bool ga = gather && !f.special && band_shaped(frames(b), 2 * L + 1, s.W);
+    if (pl->Vc && !f.special && !ga && f.distinct + 1 <= pl->Vc) {
       // compact numbering: the blank's column (0, or the CTC blank id), then the lattice's distinct label
       // columns in ascending order
       f.compact = 1;
-      int32_t *g = h_gather.data() + (size_t)b * pl->Vc;
-      g[0] = ctc ? blank : 0;
+      std::fill(seen, seen + n_mask, (int64_t)0);
+      for (int64_t l = 0; l < L; ++l) seen[lab[l] >> 6] |= (int64_t)1 << (lab[l] & 63);
+      int32_t *g = gather_rows.data() + (size_t)b * pl->Vc;
+      g[0] = s.ctc ? s.blank : 0;
       int32_t n = 1;
       for (int w = 0; w < n_mask; ++w)
-        for (int64_t m = distinct_mask[w]; m; m &= m - 1) g[n++] = w * 64 + __builtin_ctzll((unsigned long long)m);
-    }
-    facts[(size_t)b] = f;
-  });
-  {  // offsets of the padded column table (a bad-label lattice has no columns)
-    int64_t off = 0;
-    for (int64_t b = 0; b < B; ++b) {
-      if (mask && !mask[b]) continue;
-      facts[(size_t)b].col_off = off;
-      if (!facts[(size_t)b].bad) off += align_up(l_off[b + 1] - l_off[b], 8) + 8;
-    }
-    col16.assign((size_t)off, 0);
-  }
-  for_lattices([&](int64_t b, int64_t *) {  // pass B: the column table
-    const LatFacts &f = facts[(size_t)b];
-    if (f.bad) return;
-    const int64_t L = l_off[b + 1] - l_off[b];
-    const int32_t *lab = labels + l_off[b];
-    uint16_t *c = col16.data() + f.col_off;
-    if (f.compact) {
-      const int32_t *g = h_gather.data() + (size_t)b * pl->Vc;
-      const int32_t n = f.distinct + 1;
+        for (int64_t m = seen[w]; m; m &= m - 1) g[n++] = w * 64 + __builtin_ctzll((unsigned long long)m);
       for (int64_t l = 0; l < L; ++l) c[l] = (uint16_t)(std::lower_bound(g + 1, g + n, lab[l]) - g);
     } else {
-      for (int64_t l = 0; l < L; ++l) c[l] = (uint16_t)(lab[l] < 0 ? lab[l] + V : lab[l]);
+      for (int64_t l = 0; l < L; ++l) c[l] = (uint16_t)(lab[l] < 0 ? lab[l] + s.V : lab[l]);
     }
   });
+}
+
+// ---- stage 3: the work lists (warp, band, wide, generic); the offsets of all but the band list
+void Setup::classify() {
+  const int64_t W = s.W, M = s.M;
+  // resident CTAs of the wide kernel (its warps spin on each other: the whole grid must be resident)
+  Launch &lw = pl->launch[Q_WIDE];
+  lw = Launch{s.ctc ? (const void *)kab_wide_ctc_kernel : (const void *)kab_wide_kernel, dim3(), dim3(KAB_WD_THREADS),
+              kab_wide_geom(pl->stage_bytes).smem_bytes, 0, true};
+  {
+    int occ = 0;
+    if (lw.smem <= 227 * 1024 && ensure_dyn_smem(lw.fn, pl->device, lw.smem) == cudaSuccess &&
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, lw.fn, KAB_WD_THREADS, lw.smem) == cudaSuccess)
+      wide_capacity = occ * pl->sm_count;
+    (void)cudaGetLastError();
+  }
   // CTC long-form plans: the wide kernel runs its lattices one after another, each on the whole GPU; the
   // generic kernel runs them side by side, one CTA each.  A makespan estimate from measured costs (B200, V = 32,
   // tools/forced_align_long_bench.py, DESIGN.md 3.9) gives all lattices that both kernels could take to one of
@@ -541,71 +553,64 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
   // 177 ns per frame wide at Vc = 272 and 0.58 Gcells/s for a lone generic lattice at V = 1025; the constants
   // stay, DESIGN.md 3.9c.)
   bool ctc_wide = false;
-  if (ctc && ctc_long) {
-    double frames = 0.0, cells = 0.0, max_cells = 0.0;
+  if (s.ctc && s.ctc_long) {
+    double sum_t = 0.0, cells = 0.0, max_cells = 0.0;
     for (int64_t b = 0; b < B; ++b) {
-      if ((mask && !mask[b]) || facts[(size_t)b].bad) continue;
+      if (!in(b) || facts[(size_t)b].bad) continue;
       if (pl->Vc && !facts[(size_t)b].compact) continue;  // (too many distinct labels for the compact copy: generic)
-      const int64_t T = t_off[b + 1] - t_off[b], S = 2 * (l_off[b + 1] - l_off[b]) + 1;
+      const int64_t T = frames(b), S = 2 * len(b) + 1;
       if (S + 32 <= KAB_BAND_OW * BAND_MAX_WARPS) continue;  // warp or band class
-      if (((S + KAB_BAND_OW - 1) / KAB_BAND_OW + KAB_WD_CW - 1) / KAB_WD_CW + 1 > wide_capacity) continue;
-      frames += (double)T;
+      if (wide_ctas(S) + 1 > wide_capacity) continue;
+      sum_t += (double)T;
       cells += (double)T * (double)S;
       max_cells = std::max(max_cells, (double)T * (double)S);
     }
-    ctc_wide = frames * 102.0 <= std::max(max_cells / 0.68, cells / 79.0);  // (ns)
+    ctc_wide = sum_t * 102.0 <= std::max(max_cells / 0.68, cells / 79.0);  // (ns)
   }
+  kab_plan_info &info = pl->info;
+  status_init.assign((size_t)B, 0);
   for (int64_t b = 0; b < B; ++b) {
-    if (mask && !mask[b]) continue;
-    const int64_t T = t_off[b + 1] - t_off[b], L = l_off[b + 1] - l_off[b], S = 2 * L + 1;
-    const bool bad = facts[(size_t)b].bad != 0, special = facts[(size_t)b].special != 0;
-    const int64_t distinct = facts[(size_t)b].distinct;
-    if (bad) {  // reference: IndexError at align.py:77
-      status_init[(size_t)b] = KAB_ST_BAD_LABEL;
+    if (!in(b)) continue;
+    const int64_t T = frames(b), L = len(b), S = 2 * L + 1;
+    const LatFacts &f = facts[(size_t)b];
+    // reference: IndexError at align.py:77; CTC: no path fits when T < L + R (R = adjacent equal labels,
+    // which need a blank between)
+    if (f.bad || (s.ctc && T < L + f.repeats)) {
+      status_init[(size_t)b] = f.bad ? KAB_ST_BAD_LABEL : KAB_ST_DEAD_BAND;
       pl->any_bad_label = true;
       continue;
-    }
-    if (ctc) {  // CTC: no path fits when T < L + R (R = adjacent equal labels, which need a blank between)
-      const int32_t *lab = labels + l_off[b];
-      int64_t R = 0;
-      for (int64_t l = 1; l < L; ++l) R += lab[l] == lab[l - 1];
-      if (T < L + R) {
-        status_init[(size_t)b] = KAB_ST_DEAD_BAND;
-        pl->any_bad_label = true;
-        continue;
-      }
     }
     KabLattice d{};
     d.t_off = t_off[b];
     d.lab_off = l_off[b];
     d.T = (int32_t)T; d.L = (int32_t)L; d.index = (int32_t)b;
-    d.col_off = facts[(size_t)b].col_off;
-    const bool ga = pl->band_ga && !special && band_shaped(T, S);  // gather mode: the labels stay column numbers
+    d.col_off = f.col_off;
+    const bool ga = gather && !f.special && band_shaped(T, S, W);  // gather mode: the labels stay column numbers
 
     // max_move 1 .. 3 run in the same kernels (their MM instantiations turn the excluded moves'
     // candidates into -inf); more than four moves only exist in the generic kernel
-    const bool fast = M <= 4 && !special && (ga || (Veff <= MAX_STAGE_V && (!pl->Vc || distinct + 1 <= pl->Vc)));
-    const bool full = W >= S && (S * (T - 1)) / T <= W / 2;
-    const int64_t weff = ctc ? S : std::min<int64_t>(W, S);
+    const bool fast = M <= 4 && !f.special && (ga || (Veff <= MAX_STAGE_V && (!pl->Vc || f.distinct + 1 <= pl->Vc)));
+    const bool full = unbanded(T, S, W);
+    const int64_t weff = s.ctc ? S : std::min<int64_t>(W, S);
     int q;
     if (fast && !ga && full && S <= 248) {
       q = Q_WARP;
       d.k = S <= 62 ? 2 : (S <= 124 ? 4 : (S <= 186 ? 6 : 8));  // 31 lanes x K states
       d.bp_off = bp_bytes;
-      if (ctc || d.k <= 4) {  // backpointer word-rows (kab_warp_align: the BP scheme)
+      if (s.ctc || d.k <= 4) {  // backpointer word-rows (kab_warp_align: the BP scheme)
         const int fpw = d.k <= 2 ? 8 : (d.k <= 4 ? 4 : 2);
         bp_bytes += align_up((T + fpw - 1) / fpw * 128, 256);
       } else {  // score checkpoint rows, one per KAB_CKPT_C frames
         bp_bytes += align_up((T + KAB_CKPT_C - 1) / KAB_CKPT_C * kab_ckpt_stride((int)S, d.k) * 4, 256);
       }
-    } else if (fast && W >= 1 && S <= 3 * T && weff + 32 <= KAB_BAND_OW * BAND_MAX_WARPS) {
-      q = Q_BAND;  // backpointer offsets are assigned below, once the ring size is known
+    } else if (fast && band_shaped(T, S, W)) {
+      q = Q_BAND;  // backpointer offsets are assigned by lay_out_band, once the kernel is known
       max_band_weff = std::max(max_band_weff, weff);
-    } else if (fast && !ga && (ctc ? ctc_wide : M == 4) && full && ((S + KAB_BAND_OW - 1) / KAB_BAND_OW + KAB_WD_CW - 1) / KAB_WD_CW + 1 <= wide_capacity) {
+    } else if (fast && !ga && (s.ctc ? ctc_wide : M == 4) && full && wide_ctas(S) + 1 <= wide_capacity) {
       q = Q_WIDE;  // unbanded and wider than a CTA: a chain of warps over the whole GPU
       const int nww = (int)((S + KAB_BAND_OW - 1) / KAB_BAND_OW);
       d.k = nww;
-      wide_max_ctas = std::max(wide_max_ctas, (nww + KAB_WD_CW - 1) / KAB_WD_CW);
+      wide_max_ctas = std::max(wide_max_ctas, (int)wide_ctas(S));
       d.bp_off = bp_bytes;
       bp_bytes += (int64_t)nww * ((T + 7) / 8) * 256;  // [warp][group][32 lanes][8 B]
       d.scr_off = pl->wide_ws_bytes / 4;
@@ -620,139 +625,135 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
     pl->lists[q].push_back(d);
     pl->max_T[q] = std::max(pl->max_T[q], (int)T);
     info.n_class[q == Q_WARP ? KAB_CLASS_WARP : (q == Q_GENERIC ? KAB_CLASS_GENERIC : (q == Q_WIDE ? KAB_CLASS_WIDE : KAB_CLASS_BAND))]++;
-    const int64_t cells = ctc ? T * S : cells_eval_of(T, S, W);
+    const int64_t cells = s.ctc ? T * S : cells_eval_of(T, S, W);
     info.cells_eval += cells;
     info.cells_nominal += T * S;
     int bbits = 0;
     while ((1 << bbits) < M) ++bbits;
-    const int64_t dcols = std::min<int64_t>(V, distinct + 1);
+    const int64_t dcols = std::min<int64_t>(s.V, f.distinct + 1);
     info.algorithmic_bytes += 4 * dcols * T + (cells * bbits + 7) / 8 + (T * bbits + 7) / 8 + 12 * T;
   }
-  if (!pl->lists[Q_BAND].empty()) {
-    pl->band_nw = (int32_t)((max_band_weff + 32 + KAB_BAND_OW - 1) / KAB_BAND_OW);
-    // Two band kernels.  The pipelined cluster kernel (kab_bandp.cuh: rings of 4 * NC warps over a
-    // cluster of NC <= 8 CTAs, one warp per scheduler) has the shorter frame (Gon gitsune 14.2 vs
-    // 15.4 ms, config 4(i) 168 vs 188 ms) but takes NC whole SMs per lattice; the single-CTA kernel
-    // (kab_band.cuh) runs two lattices per SM.  So: the cluster kernel when every band lattice of
-    // the plan gets its own cluster at once, the single-CTA kernel for larger batches.
-    // KAB_BAND_CLUSTER=0 forces the single-CTA kernel, =N (>= 1) the cluster kernel with >= N CTAs.
-    const int nc = (pl->band_nw + KAB_BP_CW - 1) / KAB_BP_CW;
-    const char *cl = getenv("KAB_BAND_CLUSTER");
-    int want_nc = cl ? atoi(cl) : -1;
-    if (band_mode >= 0) want_nc = band_mode == 0 ? 0 : -1;  // (sub-plans of a hybrid plan: the kernel is given)
-    const bool cluster_ok = nc <= 8 && kab_bandp_geom(pl->stage_bytes).smem_bytes <= 227 * 1024;
-    // kab_bandq.cuh (two warps per scheduler, two states per lane: the shorter frame) when its ring
-    // of 40-slot warps fits a cluster of <= 8 CTAs and every lattice gets its own cluster at once;
-    // KAB_BAND_Q=0 keeps kab_bandp.cuh, =1 forces kab_bandq.cuh whenever its geometry allows
-    const int nwq = (int)((max_band_weff + 32 + KAB_BQ_OW - 1) / KAB_BQ_OW);
-    const int ncq = (nwq + KAB_BQ_CW - 1) / KAB_BQ_CW;
-    const bool q_ok = ncq <= 8 && kab_bandq_geom(pl->stage_bytes).smem_bytes <= 227 * 1024;
-    // kab_bandr.cuh: the same lanes with ONE compute warp per scheduler and the bookkeeping on helper
-    // warps -- by far the shortest frame, at 4 compute warps per CTA (7 CTAs for the 1000-wide band).
-    // Its clusters take lattices from the work queue, so a plan may hold more lattices than clusters.
-    // KAB_BAND_R=0 disables it, =1 forces it whenever its geometry allows.
-    const int ncr = (nwq + KAB_BR_CW - 1) / KAB_BR_CW;
-    const bool r_ok = pl->band_ga || (ncr <= 8 && pl->stage_frames == KAB_BR_F && kab_bandr_geom(pl->stage_bytes).smem_bytes <= 227 * 1024);
-    const char *qe = getenv("KAB_BAND_Q");
-    const int want_q = band_mode >= 0 ? (band_mode == 0 ? 0 : -1) : (qe ? atoi(qe) : -1);
-    const char *re = getenv("KAB_BAND_R");
-    const int want_r = band_mode >= 0 ? band_mode : (re ? atoi(re) : -1);
-    int64_t n_band = (int64_t)pl->lists[Q_BAND].size();
-    // Which kernel for this plan?  A makespan estimate from measured per-frame costs (B200, 1000-wide
-    // band): kab_bandr.cuh ~70 ns per frame on one of sm_count / ncr clusters that pull lattices from
-    // the work queue, kab_band.cuh ~190 ns per frame with two lattices per SM.  A book (36 chapters)
-    // is bound by its longest chapter -> bandr; hundreds of chapters at once -> the single-CTA kernel.
-    double sum_t = 0.0, max_t = 0.0, bt_steps = 0.0;
-    for (const KabLattice &d : pl->lists[Q_BAND]) {
-      sum_t += d.T; max_t = std::max(max_t, (double)d.T);
-      bt_steps += (double)d.T * (double)std::min<int64_t>(W, 2 * (int64_t)d.L + 1);
-    }
-    // (bandr: 70 ns per frame for the longest lattice; with every cluster of the GPU busy on a queue of
-    // lattices ~90 ns per frame of a cluster's share, plus the map walkers of the parallel traceback at
-    // 1.85e12 steps/s -- 162 chapters on one GPU: 60.6 ms measured, 59 estimated; the first version of
-    // this estimate (70 ns, no traceback) said 41 and took the plan away from the single-CTA kernel's 49)
-    const double est_r = std::max(max_t * 70.0, sum_t / std::max(1, pl->sm_count / std::max(1, ncr)) * 90.0) + bt_steps * 0.55e-3;
-    // (190 ns per frame is a lone lattice's latency in the single-CTA kernel; with every SM holding two of
-    // them a CTA slot's frames cost ~330 ns each -- 18 books on one GPU: 49 M frames / 296 slots, 54.5 ms.
-    // The estimates keep the one figure: with 330 in the throughput terms the split below was chosen
-    // less often and measured worse, 36.9 instead of 34.9 ms for 18 books on two GPUs.)
-    const double est_b = std::max(max_t, sum_t / (double)(pl->sm_count * (pl->band_nw <= 16 ? 2 : 1))) * 190.0;
-    const bool use_r = pl->band_ga || (r_ok && want_r != 0 && want_nc != 0 && want_q != 0 && (want_r >= 1 || want_nc >= 1 || est_r <= est_b));
-    const bool use_q = !use_r && M == 4 && q_ok && want_q != 0 && want_nc != 0 && (want_q >= 1 || n_band <= pl->sm_count / ncq);
-    // Hybrid: a plan of hundreds of chapters takes the single-CTA kernel (throughput), but its makespan
-    // is then the LONGEST chapter at that kernel's 190 ns per frame.  Give the longest ones to
-    // kab_bandr.cuh (70 ns per frame) on k clusters and the rest to the single-CTA kernel on the other
-    // SMs, side by side: the split (k clusters, the m longest lattices) with the smallest estimated
-    // makespan, taken when it beats the single kernel by 15 %.  KAB_BAND_HYBRID=0 / 1 disables / forces it.
-    {
-      const char *he = getenv("KAB_BAND_HYBRID");
-      const int want_h = he ? atoi(he) : -1;
-      if (band_mode < 0 && !mask && !use_r && !use_q && r_ok && !pl->band_ga && !pl->Vc && V <= MAX_STAGE_V && want_h != 0 &&
-          want_r < 0 && want_q < 0 && want_nc < 0 && n_band >= 2) {
-        std::vector<KabLattice> &bl = pl->lists[Q_BAND];
-        std::stable_sort(bl.begin(), bl.end(), [](const KabLattice &a, const KabLattice &b2) { return a.T > b2.T; });
-        std::vector<double> pre((size_t)n_band + 1, 0.0);
-        for (int64_t i = 0; i < n_band; ++i) pre[(size_t)i + 1] = pre[(size_t)i] + bl[(size_t)i].T;
-        const int per_sm = pl->band_nw <= 16 ? 2 : 1;
-        double best = est_b;
-        int best_k = 0;
-        int64_t best_m = 0;
-        for (int k = 1; k <= pl->sm_count / ncr / 2; ++k) {
-          const double sm_left = (double)(pl->sm_count - k * ncr) * per_sm;
-          for (int64_t m = k; m < n_band && m <= 16 * (int64_t)k; ++m) {
-            const double tr_ = std::max((double)bl[0].T, pre[(size_t)m] / k) * 70.0;
-            const double tb_ = std::max((double)bl[(size_t)m].T, (sum_t - pre[(size_t)m]) / sm_left) * 190.0;
-            const double ms = std::max(tr_, tb_);
-            if (ms < best) { best = ms; best_k = k; best_m = m; }
-          }
-        }
-        if (want_h >= 1 && best_k == 0) { best_k = 1; best_m = 1; }
-        if (best_k > 0 && (want_h >= 1 || best < 0.85 * est_b)) {
-          hyb_mask.assign((size_t)B, 0);
-          for (int64_t i = 0; i < best_m; ++i) hyb_mask[(size_t)bl[(size_t)i].index] = 1;
-          bl.erase(bl.begin(), bl.begin() + best_m);
-          hyb_k = best_k;
-          want_nc = 0;  // (the rest: the single-CTA kernel, whatever its number)
-          pl->band_sm_reserved = best_k * ncr;
-          n_band = (int64_t)bl.size();
-          pl->max_T[Q_BAND] = bl.empty() ? 0 : bl[0].T;
-        }
+}
+
+// ---- stage 4: the band list's kernel, from makespan estimates and the knobs; maybe a hybrid split
+void Setup::choose_band_kernel(int band_mode) {
+  std::vector<KabLattice> &bl = pl->lists[Q_BAND];
+  if (bl.empty()) return;
+  pl->band_nw = (int32_t)((max_band_weff + 32 + KAB_BAND_OW - 1) / KAB_BAND_OW);
+  // Two band kernels.  The pipelined cluster kernel (kab_bandp.cuh: rings of 4 * NC warps over a
+  // cluster of NC <= 8 CTAs, one warp per scheduler) has the shorter frame (Gon gitsune 14.2 vs
+  // 15.4 ms, config 4(i) 168 vs 188 ms) but takes NC whole SMs per lattice; the single-CTA kernel
+  // (kab_band.cuh) runs two lattices per SM.  So: the cluster kernel when every band lattice of
+  // the plan gets its own cluster at once, the single-CTA kernel for larger batches.
+  // KAB_BAND_CLUSTER=0 forces the single-CTA kernel, =N (>= 1) the cluster kernel with >= N CTAs.
+  const int nc = (pl->band_nw + KAB_BP_CW - 1) / KAB_BP_CW;
+  int want_nc = knob.band_cluster;
+  if (band_mode >= 0) want_nc = band_mode == 0 ? 0 : -1;  // (sub-plans of a hybrid plan: the kernel is given)
+  const bool cluster_ok = nc <= 8 && kab_bandp_geom(pl->stage_bytes).smem_bytes <= 227 * 1024;
+  // kab_bandq.cuh (two warps per scheduler, two states per lane: the shorter frame) when its ring
+  // of 40-slot warps fits a cluster of <= 8 CTAs and every lattice gets its own cluster at once;
+  // KAB_BAND_Q=0 keeps kab_bandp.cuh, =1 forces kab_bandq.cuh whenever its geometry allows
+  const int nwq = (int)((max_band_weff + 32 + KAB_BQ_OW - 1) / KAB_BQ_OW);
+  const int ncq = (nwq + KAB_BQ_CW - 1) / KAB_BQ_CW;
+  const bool q_ok = ncq <= 8 && kab_bandq_geom(pl->stage_bytes).smem_bytes <= 227 * 1024;
+  // kab_bandr.cuh: the same lanes with ONE compute warp per scheduler and the bookkeeping on helper
+  // warps -- by far the shortest frame, at 4 compute warps per CTA (7 CTAs for the 1000-wide band).
+  // Its clusters take lattices from the work queue, so a plan may hold more lattices than clusters.
+  // KAB_BAND_R=0 disables it, =1 forces it whenever its geometry allows.
+  const int ncr = (nwq + KAB_BR_CW - 1) / KAB_BR_CW;
+  const bool r_ok = gather || (ncr <= 8 && pl->stage_frames == KAB_BR_F && kab_bandr_geom(pl->stage_bytes).smem_bytes <= 227 * 1024);
+  const int want_q = band_mode >= 0 ? (band_mode == 0 ? 0 : -1) : knob.band_q;
+  const int want_r = band_mode >= 0 ? band_mode : knob.band_r;
+  int64_t n_band = (int64_t)bl.size();
+  // Which kernel for this plan?  A makespan estimate from measured per-frame costs (B200, 1000-wide
+  // band): kab_bandr.cuh ~70 ns per frame on one of sm_count / ncr clusters that pull lattices from
+  // the work queue, kab_band.cuh ~190 ns per frame with two lattices per SM.  A book (36 chapters)
+  // is bound by its longest chapter -> bandr; hundreds of chapters at once -> the single-CTA kernel.
+  double sum_t = 0.0, max_t = 0.0, bt_steps = 0.0;
+  for (const KabLattice &d : bl) {
+    sum_t += d.T; max_t = std::max(max_t, (double)d.T);
+    bt_steps += (double)d.T * (double)std::min<int64_t>(s.W, 2 * (int64_t)d.L + 1);
+  }
+  // (bandr: 70 ns per frame for the longest lattice; with every cluster of the GPU busy on a queue of
+  // lattices ~90 ns per frame of a cluster's share, plus the map walkers of the parallel traceback at
+  // 1.85e12 steps/s -- 162 chapters on one GPU: 60.6 ms measured, 59 estimated; the first version of
+  // this estimate (70 ns, no traceback) said 41 and took the plan away from the single-CTA kernel's 49)
+  const double est_r = std::max(max_t * 70.0, sum_t / std::max(1, pl->sm_count / std::max(1, ncr)) * 90.0) + bt_steps * 0.55e-3;
+  // (190 ns per frame is a lone lattice's latency in the single-CTA kernel; with every SM holding two of
+  // them a CTA slot's frames cost ~330 ns each -- 18 books on one GPU: 49 M frames / 296 slots, 54.5 ms.
+  // The estimates keep the one figure: with 330 in the throughput terms the split below was chosen
+  // less often and measured worse, 36.9 instead of 34.9 ms for 18 books on two GPUs.)
+  const double est_b = std::max(max_t, sum_t / (double)(pl->sm_count * (pl->band_nw <= 16 ? 2 : 1))) * 190.0;
+  const bool use_r = gather || (r_ok && want_r != 0 && want_nc != 0 && want_q != 0 && (want_r >= 1 || want_nc >= 1 || est_r <= est_b));
+  const bool use_q = !use_r && s.M == 4 && q_ok && want_q != 0 && want_nc != 0 && (want_q >= 1 || n_band <= pl->sm_count / ncq);
+  // Hybrid: a plan of hundreds of chapters takes the single-CTA kernel (throughput), but its makespan
+  // is then the LONGEST chapter at that kernel's 190 ns per frame.  Give the longest ones to
+  // kab_bandr.cuh (70 ns per frame) on k clusters and the rest to the single-CTA kernel on the other
+  // SMs, side by side: the split (k clusters, the m longest lattices) with the smallest estimated
+  // makespan, taken when it beats the single kernel by 15 %.  KAB_BAND_HYBRID=0 / 1 disables / forces it.
+  const int want_h = knob.band_hybrid;
+  if (band_mode < 0 && !mask && !use_r && !use_q && r_ok && !gather && !pl->Vc && s.V <= MAX_STAGE_V && want_h != 0 &&
+      want_r < 0 && want_q < 0 && want_nc < 0 && n_band >= 2) {
+    std::stable_sort(bl.begin(), bl.end(), [](const KabLattice &a, const KabLattice &b2) { return a.T > b2.T; });
+    std::vector<double> pre((size_t)n_band + 1, 0.0);
+    for (int64_t i = 0; i < n_band; ++i) pre[(size_t)i + 1] = pre[(size_t)i] + bl[(size_t)i].T;
+    const int per_sm = pl->band_nw <= 16 ? 2 : 1;
+    double best = est_b;
+    int best_k = 0;
+    int64_t best_m = 0;
+    for (int k = 1; k <= pl->sm_count / ncr / 2; ++k) {
+      const double sm_left = (double)(pl->sm_count - k * ncr) * per_sm;
+      for (int64_t m = k; m < n_band && m <= 16 * (int64_t)k; ++m) {
+        const double tr_ = std::max((double)bl[0].T, pre[(size_t)m] / k) * 70.0;
+        const double tb_ = std::max((double)bl[(size_t)m].T, (sum_t - pre[(size_t)m]) / sm_left) * 190.0;
+        const double ms = std::max(tr_, tb_);
+        if (ms < best) { best = ms; best_k = k; best_m = m; }
       }
     }
-    if (use_r || use_q) {
-      pl->band_q = true;
-      pl->band_r = use_r;
-      pl->band_cw = use_r ? KAB_BR_CW : KAB_BQ_CW;
-      pl->band_nc = use_r ? ncr : ncq;
-      const int nwt = pl->band_cw * pl->band_nc;
-      for (KabLattice &d : pl->lists[Q_BAND]) {
-        d.bp_off = bp_bytes;
-        bp_bytes += (int64_t)((d.T + 7) / 8) * 128 * nwt;  // [warp][group][32 lanes][4 B]
-        d.scr_off = pl->band_fifo_bytes / 4;
-        pl->band_fifo_bytes += (int64_t)align_up((int64_t)kab_bandq_ws_bytes(nwt), 256);
-      }
-    } else if ([&] {
-      if (want_nc < 0 && cluster_ok) {
-        // resident clusters of this size: every SM holds one CTA of the cluster kernel
-        const int64_t resident = pl->sm_count / nc;
-        want_nc = (int64_t)pl->lists[Q_BAND].size() <= resident ? nc : 0;
-      }
-      return M == 4 && cluster_ok && want_nc >= 1; }()) {
-      pl->band_nc = std::min(8, std::max(nc, want_nc));
-      const int nwt = KAB_BP_CW * pl->band_nc;
-      for (KabLattice &d : pl->lists[Q_BAND]) {
-        d.bp_off = bp_bytes;
-        bp_bytes += (int64_t)((d.T + 7) / 8) * 256 * nwt;  // [warp][group][32 lanes][8 B]
-        d.scr_off = pl->band_fifo_bytes / 4;
-        pl->band_fifo_bytes += (int64_t)align_up((int64_t)kab_bandp_ws_bytes(nwt), 256);
-      }
-    } else {
-      const KabBandGeom geo = kab_band_geom(pl->band_nw, pl->stage_bytes);
-      for (KabLattice &d : pl->lists[Q_BAND]) {
-        d.bp_off = bp_bytes;
-        bp_bytes += align_up((int64_t)d.T * geo.nbp, 256);
-      }
+    if (want_h >= 1 && best_k == 0) { best_k = 1; best_m = 1; }
+    if (best_k > 0 && (want_h >= 1 || best < 0.85 * est_b)) {
+      hyb_mask.assign((size_t)B, 0);
+      for (int64_t i = 0; i < best_m; ++i) hyb_mask[(size_t)bl[(size_t)i].index] = 1;
+      bl.erase(bl.begin(), bl.begin() + best_m);
+      hyb_k = best_k;
+      want_nc = 0;  // (the rest: the single-CTA kernel, whatever its number)
+      pl->band_sm_reserved = best_k * ncr;
+      pl->max_T[Q_BAND] = bl.empty() ? 0 : bl[0].T;
     }
+  }
+  if (use_r || use_q) {
+    pl->band_kernel = use_q ? BandKernel::Q : (gather ? BandKernel::R_GATHER : BandKernel::R);
+    pl->band_cw = use_r ? KAB_BR_CW : KAB_BQ_CW; pl->band_nc = use_r ? ncr : ncq;
+    return;
+  }
+  if (want_nc < 0 && cluster_ok) {
+    // resident clusters of this size: every SM holds one CTA of the cluster kernel
+    const int64_t resident = pl->sm_count / nc;
+    want_nc = (int64_t)bl.size() <= resident ? nc : 0;
+  }
+  if (s.M == 4 && cluster_ok && want_nc >= 1) {
+    pl->band_kernel = BandKernel::P;
+    pl->band_cw = KAB_BP_CW; pl->band_nc = std::min(8, std::max(nc, want_nc));
+  }
+}
+
+bool band_layout_q(BandKernel k) { return k == BandKernel::Q || k == BandKernel::R || k == BandKernel::R_GATHER; }
+
+// ---- stage 5: band backpointers and workspaces, longest-first order, the parallel backtrack's maps
+void Setup::lay_out_band() {
+  const BandKernel bk = pl->band_kernel;
+  const int nwt = pl->band_cw * pl->band_nc;
+  const int nbp = pl->band_nw ? kab_band_geom(pl->band_nw, pl->stage_bytes).nbp : 0;  // (single-CTA kernel)
+  for (KabLattice &d : pl->lists[Q_BAND]) {
+    d.bp_off = bp_bytes;
+    if (bk == BandKernel::CTA) {
+      bp_bytes += align_up((int64_t)d.T * nbp, 256);
+      continue;
+    }
+    // [warp][group][32 lanes][4 B] (KabBtLayoutQ) or [8 B] (KabBtLayoutP)
+    bp_bytes += (int64_t)((d.T + 7) / 8) * (band_layout_q(bk) ? 128 : 256) * nwt;
+    d.scr_off = pl->band_fifo_bytes / 4;
+    pl->band_fifo_bytes += (int64_t)align_up((int64_t)(band_layout_q(bk) ? kab_bandq_ws_bytes(nwt) : kab_bandp_ws_bytes(nwt)), 256);
   }
   // longest-processing-time-first order inside every queue
   for (int q = 0; q < N_QUEUES; ++q)
@@ -764,167 +765,223 @@ int plan_create_impl(kab_plan **out, int device, int64_t B, const int64_t *t_off
       return a.T > b2.T;
     });
 
-  // parallel backtrack of the cluster band kernel: per-lattice block maps (KAB_BAND_SERIAL_BT=1
-  // keeps the in-kernel single-thread walker: development / comparison)
-  // The maps kernel walks sum T * min(W, S) steps at ~1.85e12 steps/s (measured: the 36-chapter book,
-  // 2.7e9 steps, 1.46 ms); the in-kernel walkers run side by side, 40 ns per frame of the longest
-  // lattice.  So the parallel traceback is used when the plan is a few lattices or very unequal
+  // parallel backtrack of the cluster band kernels: per-lattice block maps.  kab_bandq.cuh and kab_bandr.cuh
+  // have no walker of their own; kab_bandp.cuh has one (KAB_BAND_SERIAL_BT=1 keeps it: development /
+  // comparison).  The maps kernel walks sum T * min(W, S) steps at ~1.85e12 steps/s (measured: the
+  // 36-chapter book, 2.7e9 steps, 1.46 ms); the in-kernel walkers run side by side, 40 ns per frame of the
+  // longest lattice.  So the parallel traceback is used when the plan is a few lattices or very unequal
   // ones (a book), not for dozens of equal ones.  KAB_BAND_SERIAL_BT=0 forces it.
-  bool par_bt = !pl->lists[Q_BAND].empty() && pl->band_nc > 0;
-  if (par_bt) {
-    const char *sb = getenv("KAB_BAND_SERIAL_BT");
+  if (pl->lists[Q_BAND].empty() || bk == BandKernel::CTA) return;
+  if (bk == BandKernel::P) {
     double steps = 0.0, tmax = 0.0;
     for (const KabLattice &d : pl->lists[Q_BAND]) {
-      steps += (double)d.T * (double)std::min<int64_t>(W, 2 * (int64_t)d.L + 1);
+      steps += (double)d.T * (double)std::min<int64_t>(s.W, 2 * (int64_t)d.L + 1);
       tmax = std::max(tmax, (double)d.T);
     }
-    par_bt = pl->band_q || (sb ? atoi(sb) == 0 : steps * 0.55e-12 <= 0.6 * tmax * 40e-9);  // (kab_bandq has no walker of its own)
+    if (knob.serial_bt >= 0 ? knob.serial_bt != 0 : steps * 0.55e-12 > 0.6 * tmax * 40e-9) return;
   }
-  if (par_bt) {
-    for (const KabLattice &d : pl->lists[Q_BAND]) {
-      KabBtMeta m{};
-      m.map_off = pl->bt_map_ints;
-      m.first_block = pl->bt_blocks;
-      m.n_blocks = (d.T + KAB_BT_BLOCK - 1) / KAB_BT_BLOCK;
-      m.wl = (int32_t)align_up(std::min<int64_t>(W, 2 * (int64_t)d.L + 1), 32);
-      pl->bt_map_ints += (int64_t)m.n_blocks * KAB_BT_NSUB * m.wl;
-      pl->bt_blocks += m.n_blocks;
-      pl->bt_max_wl = std::max(pl->bt_max_wl, m.wl);
-      pl->bt_meta.push_back(m);
-    }
+  for (const KabLattice &d : pl->lists[Q_BAND]) {
+    KabBtMeta m{};
+    m.map_off = pl->bt_map_ints;
+    m.first_block = pl->bt_blocks;
+    m.n_blocks = (d.T + KAB_BT_BLOCK - 1) / KAB_BT_BLOCK;
+    m.wl = (int32_t)align_up(std::min<int64_t>(s.W, 2 * (int64_t)d.L + 1), 32);
+    pl->bt_map_ints += (int64_t)m.n_blocks * KAB_BT_NSUB * m.wl;
+    pl->bt_blocks += m.n_blocks;
+    pl->bt_max_wl = std::max(pl->bt_max_wl, m.wl);
+    pl->bt_meta.push_back(m);
   }
+}
 
-  tr.mark("classify");
-  // ---- device allocations
+// pool_malloc (nothing for 0 bytes) and, given `src`, the upload of its bytes; a failure is cuda_fail(e, what)
+int alloc(void **dst, size_t bytes, const char *what, const void *src = nullptr) {
+  cudaError_t e = bytes ? pool_malloc(dst, bytes) : cudaSuccess;
+  if (e == cudaSuccess && bytes && src) e = cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice);
+  return e == cudaSuccess ? KAB_OK : cuda_fail(e, what);
+}
+
+cudaLaunchConfig_t launch_config(const Launch &k, cudaLaunchAttribute *at, cudaStream_t stream) {
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = k.grid; cfg.blockDim = k.block; cfg.dynamicSmemBytes = k.smem; cfg.stream = stream;
+  cfg.attrs = at;
+  cfg.numAttrs = k.cluster || k.cooperative ? 1 : 0;
+  at[0].id = k.cluster ? cudaLaunchAttributeClusterDimension : cudaLaunchAttributeCooperative;
+  if (k.cluster) at[0].val.clusterDim = {k.cluster, 1, 1};
+  else at[0].val.cooperative = 1;
+  return cfg;
+}
+
+// Launches a warp, band or wide list from its record.  The arguments are the kernel's parameters:
+// (lattices, count, KabParams[, workspace: the wide kernel][, blank column: the CTC kernels]).
+cudaError_t launch_list(const Launch &k, const KabLattice *lats, int n, KabParams p, unsigned char *const *wide_ws,
+                        const int *blank, cudaStream_t stream) {
+  void *args[5] = {&lats, &n, &p};
+  int na = 3;
+  if (wide_ws) args[na++] = (void *)wide_ws;
+  if (blank) args[na++] = (void *)blank;
+  cudaLaunchAttribute at[1];
+  const cudaLaunchConfig_t cfg = launch_config(k, at, stream);
+  return cudaLaunchKernelExC(&cfg, k.fn, args);
+}
+
+// ---- stage 6: device allocations and uploads; the launch records (kernel attributes and occupancy queries
+// on the functions launched)
+int Setup::allocate() {
   int rc = KAB_OK;
-  auto up = [&](void **dst, const void *src, size_t bytes) -> int {
-    if (!bytes) return KAB_OK;
-    KAB_CUDA(pool_malloc(dst, bytes));
-    KAB_CUDA(cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice));
-    return KAB_OK;
-  };
-  do {
-    for (int q = 0; q < N_QUEUES && rc == KAB_OK; ++q)
-      rc = up((void **)&pl->d_lists[q], pl->lists[q].data(), pl->lists[q].size() * sizeof(KabLattice));
-    if (rc) break;
-    if ((rc = up((void **)&pl->d_col16, col16.data(), col16.size() * sizeof(uint16_t)))) break;
-    if (B > 0 && (rc = up((void **)&pl->d_t_off, t_off, (size_t)(B + 1) * sizeof(int64_t)))) break;
-    if (pl->Vc) {
-      cudaError_t e3 = pool_malloc((void **)&pl->d_nonfinite, (size_t)B * sizeof(int32_t));
-      if (e3 != cudaSuccess) { rc = cuda_fail(e3, "pool_malloc(non-finite flags)"); break; }
-      if ((rc = up((void **)&pl->d_gather, h_gather.data(), h_gather.size() * sizeof(int32_t)))) break;
-      cudaError_t e2 = pool_malloc((void **)&pl->d_lpc, (size_t)pl->total_T * pl->Vc * sizeof(float));
-      if (e2 != cudaSuccess) { rc = cuda_fail(e2, "pool_malloc(compact log-probs)"); break; }
-    }
-    if (!pl->lists[Q_GENERIC].empty())
-      if ((rc = up((void **)&pl->d_raw, labels, (size_t)pl->total_L * sizeof(int32_t)))) break;
-    if (pl->any_bad_label)
-      if ((rc = up((void **)&pl->d_status_init, status_init.data(), (size_t)B * sizeof(int32_t)))) break;
-    cudaError_t e;
-    if (bp_bytes && (e = pool_malloc((void **)&pl->d_bp, (size_t)bp_bytes)) != cudaSuccess) { rc = cuda_fail(e, "pool_malloc(backpointers)"); break; }
-    if (scr_floats && (e = pool_malloc((void **)&pl->d_scratch, (size_t)scr_floats * 4)) != cudaSuccess) { rc = cuda_fail(e, "pool_malloc(scratch)"); break; }
-    if ((e = pool_malloc((void **)&pl->d_queue, N_QUEUES * sizeof(unsigned int))) != cudaSuccess) { rc = cuda_fail(e, "pool_malloc(queue)"); break; }
-
-    // ---- launch geometry
-    if (!pl->lists[Q_WARP].empty()) {
-      const size_t smem = 128 + (size_t)KAB_WARPS_PER_CTA * (KAB_WARP_STAGES * pl->stage_bytes + 256);  // + label tables
-      const void *fn = ctc ? (const void *)kab_warp_ctc_kernel
-                     : M == 4 ? (Veff == 39 ? (const void *)kab_warp_kernel<39, false> : (const void *)kab_warp_kernel<0, false>)
-                              : (Veff == 39 ? (const void *)kab_warp_kernel<39, true> : (const void *)kab_warp_kernel<0, true>);
-      if ((e = ensure_dyn_smem(fn, device, smem)) != cudaSuccess) { rc = cuda_fail(e, "cudaFuncSetAttribute(warp)"); break; }
+  cudaError_t e;
+  for (int q = 0; q < N_QUEUES; ++q)
+    if ((rc = alloc((void **)&pl->d_lists[q], pl->lists[q].size() * sizeof(KabLattice), "work list", pl->lists[q].data()))) return rc;
+  if ((rc = alloc((void **)&pl->d_col16, col16.size() * sizeof(uint16_t), "column table", col16.data()))) return rc;
+  if ((rc = alloc((void **)&pl->d_t_off, B > 0 ? (size_t)(B + 1) * sizeof(int64_t) : 0, "frame offsets", t_off))) return rc;
+  if (pl->Vc) {
+    if ((rc = alloc((void **)&pl->d_nonfinite, (size_t)B * sizeof(int32_t), "pool_malloc(non-finite flags)"))) return rc;
+    if ((rc = alloc((void **)&pl->d_gather, gather_rows.size() * sizeof(int32_t), "gather rows", gather_rows.data()))) return rc;
+    if ((rc = alloc((void **)&pl->d_lpc, (size_t)pl->total_T * pl->Vc * sizeof(float), "pool_malloc(compact log-probs)"))) return rc;
+  }
+  if (!pl->lists[Q_GENERIC].empty() && (rc = alloc((void **)&pl->d_raw, (size_t)pl->total_L * sizeof(int32_t), "labels", labels))) return rc;
+  if (pl->any_bad_label && (rc = alloc((void **)&pl->d_status_init, (size_t)B * sizeof(int32_t), "statuses", status_init.data()))) return rc;
+  if ((rc = alloc((void **)&pl->d_bp, (size_t)bp_bytes, "pool_malloc(backpointers)"))) return rc;
+  if ((rc = alloc((void **)&pl->d_scratch, (size_t)scr_floats * 4, "pool_malloc(scratch)"))) return rc;
+  if ((rc = alloc((void **)&pl->d_queue, N_QUEUES * sizeof(unsigned int), "pool_malloc(queue)"))) return rc;
+  if (!pl->bt_meta.empty()) {
+    if ((rc = alloc((void **)&pl->d_bt_meta, pl->bt_meta.size() * sizeof(KabBtMeta), "backtrack metadata", pl->bt_meta.data()))) return rc;
+    if ((rc = alloc((void **)&pl->d_bt_maps, (size_t)pl->bt_map_ints * 4, "pool_malloc(backtrack maps)"))) return rc;
+    if ((rc = alloc((void **)&pl->d_bt_entry, (size_t)pl->bt_blocks * 4, "pool_malloc(backtrack entries)"))) return rc;
+    if ((rc = alloc((void **)&pl->d_end_state, (size_t)B * 4, "pool_malloc(end states)"))) return rc;
+  }
+  if ((rc = alloc((void **)&pl->d_band_fifo, (size_t)pl->band_fifo_bytes, "pool_malloc(band FIFOs)"))) return rc;
+  if ((rc = alloc((void **)&pl->d_wide_ws, (size_t)pl->wide_ws_bytes, "pool_malloc(wide workspace)"))) return rc;
+  if (!pl->lists[Q_WARP].empty()) {
+    Launch &l = pl->launch[Q_WARP];
+    l.fn = s.ctc ? (const void *)kab_warp_ctc_kernel
+         : s.M == 4 ? (Veff == 39 ? (const void *)kab_warp_kernel<39, false> : (const void *)kab_warp_kernel<0, false>)
+                    : (Veff == 39 ? (const void *)kab_warp_kernel<39, true> : (const void *)kab_warp_kernel<0, true>);
+    l.block = dim3(KAB_WARPS_PER_CTA * 32);
+    l.smem = 128 + (size_t)KAB_WARPS_PER_CTA * (KAB_WARP_STAGES * pl->stage_bytes + 256);  // + label tables
+    if ((e = ensure_dyn_smem(l.fn, pl->device, l.smem)) != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(warp)");
+    int occ = 0;
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, l.fn, l.block.x, l.smem)) != cudaSuccess) return cuda_fail(e, "occupancy(warp)");
+    const int64_t ctas = ((int64_t)pl->lists[Q_WARP].size() + KAB_WARPS_PER_CTA - 1) / KAB_WARPS_PER_CTA;
+    occ = std::min(occ, KAB_WARP_MINBLOCKS);
+    if (knob.warp_ctas_per_sm >= 1) occ = std::min(occ, knob.warp_ctas_per_sm);
+    l.grid = dim3((unsigned)std::min<int64_t>(ctas, (int64_t)pl->sm_count * std::max(occ, 1)));
+  }
+  if (!pl->lists[Q_BAND].empty()) {
+    Launch &l = pl->launch[Q_BAND];
+    const BandKernel bk = pl->band_kernel;
+    const int64_t n_band = (int64_t)pl->lists[Q_BAND].size();
+    const bool mm = s.M != 4, small = pl->band_nw <= 16;
+    l.fn = bk == BandKernel::P ? (const void *)kab_bandp_kernel
+         : bk == BandKernel::Q ? (const void *)kab_bandq_kernel
+         : bk == BandKernel::R ? (mm ? (const void *)kab_bandr_kernel<true> : (const void *)kab_bandr_kernel<false>)
+         : bk == BandKernel::R_GATHER ? (mm ? (const void *)kab_bandr_kernel<true, true> : (const void *)kab_bandr_kernel<false, true>)
+         : s.ctc ? (small ? (const void *)kab_band_ctc_kernel<512> : (const void *)kab_band_ctc_kernel<1024>)
+         : small ? (mm ? (const void *)kab_band_kernel<512, true> : (const void *)kab_band_kernel<512, false>)
+                 : (mm ? (const void *)kab_band_kernel<1024, true> : (const void *)kab_band_kernel<1024, false>);
+    const bool ga = bk == BandKernel::R_GATHER;  // (no emission stages: the geometry's minimum)
+    l.stage_frames = ga ? KAB_BR_F : pl->stage_frames;
+    l.stage_bytes = ga ? 64 : pl->stage_bytes;
+    if (bk == BandKernel::CTA) {
+      l.block = dim3(pl->band_nw * 32);
+      l.smem = kab_band_geom(pl->band_nw, pl->stage_bytes).smem_bytes;
       int occ = 0;
-      if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, KAB_WARPS_PER_CTA * 32, smem)) != cudaSuccess) { rc = cuda_fail(e, "occupancy(warp)"); break; }
-      pl->smem[Q_WARP] = smem;
-      const int64_t ctas = ((int64_t)pl->lists[Q_WARP].size() + KAB_WARPS_PER_CTA - 1) / KAB_WARPS_PER_CTA;
-      occ = std::min(occ, KAB_WARP_MINBLOCKS);
-      if (const char *cs = getenv("KAB_WARP_CTAS_PER_SM")) {  // development knob
-        const int v = atoi(cs);
-        if (v >= 1) occ = std::min(occ, v);
-      }
-      pl->grid[Q_WARP] = (int)std::min<int64_t>(ctas, (int64_t)pl->sm_count * std::max(occ, 1));
-    }
-    if (!pl->bt_meta.empty()) {
-      if ((rc = up((void **)&pl->d_bt_meta, pl->bt_meta.data(), pl->bt_meta.size() * sizeof(KabBtMeta)))) break;
-      if ((e = pool_malloc((void **)&pl->d_bt_maps, (size_t)pl->bt_map_ints * 4)) != cudaSuccess) { rc = cuda_fail(e, "pool_malloc(backtrack maps)"); break; }
-      if ((e = pool_malloc((void **)&pl->d_bt_entry, (size_t)pl->bt_blocks * 4)) != cudaSuccess) { rc = cuda_fail(e, "pool_malloc(backtrack entries)"); break; }
-      if ((e = pool_malloc((void **)&pl->d_end_state, (size_t)pl->B * 4)) != cudaSuccess) { rc = cuda_fail(e, "pool_malloc(end states)"); break; }
-    }
-    if (!pl->lists[Q_BAND].empty() && pl->band_nc > 0) {
-      if ((e = pool_malloc((void **)&pl->d_band_fifo, (size_t)pl->band_fifo_bytes)) != cudaSuccess) { rc = cuda_fail(e, "pool_malloc(band FIFOs)"); break; }
-      const size_t smem_b = pl->band_r ? kab_bandr_geom(pl->band_ga ? 64 : pl->stage_bytes).smem_bytes
-                                       : (pl->band_q ? kab_bandq_geom(pl->stage_bytes).smem_bytes : kab_bandp_geom(pl->stage_bytes).smem_bytes);
-      const void *fn = pl->band_r ? (pl->band_ga ? (M == 4 ? (const void *)kab_bandr_kernel<false, true> : (const void *)kab_bandr_kernel<true, true>)
-                                                 : (M == 4 ? (const void *)kab_bandr_kernel<false> : (const void *)kab_bandr_kernel<true>))
-                                  : (pl->band_q ? (const void *)kab_bandq_kernel : (const void *)kab_bandp_kernel);
-      const int threads = pl->band_r ? KAB_BR_THREADS : (pl->band_q ? KAB_BQ_THREADS : KAB_BP_THREADS);
-      if ((e = ensure_dyn_smem(fn, device, smem_b)) != cudaSuccess) { rc = cuda_fail(e, "cudaFuncSetAttribute(cluster band)"); break; }
-      pl->smem[Q_BAND] = smem_b;
-      cudaLaunchConfig_t cfg{};
+      if ((e = ensure_dyn_smem(l.fn, pl->device, l.smem)) != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(band)");
+      if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, l.fn, l.block.x, l.smem)) != cudaSuccess) return cuda_fail(e, "occupancy(band)");
+      l.grid = dim3((unsigned)std::min<int64_t>(n_band, (int64_t)(pl->sm_count - pl->band_sm_reserved) * std::max(occ, 1)));
+    } else {
+      const bool r = bk == BandKernel::R || bk == BandKernel::R_GATHER;
+      l.block = dim3(r ? KAB_BR_THREADS : (bk == BandKernel::Q ? KAB_BQ_THREADS : KAB_BP_THREADS));
+      l.smem = r ? kab_bandr_geom(l.stage_bytes).smem_bytes
+                 : (bk == BandKernel::Q ? kab_bandq_geom(l.stage_bytes).smem_bytes : kab_bandp_geom(l.stage_bytes).smem_bytes);
+      l.cluster = (unsigned)pl->band_nc;
+      if ((e = ensure_dyn_smem(l.fn, pl->device, l.smem)) != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(cluster band)");
+      l.grid = dim3((unsigned)(pl->band_nc * pl->sm_count));
       cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeClusterDimension;
-      at[0].val.clusterDim.x = (unsigned)pl->band_nc; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-      cfg.gridDim = dim3((unsigned)(pl->band_nc * pl->sm_count), 1, 1);
-      cfg.blockDim = dim3((unsigned)threads, 1, 1);
-      cfg.dynamicSmemBytes = smem_b;
-      cfg.attrs = at; cfg.numAttrs = 1;
+      const cudaLaunchConfig_t cfg = launch_config(l, at, nullptr);
       int ncl = 0;
-      if ((e = cudaOccupancyMaxActiveClusters(&ncl, fn, &cfg)) != cudaSuccess) { rc = cuda_fail(e, "cudaOccupancyMaxActiveClusters(cluster band)"); break; }
-      ncl = (int)std::min<int64_t>(std::max(ncl, 1), (int64_t)pl->lists[Q_BAND].size());
-      pl->grid[Q_BAND] = ncl * pl->band_nc;
-    } else if (!pl->lists[Q_BAND].empty()) {
-      const KabBandGeom geo = kab_band_geom(pl->band_nw, pl->stage_bytes);
-      const void *fn = ctc ? (pl->band_nw <= 16 ? (const void *)kab_band_ctc_kernel<512> : (const void *)kab_band_ctc_kernel<1024>)
-                     : M == 4 ? (pl->band_nw <= 16 ? (const void *)kab_band_kernel<512, false> : (const void *)kab_band_kernel<1024, false>)
-                              : (pl->band_nw <= 16 ? (const void *)kab_band_kernel<512, true> : (const void *)kab_band_kernel<1024, true>);
-      if ((e = ensure_dyn_smem(fn, device, geo.smem_bytes)) != cudaSuccess) { rc = cuda_fail(e, "cudaFuncSetAttribute(band)"); break; }
-      int occ = 0;
-      if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, pl->band_nw * 32, geo.smem_bytes)) != cudaSuccess) { rc = cuda_fail(e, "occupancy(band)"); break; }
-      pl->smem[Q_BAND] = geo.smem_bytes;
-      pl->grid[Q_BAND] = (int)std::min<int64_t>((int64_t)pl->lists[Q_BAND].size(), (int64_t)(pl->sm_count - pl->band_sm_reserved) * std::max(occ, 1));
+      if ((e = cudaOccupancyMaxActiveClusters(&ncl, l.fn, &cfg)) != cudaSuccess) return cuda_fail(e, "cudaOccupancyMaxActiveClusters(cluster band)");
+      l.grid = dim3((unsigned)(std::min<int64_t>(std::max(ncl, 1), n_band) * pl->band_nc));
     }
-    if (!pl->lists[Q_WIDE].empty()) {
-      if ((e = pool_malloc((void **)&pl->d_wide_ws, (size_t)pl->wide_ws_bytes)) != cudaSuccess) { rc = cuda_fail(e, "pool_malloc(wide workspace)"); break; }
-      pl->smem[Q_WIDE] = kab_wide_geom(pl->stage_bytes).smem_bytes;
-      pl->grid[Q_WIDE] = wide_max_ctas + 1;  // forward CTAs + the backtrack CTA
-    }
-    if (!pl->lists[Q_GENERIC].empty())
-      pl->grid[Q_GENERIC] = (int)std::min<int64_t>((int64_t)pl->lists[Q_GENERIC].size(), (int64_t)pl->sm_count * 4);
-  } while (0);
-  tr.mark("allocate, upload, kernel attributes");
-  if (rc != KAB_OK) { plan_free(pl); return rc; }
+  }
+  if (!pl->lists[Q_WIDE].empty()) pl->launch[Q_WIDE].grid = dim3((unsigned)(wide_max_ctas + 1));  // forward CTAs + the backtrack CTA
+  if (!pl->lists[Q_GENERIC].empty())
+    pl->launch[Q_GENERIC].grid = dim3((unsigned)std::min<int64_t>((int64_t)pl->lists[Q_GENERIC].size(), (int64_t)pl->sm_count * 4));
+  return KAB_OK;
+}
 
+// ---- stage 7: the plan's info, and the sub-plan of a hybrid band plan
+int Setup::finish() {
+  kab_plan_info &info = pl->info;
   info.backptr_bytes = bp_bytes;
   info.workspace_bytes = bp_bytes + scr_floats * 4 + pl->wide_ws_bytes + pl->band_fifo_bytes + (int64_t)col16.size() * 2 +
                          (pl->d_raw ? pl->total_L * 4 : 0) + B * (int64_t)sizeof(KabLattice);
   info.kernel_launches = 0;
   for (int q = 0; q < N_QUEUES; ++q) info.kernel_launches += pl->lists[q].empty() ? 0 : 1;
+  const BandKernel bk = pl->band_kernel;
   if (!pl->lists[Q_BAND].empty()) {
-    info.band_kernel = pl->band_r ? KAB_BAND_KERNEL_SPEC : (pl->band_q ? KAB_BAND_KERNEL_CLUSTER2 : (pl->band_nc > 0 ? KAB_BAND_KERNEL_CLUSTER : KAB_BAND_KERNEL_CTA));
+    const int32_t code[] = {KAB_BAND_KERNEL_CTA, KAB_BAND_KERNEL_CLUSTER, KAB_BAND_KERNEL_CLUSTER2, KAB_BAND_KERNEL_SPEC, KAB_BAND_KERNEL_SPEC};
+    info.band_kernel = code[(int)bk];  // (in BandKernel's order)
     info.band_cluster = pl->band_nc > 0 ? pl->band_nc : 1;
   }
-  if (!pl->bt_meta.empty()) info.kernel_launches += 3;  // kab_bt_maps_kernel, kab_bt_stitch_kernel, kab_bt_gather_kernel
-  if (pl->band_r) info.kernel_launches += 1;            // kab_finite_rows_kernel
-  if (pl->Vc)                                          // kab_compact_kernel (CTC: _ctc_), kab_expand_labels_kernel
+  if (!pl->bt_meta.empty()) info.kernel_launches += 3;                      // kab_bt_maps_kernel, kab_bt_stitch_kernel, kab_bt_gather_kernel
+  if (bk == BandKernel::R || bk == BandKernel::R_GATHER) info.kernel_launches += 1;  // kab_finite_rows_kernel
+  if (pl->Vc)                                                               // kab_compact_kernel (CTC: _ctc_), kab_expand_labels_kernel
     for (int q : {Q_WARP, Q_BAND, Q_WIDE}) info.kernel_launches += pl->lists[q].empty() ? 0 : 2;
-  if (hyb_k > 0) {  // the sub-plan of a hybrid band plan: same arrays, its own lattices, workspaces and stream
-    int rcs = plan_create_impl(&pl->sub, device, B, t_off, labels, l_off, V, W, M, hyb_mask.data(), 1, pl->ctc, pl->blank, pl->ctc_long);
-    if (rcs == KAB_OK) {
-      pl->sub->is_child = true;
-      pl->sub->grid[Q_BAND] = std::min(pl->sub->grid[Q_BAND], hyb_k * pl->sub->band_nc);
-      cudaError_t e = pool_malloc((void **)&pl->sub->d_started, sizeof(unsigned int));
-      if (e == cudaSuccess) e = cudaMemset(pl->sub->d_started, 0, sizeof(unsigned int));
-      if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&pl->s_sub, cudaStreamNonBlocking);
-      if (e == cudaSuccess) e = cudaEventCreateWithFlags(&pl->ev_fork, cudaEventDisableTiming);
-      if (e == cudaSuccess) e = cudaEventCreateWithFlags(&pl->ev_join, cudaEventDisableTiming);
-      if (e != cudaSuccess) rcs = cuda_fail(e, "stream / events of the hybrid band plan");
-    }
-    if (rcs != KAB_OK) { plan_free(pl); return rcs; }
-    info.band_kernel = KAB_BAND_KERNEL_HYBRID;
-    info.band_cluster = pl->sub->band_nc;
-    info.backptr_bytes += pl->sub->info.backptr_bytes;
-    info.workspace_bytes += pl->sub->info.workspace_bytes;
-    info.kernel_launches += pl->sub->info.kernel_launches;
+  if (hyb_k == 0) return KAB_OK;
+  // the sub-plan of a hybrid band plan: same arrays, its own lattices, workspaces and stream
+  if (int rc = plan_create_impl(&pl->sub, pl->device, s, B, t_off, labels, l_off, hyb_mask.data(), 1)) return rc;
+  pl->sub->is_child = true;
+  pl->sub->launch[Q_BAND].grid.x = std::min(pl->sub->launch[Q_BAND].grid.x, (unsigned)(hyb_k * pl->sub->band_nc));
+  cudaError_t e = pool_malloc((void **)&pl->sub->d_started, sizeof(unsigned int));
+  if (e == cudaSuccess) e = cudaMemset(pl->sub->d_started, 0, sizeof(unsigned int));
+  if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&pl->s_sub, cudaStreamNonBlocking);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&pl->ev_fork, cudaEventDisableTiming);
+  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&pl->ev_join, cudaEventDisableTiming);
+  if (e != cudaSuccess) return cuda_fail(e, "stream / events of the hybrid band plan");
+  info.band_kernel = KAB_BAND_KERNEL_HYBRID;
+  info.band_cluster = pl->sub->band_nc;
+  info.backptr_bytes += pl->sub->info.backptr_bytes;
+  info.workspace_bytes += pl->sub->info.workspace_bytes;
+  info.kernel_launches += pl->sub->info.kernel_launches;
+  return KAB_OK;
+}
+
+int plan_create_impl(kab_plan **out, int device, const PlanSpec &s, int64_t B, const int64_t *t_off,
+                     const int32_t *labels, const int64_t *l_off, const uint8_t *mask, int band_mode) {
+  if (!out || B < 0 || !t_off || !l_off || s.V < 1 || s.V > 65535 || s.W < 0 || s.M < 1 || s.M > 255) return KAB_E_BAD_ARG;
+  if (B > 0 && (t_off[0] < 0 || l_off[0] < 0)) return KAB_E_BAD_ARG;
+  if (B > 0 && l_off[B] > l_off[0] && !labels) return KAB_E_BAD_ARG;
+  for (int64_t b = 0; b < B; ++b) {
+    const int64_t T = t_off[b + 1] - t_off[b], L = l_off[b + 1] - l_off[b];
+    if (T < 1 || T > 0x3fffffff || L < 0 || L > 0x3ffffff0) return KAB_E_BAD_ARG;
   }
+  DeviceGuard guard;
+  KAB_CUDA(guard.enter(device));
+  kab_plan *pl = new (std::nothrow) kab_plan();
+  if (!pl) return KAB_E_NOMEM;
+  pl->device = device; pl->B = B; pl->spec = s;
+  pl->total_T = B ? t_off[B] : 0;  // offsets are absolute rows / entries of the caller's arrays
+  pl->total_L = B ? l_off[B] : 0;
+  if (B > 0) {
+    pl->h_t_off.assign(t_off, t_off + B + 1);
+    pl->h_l_off.assign(l_off, l_off + B + 1);
+    if (pl->total_L > 0) pl->h_labels.assign(labels, labels + pl->total_L);
+  }
+  Trace tr("kab_plan_create");
+  if (int rcs = sm_count_of(device, &pl->sm_count)) { delete pl; return rcs; }
+  pl->info.n_lattices = B; pl->info.device = device; pl->info.total_frames = pl->total_T;
+
+  Setup x{pl, s, Knobs::read(), B, t_off, l_off, labels, mask};
+  x.scan_labels();
+  x.compact_vocabulary();
+  x.classify();
+  x.choose_band_kernel(band_mode);
+  x.lay_out_band();
+  tr.mark("classify");
+  int rc = x.allocate();
+  tr.mark("allocate, upload, kernel attributes");
+  if (rc == KAB_OK) rc = x.finish();
+  if (rc != KAB_OK) { plan_free(pl); return rc; }
   *out = pl;
   return KAB_OK;
 }
@@ -947,44 +1004,41 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   DeviceGuard guard;
   KAB_CUDA(guard.enter(pl->device));
+  const PlanSpec &s = pl->spec;
   KabParams p{};
   p.lp = d_log_probs;
-  p.lp_bytes = pl->total_T * (int64_t)pl->V * 4;
+  p.lp_bytes = pl->total_T * (int64_t)s.V * 4;
   p.col16 = pl->d_col16; p.raw = pl->d_raw; p.bp = pl->d_bp; p.scratch = pl->d_scratch;
   p.best_path = d_best_path; p.best_labels = d_best_labels; p.best_scores = d_best_scores;
   p.final_score = d_final_score; p.status = d_status;
-  p.V = pl->V; p.W = pl->W; p.M = pl->M;
+  p.V = s.V; p.W = s.W; p.M = s.M;
   p.stage_frames = pl->stage_frames; p.stage_bytes = pl->stage_bytes;
   p.one = 1u;
   p.started = pl->d_started;
   {  // max_move < 4: the excluded moves' candidates become -inf (kab_mm)
     const float ninf = -std::numeric_limits<float>::infinity();
-    p.mm1 = pl->M >= 2 ? 0.0f : ninf; p.mm2 = pl->M >= 3 ? 0.0f : ninf; p.mm3 = pl->M >= 4 ? 0.0f : ninf;
+    p.mm1 = s.M >= 2 ? 0.0f : ninf; p.mm2 = s.M >= 3 ? 0.0f : ninf; p.mm3 = s.M >= 4 ? 0.0f : ninf;
   }
   p.band_nw = pl->band_nw;
 
-  // the staged kernels' view of the log-probs: the caller's array, or its compact copy
+  // the staged kernels' view of the log-probs: the caller's array, or its compact copy (not the gather mode's)
   KabParams pf = p;
-  const int fast_lists[3] = {Q_WARP, Q_BAND, Q_WIDE};
+  const BandKernel bk = pl->band_kernel;
+  auto on_copy = [&](int q) { return !pl->lists[q].empty() && !(q == Q_BAND && bk == BandKernel::R_GATHER); };
   if (pl->Vc) {
     KAB_CUDA(cudaMemsetAsync(pl->d_nonfinite, 0, (size_t)pl->B * sizeof(int32_t), stream));
-    for (int q : fast_lists)
-      if (!pl->lists[q].empty() && !(q == Q_BAND && pl->band_ga)) {
+    for (int q : {Q_WARP, Q_BAND, Q_WIDE})
+      if (on_copy(q)) {
         const dim3 grid((unsigned)pl->lists[q].size(), (unsigned)((pl->max_T[q] + KAB_COMPACT_FRAMES - 1) / KAB_COMPACT_FRAMES));
-        if (pl->ctc)
-          kab_compact_ctc_kernel<<<grid, 256, 0, stream>>>(pl->d_lists[q], d_log_probs, pl->d_lpc, pl->d_gather, pl->V, pl->Vc,
-                                                           pl->d_nonfinite);
-        else
-          kab_compact_kernel<<<grid, 256, 0, stream>>>(pl->d_lists[q], d_log_probs, pl->d_lpc, pl->d_gather, pl->V, pl->Vc,
-                                                       pl->d_nonfinite);
+        (s.ctc ? kab_compact_ctc_kernel : kab_compact_kernel)<<<grid, 256, 0, stream>>>(pl->d_lists[q], d_log_probs, pl->d_lpc,
+                                                                                          pl->d_gather, s.V, pl->Vc, pl->d_nonfinite);
       }
-    pf.lp = pl->d_lpc;
-    pf.V = pl->Vc;
-    pf.lp_bytes = pl->total_T * (int64_t)pl->Vc * 4;
+    pf.lp = pl->d_lpc; pf.V = pl->Vc; pf.lp_bytes = pl->total_T * (int64_t)pl->Vc * 4;
   }
   // CTC: the blank's column in the staged kernels' view (compact column 0 of the copy); the generic kernel
   // reads the caller's array and keeps the blank id
-  const int32_t sblank = pl->Vc ? 0 : pl->blank;
+  const int sblank = pl->Vc ? 0 : s.blank;
+  const int *blank_arg = s.ctc ? &sblank : nullptr;
 
   if (pl->sub) {  // hybrid band plan: the long lattices first (their clusters need whole SMs), on the side stream
     KAB_CUDA(cudaEventRecord(pl->ev_fork, stream));
@@ -994,7 +1048,7 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
     KAB_CUDA(cudaEventRecord(pl->ev_join, pl->s_sub));
     // the single-CTA kernel below would otherwise spread one CTA over every SM before the clusters
     // (which need whole SMs) are placed, and the two kernels would run one after the other
-    pl->sub->gate_target += (unsigned int)pl->sub->grid[Q_BAND];
+    pl->sub->gate_target += pl->sub->launch[Q_BAND].grid.x;
     if (!pl->lists[Q_BAND].empty()) kab_gate_kernel<<<1, 32, 0, stream>>>(pl->sub->d_started, pl->sub->gate_target);
   }
   KAB_CUDA(cudaMemsetAsync(pl->d_queue, 0, N_QUEUES * sizeof(unsigned int), stream));
@@ -1003,87 +1057,38 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
 
   if (!pl->lists[Q_WARP].empty()) {
     KabParams pw = pf; pw.queue = pl->d_queue + Q_WARP;
-    const int nwl = (int)pl->lists[Q_WARP].size();
-    const dim3 wg((unsigned)pl->grid[Q_WARP]), wb(KAB_WARPS_PER_CTA * 32);
-    if (pl->ctc) {
-      kab_warp_ctc_kernel<<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw, sblank);
-    } else if (pl->M == 4) {
-      if (pf.V == 39) kab_warp_kernel<39, false><<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw);
-      else kab_warp_kernel<0, false><<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw);
-    } else {
-      if (pf.V == 39) kab_warp_kernel<39, true><<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw);
-      else kab_warp_kernel<0, true><<<wg, wb, pl->smem[Q_WARP], stream>>>(pl->d_lists[Q_WARP], nwl, pw);
-    }
+    KAB_CUDA(launch_list(pl->launch[Q_WARP], pl->d_lists[Q_WARP], (int)pl->lists[Q_WARP].size(), pw, nullptr, blank_arg, stream));
   }
   if (!pl->lists[Q_BAND].empty()) {
-    KabParams pb = pl->band_ga ? p : pf; pb.queue = pl->d_queue + Q_BAND;
-    if (pl->band_ga) { pb.stage_frames = KAB_BR_F; pb.stage_bytes = 64; }  // (no emission stages: the geometry's minimum)
-    KabBandTiming band_timing(pb, stream, pl->band_nw);  // (development builds only: kab_debug.h)
-    if (pl->band_nc > 0) {
-      if (!pl->band_r) KAB_CUDA(cudaMemsetAsync(pl->d_band_fifo, 0, (size_t)pl->band_fifo_bytes, stream));  // (bandr: mailboxes in shared memory)
-      pb.fifo = pl->d_band_fifo;
-      KabBandpTiming bandp_timing(pb, stream, KAB_BP_CW * pl->band_nc);
-      cudaLaunchConfig_t cfg{};
-      cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeClusterDimension;
-      at[0].val.clusterDim.x = (unsigned)pl->band_nc; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-      cfg.gridDim = dim3((unsigned)pl->grid[Q_BAND], 1, 1);
-      cfg.blockDim = dim3((unsigned)(pl->band_r ? KAB_BR_THREADS : (pl->band_q ? KAB_BQ_THREADS : KAB_BP_THREADS)), 1, 1);
-      cfg.dynamicSmemBytes = pl->smem[Q_BAND];
-      cfg.stream = stream;
-      cfg.attrs = at; cfg.numAttrs = 1;
-      pb.end_state = pl->d_end_state;  // nullptr: the kernel walks back itself
-      const int n_band = (int)pl->lists[Q_BAND].size();
+    const Launch &lb = pl->launch[Q_BAND];
+    KabParams pb = bk == BandKernel::R_GATHER ? p : pf;
+    pb.queue = pl->d_queue + Q_BAND; pb.stage_frames = lb.stage_frames; pb.stage_bytes = lb.stage_bytes;
+    pb.fifo = pl->d_band_fifo; pb.end_state = pl->d_end_state;  // (end_state nullptr: the kernel walks back itself)
+    const int n_band = (int)pl->lists[Q_BAND].size(), nwt = pl->band_cw * pl->band_nc;
+    std::optional<KabBandTiming> t_cta; std::optional<KabBandpTiming> t_p; std::optional<KabBandqTiming> t_q; std::optional<KabBandrTiming> t_r;
+    if (bk == BandKernel::CTA) t_cta.emplace(pb, stream, pl->band_nw);  // (development builds only: kab_debug.h)
+    else if (bk == BandKernel::P) t_p.emplace(pb, stream, nwt);
+    else if (bk == BandKernel::Q) t_q.emplace(pb, stream, nwt);
+    else t_r.emplace(pb, stream, nwt);
+    if (bk == BandKernel::P || bk == BandKernel::Q)  // (bandr: mailboxes in shared memory)
+      KAB_CUDA(cudaMemsetAsync(pl->d_band_fifo, 0, (size_t)pl->band_fifo_bytes, stream));
+    KAB_CUDA(launch_list(lb, pl->d_lists[Q_BAND], n_band, pb, nullptr, blank_arg, stream));
+    if (bk == BandKernel::R || bk == BandKernel::R_GATHER) {
+      const dim3 fg((unsigned)n_band, (unsigned)((pl->max_T[Q_BAND] + KAB_FIN_ROWS - 1) / KAB_FIN_ROWS));
+      kab_finite_rows_kernel<<<fg, 256, 0, stream>>>(pl->d_lists[Q_BAND], pb.lp, pb.V, d_status, d_final_score);
+    }
+    if (pl->d_end_state) {  // the parallel backtrack (kab_btpar.cuh)
       const dim3 mg((unsigned)pl->bt_blocks, (unsigned)((pl->bt_max_wl + KAB_BT_THREADS - 1) / KAB_BT_THREADS));
-      if (pl->band_q) {
-        KabBandqTiming bandq_timing(pb, stream, pl->band_cw * pl->band_nc);
-        const int nwt = pl->band_cw * pl->band_nc;
-        KabBandrTiming bandr_timing(pb, stream, nwt);
-        if (pl->band_r) {
-          if (pl->band_ga) {
-            if (pl->M == 4)
-              KAB_CUDA(cudaLaunchKernelEx(&cfg, kab_bandr_kernel<false, true>, (const KabLattice *)pl->d_lists[Q_BAND], n_band, pb));
-            else
-              KAB_CUDA(cudaLaunchKernelEx(&cfg, kab_bandr_kernel<true, true>, (const KabLattice *)pl->d_lists[Q_BAND], n_band, pb));
-          } else if (pl->M == 4)
-            KAB_CUDA(cudaLaunchKernelEx(&cfg, kab_bandr_kernel<false>, (const KabLattice *)pl->d_lists[Q_BAND], n_band, pb));
-          else
-            KAB_CUDA(cudaLaunchKernelEx(&cfg, kab_bandr_kernel<true>, (const KabLattice *)pl->d_lists[Q_BAND], n_band, pb));
-          const dim3 fg((unsigned)n_band, (unsigned)((pl->max_T[Q_BAND] + KAB_FIN_ROWS - 1) / KAB_FIN_ROWS));
-          kab_finite_rows_kernel<<<fg, 256, 0, stream>>>(pl->d_lists[Q_BAND], pb.lp, pb.V, d_status, d_final_score);
-        } else
-          KAB_CUDA(cudaLaunchKernelEx(&cfg, kab_bandq_kernel, (const KabLattice *)pl->d_lists[Q_BAND], n_band, pb));
-        kab_bt_maps_kernel<KabBtLayoutQ><<<mg, KAB_BT_THREADS, 0, stream>>>(pl->d_lists[Q_BAND], pl->d_bt_meta, n_band, pl->d_bp,
-                                                                            d_status, pl->d_bt_maps, pl->W, nwt);
-        kab_bt_stitch_kernel<KabBtLayoutQ><<<n_band, 1024, 0, stream>>>(pl->d_lists[Q_BAND], pl->d_bt_meta, pb, pl->d_end_state,
-                                                                        pl->d_bt_maps, pl->d_bt_entry, nwt);
-      } else {
-        const int nwt = KAB_BP_CW * pl->band_nc;
-        KAB_CUDA(cudaLaunchKernelEx(&cfg, kab_bandp_kernel, (const KabLattice *)pl->d_lists[Q_BAND], n_band, pb));
-        if (pl->d_end_state) {
-          kab_bt_maps_kernel<KabBtLayoutP><<<mg, KAB_BT_THREADS, 0, stream>>>(pl->d_lists[Q_BAND], pl->d_bt_meta, n_band, pl->d_bp,
-                                                                              d_status, pl->d_bt_maps, pl->W, nwt);
-          kab_bt_stitch_kernel<KabBtLayoutP><<<n_band, 1024, 0, stream>>>(pl->d_lists[Q_BAND], pl->d_bt_meta, pb, pl->d_end_state,
-                                                                          pl->d_bt_maps, pl->d_bt_entry, nwt);
-        }
-      }
-      if (pl->d_end_state) {
-        const dim3 gg((unsigned)n_band, (unsigned)((pl->max_T[Q_BAND] + KAB_BT_GATHER_FRAMES - 1) / KAB_BT_GATHER_FRAMES));
-        kab_bt_gather_kernel<<<gg, 256, 0, stream>>>(pl->d_lists[Q_BAND], pb);
-      }
-    } else {
-      const int nbl = (int)pl->lists[Q_BAND].size();
-      const dim3 bg((unsigned)pl->grid[Q_BAND]), bb((unsigned)(pl->band_nw * 32));
-      if (pl->ctc) {
-        if (pl->band_nw <= 16) kab_band_ctc_kernel<512><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb, sblank);
-        else kab_band_ctc_kernel<1024><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb, sblank);
-      } else if (pl->band_nw <= 16) {
-        if (pl->M == 4) kab_band_kernel<512, false><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb);
-        else kab_band_kernel<512, true><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb);
-      } else {
-        if (pl->M == 4) kab_band_kernel<1024, false><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb);
-        else kab_band_kernel<1024, true><<<bg, bb, pl->smem[Q_BAND], stream>>>(pl->d_lists[Q_BAND], nbl, pb);
-      }
+      auto maps_stitch = [&](auto layout) {
+        using Layout = decltype(layout);
+        kab_bt_maps_kernel<Layout><<<mg, KAB_BT_THREADS, 0, stream>>>(pl->d_lists[Q_BAND], pl->d_bt_meta, n_band, pl->d_bp, d_status,
+                                                                      pl->d_bt_maps, s.W, nwt);
+        kab_bt_stitch_kernel<Layout><<<n_band, 1024, 0, stream>>>(pl->d_lists[Q_BAND], pl->d_bt_meta, pb, pl->d_end_state,
+                                                                  pl->d_bt_maps, pl->d_bt_entry, nwt);
+      };
+      if (band_layout_q(bk)) maps_stitch(KabBtLayoutQ{}); else maps_stitch(KabBtLayoutP{});
+      const dim3 gg((unsigned)n_band, (unsigned)((pl->max_T[Q_BAND] + KAB_BT_GATHER_FRAMES - 1) / KAB_BT_GATHER_FRAMES));
+      kab_bt_gather_kernel<<<gg, 256, 0, stream>>>(pl->d_lists[Q_BAND], pb);
     }
   }
   if (!pl->lists[Q_WIDE].empty()) {
@@ -1091,29 +1096,22 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
     KabWideTiming wide_timing(pf, stream);
     // cooperative launch: the warps of the chain spin on each other, so the whole grid has to be
     // resident -- the runtime checks that instead of letting the kernel hang
-    const KabLattice *wl = pl->d_lists[Q_WIDE];
-    int wn = (int)pl->lists[Q_WIDE].size();
-    unsigned char *wws = pl->d_wide_ws;
-    int wblank = sblank;
-    void *wargs[] = {(void *)&wl, (void *)&wn, (void *)&pf, (void *)&wws, (void *)&wblank};
-    const void *wfn = pl->ctc ? (const void *)kab_wide_ctc_kernel : (const void *)kab_wide_kernel;
-    KAB_CUDA(cudaLaunchCooperativeKernel(wfn, dim3((unsigned)pl->grid[Q_WIDE]), dim3(KAB_WD_THREADS), wargs,
-                                         pl->smem[Q_WIDE], stream));
+    KAB_CUDA(launch_list(pl->launch[Q_WIDE], pl->d_lists[Q_WIDE], (int)pl->lists[Q_WIDE].size(), pf, &pl->d_wide_ws, blank_arg, stream));
   }
   if (pl->Vc)  // best_labels of the staged kernels: compact index -> label value
-    for (int q : fast_lists)
-      if (!pl->lists[q].empty() && !(q == Q_BAND && pl->band_ga)) {
+    for (int q : {Q_WARP, Q_BAND, Q_WIDE})
+      if (on_copy(q)) {
         const dim3 grid((unsigned)pl->lists[q].size(), (unsigned)((pl->max_T[q] + KAB_COMPACT_FRAMES - 1) / KAB_COMPACT_FRAMES));
         kab_expand_labels_kernel<<<grid, 64, 0, stream>>>(pl->d_lists[q], d_best_labels, d_status, d_final_score,
                                                           pl->d_gather, pl->Vc, pl->d_nonfinite);
       }
   if (!pl->lists[Q_GENERIC].empty()) {
     KabParams pg = p; pg.queue = pl->d_queue + Q_GENERIC;
-    if (pl->ctc)
-      kab_generic_ctc_kernel<GENERIC_NT><<<pl->grid[Q_GENERIC], GENERIC_NT, 0, stream>>>(
-          pl->d_lists[Q_GENERIC], (int)pl->lists[Q_GENERIC].size(), pg, pl->blank);
+    if (s.ctc)
+      kab_generic_ctc_kernel<GENERIC_NT><<<pl->launch[Q_GENERIC].grid, GENERIC_NT, 0, stream>>>(
+          pl->d_lists[Q_GENERIC], (int)pl->lists[Q_GENERIC].size(), pg, s.blank);
     else
-      kab_generic_kernel<GENERIC_NT><<<pl->grid[Q_GENERIC], GENERIC_NT, 0, stream>>>(
+      kab_generic_kernel<GENERIC_NT><<<pl->launch[Q_GENERIC].grid, GENERIC_NT, 0, stream>>>(
           pl->d_lists[Q_GENERIC], (int)pl->lists[Q_GENERIC].size(), pg);
   }
   KAB_CUDA(cudaGetLastError());
@@ -1253,7 +1251,7 @@ int kab_plan_segment_stats_device(kab_plan *pl, const int32_t *d_best_path, cons
                                   const int64_t *d_seg_lat_off, const int64_t *d_seg_end,
                                   kab_segment_record *d_records, uint8_t *d_labels_u8, void *stream_) {
   if (!pl || n_segments < 0) return KAB_E_BAD_ARG;
-  if (pl->ctc) return KAB_E_UNSUPPORTED;  // (the records are those of Kokoro-Align's align())
+  if (pl->spec.ctc) return KAB_E_UNSUPPORTED;  // (the records are those of Kokoro-Align's align())
   if (pl->B == 0) return n_segments == 0 ? KAB_OK : KAB_E_BAD_ARG;
   if (!d_best_path || !d_best_labels || !d_best_scores || !d_status) return KAB_E_BAD_ARG;
   if (n_segments > 0 && (!d_seg_lat_off || !d_seg_end || !d_records)) return KAB_E_BAD_ARG;
@@ -1286,7 +1284,7 @@ struct HostRun {  // what one kab_plan_run_host* call asks for
 int host_setup(kab_plan *pl) {
   if (pl->host_ready) return KAB_OK;
   const size_t n = (size_t)pl->total_T, B = (size_t)pl->B;
-  const int64_t V = pl->V;
+  const int64_t V = pl->spec.V;
   auto fail = [&](int rc) { host_teardown(pl); return rc; };
 #define KAB_SETUP(call)                                                  \
   do {                                                                   \
@@ -1335,8 +1333,8 @@ int host_setup(kab_plan *pl) {
         for (auto &x : lo) x -= l0;
         const int32_t *lab = pl->h_labels.empty() ? nullptr : pl->h_labels.data() + l0;
         child_rc[k] = (inject && atoi(inject) == (int)k) ? KAB_E_NOMEM
-                                                        : plan_create_impl(&child[k], pl->device, b1 - b0, to.data(), lab, lo.data(), pl->V, pl->W, pl->M,
-                                                                           nullptr, pl->ctc ? 0 : -1, pl->ctc, pl->blank, pl->ctc_long);
+                                                        : plan_create_impl(&child[k], pl->device, pl->spec, b1 - b0, to.data(), lab, lo.data(), nullptr,
+                                                                           pl->spec.ctc ? 0 : -1);
       };
       if (std::thread::hardware_concurrency() >= 4 && !getenv("KAB_SERIAL_SETUP")) {
         std::vector<std::thread> th;
@@ -1371,7 +1369,7 @@ int host_setup(kab_plan *pl) {
   {
     const char *be = getenv("KAB_HOST_BOOK");
     const std::vector<KabLattice> &bl = pl->lists[Q_BAND];  // (longest first)
-    if (pl->segs.empty() && !pl->sub && !pl->is_child && pl->band_r && !pl->band_ga && !pl->Vc && !pl->any_bad_label &&
+    if (pl->segs.empty() && !pl->sub && !pl->is_child && pl->band_kernel == BandKernel::R && !pl->Vc && !pl->any_bad_label &&
         pl->h_t_off[0] == 0 && bl.size() >= 4 && !(be && atoi(be) == 0) && (bytes_total >= (48ll << 20) || (be && atoi(be) >= 1))) {
       double band_t = 0.0;
       for (const KabLattice &d : bl) band_t += d.T;
@@ -1401,8 +1399,8 @@ int host_setup(kab_plan *pl) {
       int rcs[NP] = {KAB_OK, KAB_OK, KAB_OK};
       auto make = [&](int k) {
         if (k + 1 < NP && cnt[k] == 0) return;
-        rcs[k] = plan_create_impl(&pl->pipe[k], pl->device, (int64_t)B, pl->h_t_off.data(), lab, pl->h_l_off.data(), pl->V, pl->W, pl->M,
-                                  m[k].data(), k + 1 < NP ? 1 : -1, pl->ctc, pl->blank, pl->ctc_long);
+        rcs[k] = plan_create_impl(&pl->pipe[k], pl->device, pl->spec, (int64_t)B, pl->h_t_off.data(), lab, pl->h_l_off.data(),
+                                  m[k].data(), k + 1 < NP ? 1 : -1);
       };
       {
         std::vector<std::thread> th;
@@ -1419,7 +1417,8 @@ int host_setup(kab_plan *pl) {
         pl->pipe[k]->is_child = true;
         if (pl->pipe[k]->band_nc > 0 && !pl->pipe[k]->lists[Q_BAND].empty()) {
           const int want_cl = k + 1 < NP ? (int)cnt[k] : std::max(1, ncl_left);
-          pl->pipe[k]->grid[Q_BAND] = std::min(pl->pipe[k]->grid[Q_BAND], want_cl * pl->pipe[k]->band_nc);
+          unsigned &grid = pl->pipe[k]->launch[Q_BAND].grid.x;
+          grid = std::min(grid, (unsigned)(want_cl * pl->pipe[k]->band_nc));
           ncl_left -= want_cl;
         }
         if (k > 0) KAB_SETUP(cudaStreamCreateWithFlags(&pl->s_pipe[k], cudaStreamNonBlocking));
@@ -1456,7 +1455,7 @@ int run_host_impl(kab_plan *pl, const HostRun &r) {
   KAB_CUDA(guard.enter(pl->device));
   Trace tr("kab_plan_run_host");
   const size_t n = (size_t)pl->total_T, B = (size_t)pl->B;
-  const int64_t V = pl->V;
+  const int64_t V = pl->spec.V;
   if (int rc = host_setup(pl)) return rc;
   const bool want_stats = r.n_seg > 0 || r.h_lab8;
   if (want_stats) {
@@ -1504,7 +1503,7 @@ int run_host_impl(kab_plan *pl, const HostRun &r) {
         KAB_CUDA(cudaStreamWaitEvent(ck, pl->ev_pipe_in[k], 0));
         if (r.logits)
           for (const auto &rr : pl->pipe_rows[k])
-            if ((rc = kab_log_softmax_device(pl->d_lp + rr.first * V, pl->d_lp + rr.first * V, rr.second, pl->V, ck)) != KAB_OK) return rc;
+            if ((rc = kab_log_softmax_device(pl->d_lp + rr.first * V, pl->d_lp + rr.first * V, rr.second, pl->spec.V, ck)) != KAB_OK) return rc;
         rc = kab_plan_run_device(pl->pipe[k], pl->d_lp, pl->d_path, pl->d_lab, pl->d_sc, pl->d_fs, pl->d_st, ck);
         if (rc != KAB_OK) return rc;
         if (k > 0) {
@@ -1514,7 +1513,7 @@ int run_host_impl(kab_plan *pl, const HostRun &r) {
       }
     } else {
       KAB_CUDA(cudaMemcpyAsync(pl->d_lp, r.h_in, n * V * 4, cudaMemcpyHostToDevice, s));
-      if (r.logits && (rc = kab_log_softmax_device(pl->d_lp, pl->d_lp, (int64_t)n, pl->V, s)) != KAB_OK) return rc;
+      if (r.logits && (rc = kab_log_softmax_device(pl->d_lp, pl->d_lp, (int64_t)n, pl->spec.V, s)) != KAB_OK) return rc;
       rc = kab_plan_run_device(pl, pl->d_lp, pl->d_path, pl->d_lab, pl->d_sc, pl->d_fs, pl->d_st, s);
       if (rc != KAB_OK) return rc;
     }
@@ -1541,7 +1540,7 @@ int run_host_impl(kab_plan *pl, const HostRun &r) {
     KAB_CUDA(cudaEventRecord(pl->ev_in[k], pl->s_in));
     KAB_CUDA(cudaStreamWaitEvent(pl->stream, pl->ev_in[k], 0));
     int rc = KAB_OK;
-    if (r.logits && (rc = kab_log_softmax_device(pl->d_lp + t0 * V, pl->d_lp + t0 * V, (int64_t)nk, pl->V, pl->stream)) != KAB_OK)
+    if (r.logits && (rc = kab_log_softmax_device(pl->d_lp + t0 * V, pl->d_lp + t0 * V, (int64_t)nk, pl->spec.V, pl->stream)) != KAB_OK)
       return rc;
     rc = kab_plan_run_device(c, pl->d_lp + t0 * V, pl->d_path + t0, pl->d_lab + t0, pl->d_sc + t0,
                              pl->d_fs + b0, pl->d_st + b0, pl->stream);
@@ -1591,7 +1590,7 @@ int kab_plan_run_host_segments(kab_plan *pl, const float *h_in, int32_t is_logit
                                kab_segment_record *h_records, uint8_t *h_labels_u8, int32_t *h_best_path,
                                int32_t *h_best_labels, float *h_best_scores, float *h_final_score,
                                int32_t *h_status) {
-  if (pl && pl->ctc) return KAB_E_UNSUPPORTED;  // (the records are those of Kokoro-Align's align())
+  if (pl && pl->spec.ctc) return KAB_E_UNSUPPORTED;  // (the records are those of Kokoro-Align's align())
   HostRun r;
   r.h_in = h_in; r.logits = is_logits != 0;
   r.n_seg = n_segments; r.h_seg_lat_off = h_seg_lat_off; r.h_seg_end = h_seg_end; r.h_rec = h_records;
