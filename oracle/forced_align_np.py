@@ -23,8 +23,10 @@ NEG_INF = np.float32(-np.inf)
 
 
 def forced_align_np(lp, targets, blank=0):
-    """lp float32 [T, V], targets int [L] (L >= 1, no blank, T >= L + repeats).
-    Returns (state path int32 [T], paths int32 [T], scores float32 [T], final score float32)."""
+    """lp float32 [T, V], targets int [L] (no blank, T >= L + repeats).
+    Returns (state path int32 [T], paths int32 [T], scores float32 [T], final score float32).
+    L = 0 (S = 1, which the C ABI accepts and torchaudio does not): the path is all blank and the
+    final score is the float32 running sum of lp[:, blank] from 0, in frame order."""
     lp = np.ascontiguousarray(lp, dtype=np.float32)
     tg = np.asarray(targets, dtype=np.int64)
     T = lp.shape[0]
@@ -41,7 +43,7 @@ def forced_align_np(lp, targets, blank=0):
     for t in range(T):
         x0 = prev
         x1 = np.concatenate([[NEG_INF], prev[:-1]]).astype(np.float32)
-        x2 = np.where(allow2, np.concatenate([[NEG_INF, NEG_INF], prev[:-2]]), NEG_INF).astype(np.float32)
+        x2 = np.where(allow2, np.concatenate([[NEG_INF, NEG_INF], prev[:-2]])[:S], NEG_INF).astype(np.float32)
         j2 = (x2 > x1) & (x2 > x0)
         j1 = (x1 > x0) & (x1 > x2)
         best = np.where(j2, x2, np.where(j1, x1, x0))

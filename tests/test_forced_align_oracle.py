@@ -89,6 +89,83 @@ def test_restatement_matches_live_torchaudio(seed):
         assert s[0].numpy().tobytes() == scores.tobytes()
 
 
+@pytest.mark.parametrize("blank", [0, 3, 6])
+def test_restatement_empty_transcript(blank):
+    """L = 0 (S = 1): state 0 and the blank in every frame, scores lp[:, blank], and as final score their
+    float32 running sum from 0 in frame order (-inf from a -inf blank log-prob on)."""
+    rng = np.random.default_rng(blank)
+    for T in (1, 2, 9, 50):
+        lp = np.log(rng.dirichlet(np.ones(7), T)).astype(np.float32)
+        if T == 50:
+            lp[31, blank] = -np.inf
+        states, paths, scores, final = forced_align_np(lp, np.zeros(0, np.int32), blank)
+        f = np.float32(0.0)
+        for t in range(T):
+            f = np.float32(f + lp[t, blank])
+        assert (states == 0).all() and (paths == blank).all() and states.dtype == paths.dtype == np.int32
+        assert scores.tobytes() == np.ascontiguousarray(lp[:, blank]).tobytes()
+        assert final.tobytes() == f.tobytes() and (np.isneginf(final) == (T == 50))
+    _, _, _, final, status = forced_align_batch_np(lp, np.array([0, 20, 50]), np.array([(blank + 1) % 7], np.int32),
+                                                   np.array([0, 0, 1]), blank)
+    assert status.tolist() == [0, 0]
+
+
+def test_edge_case_generator():
+    """The cases of test_gpu_forced_align_edges.py are what their names say."""
+    from tests.test_gpu_forced_align_edges import COMPACT_CASES, EDGE_CASES, make_case
+    for case in EDGE_CASES + COMPACT_CASES:
+        S, V, blank, t_kind, content = case
+        lp, tg = make_case(case)
+        L, T = len(tg), lp.shape[0]
+        R = int((tg[1:] == tg[:-1]).sum())
+        assert lp.dtype == np.float32 and lp.shape[1] == V and S == 2 * L + 1, case
+        assert ((tg >= 0) & (tg < V) & (tg != blank)).all() and T >= L + R, case
+        assert blank == 0 or V == 2 or content == "allrep" or (tg == 0).any(), case
+        if t_kind in ("tight", "tight1"):
+            assert T == L + R + (t_kind == "tight1"), case
+        elif isinstance(t_kind, int):
+            assert T == t_kind, case
+        else:
+            assert T % t_kind[1] == t_kind[0], case
+        if content in ("climb", "blankmask"):
+            assert R == 0
+        if content == "climb":
+            assert T == L
+        if content == "allrep":
+            assert (tg == tg[0]).all()
+        if content in ("zero", "const"):
+            assert (lp == lp[:, :1]).all()
+        if V > 512:
+            assert len(set(tg.tolist())) <= 300
+    S = np.array([c[0] for c in EDGE_CASES])
+    for s in (3, 61, 63, 123, 125, 185, 187, 247, 249, 279, 281, 1631, 1633, 3295):
+        assert (S == s).any(), s
+    assert {2, 5, 32, 64, 65, 129, 512} == {c[1] for c in EDGE_CASES}
+
+
+def test_edge_cases_match_live_torchaudio():
+    """The restatement against torchaudio's CPU forced_align on every case of test_gpu_forced_align_edges.py
+    whose chosen end state is finite; the -inf row and -inf end cases end -inf."""
+    torch, F = _torchaudio()
+    from tests.test_gpu_forced_align_edges import COMPACT_CASES, EDGE_CASES, case_data, case_id
+    n = 0
+    for case in EDGE_CASES + COMPACT_CASES:
+        blank, content = case[2], case[4]
+        lp, tg, (_, paths, scores, final) = case_data(case)
+        if content in ("row", "end"):
+            assert np.isneginf(final), case_id(case)
+            continue
+        if content != "mask":
+            assert np.isfinite(final), case_id(case)
+        if not np.isfinite(final):
+            continue
+        p, s = F.forced_align(torch.from_numpy(lp)[None], torch.from_numpy(tg)[None], blank=blank)
+        np.testing.assert_array_equal(p[0].numpy(), paths, err_msg=case_id(case))
+        assert s[0].numpy().tobytes() == scores.tobytes(), case_id(case)
+        n += 1
+    assert n >= 60
+
+
 def test_batch_restatement_statuses():
     rng = np.random.default_rng(7)
     lp = np.log(rng.dirichlet(np.ones(5), 13)).astype(np.float32)
