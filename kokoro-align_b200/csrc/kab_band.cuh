@@ -57,16 +57,44 @@ __host__ __device__ inline KabBandGeom kab_band_geom(int nw, int stage_bytes) {
   return g;
 }
 
-__device__ __forceinline__ void kab_bulk_s2g(void *dst, const void *src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(kab_smem_u32(src)),
-               "r"(bytes)
-               : "memory");
-  asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+// Backtrack of ONE full group (8 frames, descending) from registers, in the backpointer words of the
+// cluster and wide kernels (kab_bandp.cuh, kab_wide.cuh: a lane of four states keeps one byte per
+// frame, 8 frames per 64-bit word): w0 holds the 8 backpointer bytes of the walker's byte column, w1
+// those of the column below (have1: it is available).
+// No load sits on the dependent chain (shift -> mask -> subtract -> compare).  Stops before the
+// frame that would need a third column; returns the next frame to process (-1: group done) and
+// the number of column steps taken (0..2, the last one not yet served when it stopped early).
+__device__ __forceinline__ int kab_walk_group8(const uint2 w0, const uint2 w1, const bool have1, int &v, int &k2,
+                                               int *pg, int &nchg) {
+  // Branch-free on purpose (selects only): with one active thread every taken branch costs a
+  // convergence-barrier round trip (~40 cycles, measured), several times the chain itself.  Frames
+  // after the stop point are computed and discarded (the caller overwrites their path entries).
+  uint32_t cx = w0.x, cy = w0.y;
+  int n = 0, f_next = -1, v_s = 0, k2_s = 0, n_s = 0;
+  bool stopped = false;
+#pragma unroll
+  for (int f = 7; f >= 0; --f) {
+    const uint32_t word = (f >= 4 ? cy : cx) >> (8 * (f & 3));
+    const int mv = (int)((word >> k2) & 3u);
+    pg[f] = v;
+    v -= mv;
+    k2 -= 2 * mv;
+    const bool neg = k2 < 0;  // left the byte column
+    k2 += neg ? 8 : 0;
+    n += neg ? 1 : 0;
+    const bool stop_now = neg && !stopped && (n == 2 || !have1);
+    f_next = stop_now ? f - 1 : f_next;
+    v_s = stop_now ? v : v_s;
+    k2_s = stop_now ? k2 : k2_s;
+    n_s = stop_now ? n : n_s;
+    stopped = stopped || stop_now;
+    cx = neg ? w1.x : cx;
+    cy = neg ? w1.y : cy;
+  }
+  if (stopped) { v = v_s; k2 = k2_s; n = n_s; }
+  nchg = n;
+  return stopped ? f_next : -1;
 }
-__device__ __forceinline__ void kab_bulk_wait_read0() {
-  asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-}
-__device__ __forceinline__ void kab_bulk_wait0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
 // CTC: the CTC forced-alignment recurrence (kab_common.cuh) over the whole lattice: the host sets W so
 // that the window is [0, S) in every frame, and S + 32 <= R, so no chunk is ever recycled.  Junk from
@@ -458,7 +486,7 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
             for (int i = i1 - 1; i >= i0; --i, rowp -= NBP) {
               const unsigned char byte = rowp[slot >> 2];
               pbuf[i - i0] = v;
-              const int mv = kab_decode_move((byte >> (2 * (slot & 3))) & 3u, v);
+              const int mv = kab_decode_move((byte >> (2 * (slot & 3))) & 3u);
               v -= mv;
               slot -= mv;
               if (slot < 0) slot += R;

@@ -36,7 +36,7 @@
 //     frames of the current region and the two below it is staged by bulk copies (double
 //     buffered); the other warps write the previous block's outputs.
 #pragma once
-#include "kab_band.cuh"
+#include "kab_band.cuh"  // KAB_BAND_G / GHOST / OW: the lanes of kab_band.cuh; kab_walk_group8
 #include "kab_common.cuh"
 
 #define KAB_BP_CW 4      // compute warps per CTA
@@ -62,128 +62,9 @@ __host__ __device__ inline KabBandpGeom kab_bandp_geom(int stage_bytes) {
   return g;
 }
 
-// ---------------------------------------------------------------- cluster helpers
-__device__ __forceinline__ uint32_t kab_cluster_rank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ uint32_t kab_cluster_size() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void kab_cluster_sync() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// shared::cta address -> shared::cluster address of the same variable in CTA `rank`
-__device__ __forceinline__ uint32_t kab_mapa(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void kab_st_cluster_u32(uint32_t addr, uint32_t v) {
-  asm volatile("st.shared::cluster.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
-}
-__device__ __forceinline__ void kab_red_max_cluster_s32(uint32_t addr, int v) {
-  asm volatile("red.relaxed.cluster.shared::cluster.max.s32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
-}
-__device__ __forceinline__ void kab_red_or_cluster_u32(uint32_t addr, uint32_t v) {
-  asm volatile("red.relaxed.cluster.shared::cluster.or.b32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
-}
-__device__ __forceinline__ void kab_mbar_arrive(uint64_t *bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(kab_smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool kab_mbar_try_wait_addr(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"  // non-blocking: try_wait may suspend the
-      "selp.u32 %0, 1, 0, p;\n\t}"                                     // warp for ~800 cycles (measured) when it
-      : "=r"(ok)                                                         // races with the arming arrive
-      : "r"(bar), "r"(parity)
-      : "memory");
-  return ok != 0;
-}
-__device__ __forceinline__ void kab_mbar_spin(uint64_t *bar, uint32_t parity) {  // non-blocking poll
-  const uint32_t a = kab_smem_u32(bar);
-  while (!kab_mbar_try_wait_addr(a, parity)) {
-  }
-}
-__device__ __forceinline__ void kab_bulk_wait_read1() {
-  asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-}
-
-// Global scratch of one lattice in cluster mode (zeroed before every run), at p.fifo + lat.scr_off * 4:
-// cons[nwt] (messages warp w is done with), then fifo[nwt][D][192 B]
-__host__ __device__ inline size_t kab_bandp_fifo_off(int nwt) { return ((size_t)nwt * 4 + 255) & ~(size_t)255; }
+// Bytes of the global scratch of one lattice (layout: kab_cluster_fifo_off)
 __host__ __device__ inline size_t kab_bandp_ws_bytes(int nwt) {
-  return kab_bandp_fifo_off(nwt) + (size_t)nwt * KAB_BP_D * KAB_BP_MSG_BYTES;
-}
-// (score, seq) travel as ONE 64-bit access: PTX guarantees single-copy atomicity for a naturally
-// aligned .b64 access, not for a .v2.b32 vector (which the memory model treats as two accesses).
-__device__ __forceinline__ void kab_st_volatile_b64(void *p, uint32_t lo, uint32_t hi) {
-  asm volatile(
-      "{\n\t.reg .b64 q;\n\t"
-      "mov.b64 q, {%1, %2};\n\t"
-      "st.relaxed.gpu.global.b64 [%0], q;\n\t}" ::"l"(p), "r"(lo), "r"(hi)
-      : "memory");
-}
-__device__ __forceinline__ uint2 kab_ld_volatile_b64(const void *p) {
-  uint2 v;
-  asm volatile(
-      "{\n\t.reg .b64 q;\n\t"
-      "ld.relaxed.gpu.global.b64 q, [%2];\n\t"
-      "mov.b64 {%0, %1}, q;\n\t}"
-      : "=r"(v.x), "=r"(v.y)
-      : "l"(p)
-      : "memory");
-  return v;
-}
-__device__ __forceinline__ uint32_t kab_ld_volatile_u32(const void *p) {
-  uint32_t v;
-  asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void kab_st_volatile_u32(void *p, uint32_t v) {
-  asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-
-// Backtrack of ONE full group (8 frames, descending) from registers: w0 holds the 8 backpointer
-// bytes of the walker's byte column, w1 those of the column below (have1: it is available).
-// No load sits on the dependent chain (shift -> mask -> subtract -> compare).  Stops before the
-// frame that would need a third column; returns the next frame to process (-1: group done) and
-// the number of column steps taken (0..2, the last one not yet served when it stopped early).
-__device__ __forceinline__ int kab_walk_group8(const uint2 w0, const uint2 w1, const bool have1, int &v, int &k2,
-                                               int *pg, int &nchg) {
-  // Branch-free on purpose (selects only): with one active thread every taken branch costs a
-  // convergence-barrier round trip (~40 cycles, measured), several times the chain itself.  Frames
-  // after the stop point are computed and discarded (the caller overwrites their path entries).
-  uint32_t cx = w0.x, cy = w0.y;
-  int n = 0, f_next = -1, v_s = 0, k2_s = 0, n_s = 0;
-  bool stopped = false;
-#pragma unroll
-  for (int f = 7; f >= 0; --f) {
-    const uint32_t word = (f >= 4 ? cy : cx) >> (8 * (f & 3));
-    const int mv = (int)((word >> k2) & 3u);
-    pg[f] = v;
-    v -= mv;
-    k2 -= 2 * mv;
-    const bool neg = k2 < 0;  // left the byte column
-    k2 += neg ? 8 : 0;
-    n += neg ? 1 : 0;
-    const bool stop_now = neg && !stopped && (n == 2 || !have1);
-    f_next = stop_now ? f - 1 : f_next;
-    v_s = stop_now ? v : v_s;
-    k2_s = stop_now ? k2 : k2_s;
-    n_s = stop_now ? n : n_s;
-    stopped = stopped || stop_now;
-    cx = neg ? w1.x : cx;
-    cy = neg ? w1.y : cy;
-  }
-  if (stopped) { v = v_s; k2 = k2_s; n = n_s; }
-  nchg = n;
-  return stopped ? f_next : -1;
+  return kab_cluster_fifo_off(nwt) + (size_t)nwt * KAB_BP_D * KAB_BP_MSG_BYTES;
 }
 
 #ifdef KAB_BANDP_TIMING
@@ -371,7 +252,7 @@ __global__ void __launch_bounds__(KAB_BP_THREADS, 1)
       // neighbour FIFO in global memory: my inbox (messages of warp pgw) and the inbox of warp ngw
       unsigned char *gws = p.fifo + (size_t)lat.scr_off * 4;
       unsigned int *cons = reinterpret_cast<unsigned int *>(gws);
-      unsigned char *gfifo = gws + kab_bandp_fifo_off(NWT);
+      unsigned char *gfifo = gws + kab_cluster_fifo_off(NWT);
       const unsigned char *inbox = gfifo + (size_t)gw * D * KAB_BP_MSG_BYTES + (lane < GH ? lane : 0) * 32;
       unsigned char *outbox = gfifo + (size_t)ngw * D * KAB_BP_MSG_BYTES + (lane >= 32 - GH ? lane - (32 - GH) : 0) * 32;
       uint32_t cons_seen = 0;      // messages the warp above is known to be done with

@@ -27,13 +27,10 @@
 // written with bulk stores.  The traceback is always the parallel map composition of
 // kab_btpar.cuh (KabBtLayoutQ); this kernel publishes the forced end state.
 #pragma once
-#include "kab_band.cuh"
-#include "kab_bandp.cuh"
+#include "kab_band.cuh"  // KAB_BAND_G: frames per group
 #include "kab_common.cuh"
 
-#ifndef KAB_BQ_CW
 #define KAB_BQ_CW 8      // compute warps per CTA
-#endif
 #define KAB_BQ_GH 12     // ghost lanes per warp = 3 * G / 2
 #define KAB_BQ_OW 40     // ring slots owned by a warp = (32 - GH) * 2
 #define KAB_BQ_NS 48     // emission stages per CTA.  The ring of 8 * NC warps is a CHAIN in time: every warp trails its
@@ -56,11 +53,9 @@ __host__ __device__ inline KabBandqGeom kab_bandq_geom(int stage_bytes) {
   g.smem_bytes = g.stage_off + (size_t)KAB_BQ_NS * stage_bytes;
   return g;
 }
-// Global scratch of one lattice (zeroed before every run), at p.fifo + lat.scr_off * 4:
-// cons[nwt] (messages warp w is done with), then fifo[nwt][D][192 B]
-__host__ __device__ inline size_t kab_bandq_fifo_off(int nwt) { return ((size_t)nwt * 4 + 255) & ~(size_t)255; }
+// Bytes of the global scratch of one lattice (layout: kab_cluster_fifo_off)
 __host__ __device__ inline size_t kab_bandq_ws_bytes(int nwt) {
-  return kab_bandq_fifo_off(nwt) + (size_t)nwt * KAB_BQ_D * KAB_BQ_MSG_BYTES;
+  return kab_cluster_fifo_off(nwt) + (size_t)nwt * KAB_BQ_D * KAB_BQ_MSG_BYTES;
 }
 
 #ifdef KAB_BANDQ_TIMING
@@ -230,7 +225,7 @@ __global__ void __launch_bounds__(KAB_BQ_THREADS, 1)
       // neighbour FIFO in global memory: my inbox (messages of the warp below) and the inbox of warp ngw
       unsigned char *gws = p.fifo + (size_t)lat.scr_off * 4;
       unsigned int *cons = reinterpret_cast<unsigned int *>(gws);
-      unsigned char *gfifo = gws + kab_bandq_fifo_off(NWT);
+      unsigned char *gfifo = gws + kab_cluster_fifo_off(NWT);
       const unsigned char *inbox = gfifo + (size_t)gw * D * KAB_BQ_MSG_BYTES + (lane < GH ? lane : 0) * 16;
       unsigned char *outbox = gfifo + (size_t)ngw * D * KAB_BQ_MSG_BYTES + (lane >= 32 - GH ? lane - (32 - GH) : 0) * 16;
       uint32_t cons_seen = 0;   // messages the warp above is known to be done with

@@ -35,36 +35,24 @@
 // GA (template parameter): gather mode for wide vocabularies -- the prep warps read the emissions
 // from global memory, the producer warp prefetches the rows into L2.
 #pragma once
-#include "kab_band.cuh"
-#include "kab_bandp.cuh"
-#include "kab_bandq.cuh"
+#include "kab_band.cuh"   // KAB_BAND_G: frames per group
+#include "kab_bandq.cuh"  // KAB_BQ_GH / KAB_BQ_OW: the lanes of kab_bandq.cuh
 #include "kab_common.cuh"
 
-#ifndef KAB_BR_EXP_FRAMES
-#define KAB_BR_EXP_FRAMES 8   // what-if builds only: frames executed per group (results are wrong below 8)
-#endif
-#ifndef KAB_BR_CW
 #define KAB_BR_CW 4           // compute warps per CTA (and as many prep warps): ONE compute warp per scheduler.  The
                               // SM sub-partition issues ~1 instruction per cycle and a warp at most every other
                               // cycle; with two compute + two prep warps per scheduler the compute warps got a
                               // quarter of the slots each (measured: 940 cycles for the 230 instructions of a group)
-#endif
 #define KAB_BR_GH KAB_BQ_GH   // ghost lanes
 #define KAB_BR_OW KAB_BQ_OW   // owned ring slots per warp
-#ifndef KAB_BR_NS
 #define KAB_BR_NS 40          // emission stages per CTA (head and tail of the chain can sit in one CTA)
-#endif
 #define KAB_BR_F 16           // frames per emission stage this kernel is built for (two groups; the plan checks it)
 #define KAB_BR_TD 8           // emission tiles per compute warp (groups the prep warps may run ahead)
 #define KAB_BR_MD 16          // mailbox depth (messages)
 #define KAB_BR_GA_AHEAD 12    // gather mode: chunks (of 16 frames) the L2 prefetch runs ahead of the producer
 #define KAB_BR_BG 16          // groups per backpointer block (2 KB)
 #define KAB_BR_NBB 4          // backpointer staging buffers per compute warp
-#ifdef KAB_BR_ISOLATE          // experiment: 2 compute warps alone on schedulers 0 and 1, the helpers on 2 and 3
-#define KAB_BR_THREADS (12 * 32)
-#else
 #define KAB_BR_THREADS ((3 * KAB_BR_CW + 1) * 32)
-#endif
 
 struct KabBandrGeom {
   size_t ctrl_off, tile_off, mbox_off, bp_off, vbf_off, wtab_off, stage_off, smem_bytes;
@@ -92,46 +80,6 @@ __host__ __device__ inline KabBandrGeom kab_bandr_geom(int stage_bytes) {
 #define KAB_BR_C_UPDONE 19    // last warp of a CTA: copy of the COMPDONE word of the warp above, which lives in the
                               // next CTA and PUSHES its progress here (a remote load per group stalled this warp
                               // for ~1 200 cycles and made it the slowest link of the chain)
-
-__device__ __forceinline__ uint32_t kab_lds_relaxed_u32(uint32_t addr) {
-  uint32_t v;
-  asm volatile("ld.relaxed.cluster.shared::cta.u32 %0, [%1];" : "=r"(v) : "r"(addr) : "memory");
-  return v;
-}
-__device__ __forceinline__ void kab_sts_relaxed_u32(uint32_t addr, uint32_t v) {
-  asm volatile("st.relaxed.cluster.shared::cta.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
-}
-__device__ __forceinline__ uint2 kab_lds_relaxed_b64(uint32_t addr) {
-  uint2 v;
-  asm volatile(
-      "{\n\t.reg .b64 q;\n\t"
-      "ld.relaxed.cluster.shared::cta.b64 q, [%2];\n\t"
-      "mov.b64 {%0, %1}, q;\n\t}"
-      : "=r"(v.x), "=r"(v.y)
-      : "r"(addr)
-      : "memory");
-  return v;
-}
-// (score, seq) as ONE 64-bit store into the shared memory of any CTA of the cluster (addr from mapa)
-__device__ __forceinline__ void kab_st_cluster_b64(uint32_t addr, uint32_t lo, uint32_t hi) {
-  asm volatile(
-      "{\n\t.reg .b64 q;\n\t"
-      "mov.b64 q, {%1, %2};\n\t"
-      "st.relaxed.cluster.shared::cluster.b64 [%0], q;\n\t}" ::"r"(addr), "r"(lo), "r"(hi)
-      : "memory");
-}
-__device__ __forceinline__ void kab_sts_b64(uint32_t addr, uint32_t lo, uint32_t hi) {  // own CTA: a plain STS.64
-  asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(addr), "r"(lo), "r"(hi) : "memory");
-}
-__device__ __forceinline__ uint32_t kab_ld_cluster_u32(uint32_t addr) {
-  uint32_t v;
-  asm volatile("ld.relaxed.cluster.shared::cluster.u32 %0, [%1];" : "=r"(v) : "r"(addr) : "memory");
-  return v;
-}
-__device__ __forceinline__ void kab_fence_cta() { asm volatile("fence.acq_rel.cta;" ::: "memory"); }
-__device__ __forceinline__ void kab_mbar_arrive_addr(uint32_t bar) {  // (32-bit shared address: no conversion per call)
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
 
 #ifdef KAB_BANDR_TIMING
 #define KAB_RTM(var) const long long var = clock64()
@@ -170,27 +118,9 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
   // ids and the helpers, which poll while they wait, the low ones: warp 0 producer, 1 .. 2 CW prep
   // (two per compute warp: one builds the tiles of the even groups, the other those of the odd
   // ones), 2 CW + 1 .. 3 CW compute -- one compute warp and two prep warps per scheduler.
-#ifdef KAB_BR_EXP_PRODLAST
-  // experiment: the producer is warp 1 (scheduler 1), warp 0 takes the prep role warp 1 had
-  const int vw = warp == 1 ? 0 : (warp == 0 ? 1 : warp);   // virtual warp id with the standard roles
-  const bool is_prod = vw == 0, is_prep = vw >= 1 && vw <= 2 * CW;
-  const int pp = is_prep ? (vw - 1) & 1 : 0;
-  const int cw = is_prep ? (vw - 1) >> 1 : (vw > 2 * CW ? vw - 1 - 2 * CW : 0);
-#elif defined(KAB_BR_ISOLATE)
-  static_assert(CW == 2, "isolated layout: two compute warps");
-  // ids 8, 9 compute (schedulers 0, 1, alone); 2, 3 / 6, 7 prep; 10 producer; 0, 1, 4, 5, 11 idle at the barriers
-  const bool is_prod = warp == 10, is_prep = warp == 2 || warp == 3 || warp == 6 || warp == 7;
-  const bool is_idle = warp == 0 || warp == 1 || warp == 4 || warp == 5 || warp == 11;
-  const int pp = is_prep ? (warp >> 2) : 0;
-  const int cw = is_prep ? (warp & 1) : (warp == 9 ? 1 : 0);
-#else
   const bool is_prod = warp == 0, is_prep = warp >= 1 && warp <= 2 * CW;
   const int pp = is_prep ? (warp - 1) & 1 : 0;                                        // parity a prep warp builds
   const int cw = is_prep ? (warp - 1) >> 1 : (warp > 2 * CW ? warp - 1 - 2 * CW : 0);  // the compute warp this warp is / serves
-#endif
-#ifndef KAB_BR_ISOLATE
-  constexpr bool is_idle = false;
-#endif
   const int gw = (int)rank * CW + cw;         // its global index in the ring
   const bool owned = lane >= GH;
   // ring slot of this lane's blank state: owned lanes tile the warp's 40 slots, ghost lanes mirror
@@ -260,9 +190,7 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
       const int wqF = (int)(((long long)S * F) / T), wrF = (int)(((long long)S * F) % T);
       for (int c = 0; c < n_chunks; ++c) {
         const uint32_t gc = ec0 + (uint32_t)c, stg = gc % NS, use = gc / NS;
-#ifndef KAB_BR_EXP_NOSTAGE
         if (use > 0) kab_mbar_wait(&eempty[stg], (use - 1u) & 1u);  // all prep warps released it
-#endif
         float *dst = stage_base + stg * stage_words;
         // the window of align.py:64 for the frames of this chunk (and the first frame behind it): lo_i =
         // max(0, S*i // T - W // 2) -- here, where nobody waits for it, instead of an incremental
@@ -405,16 +333,8 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
           }
           if (!own) continue;
           const int hi0 = min(lo0 + W, S);
-#ifdef KAB_BR_EXP_ALLSAFE
-          const bool safe = nfr == G;
-#else
           const bool safe = __all_sync(KAB_FULL_MASK, nfr == G && vb >= lo1 && vb + 2 <= hi0);
-#endif
           float2 *tile = reinterpret_cast<float2 *>(kab_smem + geo.tile_off + (size_t)cw * (TD * 2048) + (size_t)t * 2048) + lane;
-#ifdef KAB_BR_EXP_NOTILE
-          if (true) {
-          } else
-#endif
           if (safe) {
 #pragma unroll
             for (int f = 0; f < G; ++f)
@@ -463,7 +383,7 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
         while (bp_issued < n_blocks) service_bp();
         if (lane == 0) kab_bulk_wait0();  // the compute warp's backpointer blocks are in global memory
       }
-    } else if (!is_idle) {
+    } else {
       // ================= compute warp: the recurrence
       // Nothing here waits on a fence: every hand-over is a word that carries its own sequence
       // number, polled in shared memory (the LSU of an SM executes a warp's shared-memory accesses in
@@ -498,11 +418,7 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
       // (st.shared::cluster compiles to a generic ST through the shared window -- hundreds of cycles even
       // when the target is this CTA -- so the seven links inside a CTA use plain STS / LDS)
       const uint32_t up_lane_off = (uint32_t)(lane >= 32 - GH ? lane - (32 - GH) : 0) * 16u;
-#ifdef KAB_BR_EXP_ALLREMOTE
-      const uint32_t up_mbox = kab_mapa(up_mbox_local, up_rank) + up_lane_off;
-#else
       const uint32_t up_mbox = (remote_up ? kab_mapa(up_mbox_local, up_rank) : up_mbox_local) + up_lane_off;
-#endif
       const uint32_t up_done = remote_up ? ctrl + 4 * KAB_BR_C_UPDONE : up_ctrl_local + 4 * KAB_BR_C_COMPDONE;
       auto read_up_done = [&]() { return kab_lds_relaxed_u32(up_done); };
       // first warp of a CTA: its progress also goes to the warp below, in the previous CTA of the cluster
@@ -510,11 +426,7 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
       const uint32_t down_done = kab_mapa(smem0 + (uint32_t)geo.ctrl_off + (uint32_t)(CW - 1) * 128u + 4 * KAB_BR_C_UPDONE,
                                           rank == 0 ? NC - 1 : rank - 1);
       auto publish = [&](uint32_t slot, uint32_t seq) {  // lanes 20..31: the two (score, seq) words of message seq - 1
-#ifdef KAB_BR_EXP_ALLREMOTE
-        if (true) {
-#else
         if (remote_up) {
-#endif
           kab_st_cluster_b64(slot, __float_as_uint(s0), seq);
           kab_st_cluster_b64(slot + 8, __float_as_uint(s1), seq);
         } else {
@@ -560,9 +472,6 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
         pf0 = kab_lds_relaxed_b64(nslot);
         pf1 = kab_lds_relaxed_b64(nslot + 8);
       };
-#ifdef KAB_BANDR_TOTAL
-      const long long tot0 = clock64();
-#endif
       for (int g = 0; g < n_groups;) {
         // ---- COMMON PATH: two groups (one emission chunk) per pass -- all of them but the first two,
         // the last ones and the rare wait for mailbox room.  Straight-line code: a lone warp pays ~15
@@ -581,11 +490,7 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
           KAB_RTM(fa);
           // the chunk's second tile word (published last) carries both need flags
           while ((tw & 0x3fffffffu) != (uint32_t)g + 2u) tw = kab_lds_relaxed_u32(ctrl + 4 * (KAB_BR_C_TILESEQ + t + 1));
-#ifdef KAB_BR_EXP_NOMSG
-          const bool need0 = false, need1 = false;
-#else
           const bool need0 = (tw & 0x40000000u) != 0u, need1 = (tw >> 31) != 0u;
-#endif
           const uint32_t tl = tiles_lane + (uint32_t)t * 2048u;
           float2 e[G], e2[G];
 #pragma unroll
@@ -602,7 +507,7 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
           bw = 0;
           KAB_RTM(ff0);
 #pragma unroll
-          for (int f = 0; f < KAB_BR_EXP_FRAMES; ++f) frame(e[f].x, e[f].y, 4 * f);
+          for (int f = 0; f < G; ++f) frame(e[f].x, e[f].y, 4 * f);
           KAB_RTM(ff1);
           // message g at once: the warp above is waiting for it
           asm volatile(
@@ -623,7 +528,7 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
           KAB_RTM(fx1);
           bw = 0;
 #pragma unroll
-          for (int f = 0; f < KAB_BR_EXP_FRAMES; ++f) frame(e2[f].x, e2[f].y, 4 * f);
+          for (int f = 0; f < G; ++f) frame(e2[f].x, e2[f].y, 4 * f);
           KAB_RTM(fx2);
           // message g + 1, then: both groups are finished, their tiles have been read (the prep warps
           // may reuse the slots), progress for the warp below
@@ -787,9 +692,6 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
         KAB_RTM_ADD(tm_bp, te, tf);
         }
       }
-#ifdef KAB_BANDR_TOTAL
-      if (lane == 0 && (gw & 3) == 0) printf("warp %2d: %lld cycles per group (compute loop, %d groups)\n", gw, (clock64() - tot0) / n_groups, n_groups);
-#endif
 #ifdef KAB_BANDR_TIMING
       if (lane == 0 && p.debug) {
         long long *d = p.debug + gw * 16;
@@ -818,7 +720,7 @@ __global__ void __launch_bounds__(KAB_BR_THREADS, 1)
 
     const int v = *s_vmax;
     const int status = *s_bad ? 3 : (v < 0 ? 1 : 0);
-    if (!is_prod && !is_prep && !is_idle && owned && status == 0 && p.final_score) {  // (compute warps)
+    if (!is_prod && !is_prep && owned && status == 0 && p.final_score) {  // (compute warps)
       if (vb + 0 == v) p.final_score[lat.index] = s0;
       if (vb + 1 == v) p.final_score[lat.index] = s1;
     }

@@ -30,8 +30,8 @@
 //     bp[((reg * n_groups + t / 8) * 32 + 12 + (slot % 40) / 2) * 4],   reg = slot / 40,
 //     move = (word >> (4 * (t % 8) + 2 * (slot & 1))) & 3.
 #pragma once
-#include "kab_band.cuh"
-#include "kab_bandq.cuh"
+#include "kab_band.cuh"   // KAB_BAND_OW: KabBtLayoutP
+#include "kab_bandq.cuh"  // KAB_BQ_GH / KAB_BQ_OW: KabBtLayoutQ
 #include "kab_common.cuh"
 
 struct KabBtLayoutP {

@@ -108,10 +108,13 @@ __device__ __forceinline__ float kab_ctc_label_sel(float x0, float x1, float x2,
   return p2 ? x2 : (p1 ? x1 : x0);
 }
 
-// ---------------------------------------------------------------- mbarrier + 1-D bulk copy (TMA)
+// ---------------------------------------------------------------- inline-PTX memory and synchronisation wrappers
+// (mbarriers, 1-D bulk copies, fences, clusters / distributed shared memory, relaxed accesses)
 __device__ __forceinline__ uint32_t kab_smem_u32(const void *p) {
   return (uint32_t)__cvta_generic_to_shared(p);
 }
+
+// ---- mbarriers
 __device__ __forceinline__ void kab_mbar_init(uint64_t *bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(kab_smem_u32(bar)), "r"(count) : "memory");
 }
@@ -122,6 +125,12 @@ __device__ __forceinline__ void kab_mbar_expect_tx(uint64_t *bar, uint32_t bytes
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(kab_smem_u32(bar)), "r"(bytes)
                : "memory");
 }
+__device__ __forceinline__ void kab_mbar_arrive(uint64_t *bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(kab_smem_u32(bar)) : "memory");
+}
+// Two ways to wait for a phase: try_wait may suspend the warp (kab_mbar_wait), test_wait never does
+// (kab_mbar_spin: try_wait may suspend the warp for ~800 cycles (measured) when it races with the
+// arming arrive).
 __device__ __forceinline__ bool kab_mbar_try_wait(uint64_t *bar, uint32_t parity) {
   uint32_t ok;
   asm volatile(
@@ -137,16 +146,30 @@ __device__ __forceinline__ void kab_mbar_wait(uint64_t *bar, uint32_t parity) {
   while (!kab_mbar_try_wait(bar, parity)) {
   }
 }
+__device__ __forceinline__ bool kab_mbar_test_wait(uint32_t bar, uint32_t parity) {
+  uint32_t ok;
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
+      "selp.u32 %0, 1, 0, p;\n\t}"
+      : "=r"(ok)
+      : "r"(bar), "r"(parity)
+      : "memory");
+  return ok != 0;
+}
+__device__ __forceinline__ void kab_mbar_spin(uint64_t *bar, uint32_t parity) {
+  const uint32_t a = kab_smem_u32(bar);
+  while (!kab_mbar_test_wait(a, parity)) {
+  }
+}
+
+// ---- 1-D bulk copies (TMA)
 // global -> shared bulk copy; completion is signalled on `bar` (complete_tx::bytes).
 __device__ __forceinline__ void kab_bulk_g2s(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
                    kab_smem_u32(dst)),
                "l"(src), "r"(bytes), "r"(kab_smem_u32(bar))
                : "memory");
-}
-// Bulk prefetch of a global range into L2 (no destination): address 16-byte aligned, size a multiple of 16.
-__device__ __forceinline__ void kab_bulk_prefetch_l2(const void *src, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
 }
 // Same, with an L2 eviction-priority hint (createpolicy); the warp kernel passes evict_normal.
 __device__ __forceinline__ void kab_bulk_g2s_hint(void *dst, const void *src, uint32_t bytes, uint64_t *bar,
@@ -157,10 +180,127 @@ __device__ __forceinline__ void kab_bulk_g2s_hint(void *dst, const void *src, ui
       "l"(src), "r"(bytes), "r"(kab_smem_u32(bar)), "l"(policy)
       : "memory");
 }
+// Bulk prefetch of a global range into L2 (no destination): address 16-byte aligned, size a multiple of 16.
+__device__ __forceinline__ void kab_bulk_prefetch_l2(const void *src, uint32_t bytes) {
+  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
+}
+// shared -> global bulk copy, committed as its own bulk group
+__device__ __forceinline__ void kab_bulk_s2g(void *dst, const void *src, uint32_t bytes) {
+  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(kab_smem_u32(src)),
+               "r"(bytes)
+               : "memory");
+  asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+}
+// wait until at most 0 / 1 bulk groups still read their source; until all bulk groups are complete
+__device__ __forceinline__ void kab_bulk_wait_read0() {
+  asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+}
+__device__ __forceinline__ void kab_bulk_wait_read1() {
+  asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+}
+__device__ __forceinline__ void kab_bulk_wait0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+
+// ---- fences
 __device__ __forceinline__ void kab_fence_proxy_async() { asm volatile("fence.proxy.async;" ::: "memory"); }
 // shared-memory-only form: SASS FENCE.VIEW.ASYNC.S without the MEMBAR.ALL.GPU of the generic one
 __device__ __forceinline__ void kab_fence_proxy_async_smem() {
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+}
+__device__ __forceinline__ void kab_fence_cta() { asm volatile("fence.acq_rel.cta;" ::: "memory"); }
+
+// ---- clusters and distributed shared memory
+__device__ __forceinline__ uint32_t kab_cluster_rank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+__device__ __forceinline__ uint32_t kab_cluster_size() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(r));
+  return r;
+}
+__device__ __forceinline__ void kab_cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// shared::cta address -> shared::cluster address of the same variable in CTA `rank`
+__device__ __forceinline__ uint32_t kab_mapa(uint32_t addr, uint32_t rank) {
+  uint32_t r;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
+  return r;
+}
+__device__ __forceinline__ void kab_st_cluster_u32(uint32_t addr, uint32_t v) {
+  asm volatile("st.shared::cluster.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
+}
+// (score, seq) as ONE 64-bit store into the shared memory of any CTA of the cluster (addr from mapa)
+__device__ __forceinline__ void kab_st_cluster_b64(uint32_t addr, uint32_t lo, uint32_t hi) {
+  asm volatile(
+      "{\n\t.reg .b64 q;\n\t"
+      "mov.b64 q, {%1, %2};\n\t"
+      "st.relaxed.cluster.shared::cluster.b64 [%0], q;\n\t}" ::"r"(addr), "r"(lo), "r"(hi)
+      : "memory");
+}
+__device__ __forceinline__ void kab_red_max_cluster_s32(uint32_t addr, int v) {
+  asm volatile("red.relaxed.cluster.shared::cluster.max.s32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
+}
+__device__ __forceinline__ void kab_red_or_cluster_u32(uint32_t addr, uint32_t v) {
+  asm volatile("red.relaxed.cluster.shared::cluster.or.b32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
+}
+// Global scratch of one lattice of the cluster band kernels kab_bandp / kab_bandq (zeroed before every
+// run), at p.fifo + lat.scr_off * 4: cons[nwt] (messages warp w is done with), then fifo[nwt][D][192 B]
+__host__ __device__ inline size_t kab_cluster_fifo_off(int nwt) { return ((size_t)nwt * 4 + 255) & ~(size_t)255; }
+
+// ---- relaxed accesses
+// Global memory, .gpu scope.  (score, seq) travel as ONE 64-bit access: PTX guarantees single-copy
+// atomicity for a naturally aligned .b64 access, not for a .v2.b32 vector (which the memory model
+// treats as two accesses).
+__device__ __forceinline__ void kab_st_volatile_b64(void *p, uint32_t lo, uint32_t hi) {
+  asm volatile(
+      "{\n\t.reg .b64 q;\n\t"
+      "mov.b64 q, {%1, %2};\n\t"
+      "st.relaxed.gpu.global.b64 [%0], q;\n\t}" ::"l"(p), "r"(lo), "r"(hi)
+      : "memory");
+}
+__device__ __forceinline__ uint2 kab_ld_volatile_b64(const void *p) {
+  uint2 v;
+  asm volatile(
+      "{\n\t.reg .b64 q;\n\t"
+      "ld.relaxed.gpu.global.b64 q, [%2];\n\t"
+      "mov.b64 {%0, %1}, q;\n\t}"
+      : "=r"(v.x), "=r"(v.y)
+      : "l"(p)
+      : "memory");
+  return v;
+}
+__device__ __forceinline__ uint32_t kab_ld_volatile_u32(const void *p) {
+  uint32_t v;
+  asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void kab_st_volatile_u32(void *p, uint32_t v) {
+  asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+// The own CTA's shared memory (32-bit shared::cta addresses), .cluster scope.
+__device__ __forceinline__ uint32_t kab_lds_relaxed_u32(uint32_t addr) {
+  uint32_t v;
+  asm volatile("ld.relaxed.cluster.shared::cta.u32 %0, [%1];" : "=r"(v) : "r"(addr) : "memory");
+  return v;
+}
+__device__ __forceinline__ void kab_sts_relaxed_u32(uint32_t addr, uint32_t v) {
+  asm volatile("st.relaxed.cluster.shared::cta.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
+}
+__device__ __forceinline__ uint2 kab_lds_relaxed_b64(uint32_t addr) {
+  uint2 v;
+  asm volatile(
+      "{\n\t.reg .b64 q;\n\t"
+      "ld.relaxed.cluster.shared::cta.b64 q, [%2];\n\t"
+      "mov.b64 {%0, %1}, q;\n\t}"
+      : "=r"(v.x), "=r"(v.y)
+      : "r"(addr)
+      : "memory");
+  return v;
+}
+__device__ __forceinline__ void kab_sts_b64(uint32_t addr, uint32_t lo, uint32_t hi) {  // own CTA: a plain STS.64
+  asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(addr), "r"(lo), "r"(hi) : "memory");
 }
 
 // ---------------------------------------------------------------- emission staging
@@ -262,20 +402,11 @@ __device__ __forceinline__ float kab_max3(float a, float b, float c) {
 // both pipes issue at half rate on sm_100 -- this keeps them balanced.  The bits touched by one
 // frame are disjoint, so the adds never carry.
 // Backpointer codes: a label state stores its move (0..3); a blank state stores 0, 1 or 3 (bit 0 =
-// move != 0, bit 1 = move 3), so the 2-bit code is the move for both.  (The KAB_SEL_V1 selects set
-// blank bit 1 alone for move 3: there code >= 2 decodes to 3.)
-__device__ __forceinline__ int kab_decode_move(uint32_t code, int v) {
-#ifndef KAB_SEL_V1
-  (void)v;
-  return (int)code;
-#else
-  return ((v & 1) == 0 && code >= 2u) ? 3 : (int)code;
-#endif
-}
+// move != 0, bit 1 = move 3), so the 2-bit code is the move for both.
+__device__ __forceinline__ int kab_decode_move(uint32_t code) { return (int)code; }
 __device__ __forceinline__ float kab_blank_sel(float a0, float a1, float a3, uint32_t &w, const uint32_t bit1,
                                                const uint32_t bit2, const uint32_t one) {
   float best;
-#ifndef KAB_SEL_V1
   // The first maximum is the smallest move whose candidate EQUALS the 3-input maximum (FMNMX3):
   // bit 0 = (move != 0), bit 1 = (move != 0 and move != 1), i.e. codes 0, 1, 3.
   asm("{\n\t"
@@ -288,20 +419,6 @@ __device__ __forceinline__ float kab_blank_sel(float a0, float a1, float a3, uin
       "}"
       : "=f"(best), "+r"(w)
       : "f"(a0), "f"(a1), "f"(a3), "r"(bit1), "r"(bit2), "r"(one));
-#else
-  asm("{\n\t"
-      ".reg .f32 m;\n\t"
-      ".reg .pred p1, p3;\n\t"
-      "max.f32 m, %2, %3;\n\t"
-      "setp.gt.f32 p1, %3, %2;\n\t"
-      "setp.gt.f32 p3, %4, m;\n\t"
-      "max.f32 %0, m, %4;\n\t"
-      "@p1 mad.lo.u32 %1, %7, %5, %1;\n\t"   // code bit 0: move 1 beat move 0
-      "@p3 mad.lo.u32 %1, %7, %6, %1;\n\t"   // code bit 1: move 3 beat both (bit 0 is then don't-care)
-      "}"
-      : "=f"(best), "+r"(w)
-      : "f"(a0), "f"(a1), "f"(a3), "r"(bit1), "r"(bit2), "r"(one));
-#endif
   return best;
 }
 // Label state: candidates a0..a3; tournament form of the ascending strict-'>' scan: the winner
@@ -309,7 +426,6 @@ __device__ __forceinline__ float kab_blank_sel(float a0, float a1, float a3, uin
 __device__ __forceinline__ float kab_label_sel(float a0, float a1, float a2, float a3, uint32_t &w,
                                                const uint32_t bit1, const uint32_t bit2, const uint32_t one) {
   float best;
-#ifndef KAB_SEL_V1
   // m01 = max(a0, a1); best = max3(m01, a2, a3); the upper pair won iff best != m01 (strictly
   // greater); the odd candidate of the winning pair won iff its even candidate != best.
   asm("{\n\t"
@@ -325,21 +441,5 @@ __device__ __forceinline__ float kab_label_sel(float a0, float a1, float a2, flo
       "}"
       : "=f"(best), "+r"(w)
       : "f"(a0), "f"(a1), "f"(a2), "f"(a3), "r"(bit1), "r"(bit2), "r"(one));
-#else
-  asm("{\n\t"
-      ".reg .f32 m01, m23, z;\n\t"
-      ".reg .pred ph, pl;\n\t"
-      "max.f32 m01, %2, %3;\n\t"
-      "max.f32 m23, %4, %5;\n\t"
-      "setp.gt.f32 ph, m23, m01;\n\t"
-      "selp.f32 %0, m23, m01, ph;\n\t"
-      "selp.f32 z, %4, %2, ph;\n\t"    // even candidate of the winning pair
-      "setp.gt.f32 pl, %0, z;\n\t"     // low bit: the odd candidate won its pair strictly
-      "@pl mad.lo.u32 %1, %8, %6, %1;\n\t"
-      "@ph mad.lo.u32 %1, %8, %7, %1;\n\t"     // high bit = ph
-      "}"
-      : "=f"(best), "+r"(w)
-      : "f"(a0), "f"(a1), "f"(a2), "f"(a3), "r"(bit1), "r"(bit2), "r"(one));
-#endif
   return best;
 }

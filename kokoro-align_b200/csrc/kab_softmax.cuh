@@ -18,8 +18,6 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include "kab_band.cuh"    // kab_bulk_s2g
-#include "kab_bandp.cuh"   // kab_bulk_wait_read1
 #include "kab_common.cuh"  // mbarrier + bulk-copy helpers
 
 #define KAB_SM_ROWS 256     // rows per tile = threads per CTA

@@ -27,11 +27,15 @@
 //     like kab_bandp.cuh (blocks of 128 frames of the current warp region and the two below it
 //     by bulk copies) while the other CTAs are already running the next lattice.
 #pragma once
-#include "kab_bandp.cuh"
+#include "kab_band.cuh"  // KAB_BAND_G / GHOST / OW: the lanes of kab_band.cuh; kab_walk_group8
+#include "kab_common.cuh"
 
-#ifdef KAB_WIDE_TIMING
-#undef KAB_TM
-#define KAB_TM(var) const long long var = clock64()
+// Group timestamps of the KAB_WIDE_TIMING build.  The KAB_BANDP_TIMING build takes them as well (the
+// two kernels shared one timing macro), so that build keeps compiling this kernel as it always did.
+#if defined(KAB_WIDE_TIMING) || defined(KAB_BANDP_TIMING)
+#define KAB_WTM(var) const long long var = clock64()
+#else
+#define KAB_WTM(var)
 #endif
 
 #define KAB_WD_CW 4      // compute warps per CTA
@@ -274,7 +278,7 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
         for (int g = 0; g < n_groups; ++g) {
           const int i0 = g * G, nfr = min(G, T - i0);
           const bool more = i0 + G < T;
-          KAB_TM(ta);
+          KAB_WTM(ta);
           // ---- ghost lanes: message g-1 of the warp below (its top 24 states after its group g-1)
           if (g > 0 && !owned) {
             if (has_below) {
@@ -305,12 +309,12 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
             pf2 = kab_ld_volatile_b64(slot + 16);
             pf3 = kab_ld_volatile_b64(slot + 24);
           }
-          KAB_TM(tb);
+          KAB_WTM(tb);
           const bool next_crosses = fic + G == F;
           const uint32_t nst = st + 1 == NS ? 0 : st + 1;
           const uint32_t nph = nst == 0 ? ph ^ 1u : ph;
           if (next_crosses && more) kab_mbar_spin(&efull[nst], nph);
-          KAB_TM(tc);
+          KAB_WTM(tc);
           const char *rowng = next_crosses ? chunk_ptr(nst) : rowc + G * VB;
           if (more) load_group(rowng, nb, n1, n3);
           uint32_t wlo = 0, whi = 0;
@@ -328,7 +332,7 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
                 else frame(eb[f], e1[f], e3[f], f < 4 ? wlo : whi, 8 * (f & 3));
               }
           }
-          KAB_TM(td);
+          KAB_WTM(td);
           // ---- message g for the warp above: (score, seq) pairs, one 8-byte store each
           if (more && has_above) {
             if (g >= D && (uint32_t)(g - D) >= cons_seen) {  // about to lap the consumer: read its progress
@@ -345,7 +349,7 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
               kab_st_volatile_b64(slot + 24, __float_as_uint(s3), seq);
             }
           }
-          KAB_TM(te);
+          KAB_WTM(te);
           // ---- backpointer word of this group -> staging; block finished?
           if (owned) *reinterpret_cast<uint2 *>(bpbuf + ((blk & 1) * FBW + fib) * 32 + (lane - GH) * 8) = make_uint2(wlo, whi);
           fib += G;
@@ -516,7 +520,7 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
           int *pbuf = pathbuf + buf * FBK;
           const unsigned char *rows = btbuf + ((size_t)buf * NREG + jreg) * RSZ;
           int col = (v - wreg * OW) >> 2, k2 = 2 * (v & 3);  // byte column of the walker, bit offset in it
-          // Full groups are walked from registers (kab_walk_group8 in kab_bandp.cuh: two 64-bit loads
+          // Full groups are walked from registers (kab_walk_group8 in kab_band.cuh: two 64-bit loads
           // per group, loaded a group early, and a branch-free 8-frame body); what it leaves takes the
           // generic step, which also handles the step into the warp region below.
           auto step_column = [&]() {
