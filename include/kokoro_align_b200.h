@@ -126,6 +126,30 @@ int kab_plan_create_ctc(kab_plan **plan, int device, int64_t n_lattices, const i
 int kab_plan_create_ctc_long(kab_plan **plan, int device, int64_t n_lattices, const int64_t *t_off,
                              const int32_t *labels, const int64_t *l_off, int32_t vocab_size,
                              int32_t blank);
+/*
+ * Banded CTC forced alignment (long recordings, long batches): kab_plan_create_ctc with the
+ * recurrence limited to a window of beam_size = W >= 1 states around the diagonal, the window of
+ * kab_plan_create (align.py:64-65).  Lattice b (T frames, S = 2L+1 states) at frame i:
+ *     lo_i = max(0, floor(S*i/T) - floor(W/2)),   hi_i = min(lo_i + W, S)
+ * Every frame applies the CTC recurrence unchanged and then sets every state outside [lo_i, hi_i)
+ * to -inf.  The result is the best path INSIDE the band: it equals the unbanded one when that path
+ * lies inside the band.
+ *   - Covering lattices (W >= S and floor(S*(T-1)/T) <= floor(W/2): the window never clips) are
+ *     routed and computed as by kab_plan_create_ctc_long; their outputs are byte-identical to it,
+ *     including its "both end states -inf: follow the recurrence" case.
+ *   - Any other lattice ends in S-1 if a[S-1] > a[S-2], else S-2; when both are -inf no path stays
+ *     inside the band: KAB_ST_DEAD_BAND with a NaN final_score (outputs unspecified).
+ *   - The other statuses are those of kab_plan_create_ctc.
+ * Routing of a lattice whose window clips: KAB_CLASS_BAND (single-CTA band kernel, T * NBP bytes of
+ * backpointers, NBP = (26 * NW + 15) & ~15, NW = ceil((min(W, S) + 32) / 104) warps) when
+ * min(W, S) <= 3264 and its columns are staged (vocab_size <= 512, or at most 511 distinct labels
+ * through the compact copy); otherwise KAB_CLASS_GENERIC, T * min(W, S) bytes.  kab_plan_info's
+ * cells_eval and algorithmic_bytes count the windowed cells.
+ * KAB_E_BAD_ARG for a blank outside [0, vocab_size) or beam_size < 1.
+ */
+int kab_plan_create_ctc_band(kab_plan **plan, int device, int64_t n_lattices, const int64_t *t_off,
+                             const int32_t *labels, const int64_t *l_off, int32_t vocab_size,
+                             int32_t blank, int32_t beam_size);
 int kab_plan_get_info(const kab_plan *plan, kab_plan_info *info);
 int kab_plan_destroy(kab_plan *plan);
 

@@ -21,7 +21,7 @@ KAB_OK, KAB_E_CUDA, KAB_E_BAD_ARG, KAB_E_NOMEM, KAB_E_UNSUPPORTED = 0, -1, -2, -
 ST_OK, ST_DEAD_BAND, ST_BAD_LABEL, ST_NONFINITE = 0, 1, 2, 3
 
 EXPORTS = ["kab_version", "kab_error_string", "kab_last_cuda_error", "kab_device_count",
-           "kab_plan_create", "kab_plan_create_ctc", "kab_plan_create_ctc_long", "kab_plan_get_info", "kab_plan_destroy", "kab_plan_run_device",
+           "kab_plan_create", "kab_plan_create_ctc", "kab_plan_create_ctc_long", "kab_plan_create_ctc_band", "kab_plan_get_info", "kab_plan_destroy", "kab_plan_run_device",
            "kab_plan_run_host", "kab_plan_run_host_logits", "kab_plan_run_host_segments", "kab_plan_segment_stats_device", "kab_log_softmax_device", "kab_log_softmax_pack_device", "kab_merge_tokens_device", "kab_word_spans_device", "kab_ctc_best_path", "kab_encode_transcript", "kab_merge_repeated", "kab_pool_trim", "kab_host_alloc", "kab_host_free"]
 
 
@@ -103,6 +103,7 @@ def lib():
     L.kab_plan_create.argtypes = [ctypes.POINTER(vp), ctypes.c_int, i64, vp, vp, vp, i32, i32, i32]
     L.kab_plan_create_ctc.argtypes = [ctypes.POINTER(vp), ctypes.c_int, i64, vp, vp, vp, i32, i32]
     L.kab_plan_create_ctc_long.argtypes = [ctypes.POINTER(vp), ctypes.c_int, i64, vp, vp, vp, i32, i32]
+    L.kab_plan_create_ctc_band.argtypes = [ctypes.POINTER(vp), ctypes.c_int, i64, vp, vp, vp, i32, i32, i32]
     L.kab_plan_get_info.argtypes = [vp, ctypes.POINTER(PlanInfo)]
     L.kab_plan_destroy.argtypes = [vp]
     L.kab_plan_run_device.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp]

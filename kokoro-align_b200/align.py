@@ -67,7 +67,7 @@ class AlignPlan:
         self._create(_lib.lib().kab_plan_create, int(beam_size), int(max_move))
 
     @classmethod
-    def ctc(cls, t_off, labels, l_off, vocab_size, blank=0, device=0, long_form=False):
+    def ctc(cls, t_off, labels, l_off, vocab_size, blank=0, device=0, long_form=False, beam_size=None):
         """A plan in CTC forced-alignment mode (kab_plan_create_ctc): torchaudio's forced_align
         recurrence for every lattice of the batch; labels are token ids in [0, vocab_size) other
         than ``blank``.  best_labels are then token ids per frame (``blank`` on even states).
@@ -76,11 +76,19 @@ class AlignPlan:
         same outputs.  Wide vocabularies (vocab_size > 512, e.g. NeMo's 1025) reach the warp, band
         and wide kernels through a compact copy of every lattice's own columns; a lattice with more
         than 511 distinct labels runs on the generic kernel on its own, and the wide kernel takes
-        long lattices while no compact lattice of the plan has more than 335 distinct labels."""
+        long lattices while no compact lattice of the plan has more than 335 distinct labels.
+        beam_size=W (kab_plan_create_ctc_band; long_form makes no difference): the recurrence is limited to
+        the window of W states around the diagonal of the Kokoro plans (align.py:64-65), so a lattice costs
+        T * W cells instead of T * S.  A lattice the window never clips is computed as by long_form=True;
+        for any other the result is the best path INSIDE the band, which equals torchaudio's only when the
+        unbanded best path lies inside it, and status 1 (ST_DEAD_BAND) says no path stays inside."""
         plan = cls.__new__(cls)
         plan._setup(t_off, labels, l_off, vocab_size, device)
         L = _lib.lib()
-        plan._create(L.kab_plan_create_ctc_long if long_form else L.kab_plan_create_ctc, int(blank))
+        if beam_size is not None:
+            plan._create(L.kab_plan_create_ctc_band, int(blank), int(beam_size))
+        else:
+            plan._create(L.kab_plan_create_ctc_long if long_form else L.kab_plan_create_ctc, int(blank))
         return plan
 
     def _setup(self, t_off, labels, l_off, vocab_size, device):
@@ -298,7 +306,17 @@ def _ctc_lengths(lengths, B, full, what):
     return n
 
 
-def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, blank=0, *, long_form=False):
+def _check_beam(beam_size):
+    if beam_size is not None and int(beam_size) < 1:
+        raise ValueError(f"beam_size must be >= 1, got {beam_size}")
+
+
+def _band_lost(beam_size, where=""):
+    return ValueError(f"{where}no CTC path stays within beam_size={beam_size}; widen the beam")
+
+
+def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, blank=0, *, long_form=False,
+                 beam_size=None):
     """Drop-in for torchaudio.functional.forced_align (same arguments, output shapes and dtypes,
     exception types): log_probs float32 [1, T, V], targets int32 / int64 [1, L] on the same device
     (CPU or CUDA).  Returns (paths [1, T] of the targets' dtype: the token id of every frame,
@@ -309,8 +327,14 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
     log-probs raise ValueError (-inf, for masking, is accepted), in any column of the row.
     long_form=True: a lattice of more than 3296 states (2 L + 1) runs on the wide kernel, with the
     same outputs.  Any vocabulary size up to 65535 reaches the staged kernels while the target has at
-    most 511 distinct ids (AlignPlan.ctc)."""
+    most 511 distinct ids (AlignPlan.ctc).
+    beam_size=W: banded alignment for long recordings (AlignPlan.ctc): only the W states of the window
+    around the diagonal S*t/T are kept in frame t, which takes T * W cells of work and backpointers instead
+    of T * S.  The result is the best path INSIDE the band; it equals torchaudio's only when the unbanded
+    best path lies inside the band.  ValueError when no path stays inside it (widen the beam) and for
+    beam_size < 1."""
     import torch
+    _check_beam(beam_size)
     _ctc_tensor_checks(log_probs, targets, blank)
     if log_probs.size(0) != 1 or targets.size(0) != 1:
         raise RuntimeError("The batch dimension for log_probs and targets must be 1 (forced_align_batch takes batches)")
@@ -327,7 +351,7 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
                            f"and number of repeats: {R}")
     dev = log_probs.device
     with AlignPlan.ctc([0, T], tg, [0, L], V, blank, device=dev.index if dev.type == "cuda" else _current_device(),
-                       long_form=long_form) as plan:
+                       long_form=long_form, beam_size=beam_size) as plan:
         if dev.type == "cuda":
             with torch.cuda.device(dev):
                 _, labs, scores, _, status = plan.run_torch(log_probs[0].contiguous())
@@ -337,11 +361,14 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
             labs, scores, status = torch.from_numpy(labs), torch.from_numpy(scores), int(st[0])
     if status == ST_NONFINITE:
         raise ValueError("log_probs must not contain NaN or +inf")
+    if status == ST_DEAD_BAND and beam_size is not None:
+        raise _band_lost(beam_size)
     raise_for_status(status, V)
     return labs.to(targets.dtype).view(1, T), scores.view(1, T)
 
 
-def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=None, blank=0, *, long_form=False):
+def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=None, blank=0, *, long_form=False,
+                       beam_size=None):
     """forced_align for a padded batch, in one plan: log_probs float32 [B, T_max, V], targets
     int32 / int64 [B, L_max], input_lengths / target_lengths [B] (None: all full length).  Item b
     is aligned over its first input_lengths[b] frames and target_lengths[b] targets.  Returns
@@ -349,8 +376,11 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
     frames past an item's length hold the blank and score 0.  Raises, like forced_align, for the
     first item that fails, naming its index.  On CUDA the valid rows are packed on the device.
     long_form: as in forced_align.  With more than 512 classes, the items with at most 511 distinct
-    target ids run on the staged kernels and the others on the generic kernel (AlignPlan.ctc)."""
+    target ids run on the staged kernels and the others on the generic kernel (AlignPlan.ctc).
+    beam_size: as in forced_align (each item's band follows its own T and S; the results are the best
+    paths inside the bands); an item with no path inside its band raises ValueError naming it."""
     import torch
+    _check_beam(beam_size)
     _ctc_tensor_checks(log_probs, targets, blank)
     B, T_max, V = (int(x) for x in log_probs.shape)
     if targets.size(0) != B:
@@ -377,7 +407,7 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
     if B == 0:
         return paths, scores
     with AlignPlan.ctc(t_off, labels, l_off, V, blank, device=dev.index if dev.type == "cuda" else _current_device(),
-                       long_form=long_form) as plan:
+                       long_form=long_form, beam_size=beam_size) as plan:
         if dev.type == "cuda":
             with torch.cuda.device(dev):
                 _, labs, sc, _, status = plan.run_torch(log_probs[valid].contiguous())   # rows packed on the device
@@ -388,6 +418,8 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
     for b in np.flatnonzero(status != ST_OK):
         if status[b] == ST_NONFINITE:
             raise ValueError(f"item {b}: log_probs must not contain NaN or +inf")
+        if status[b] == ST_DEAD_BAND and beam_size is not None:
+            raise _band_lost(beam_size, f"item {b}: ")
         raise_for_status(int(status[b]), V)
     paths[valid] = labs.to(targets.dtype)
     scores[valid] = sc

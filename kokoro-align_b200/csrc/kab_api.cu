@@ -145,7 +145,7 @@ int64_t cells_eval_of(int64_t T, int64_t S, int64_t W) {
 
 // What a plan computes.  Child plans (segments, book pipes, the hybrid sub-plan) take their parent's.
 struct PlanSpec {
-  int32_t V = 0, W = 0, M = 0;
+  int32_t V = 0, W = 0, M = 0;  // (CTC: W is CTC_W, or beam_size of a banded plan, kab_plan_create_ctc_band)
   bool ctc = false;       // CTC forced-alignment plan (kab_plan_create_ctc)
   int32_t blank = 0;      // ... and its blank id
   bool ctc_long = false;  // ... whose lattices too wide for the band kernel go to the wide kernel (kab_plan_create_ctc_long)
@@ -356,9 +356,13 @@ namespace {
 // plan chooses (and may go hybrid), 0 the single-CTA band kernel, 1 kab_bandr.cuh
 int plan_create_impl(kab_plan **out, int device, const PlanSpec &s, int64_t B, const int64_t *t_off,
                      const int32_t *labels, const int64_t *l_off, const uint8_t *mask, int band_mode);
-// CTC plans: every lattice is unbanded -- a window this wide is [0, S) in every frame of the band
-// kernel (S <= 3296 there) -- and has three moves
+// CTC plans: three moves; default and long-form plans leave every lattice unbanded -- a window this wide
+// is [0, S) in every frame of the band kernel (S <= 3296 there)
 constexpr int32_t CTC_W = 0x3fffffff, CTC_M = 3;
+// banded CTC plans: a lattice whose window clips runs on the single-CTA band kernel while min(W, S) is at
+// most this, otherwise on the generic kernel (the NW = 32 ring holds 3328 states: 64 to spare, where
+// band_shaped asks for 32)
+constexpr int64_t CTC_BAND_MAX_W = 3264;
 }  // namespace
 
 int kab_plan_create(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
@@ -378,6 +382,13 @@ int kab_plan_create_ctc_long(kab_plan **out, int device, int64_t B, const int64_
   if (blank < 0 || blank >= V) return KAB_E_BAD_ARG;
   // (the single-CTA band kernel below S = 3297, the wide kernel above it where it fits)
   return plan_create_impl(out, device, PlanSpec{V, CTC_W, CTC_M, true, blank, true}, B, t_off, labels, l_off, nullptr, 0);
+}
+
+int kab_plan_create_ctc_band(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
+                             const int64_t *l_off, int32_t V, int32_t blank, int32_t beam_size) {
+  if (blank < 0 || blank >= V || beam_size < 1) return KAB_E_BAD_ARG;
+  // (lattices the window covers are routed as by kab_plan_create_ctc_long)
+  return plan_create_impl(out, device, PlanSpec{V, beam_size, CTC_M, true, blank, true}, B, t_off, labels, l_off, nullptr, 0);
 }
 
 namespace {
@@ -559,6 +570,7 @@ void Setup::classify() {
       if (!in(b) || facts[(size_t)b].bad) continue;
       if (pl->Vc && !facts[(size_t)b].compact) continue;  // (too many distinct labels for the compact copy: generic)
       const int64_t T = frames(b), S = 2 * len(b) + 1;
+      if (!unbanded(T, S, W)) continue;                      // (banded plans: band or generic class)
       if (S + 32 <= KAB_BAND_OW * BAND_MAX_WARPS) continue;  // warp or band class
       if (wide_ctas(S) + 1 > wide_capacity) continue;
       sum_t += (double)T;
@@ -591,7 +603,7 @@ void Setup::classify() {
     // candidates into -inf); more than four moves only exist in the generic kernel
     const bool fast = M <= 4 && !f.special && (ga || (Veff <= MAX_STAGE_V && (!pl->Vc || f.distinct + 1 <= pl->Vc)));
     const bool full = unbanded(T, S, W);
-    const int64_t weff = s.ctc ? S : std::min<int64_t>(W, S);
+    const int64_t weff = std::min<int64_t>(W, S);
     int q;
     if (fast && !ga && full && S <= 248) {
       q = Q_WARP;
@@ -603,7 +615,7 @@ void Setup::classify() {
       } else {  // score checkpoint rows, one per KAB_CKPT_C frames
         bp_bytes += align_up((T + KAB_CKPT_C - 1) / KAB_CKPT_C * kab_ckpt_stride((int)S, d.k) * 4, 256);
       }
-    } else if (fast && band_shaped(T, S, W)) {
+    } else if (fast && band_shaped(T, S, W) && (!s.ctc || full || weff <= CTC_BAND_MAX_W)) {
       q = Q_BAND;  // backpointer offsets are assigned by lay_out_band, once the kernel is known
       max_band_weff = std::max(max_band_weff, weff);
     } else if (fast && !ga && (s.ctc ? ctc_wide : M == 4) && full && wide_ctas(S) + 1 <= wide_capacity) {
@@ -625,7 +637,7 @@ void Setup::classify() {
     pl->lists[q].push_back(d);
     pl->max_T[q] = std::max(pl->max_T[q], (int)T);
     info.n_class[q == Q_WARP ? KAB_CLASS_WARP : (q == Q_GENERIC ? KAB_CLASS_GENERIC : (q == Q_WIDE ? KAB_CLASS_WIDE : KAB_CLASS_BAND))]++;
-    const int64_t cells = s.ctc ? T * S : cells_eval_of(T, S, W);
+    const int64_t cells = cells_eval_of(T, S, W);
     info.cells_eval += cells;
     info.cells_nominal += T * S;
     int bbits = 0;

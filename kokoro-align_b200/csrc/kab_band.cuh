@@ -96,9 +96,12 @@ __device__ __forceinline__ int kab_walk_group8(const uint2 w0, const uint2 w1, c
   return stopped ? f_next : -1;
 }
 
-// CTC: the CTC forced-alignment recurrence (kab_common.cuh) over the whole lattice: the host sets W so
-// that the window is [0, S) in every frame, and S + 32 <= R, so no chunk is ever recycled.  Junk from
-// lane 0 climbs at most two states per frame there (16 in a group), so the 24 ghost states still cover it.
+// CTC: the CTC forced-alignment recurrence (kab_common.cuh) in the same window.  Default and long-form
+// plans set W so wide that the window is [0, S) in every frame (S + 32 <= R: no chunk is ever recycled);
+// banded plans (kab_plan_create_ctc_band) pass beam_size, and a recycled chunk recomputes its repeat bits
+// for its new states.  A lattice whose window clips somewhere and whose two end states are both -inf has
+// no path inside the band: status 1.  Junk from lane 0 climbs at most two states per frame (16 in a
+// group), so the 24 ghost states still cover it; the window advances <= 3 states per frame (S <= 2T + 1).
 template <int MAXT, bool MM, bool CTC>
 __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lats, int n_lat, const KabParams &p,
                                               const int blank) {
@@ -140,6 +143,7 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
     if (tid == 0) {
       s_item = atomicAdd(p.queue, 1u);
       s_vmax = -1;
+      if (CTC) s_end[0] = s_end[1] = kab_neg_inf();  // (an end state outside the last window has no owner)
     }
     __syncthreads();
     const unsigned int item = s_item;
@@ -198,10 +202,15 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
     const uint32_t boff = CTC ? 4u * (uint32_t)blank : 0u;  // byte offset of the blank's column
     // CTC: bit 0 / 1 = move 2 forbidden into label state vb+1 / vb+3 (state 1, or a repeated label)
     uint32_t rep = 0;
+    // CTC, next alias: byte offset of the label column of state vb+R-1 (the one below vb+R+1), prefetched
+    // with nc1 / nc3 so that recycling a chunk recomputes its repeat bits without waiting for a load
+    uint32_t ncm = 0;
+    auto load_below = [&](int base) { return base + 1 < S ? 4u * col16[(base >> 1) - 1] : 0u; };
     if (CTC) {
       const int l1 = vb >> 1;  // label index of state vb+1
       if (vb + 1 < 3 || vb + 1 >= S || col16[l1] == col16[l1 - 1]) rep |= 1u;
       if (vb + 3 >= S || col16[l1 + 1] == col16[l1]) rep |= 2u;
+      ncm = load_below(vb + R);
     }
 
     float poison = kab_poison_init<CTC>();  // NaN once a rejected log-prob was staged (kab_poison_t)
@@ -315,6 +324,10 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
       // before the next group boundary (the window advances <= 3 states per frame)
       while (vb + 3 < lo0 - 3) {
         vb += R;
+        if (CTC) {  // the repeat bits of the new states, as at lattice start (vb >= R: state vb+1 is not state 1)
+          rep = (vb + 1 >= S || nc1 == ncm ? 1u : 0u) | (vb + 3 >= S || nc3 == nc1 ? 2u : 0u);
+          ncm = load_below(vb + R);
+        }
         c1 = nc1; c3 = nc3;
         load_cols(vb + R, nc1, nc3);
         e1 = *reinterpret_cast<const float *>(rowc + c1);  // the prefetched emissions belonged
@@ -431,7 +444,12 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
     if (tid == 0) kab_bulk_wait0();  // all backpointer blocks are in global memory
     const int any_bad = __syncthreads_or(poison != poison ? 1 : 0);
     int v = s_vmax;
-    if (CTC) v = (S >= 2 && !(s_end[0] > s_end[1])) ? S - 2 : S - 1;
+    if (CTC) {
+      v = (S >= 2 && !(s_end[0] > s_end[1])) ? S - 2 : S - 1;
+      // no path stays inside a window that clips (a covering window follows the recurrence instead)
+      const bool clips = W < S || (int)(((int64_t)S * (T - 1)) / T) > half;
+      if (clips && !(s_end[0] > ninf) && !(s_end[1] > ninf)) v = -1;
+    }
     const int status = any_bad ? 3 : (v < 0 ? 1 : 0);
     if (owned && status == 0) {
       if (vb + 0 == v) s_final = s0;

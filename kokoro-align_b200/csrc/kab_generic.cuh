@@ -7,8 +7,10 @@
 #pragma once
 #include "kab_common.cuh"
 
-// CTC: the CTC forced-alignment recurrence (kab_common.cuh) over the whole lattice (no window,
-// value-independent blank test: the state's parity), blank column `blank`.
+// CTC: the CTC forced-alignment recurrence (kab_common.cuh) in the same window (value-independent blank
+// test: the state's parity), blank column `blank`.  Default and long-form plans pass a W so wide that the
+// window is [0, S) in every frame; banded plans (kab_plan_create_ctc_band) pass beam_size.  A window that
+// clips somewhere and leaves both end states -inf: no path inside the band, status 1.
 template <int NT, bool CTC>
 __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ lats, int n_lat, const KabParams &p,
                                                  const int blank) {
@@ -26,7 +28,7 @@ __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ 
     if (item >= (unsigned int)n_lat) break;
     const KabLattice lat = lats[item];
     const int64_t T = lat.T, S = 2 * (int64_t)lat.L + 1, W = p.W, M = p.M, V = p.V;
-    const int64_t Wc = CTC ? S : max((int64_t)1, min(W, S));
+    const int64_t Wc = max((int64_t)1, min(W, S));
     const int32_t *raw = p.raw + lat.lab_off;
     const float *lp = p.lp + lat.t_off * V;
     uint8_t *bp = p.bp + lat.bp_off;
@@ -40,8 +42,8 @@ __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ 
     bool bad = false;
     for (int64_t i = 0; i < T; ++i) {
       int64_t lo = (S * i) / T - W / 2;  // align.py:64 (64-bit: S*i reaches 1e11)
-      if (lo < 0 || CTC) lo = 0;
-      int64_t hi = CTC ? S : min(lo + W, S);  // align.py:65
+      if (lo < 0) lo = 0;
+      int64_t hi = min(lo + W, S);  // align.py:65
       if (hi < lo) hi = lo;
       const float *row = lp + i * V;
       for (int64_t c = tid; c < V; c += NT) {
@@ -49,17 +51,18 @@ __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ 
         bad |= CTC ? !(x < __int_as_float(0x7f800000)) : !kab_finite(x);  // CTC: -inf is accepted
       }
       if (CTC) {
-        for (int64_t v = tid; v < S; v += NT) {
+        for (int64_t v = lo + tid; v < hi; v += NT) {
           const bool lab = (v & 1) != 0;
           const int32_t ext = lab ? raw[(v - 1) >> 1] : blank;
           const float e = __ldg(&row[ext]);
-          const float x0 = v < phi ? __ldcg(&prev[v]) : kab_neg_inf();
-          const float x1 = v >= 1 && v - 1 < phi ? __ldcg(&prev[v - 1]) : kab_neg_inf();
-          const float x2 = lab && v >= 3 && v - 2 < phi && ext != raw[(v - 3) >> 1] ? __ldcg(&prev[v - 2]) : kab_neg_inf();
+          // predecessors outside the previous window are -inf
+          const float x0 = v >= plo && v < phi ? __ldcg(&prev[v]) : kab_neg_inf();
+          const float x1 = v - 1 >= plo && v - 1 < phi ? __ldcg(&prev[v - 1]) : kab_neg_inf();
+          const float x2 = lab && v >= 3 && v - 2 >= plo && v - 2 < phi && ext != raw[(v - 3) >> 1] ? __ldcg(&prev[v - 2]) : kab_neg_inf();
           uint32_t code = 0;
           const float best = lab ? kab_ctc_label_sel(x0, x1, x2, code, 0) : kab_ctc_blank_sel(x0, x1, code, 0);
           __stcg(&cur[v], __fadd_rn(best, e));
-          bp[i * Wc + v] = (uint8_t)code;
+          bp[i * Wc + (v - lo)] = (uint8_t)code;
         }
       } else
       for (int64_t v = lo + tid; v < hi; v += NT) {
@@ -91,8 +94,15 @@ __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ 
     if (vmax >= 0) atomicMax(&s_vmax, vmax);
     const int any_bad = __syncthreads_or(bad ? 1 : 0);
     int64_t v = s_vmax;
-    // CTC end rule: the better of the last two states, S-2 on a tie
-    if (CTC) v = (S >= 2 && !(__ldcg(&prev[S - 1]) > __ldcg(&prev[S - 2]))) ? S - 2 : S - 1;
+    // CTC end rule: the better of the last two states, S-2 on a tie (a state outside the last window: -inf);
+    // none of them finite in a window that clips: no path inside the band
+    if (CTC) {
+      const float e1 = S - 1 >= plo && S - 1 < phi ? __ldcg(&prev[S - 1]) : kab_neg_inf();
+      const float e2 = S >= 2 && S - 2 >= plo && S - 2 < phi ? __ldcg(&prev[S - 2]) : kab_neg_inf();
+      v = (S >= 2 && !(e1 > e2)) ? S - 2 : S - 1;
+      const bool clips = W < S || (S * (T - 1)) / T > W / 2;
+      if (clips && !(e1 > kab_neg_inf()) && !(e2 > kab_neg_inf())) v = -1;
+    }
 
     if (tid == 0) {
       int st = 0;
@@ -106,7 +116,7 @@ __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ 
         float *out_sc = p.best_scores + lat.t_off;
         for (int64_t i = T - 1; i >= 0; --i) {  // == flush_determined_path, align.py:21-40
           int64_t lo = (S * i) / T - W / 2;
-          if (lo < 0 || CTC) lo = 0;
+          if (lo < 0) lo = 0;
           const int32_t ext = (v & 1) ? raw[(v - 1) >> 1] : (CTC ? blank : 0);
           const int32_t col = ext < 0 ? ext + (int32_t)V : ext;
           out_path[i] = (int32_t)v;
