@@ -127,6 +127,23 @@ int kab_plan_create_ctc_long(kab_plan **plan, int device, int64_t n_lattices, co
                              const int32_t *labels, const int64_t *l_off, int32_t vocab_size,
                              int32_t blank);
 /*
+ * CTC forced alignment with free ends (recordings with untranscribed speech before or after the
+ * transcript, a passage inside a longer recording): kab_plan_create_ctc_long's recurrence with
+ *   - a virtual state -1 of score 0 in EVERY frame, state 0's move-1 and state 1's move-2 predecessor
+ *     (torchaudio's select and tie rules unchanged; frame 0 gets the usual initialisation); the walk
+ *     stops there, at the window's first frame t0;
+ *   - the end at the maximum of a_t[v] over every frame t and v in {S-1, S-2}: a tie between frames
+ *     picks the later frame, within a frame S-2; every candidate -inf: (T-1, S-2).  That frame is t1.
+ * Frames outside [t0, t1] get best_path -1, best_labels = blank, best_scores = log_probs[t, blank];
+ * final_score = a_t1[v_end], the path score over [t0, t1].  The statuses are kab_plan_create_ctc's;
+ * a lattice with L = 0 has every frame outside, final_score 0 and status 0.  Routed as by
+ * kab_plan_create_ctc_long (every lattice unbanded); there is no banded free-ends plan.
+ * KAB_E_BAD_ARG for a blank outside [0, vocab_size).
+ */
+int kab_plan_create_ctc_free(kab_plan **plan, int device, int64_t n_lattices, const int64_t *t_off,
+                             const int32_t *labels, const int64_t *l_off, int32_t vocab_size,
+                             int32_t blank);
+/*
  * Banded CTC forced alignment (long recordings, long batches): kab_plan_create_ctc with the
  * recurrence limited to a window of beam_size = W >= 1 states around the diagonal, the window of
  * kab_plan_create (align.py:64-65).  Lattice b (T frames, S = 2L+1 states) at frame i:

@@ -67,7 +67,8 @@ class AlignPlan:
         self._create(_lib.lib().kab_plan_create, int(beam_size), int(max_move))
 
     @classmethod
-    def ctc(cls, t_off, labels, l_off, vocab_size, blank=0, device=0, long_form=False, beam_size=None):
+    def ctc(cls, t_off, labels, l_off, vocab_size, blank=0, device=0, long_form=False, beam_size=None, *,
+            free_ends=False):
         """A plan in CTC forced-alignment mode (kab_plan_create_ctc): torchaudio's forced_align
         recurrence for every lattice of the batch; labels are token ids in [0, vocab_size) other
         than ``blank``.  best_labels are then token ids per frame (``blank`` on even states).
@@ -81,11 +82,20 @@ class AlignPlan:
         the window of W states around the diagonal of the Kokoro plans (align.py:64-65), so a lattice costs
         T * W cells instead of T * S.  A lattice the window never clips is computed as by long_form=True;
         for any other the result is the best path INSIDE the band, which equals torchaudio's only when the
-        unbanded best path lies inside it, and status 1 (ST_DEAD_BAND) says no path stays inside."""
+        unbanded best path lies inside it, and status 1 (ST_DEAD_BAND) says no path stays inside.
+        free_ends=True (kab_plan_create_ctc_free; routed as long_form=True): the transcript may cover any
+        window of frames [t0, t1] of its lattice, for recordings with untranscribed speech at the edges.
+        The path is the best one over every window of at least L + R frames (ties: the later end, the
+        earlier start); frames outside the window get state -1, the blank and its log-prob, so
+        merge_tokens_batch's spans give where the text starts and ends, and final_score is the score over
+        the window.  Not combined with beam_size (ValueError)."""
+        _check_free_ends(free_ends, beam_size)
         plan = cls.__new__(cls)
         plan._setup(t_off, labels, l_off, vocab_size, device)
         L = _lib.lib()
-        if beam_size is not None:
+        if free_ends:
+            plan._create(L.kab_plan_create_ctc_free, int(blank))
+        elif beam_size is not None:
             plan._create(L.kab_plan_create_ctc_band, int(blank), int(beam_size))
         else:
             plan._create(L.kab_plan_create_ctc_long if long_form else L.kab_plan_create_ctc, int(blank))
@@ -311,12 +321,18 @@ def _check_beam(beam_size):
         raise ValueError(f"beam_size must be >= 1, got {beam_size}")
 
 
+def _check_free_ends(free_ends, beam_size):
+    if free_ends and beam_size is not None:
+        raise ValueError("free_ends=True does not combine with beam_size: the band assumes that the transcript "
+                         "spans the whole recording")
+
+
 def _band_lost(beam_size, where=""):
     return ValueError(f"{where}no CTC path stays within beam_size={beam_size}; widen the beam")
 
 
 def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, blank=0, *, long_form=False,
-                 beam_size=None):
+                 beam_size=None, free_ends=False):
     """Drop-in for torchaudio.functional.forced_align (same arguments, output shapes and dtypes,
     exception types): log_probs float32 [1, T, V], targets int32 / int64 [1, L] on the same device
     (CPU or CUDA).  Returns (paths [1, T] of the targets' dtype: the token id of every frame,
@@ -332,9 +348,15 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
     around the diagonal S*t/T are kept in frame t, which takes T * W cells of work and backpointers instead
     of T * S.  The result is the best path INSIDE the band; it equals torchaudio's only when the unbanded
     best path lies inside the band.  ValueError when no path stays inside it (widen the beam) and for
-    beam_size < 1."""
+    beam_size < 1.
+    free_ends=True: the targets are aligned to the best window [t0, t1] of the recording rather than to all
+    of it (speech before or after the transcript, a passage inside a longer recording; AlignPlan.ctc).
+    Frames outside the window hold the blank and its log-prob, so merge_tokens gives the spans of the
+    text.  For a gap in the middle of the transcript, append a zero log-prob column as a <star> token
+    (the MMS recipe) and put it in the targets.  Not combined with beam_size (ValueError)."""
     import torch
     _check_beam(beam_size)
+    _check_free_ends(free_ends, beam_size)
     _ctc_tensor_checks(log_probs, targets, blank)
     if log_probs.size(0) != 1 or targets.size(0) != 1:
         raise RuntimeError("The batch dimension for log_probs and targets must be 1 (forced_align_batch takes batches)")
@@ -351,7 +373,7 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
                            f"and number of repeats: {R}")
     dev = log_probs.device
     with AlignPlan.ctc([0, T], tg, [0, L], V, blank, device=dev.index if dev.type == "cuda" else _current_device(),
-                       long_form=long_form, beam_size=beam_size) as plan:
+                       long_form=long_form, beam_size=beam_size, free_ends=free_ends) as plan:
         if dev.type == "cuda":
             with torch.cuda.device(dev):
                 _, labs, scores, _, status = plan.run_torch(log_probs[0].contiguous())
@@ -368,7 +390,7 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
 
 
 def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=None, blank=0, *, long_form=False,
-                       beam_size=None):
+                       beam_size=None, free_ends=False):
     """forced_align for a padded batch, in one plan: log_probs float32 [B, T_max, V], targets
     int32 / int64 [B, L_max], input_lengths / target_lengths [B] (None: all full length).  Item b
     is aligned over its first input_lengths[b] frames and target_lengths[b] targets.  Returns
@@ -378,9 +400,11 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
     long_form: as in forced_align.  With more than 512 classes, the items with at most 511 distinct
     target ids run on the staged kernels and the others on the generic kernel (AlignPlan.ctc).
     beam_size: as in forced_align (each item's band follows its own T and S; the results are the best
-    paths inside the bands); an item with no path inside its band raises ValueError naming it."""
+    paths inside the bands); an item with no path inside its band raises ValueError naming it.
+    free_ends: as in forced_align, per item (each item's best window of its own frames)."""
     import torch
     _check_beam(beam_size)
+    _check_free_ends(free_ends, beam_size)
     _ctc_tensor_checks(log_probs, targets, blank)
     B, T_max, V = (int(x) for x in log_probs.shape)
     if targets.size(0) != B:
@@ -407,7 +431,7 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
     if B == 0:
         return paths, scores
     with AlignPlan.ctc(t_off, labels, l_off, V, blank, device=dev.index if dev.type == "cuda" else _current_device(),
-                       long_form=long_form, beam_size=beam_size) as plan:
+                       long_form=long_form, beam_size=beam_size, free_ends=free_ends) as plan:
         if dev.type == "cuda":
             with torch.cuda.device(dev):
                 _, labs, sc, _, status = plan.run_torch(log_probs[valid].contiguous())   # rows packed on the device

@@ -149,6 +149,7 @@ struct PlanSpec {
   bool ctc = false;       // CTC forced-alignment plan (kab_plan_create_ctc)
   int32_t blank = 0;      // ... and its blank id
   bool ctc_long = false;  // ... whose lattices too wide for the band kernel go to the wide kernel (kab_plan_create_ctc_long)
+  bool free_ends = false; // ... with free ends: the transcript may cover any window of frames (kab_plan_create_ctc_free)
 };
 
 // The kernel of a plan's band list.  CTA: kab_band.cuh (two lattices per SM).  The cluster kernels: P kab_bandp.cuh
@@ -384,6 +385,13 @@ int kab_plan_create_ctc_long(kab_plan **out, int device, int64_t B, const int64_
   return plan_create_impl(out, device, PlanSpec{V, CTC_W, CTC_M, true, blank, true}, B, t_off, labels, l_off, nullptr, 0);
 }
 
+int kab_plan_create_ctc_free(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
+                             const int64_t *l_off, int32_t V, int32_t blank) {
+  if (blank < 0 || blank >= V) return KAB_E_BAD_ARG;
+  // (routed as by kab_plan_create_ctc_long: every lattice is unbanded)
+  return plan_create_impl(out, device, PlanSpec{V, CTC_W, CTC_M, true, blank, true, true}, B, t_off, labels, l_off, nullptr, 0);
+}
+
 int kab_plan_create_ctc_band(kab_plan **out, int device, int64_t B, const int64_t *t_off, const int32_t *labels,
                              const int64_t *l_off, int32_t V, int32_t blank, int32_t beam_size) {
   if (blank < 0 || blank >= V || beam_size < 1) return KAB_E_BAD_ARG;
@@ -546,7 +554,8 @@ void Setup::classify() {
   const int64_t W = s.W, M = s.M;
   // resident CTAs of the wide kernel (its warps spin on each other: the whole grid must be resident)
   Launch &lw = pl->launch[Q_WIDE];
-  lw = Launch{s.ctc ? (const void *)kab_wide_ctc_kernel : (const void *)kab_wide_kernel, dim3(), dim3(KAB_WD_THREADS),
+  lw = Launch{s.free_ends ? (const void *)kab_wide_ctc_free_kernel
+              : s.ctc ? (const void *)kab_wide_ctc_kernel : (const void *)kab_wide_kernel, dim3(), dim3(KAB_WD_THREADS),
               kab_wide_geom(pl->stage_bytes).smem_bytes, 0, true};
   {
     int occ = 0;
@@ -865,7 +874,8 @@ int Setup::allocate() {
   if ((rc = alloc((void **)&pl->d_wide_ws, (size_t)pl->wide_ws_bytes, "pool_malloc(wide workspace)"))) return rc;
   if (!pl->lists[Q_WARP].empty()) {
     Launch &l = pl->launch[Q_WARP];
-    l.fn = s.ctc ? (const void *)kab_warp_ctc_kernel
+    l.fn = s.free_ends ? (const void *)kab_warp_ctc_free_kernel
+         : s.ctc ? (const void *)kab_warp_ctc_kernel
          : s.M == 4 ? (Veff == 39 ? (const void *)kab_warp_kernel<39, false> : (const void *)kab_warp_kernel<0, false>)
                     : (Veff == 39 ? (const void *)kab_warp_kernel<39, true> : (const void *)kab_warp_kernel<0, true>);
     l.block = dim3(KAB_WARPS_PER_CTA * 32);
@@ -887,6 +897,7 @@ int Setup::allocate() {
          : bk == BandKernel::Q ? (const void *)kab_bandq_kernel
          : bk == BandKernel::R ? (mm ? (const void *)kab_bandr_kernel<true> : (const void *)kab_bandr_kernel<false>)
          : bk == BandKernel::R_GATHER ? (mm ? (const void *)kab_bandr_kernel<true, true> : (const void *)kab_bandr_kernel<false, true>)
+         : s.free_ends ? (small ? (const void *)kab_band_ctc_free_kernel<512> : (const void *)kab_band_ctc_free_kernel<1024>)
          : s.ctc ? (small ? (const void *)kab_band_ctc_kernel<512> : (const void *)kab_band_ctc_kernel<1024>)
          : small ? (mm ? (const void *)kab_band_kernel<512, true> : (const void *)kab_band_kernel<512, false>)
                  : (mm ? (const void *)kab_band_kernel<1024, true> : (const void *)kab_band_kernel<1024, false>);
@@ -1119,7 +1130,10 @@ int kab_plan_run_device(kab_plan *pl, const float *d_log_probs, int32_t *d_best_
       }
   if (!pl->lists[Q_GENERIC].empty()) {
     KabParams pg = p; pg.queue = pl->d_queue + Q_GENERIC;
-    if (s.ctc)
+    if (s.free_ends)
+      kab_generic_ctc_free_kernel<GENERIC_NT><<<pl->launch[Q_GENERIC].grid, GENERIC_NT, 0, stream>>>(
+          pl->d_lists[Q_GENERIC], (int)pl->lists[Q_GENERIC].size(), pg, s.blank);
+    else if (s.ctc)
       kab_generic_ctc_kernel<GENERIC_NT><<<pl->launch[Q_GENERIC].grid, GENERIC_NT, 0, stream>>>(
           pl->d_lists[Q_GENERIC], (int)pl->lists[Q_GENERIC].size(), pg, s.blank);
     else

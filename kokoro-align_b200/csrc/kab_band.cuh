@@ -102,7 +102,10 @@ __device__ __forceinline__ int kab_walk_group8(const uint2 w0, const uint2 w1, c
 // for its new states.  A lattice whose window clips somewhere and whose two end states are both -inf has
 // no path inside the band: status 1.  Junk from lane 0 climbs at most two states per frame (16 in a
 // group), so the 24 ghost states still cover it; the window advances <= 3 states per frame (S <= 2T + 1).
-template <int MAXT, bool MM, bool CTC>
+// FREE: CTC with free ends (kab_plan_create_ctc_free; always unbanded): the lane of state 0 takes the
+// virtual state -1 (score 0 in every frame) as its halo, the owners of S-1 and S-2 keep running (score,
+// frame) maxima (>=: the later frame), and the walk starts at the chosen end (t1, v) and stops at state -1.
+template <int MAXT, bool MM, bool CTC, bool FREE = false>
 __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lats, int n_lat, const KabParams &p,
                                               const int blank) {
   constexpr int G = KAB_BAND_G, GH = KAB_BAND_GHOST, OW = KAB_BAND_OW;
@@ -119,7 +122,8 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
   __shared__ unsigned int s_item;
   __shared__ int s_vmax;
   __shared__ float s_final;
-  __shared__ float s_end[2];  // CTC: scores of states S-1, S-2 of the last frame
+  __shared__ float s_end[2];  // CTC: scores of states S-1, S-2 of the last frame (FREE: their maxima)
+  __shared__ int s_endf[2];   // FREE: ... and the frames of those maxima
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const bool owned = lane >= GH;
@@ -189,8 +193,13 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
     for (int c = 0; c < min(n_chunks, KAB_BAND_STAGES); ++c) issue(c, (st + c) % KAB_BAND_STAGES);
 
     // ---- register state: everything inactive except the virtual start state 0 (align.py:57-58)
-    float s0 = (owned && slot0 == 0) ? 0.0f : ninf, s1 = ninf, s2 = ninf, s3 = ninf;
+    float s0 = (owned && slot0 == 0 && !FREE) ? 0.0f : ninf, s1 = ninf, s2 = ninf, s3 = ninf;
     int vb = slot0;  // first state of this lane's chunk (alias level 0)
+    const bool first = FREE && owned && vb == 0;  // FREE: the lane whose halo is the virtual state -1
+    // FREE: running end maxima; state S-1 is register 0 or 2 of its owner, S-2 register 1 or 3
+    const bool e1hi = (S - 1 - vb) == 2, e2hi = (S - 2 - vb) == 3;
+    float m1 = ninf, m2 = ninf;
+    int f1 = T - 1, f2 = T - 1;
     auto load_cols = [&](int base, uint32_t &ca, uint32_t &cb) {
       ca = base + 1 < S ? 4u * col16[base >> 1] : 0u;
       cb = base + 3 < S ? 4u * col16[(base >> 1) + 1] : 0u;
@@ -208,7 +217,9 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
     auto load_below = [&](int base) { return base + 1 < S ? 4u * col16[(base >> 1) - 1] : 0u; };
     if (CTC) {
       const int l1 = vb >> 1;  // label index of state vb+1
-      if (vb + 1 < 3 || vb + 1 >= S || col16[l1] == col16[l1 - 1]) rep |= 1u;
+      // (FREE: state 1 takes move 2 from the virtual state -1, and has no label below to repeat)
+      if (FREE ? vb + 1 >= S || (vb + 1 >= 3 && col16[l1] == col16[l1 - 1])
+               : vb + 1 < 3 || vb + 1 >= S || col16[l1] == col16[l1 - 1]) rep |= 1u;
       if (vb + 3 >= S || col16[l1 + 1] == col16[l1]) rep |= 2u;
       ncm = load_below(vb + R);
     }
@@ -245,7 +256,7 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
     unsigned char *bpst = bpblk + (slot0 >> 2);  // this lane's byte of the group's first staging row
 
     // One frame.  No barrier: everything a lane needs from other lanes comes by shuffle.
-    auto frame = [&](auto slow_tag, unsigned char *bpdst, const char *rownext, const bool has_next) {
+    auto frame = [&](auto slow_tag, unsigned char *bpdst, const char *rownext, const bool has_next, const int i) {
       constexpr bool SLOW = decltype(slow_tag)::value;
       int lo = 0, hi = 0;
       if (SLOW) {
@@ -255,9 +266,10 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
         if (r >= T) { r -= T; ++q; }
       }
       // previous-frame scores of the three states below this lane's chunk (lane 0: junk, see top)
-      const float h1 = __shfl_up_sync(KAB_FULL_MASK, s3, 1);
+      float h1 = __shfl_up_sync(KAB_FULL_MASK, s3, 1);
       const float h2 = __shfl_up_sync(KAB_FULL_MASK, s2, 1);
       const float h3 = __shfl_up_sync(KAB_FULL_MASK, s1, 1);
+      if constexpr (FREE) if (first) h1 = 0.0f;
       // candidates: (even, odd) state pairs share one packed add
       float t0, t1, t2, t3;
       kab_add2(s0, s1, eb, t0, t1);
@@ -289,6 +301,11 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
         n3 = (a + 3u < wd) ? n3 : ninf;
       }
       s0 = n0; s1 = n1; s2 = n2; s3 = n3;
+      if constexpr (FREE) {
+        const float x1 = e1hi ? n2 : n0, x2 = e2hi ? n3 : n1;
+        if (x1 >= m1) { m1 = x1; f1 = i; }
+        if (x2 >= m2) { m2 = x2; f2 = i; }
+      }
       if (owned) *bpdst = (unsigned char)m;
       if (has_next) {  // emissions of frame i+1 (its chunk was published by an earlier barrier)
         rowc = rownext;
@@ -341,15 +358,15 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
       if (safe) {
 #pragma unroll
         for (int f = 0; f < G; ++f)
-          frame(KabFalse{}, bpst + f * NBP, f + 1 < G ? row0 + (f + 1) * VB : rowng, f + 1 < G || i0 + G < T);
+          frame(KabFalse{}, bpst + f * NBP, f + 1 < G ? row0 + (f + 1) * VB : rowng, f + 1 < G || i0 + G < T, i0 + f);
       } else if (nfr == G) {
         q = qg; r = rg;
 #pragma unroll
         for (int f = 0; f < G; ++f)
-          frame(KabTrue{}, bpst + f * NBP, f + 1 < G ? row0 + (f + 1) * VB : rowng, f + 1 < G || i0 + G < T);
+          frame(KabTrue{}, bpst + f * NBP, f + 1 < G ? row0 + (f + 1) * VB : rowng, f + 1 < G || i0 + G < T, i0 + f);
       } else {
         q = qg; r = rg;
-        for (int f = 0; f < nfr; ++f) frame(KabTrue{}, bpst + f * NBP, row0 + (f + 1) * VB, f + 1 < nfr);
+        for (int f = 0; f < nfr; ++f) frame(KabTrue{}, bpst + f * NBP, row0 + (f + 1) * VB, f + 1 < nfr, i0 + f);
       }
       qg = qn; rg = rn;
       bpst += G * NBP;
@@ -419,7 +436,10 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
 #endif
     echunks = ec0 + n_chunks;
 
-    if (CTC) {  // CTC end rule: the better of the last two states, S-2 on a tie (kab_common.cuh)
+    if constexpr (FREE) {  // the owners' maxima
+      if (owned && (vb == S - 1 || vb + 2 == S - 1)) { s_end[0] = m1; s_endf[0] = f1; }
+      if (owned && (vb + 1 == S - 2 || vb + 3 == S - 2)) { s_end[1] = m2; s_endf[1] = f2; }
+    } else if (CTC) {  // CTC end rule: the better of the last two states, S-2 on a tie (kab_common.cuh)
       if (owned) {
         if (vb + 0 == S - 1) s_end[0] = s0;
         if (vb + 1 == S - 1) s_end[0] = s1;
@@ -443,15 +463,22 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
     }
     if (tid == 0) kab_bulk_wait0();  // all backpointer blocks are in global memory
     const int any_bad = __syncthreads_or(poison != poison ? 1 : 0);
-    int v = s_vmax;
-    if (CTC) {
+    int v = s_vmax, t1 = T - 1;
+    if constexpr (FREE) {  // free end: the larger maximum, on a tie the later frame, then S-2 (L = 0: no frame is inside)
+      const bool top = s_end[0] > s_end[1] || (s_end[0] == s_end[1] && s_endf[0] > s_endf[1]);
+      v = top ? S - 1 : S - 2;
+      t1 = top ? s_endf[0] : s_endf[1];
+      if (S == 1) { v = -1; t1 = -1; }
+    } else if (CTC) {
       v = (S >= 2 && !(s_end[0] > s_end[1])) ? S - 2 : S - 1;
       // no path stays inside a window that clips (a covering window follows the recurrence instead)
       const bool clips = W < S || (int)(((int64_t)S * (T - 1)) / T) > half;
       if (clips && !(s_end[0] > ninf) && !(s_end[1] > ninf)) v = -1;
     }
-    const int status = any_bad ? 3 : (v < 0 ? 1 : 0);
-    if (owned && status == 0) {
+    const int status = any_bad ? 3 : (v < 0 && !FREE ? 1 : 0);
+    if constexpr (FREE) {
+      if (tid == 0) s_final = S == 1 ? 0.0f : (v == S - 1 ? s_end[0] : s_end[1]);
+    } else if (owned && status == 0) {
       if (vb + 0 == v) s_final = s0;
       if (vb + 1 == v) s_final = s1;
       if (vb + 2 == v) s_final = s2;
@@ -480,12 +507,16 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
       const float *lp = p.lp + lat.t_off * (int64_t)V;
       // Warp 0 walks a block while the other warps write the previous block's outputs.
       int slot = v % R;  // ring slot of the walker's state
+      // FREE: the walker is at state -1 (move 0) outside [t0, t1]; an unbanded ring slot is the state itself
+      const int vend = v;
+      if constexpr (FREE) v = -1;
       auto flush_block = [&](int blk, int first_thread, int n_threads) {
         const int i0 = blk * FB, i1 = min(T, i0 + FB);
         const int *pbuf = pathbuf + (blk & 1) * FB;
         for (int i = i0 + (tid - first_thread); i < i1; i += n_threads) {
           const int pv = pbuf[i - i0];
-          const int lab = (pv & 1) ? (int)col16[(pv - 1) >> 1] : (CTC ? blank : 0);
+          const bool is_lab = FREE ? (pv & 1) && pv > 0 : (pv & 1);  // (FREE: -1 outside [t0, t1])
+          const int lab = is_lab ? (int)col16[(pv - 1) >> 1] : (CTC ? blank : 0);
           out_path[i] = pv;
           out_lab[i] = lab;                              // align.py:106
           out_sc[i] = __ldg(&lp[(int64_t)i * V + lab]);  // align.py:107
@@ -502,9 +533,11 @@ __device__ __forceinline__ void kab_band_body(const KabLattice *__restrict__ lat
           if (lane == 0) {  // the walk itself is a dependent chain: one lane, shared-memory latency
             const unsigned char *rowp = blkp + (size_t)(i1 - 1 - i0) * NBP;
             for (int i = i1 - 1; i >= i0; --i, rowp -= NBP) {
+              if constexpr (FREE) if (i == t1) { v = vend; slot = vend; }
               const unsigned char byte = rowp[slot >> 2];
               pbuf[i - i0] = v;
-              const int mv = kab_decode_move((byte >> (2 * (slot & 3))) & 3u);
+              int mv = kab_decode_move((byte >> (2 * (slot & 3))) & 3u);
+              if constexpr (FREE) if (v < 0) mv = 0;
               v -= mv;
               slot -= mv;
               if (slot < 0) slot += R;
@@ -537,4 +570,11 @@ template <int MAXT>
 __global__ void __launch_bounds__(MAXT, 1) kab_band_ctc_kernel(const KabLattice *__restrict__ lats, int n_lat,
                                                                KabParams p, int blank) {
   kab_band_body<MAXT, false, true>(lats, n_lat, p, blank);
+}
+
+// CTC forced alignment with free ends (kab_plan_create_ctc_free)
+template <int MAXT>
+__global__ void __launch_bounds__(MAXT, 1) kab_band_ctc_free_kernel(const KabLattice *__restrict__ lats, int n_lat,
+                                                                    KabParams p, int blank) {
+  kab_band_body<MAXT, false, true, true>(lats, n_lat, p, blank);
 }

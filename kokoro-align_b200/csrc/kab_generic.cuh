@@ -11,7 +11,11 @@
 // test: the state's parity), blank column `blank`.  Default and long-form plans pass a W so wide that the
 // window is [0, S) in every frame; banded plans (kab_plan_create_ctc_band) pass beam_size.  A window that
 // clips somewhere and leaves both end states -inf: no path inside the band, status 1.
-template <int NT, bool CTC>
+// FREE: CTC with free ends (kab_plan_create_ctc_free; always unbanded): a virtual state -1 of score 0 in
+// every frame is state 0's move-1 and state 1's move-2 predecessor, thread 0 keeps running (score, frame)
+// maxima of the end states (>=: the later frame), and the walk starts at the chosen end (t1, v) and stops
+// at state -1; frames outside [t0, t1] get state -1 and the blank.
+template <int NT, bool CTC, bool FREE = false>
 __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ lats, int n_lat, const KabParams &p,
                                                  const int blank) {
   __shared__ unsigned int s_item;
@@ -35,10 +39,12 @@ __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ 
     float *prev = p.scratch + lat.scr_off;
     float *cur = prev + (S + 16);
 
-    if (tid == 0) __stcg(&prev[0], 0.0f);  // virtual start, align.py:57-58
+    if (tid == 0 && !FREE) __stcg(&prev[0], 0.0f);  // virtual start, align.py:57-58
     __syncthreads();
 
-    int64_t plo = 0, phi = 1;
+    int64_t plo = 0, phi = FREE ? 0 : 1;
+    float m1 = kab_neg_inf(), m2 = kab_neg_inf();  // FREE (thread 0): end maxima of S-1, S-2 and their frames
+    int64_t f1 = T - 1, f2 = T - 1;
     bool bad = false;
     for (int64_t i = 0; i < T; ++i) {
       int64_t lo = (S * i) / T - W / 2;  // align.py:64 (64-bit: S*i reaches 1e11)
@@ -57,8 +63,10 @@ __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ 
           const float e = __ldg(&row[ext]);
           // predecessors outside the previous window are -inf
           const float x0 = v >= plo && v < phi ? __ldcg(&prev[v]) : kab_neg_inf();
-          const float x1 = v - 1 >= plo && v - 1 < phi ? __ldcg(&prev[v - 1]) : kab_neg_inf();
-          const float x2 = lab && v >= 3 && v - 2 >= plo && v - 2 < phi && ext != raw[(v - 3) >> 1] ? __ldcg(&prev[v - 2]) : kab_neg_inf();
+          float x1 = v - 1 >= plo && v - 1 < phi ? __ldcg(&prev[v - 1]) : kab_neg_inf();
+          float x2 = lab && v >= 3 && v - 2 >= plo && v - 2 < phi && ext != raw[(v - 3) >> 1] ? __ldcg(&prev[v - 2]) : kab_neg_inf();
+          if constexpr (FREE) if (v == 0) x1 = 0.0f;  // the virtual state -1
+          if constexpr (FREE) if (v == 1) x2 = 0.0f;
           uint32_t code = 0;
           const float best = lab ? kab_ctc_label_sel(x0, x1, x2, code, 0) : kab_ctc_blank_sel(x0, x1, code, 0);
           __stcg(&cur[v], __fadd_rn(best, e));
@@ -84,6 +92,11 @@ __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ 
       __syncthreads();
       float *t = prev; prev = cur; cur = t;
       plo = lo; phi = hi;
+      if constexpr (FREE) if (tid == 0 && S >= 3) {
+        const float a1 = __ldcg(&prev[S - 1]), a2 = __ldcg(&prev[S - 2]);
+        if (a1 >= m1) { m1 = a1; f1 = i; }
+        if (a2 >= m2) { m2 = a2; f2 = i; }
+      }
     }
 
     // forced end state: highest active state of the last frame, align.py:99-101
@@ -96,7 +109,15 @@ __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ 
     int64_t v = s_vmax;
     // CTC end rule: the better of the last two states, S-2 on a tie (a state outside the last window: -inf);
     // none of them finite in a window that clips: no path inside the band
-    if (CTC) {
+    int64_t t1 = T - 1;
+    float fs_free = 0.0f;
+    if constexpr (FREE) {  // free end (thread 0's maxima): the larger one, on a tie the later frame, then S-2
+      const bool top = m1 > m2 || (m1 == m2 && f1 > f2);
+      v = top ? S - 1 : S - 2;
+      t1 = top ? f1 : f2;
+      fs_free = top ? m1 : m2;
+      if (S == 1) { v = -1; t1 = -1; fs_free = 0.0f; }  // L = 0: no frame is inside
+    } else if (CTC) {
       const float e1 = S - 1 >= plo && S - 1 < phi ? __ldcg(&prev[S - 1]) : kab_neg_inf();
       const float e2 = S >= 2 && S - 2 >= plo && S - 2 < phi ? __ldcg(&prev[S - 2]) : kab_neg_inf();
       v = (S >= 2 && !(e1 > e2)) ? S - 2 : S - 1;
@@ -107,16 +128,25 @@ __device__ __forceinline__ void kab_generic_body(const KabLattice *__restrict__ 
     if (tid == 0) {
       int st = 0;
       if (any_bad) st = 3;
-      else if (v < 0) st = 1;
+      else if (v < 0 && !FREE) st = 1;
       p.status[lat.index] = st;
-      if (p.final_score) p.final_score[lat.index] = st == 0 ? __ldcg(&prev[v]) : __int_as_float(0x7fc00000);
+      if (p.final_score) p.final_score[lat.index] = st == 0 ? (FREE ? fs_free : __ldcg(&prev[v])) : __int_as_float(0x7fc00000);
       if (st == 0) {
         int32_t *out_path = p.best_path + lat.t_off;
         int32_t *out_lab = p.best_labels + lat.t_off;
         float *out_sc = p.best_scores + lat.t_off;
+        const int64_t vend = v;
+        if constexpr (FREE) v = -1;
         for (int64_t i = T - 1; i >= 0; --i) {  // == flush_determined_path, align.py:21-40
           int64_t lo = (S * i) / T - W / 2;
           if (lo < 0) lo = 0;
+          if constexpr (FREE) if (i == t1) v = vend;
+          if constexpr (FREE) if (v < 0) {  // outside [t0, t1]
+            out_path[i] = -1;
+            out_lab[i] = blank;
+            out_sc[i] = __ldg(&lp[i * V + blank]);
+            continue;
+          }
           const int32_t ext = (v & 1) ? raw[(v - 1) >> 1] : (CTC ? blank : 0);
           const int32_t col = ext < 0 ? ext + (int32_t)V : ext;
           out_path[i] = (int32_t)v;
@@ -140,4 +170,11 @@ template <int NT>
 __global__ void __launch_bounds__(NT) kab_generic_ctc_kernel(const KabLattice *__restrict__ lats, int n_lat,
                                                              KabParams p, int blank) {
   kab_generic_body<NT, true>(lats, n_lat, p, blank);
+}
+
+// CTC forced alignment with free ends (kab_plan_create_ctc_free)
+template <int NT>
+__global__ void __launch_bounds__(NT) kab_generic_ctc_free_kernel(const KabLattice *__restrict__ lats, int n_lat,
+                                                                  KabParams p, int blank) {
+  kab_generic_body<NT, true, true>(lats, n_lat, p, blank);
 }

@@ -145,10 +145,12 @@ __device__ __forceinline__ void kab_ckpt_store(float *row, const float (&s)[K]) 
 // CTC forced alignment (kab_common.cuh): lane l >= 1 owns the same K states; the only halo is state
 // K*(l-1)-1 (moves reach two states down, and state v-2 of a label state v is inside the lane for
 // v >= 3 of the lane).  rep bit q = move 2 is forbidden into the lane's label state 2q+1.
-template <int K>
+// FREE (free-ends plans): lane 1's halo is the virtual state -1, score 0 in every frame.
+template <int K, bool FREE>
 __device__ __forceinline__ void kab_warp_frame_ctc(float (&s)[K], const float eb, const float (&el)[K / 2],
-                                                   const uint32_t rep, uint32_t &w, const int shift) {
-  const float h1 = __shfl_up_sync(KAB_FULL_MASK, s[K - 1], 1);
+                                                   const uint32_t rep, uint32_t &w, const int shift, const bool lane1) {
+  float h1 = __shfl_up_sync(KAB_FULL_MASK, s[K - 1], 1);
+  if (FREE && lane1) h1 = 0.0f;
   float n[K];
 #pragma unroll
   for (int q = 0; q < K / 2; ++q) {
@@ -162,7 +164,10 @@ __device__ __forceinline__ void kab_warp_frame_ctc(float (&s)[K], const float eb
 }
 
 // VCT: compile-time vocabulary (39) or 0 = runtime p.V.  CTC: the CTC forced-alignment recurrence.
-template <int K, int VCT, bool MM, bool CTC>
+// FREE: CTC with free ends (kab_plan_create_ctc_free): a virtual state -1 of score 0 below state 0 in every
+// frame, running (score, frame) maxima of the end states S-1 and S-2 (>=: the later frame), the walk starts
+// at the chosen end (t1, v) and stops at state -1; frames outside [t0, t1] get state -1 and the blank.
+template <int K, int VCT, bool MM, bool CTC, bool FREE = false>
 __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float *stage_base, uint64_t *bars,
                                uint16_t *labtab, const uint64_t policy, uint32_t &chunk_counter, const int lane,
                                const int blank) {
@@ -195,14 +200,30 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
     const uint32_t col = (v > 0 && v < S) ? col16[(v - 1) >> 1] : 0u;
     coff[q] = 4u * col;
     if (v > 0 && v < S) labtab[(v - 1) >> 1] = (uint16_t)col;  // per-warp copy for the backtrack's output rows
-    if (CTC && (v < 3 || v >= S || col == col16[(v - 3) >> 1])) rep |= 1u << q;
+    // (FREE: state 1 takes move 2 from the virtual state -1, and has no label below to repeat)
+    if (CTC && (FREE ? v < 1 || v >= S || (v >= 3 && col == col16[(v - 3) >> 1])
+                     : v < 3 || v >= S || col == col16[(v - 3) >> 1])) rep |= 1u << q;
   }
   const uint32_t boff = CTC ? 4u * (uint32_t)blank : 0u;  // byte offset of the blank's column
 
   float s[K];
 #pragma unroll
   for (int k = 0; k < K; ++k) s[k] = kab_neg_inf();
-  if (lane1) s[0] = 0.0f;  // virtual start state 0, score 0 (align.py:57-58)
+  if (lane1 && !FREE) s[0] = 0.0f;  // virtual start state 0, score 0 (align.py:57-58)
+  // FREE: running maxima (score, frame) of the end states in their owner lanes: register k1e holds state
+  // S-1 there (an even state, so an even register), k2e state S-2 (odd)
+  const int k1e = (S - 1) % K, k2e = (S - 2) % K;
+  float m1 = kab_neg_inf(), m2 = kab_neg_inf();
+  int f1 = T - 1, f2 = T - 1;
+  auto track_end = [&](const int t) {
+    float e1 = s[0], e2 = s[1];
+#pragma unroll
+    for (int k = 2; k < K; k += 2) if (k == k1e) e1 = s[k];
+#pragma unroll
+    for (int k = 3; k < K; k += 2) if (k == k2e) e2 = s[k];
+    if (e1 >= m1) { m1 = e1; f1 = t; }
+    if (e2 >= m2) { m2 = e2; f2 = t; }
+  };
 
   // -- emission pipeline: the k-th chunk issued uses stage (chunk_counter + k) % STAGES.  F * V * 4 is a multiple
   // of 16, so every chunk of the lattice has the same 16-byte skew and all but the last one are
@@ -274,8 +295,9 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
           float el[K / 2];
 #pragma unroll
           for (int q = 0; q < K / 2; ++q) el[q] = *reinterpret_cast<const float *>(rb + coff[q]);
-          if (CTC) kab_warp_frame_ctc<K>(s, eb, el, rep, word, f * BPF);
+          if (CTC) kab_warp_frame_ctc<K, FREE>(s, eb, el, rep, word, f * BPF, lane1);
           else kab_warp_frame_bp<K, MM>(s, eb, el, lane1, word, f * BPF, one, mm1, mm2, mm3);
+          if (FREE) track_end(c * F + gi * FPW + f);
         }
         *bprow = word;
         bprow += 32;
@@ -290,8 +312,9 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
 #pragma unroll
           for (int q = 0; q < K / 2; ++q) el[q] = *reinterpret_cast<const float *>(rowb + coff[q]);
           uint32_t fw = 0;
-          if (CTC) kab_warp_frame_ctc<K>(s, eb, el, rep, fw, 0);
+          if (CTC) kab_warp_frame_ctc<K, FREE>(s, eb, el, rep, fw, 0, lane1);
           else kab_warp_frame_bp<K, MM>(s, eb, el, lane1, fw, 0, one, mm1, mm2, mm3);
+          if (FREE) track_end(c * F + n_groups * FPW + f);
           word |= fw << (f * BPF);
         }
         *bprow = word;
@@ -332,8 +355,18 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
     for (int k = 1; k < K; ++k) if (k == u % K) mine = s[k];
     return __shfl_sync(KAB_FULL_MASK, mine, u / K + 1);
   };
-  int v;
-  if (CTC) {  // CTC end rule: the better of the last two states, S-2 on a tie (kab_common.cuh)
+  int v, t1 = T - 1;
+  float fs_free = 0.0f;
+  if (FREE) {  // free end: the larger maximum, on a tie the later frame, then S-2 (L = 0: no frame is inside)
+    const int o1 = (S - 1) / K + 1, o2 = (S - 2) / K + 1;
+    const float a1 = __shfl_sync(KAB_FULL_MASK, m1, o1), a2 = __shfl_sync(KAB_FULL_MASK, m2, o2);
+    const int g1 = __shfl_sync(KAB_FULL_MASK, f1, o1), g2 = __shfl_sync(KAB_FULL_MASK, f2, o2);
+    const bool top = a1 > a2 || (a1 == a2 && g1 > g2);
+    v = top ? S - 1 : S - 2;
+    t1 = top ? g1 : g2;
+    fs_free = top ? a1 : a2;
+    if (S == 1) { v = -1; t1 = -1; fs_free = 0.0f; }
+  } else if (CTC) {  // CTC end rule: the better of the last two states, S-2 on a tie (kab_common.cuh)
     v = S - 1;
     if (S >= 2) {
       const float a1 = score_of(S - 1), a2 = score_of(S - 2);
@@ -349,10 +382,12 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
     v = __reduce_max_sync(KAB_FULL_MASK, cand);
   }
   const bool any_bad = __any_sync(KAB_FULL_MASK, poison != poison);
-  const int status = any_bad ? 3 : (v < 0 ? 1 : 0);
+  const int status = any_bad ? 3 : (v < 0 && !FREE ? 1 : 0);
   {
     float fs = __int_as_float(0x7fc00000);
-    if (status == 0) {
+    if (FREE) {
+      if (status == 0) fs = fs_free;
+    } else if (status == 0) {
       float mine = s[0];
 #pragma unroll
       for (int k = 1; k < K; ++k) if (k == v % K) mine = s[k];
@@ -468,9 +503,12 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
     // so a frame costs one shuffle, one shift/mask and a few adds: the 2-bit code IS the move
     // (kab_decode_move).  Frames >= T of the last block have all-zero codes (moves 0), so the
     // block bodies need no bounds checks.
-    int myv = 0, pend_t = -1;
+    // FREE: the walk is at state -1 (lane 0's register K-1, whose codes are all 0) until frame t1
+    const int vend = v;
+    if (FREE) v = -1;
+    int myv = FREE ? -1 : 0, pend_t = -1;
     float pend_s = 0.0f;
-    int own1 = v / K + 1, k2 = 2 * (v - (v / K) * K);
+    int own1 = FREE ? 0 : v / K + 1, k2 = FREE ? 2 * K - 2 : 2 * (v - (v / K) * K);
     uint32_t wr[RB], wn[RB];
     const int rb_last = ((n_rows - 1) / RB) * RB;
     fetch(rb_last, wr);
@@ -482,6 +520,7 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
       for (int r = RB - 1; r >= 0; --r) {
 #pragma unroll
         for (int f = FPW - 1; f >= 0; --f) {
+          if (FREE && fb + r * FPW + f == t1) { v = vend; own1 = vend / K + 1; k2 = 2 * (vend % K); }
           const uint32_t w = __shfl_sync(KAB_FULL_MASK, wr[r], own1);
           if (lb == r * FPW + f) myv = v;
           const int mv = (int)((w >> (f * BPF + k2)) & 3u);
@@ -496,7 +535,8 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
         const int t = fb + lane;
         pend_t = -1;
         if (t < T) {
-          const int lab = (myv & 1) ? (int)labtab[(myv - 1) >> 1] : (CTC ? blank : 0);
+          const bool is_lab = FREE ? (myv & 1) && myv > 0 : (myv & 1);  // (FREE: -1 outside [t0, t1])
+          const int lab = is_lab ? (int)labtab[(myv - 1) >> 1] : (CTC ? blank : 0);
           out_path[t] = myv;
           out_lab[t] = lab;                           // align.py:106
           pend_s = __ldg(&lp[(int64_t)t * V + lab]);  // align.py:107
@@ -510,7 +550,7 @@ __device__ void kab_warp_align(const KabLattice &lat, const KabParams &p, float 
   }
 }
 
-template <int VCT, bool MM, bool CTC>
+template <int VCT, bool MM, bool CTC, bool FREE = false>
 __device__ __forceinline__ void kab_warp_body(const KabLattice *__restrict__ lats, int n_lat, const KabParams &p,
                                               const int blank) {
   extern __shared__ __align__(128) unsigned char kab_smem[];
@@ -540,10 +580,10 @@ __device__ __forceinline__ void kab_warp_body(const KabLattice *__restrict__ lat
     if (item >= (unsigned int)n_lat) break;
     const KabLattice lat = lats[item];
     switch (lat.k) {
-      case 2: kab_warp_align<2, VCT, MM, CTC>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
-      case 4: kab_warp_align<4, VCT, MM, CTC>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
-      case 6: kab_warp_align<6, VCT, MM, CTC>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
-      default: kab_warp_align<8, VCT, MM, CTC>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
+      case 2: kab_warp_align<2, VCT, MM, CTC, FREE>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
+      case 4: kab_warp_align<4, VCT, MM, CTC, FREE>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
+      case 6: kab_warp_align<6, VCT, MM, CTC, FREE>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
+      default: kab_warp_align<8, VCT, MM, CTC, FREE>(lat, p, stage_base, bars, labtab, policy, chunk_counter, lane, blank); break;
     }
     __syncwarp();
   }
@@ -560,4 +600,10 @@ __global__ void __launch_bounds__(KAB_WARPS_PER_CTA * 32, KAB_WARP_MINBLOCKS)
 __global__ void __launch_bounds__(KAB_WARPS_PER_CTA * 32, KAB_WARP_MINBLOCKS)
     kab_warp_ctc_kernel(const KabLattice *__restrict__ lats, int n_lat, KabParams p, int blank) {
   kab_warp_body<0, false, true>(lats, n_lat, p, blank);
+}
+
+// CTC forced alignment with free ends (kab_plan_create_ctc_free)
+__global__ void __launch_bounds__(KAB_WARPS_PER_CTA * 32, KAB_WARP_MINBLOCKS)
+    kab_warp_ctc_free_kernel(const KabLattice *__restrict__ lats, int n_lat, KabParams p, int blank) {
+  kab_warp_body<0, false, true, true>(lats, n_lat, p, blank);
 }

@@ -91,7 +91,11 @@ __host__ __device__ inline KabWideGeom kab_wide_geom(int stage_bytes) {
 // still absorb it.  The end states S-1 and S-2 may sit in different warps (S = 1 mod 104: S-1 is the
 // first state of the top warp), so their owners publish both scores to the lattice's scratch and the
 // backtrack CTA applies the end rule.
-template <bool CTC>
+// FREE: CTC with free ends (kab_plan_create_ctc_free): the lane of state 0 takes the virtual state -1 (score
+// 0 in every frame) as its halo, the owners of S-1 and S-2 keep running (score, frame) maxima (>=: the later
+// frame) and publish them (frames: the two words at kab_wide_cand_off, unused by CTC plans), and the
+// backtrack CTA starts the walk at the chosen end (t1, v), possibly mid-group, and stops it at state -1.
+template <bool CTC, bool FREE = false>
 __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lats, int n_lat, const KabParams &p,
                                               unsigned char *wide_ws, const int blank) {
   constexpr int G = KAB_BAND_G, GH = KAB_BAND_GHOST, OW = KAB_BAND_OW;
@@ -107,6 +111,7 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
   float *stage_base = reinterpret_cast<float *>(kab_smem + geo.stage_off);
   __shared__ int s_v;
   __shared__ int s_status;
+  __shared__ int s_t1;  // FREE: end frame
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const bool is_bt = blockIdx.x == gridDim.x - 1;
@@ -195,7 +200,12 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
         const uint16_t *col16 = p.col16 + lat.col_off;
         const uint32_t one = p.one;
         const int vb = OW * gw + 4 * (lane - GH);  // first state of this lane (ghost lanes: the 24 below)
-        float s0 = (vb == 0) ? 0.0f : ninf, s1 = ninf, s2 = ninf, s3 = ninf;  // start state 0 (align.py:57-58)
+        float s0 = (vb == 0 && !FREE) ? 0.0f : ninf, s1 = ninf, s2 = ninf, s3 = ninf;  // start state 0 (align.py:57-58)
+        const bool first = FREE && vb == 0;  // FREE: the lane whose halo is the virtual state -1
+        // FREE: running end maxima; state S-1 is register 0 or 2 of its owner, S-2 register 1 or 3
+        const bool e1hi = (S - 1 - vb) == 2, e2hi = (S - 2 - vb) == 3;
+        float m1 = ninf, m2 = ninf;
+        int f1 = T - 1, f2 = T - 1;
         const uint32_t c1 = (vb + 1 > 0 && vb + 1 < S) ? 4u * col16[vb >> 1] : 0u;
         const uint32_t c3 = (vb + 3 > 0 && vb + 3 < S) ? 4u * col16[(vb >> 1) + 1] : 0u;
         const uint32_t boff = CTC ? 4u * (uint32_t)blank : 0u;  // byte offset of the blank's column
@@ -204,7 +214,9 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
         uint32_t rep = 0;
         if (CTC) {
           const int l1 = vb >> 1;  // label index of state vb+1
-          if (vb + 1 < 3 || vb + 1 >= S || col16[l1] == col16[l1 - 1]) rep |= 1u;
+          // (FREE: state 1 takes move 2 from the virtual state -1, and has no label below to repeat)
+          if (FREE ? vb + 1 < 1 || vb + 1 >= S || (vb + 1 >= 3 && col16[l1] == col16[l1 - 1])
+                   : vb + 1 < 3 || vb + 1 >= S || col16[l1] == col16[l1 - 1]) rep |= 1u;
           if (vb + 3 < 3 || vb + 3 >= S || col16[l1 + 1] == col16[l1]) rep |= 2u;
         }
         uint32_t st = ec0 % NS, ph = (ec0 / NS) & 1u;
@@ -256,12 +268,18 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
         };
         // CTC: select on the previous scores, then one add; only h1 comes from the lane below
         auto frame_ctc = [&](const float xb, const float x1, const float x3, uint32_t &w, const int sh) {
-          const float h1 = __shfl_up_sync(KAB_FULL_MASK, s3, 1);
+          float h1 = __shfl_up_sync(KAB_FULL_MASK, s3, 1);
+          if constexpr (FREE) if (first) h1 = 0.0f;
           const float n0 = __fadd_rn(kab_ctc_blank_sel(s0, h1, w, sh + 0), xb);
           const float n1 = __fadd_rn(kab_ctc_label_sel(s1, s0, rep & 1u ? ninf : h1, w, sh + 2), x1);
           const float n2 = __fadd_rn(kab_ctc_blank_sel(s2, s1, w, sh + 4), xb);
           const float n3 = __fadd_rn(kab_ctc_label_sel(s3, s2, rep & 2u ? ninf : s1, w, sh + 6), x3);
           s0 = n0; s1 = n1; s2 = n2; s3 = n3;
+        };
+        auto track_end = [&](const int t) {
+          const float x1 = e1hi ? s2 : s0, x2 = e2hi ? s3 : s1;
+          if (x1 >= m1) { m1 = x1; f1 = t; }
+          if (x2 >= m2) { m2 = x2; f2 = t; }
         };
 
         // ---- build the wavefront: wait until the warp below is KAB_WD_LAG groups ahead (its message
@@ -323,6 +341,7 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
             for (int f = 0; f < G; ++f) {
               if (CTC) frame_ctc(eb[f], e1[f], e3[f], f < 4 ? wlo : whi, 8 * (f & 3));
               else frame(eb[f], e1[f], e3[f], f < 4 ? wlo : whi, 8 * (f & 3));
+              if constexpr (FREE) track_end(i0 + f);
             }
           } else {
 #pragma unroll
@@ -330,6 +349,7 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
               if (f < nfr) {
                 if (CTC) frame_ctc(eb[f], e1[f], e3[f], f < 4 ? wlo : whi, 8 * (f & 3));
                 else frame(eb[f], e1[f], e3[f], f < 4 ? wlo : whi, 8 * (f & 3));
+                if constexpr (FREE) track_end(i0 + f);
               }
           }
           KAB_WTM(td);
@@ -392,7 +412,11 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
         // ---- this warp's highest active state and its score (align.py:99-101), then "finished"
         int cand = -1;
         float cs = 0.0f;
-        if (CTC) {  // the scores of the two end states S-1 -> ctl[3], S-2 -> ctl[0] (end rule: backtrack CTA)
+        if constexpr (FREE) {  // the end states' maxima S-1 -> ctl[3], S-2 -> ctl[0], and their frames
+          unsigned int *ef = reinterpret_cast<unsigned int *>(ws + kab_wide_cand_off());
+          if (owned && (vb == S - 1 || vb + 2 == S - 1)) { ctl[3] = __float_as_uint(m1); ef[0] = (unsigned int)f1; }
+          if (owned && (vb + 1 == S - 2 || vb + 3 == S - 2)) { ctl[0] = __float_as_uint(m2); ef[1] = (unsigned int)f2; }
+        } else if (CTC) {  // the scores of the two end states S-1 -> ctl[3], S-2 -> ctl[0] (end rule: backtrack CTA)
           if (owned) {
             if (vb + 0 == S - 1) ctl[3] = __float_as_uint(s0);
             if (vb + 2 == S - 1) ctl[3] = __float_as_uint(s2);
@@ -439,7 +463,19 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
         if (done >= (unsigned int)nww) break;
         __nanosleep(500);
       }
-      if (CTC) {  // end rule: S-1 if a[S-1] > a[S-2], else S-2 (a tie, and two -inf, pick S-2)
+      if constexpr (FREE) {  // free end: the larger maximum, on a tie the later frame, then S-2
+        const int S = 2 * lat.L + 1;
+        const float a1 = __uint_as_float(kab_ld_volatile_u32(&ctl[3])), a2 = __uint_as_float(kab_ld_volatile_u32(&ctl[0]));
+        const unsigned int *ef = reinterpret_cast<const unsigned int *>(ws + kab_wide_cand_off());
+        const int g1 = (int)kab_ld_volatile_u32(&ef[0]), g2 = (int)kab_ld_volatile_u32(&ef[1]);
+        const bool top = a1 > a2 || (a1 == a2 && g1 > g2);
+        const int status = kab_ld_volatile_u32(&ctl[1]) ? 3 : 0;
+        s_v = top ? S - 1 : S - 2;
+        s_t1 = top ? g1 : g2;
+        s_status = status;
+        p.status[lat.index] = status;
+        if (p.final_score) p.final_score[lat.index] = status == 0 ? (top ? a1 : a2) : __int_as_float(0x7fc00000);
+      } else if (CTC) {  // end rule: S-1 if a[S-1] > a[S-2], else S-2 (a tie, and two -inf, pick S-2)
         const int S = 2 * lat.L + 1;
         const float a1 = __uint_as_float(kab_ld_volatile_u32(&ctl[3])), a2 = __uint_as_float(kab_ld_volatile_u32(&ctl[0]));
         const int v = a1 > a2 ? S - 1 : S - 2;
@@ -463,6 +499,7 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
     }
     __syncthreads();
     int v = s_v;
+    const int t1 = FREE ? s_t1 : 0;
     if (s_status == 0) {
       const int NT = KAB_WD_THREADS;
       const uint16_t *col16 = p.col16 + lat.col_off;
@@ -489,7 +526,8 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
         const int *pbuf = pathbuf + (b & 1) * FBK;
         for (int i = i0 + (tid - first_thread); i < i1; i += n_threads) {
           const int pv = pbuf[i - i0];
-          const int lab = (pv & 1) ? (int)col16[(pv - 1) >> 1] : (CTC ? blank : 0);
+          const bool is_lab = FREE ? (pv & 1) && pv > 0 : (pv & 1);  // (FREE: -1 outside [t0, t1])
+          const int lab = is_lab ? (int)col16[(pv - 1) >> 1] : (CTC ? blank : 0);
           out_path[i] = pv;
           out_lab[i] = lab;                              // align.py:106
           out_sc[i] = __ldg(&lp[(int64_t)i * V + lab]);  // align.py:107
@@ -533,8 +571,14 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
           };
           uint2 pw0 = make_uint2(0u, 0u), pw1 = pw0;
           const unsigned char *pfrom = nullptr;
-          for (int gq = (i1 - 1 - i0) >> 3; gq >= 0; --gq) {
-            int f = min(7, i1 - 1 - i0 - gq * 8);
+          // FREE: frames above t1 and, once the walk has reached state -1, every frame below are outside
+          int top = i1 - 1 - i0;
+          if constexpr (FREE) {
+            top = v < 0 ? -1 : min(top, t1 - i0);
+            for (int j = max(top + 1, 0); j < i1 - i0; ++j) pbuf[j] = -1;
+          }
+          for (int gq = top >> 3; gq >= 0; --gq) {
+            int f = min(7, top - gq * 8);
             int *pg = pbuf + gq * 8;
             if (f == 7) {
               const unsigned char *grow = rows + gq * 256;
@@ -555,6 +599,11 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
               }
               int nchg;
               f = kab_walk_group8(w0, w1, have1, v, k2, pg, nchg);
+              if constexpr (FREE) if (v < 0) {  // reached state -1 (column 0 of region 0: the walk stopped there)
+                for (; f >= 0; --f) pg[f] = -1;
+                for (int j = 0; j < gq * 8; ++j) pbuf[j] = -1;
+                break;
+              }
               for (int c = 0; c < nchg; ++c) step_column();
             }
             for (; f >= 0; --f) {  // generic step
@@ -563,10 +612,16 @@ __device__ __forceinline__ void kab_wide_body(const KabLattice *__restrict__ lat
               const int mv = (int)((byte >> k2) & 3u);
               v -= mv;
               k2 -= 2 * mv;
+              if constexpr (FREE) if (v < 0) break;
               if (k2 < 0) {
                 k2 += 8;
                 step_column();
               }
+            }
+            if constexpr (FREE) if (v < 0) {
+              for (--f; f >= 0; --f) pg[f] = -1;
+              for (int j = 0; j < gq * 8; ++j) pbuf[j] = -1;
+              break;
             }
           }
         } else if (tid >= 32 && b + 1 < n_blocks) {
@@ -589,4 +644,10 @@ __global__ void __launch_bounds__(KAB_WD_THREADS, 1)
 __global__ void __launch_bounds__(KAB_WD_THREADS, 1)
     kab_wide_ctc_kernel(const KabLattice *__restrict__ lats, int n_lat, KabParams p, unsigned char *wide_ws, int blank) {
   kab_wide_body<true>(lats, n_lat, p, wide_ws, blank);
+}
+
+// CTC forced alignment with free ends (kab_plan_create_ctc_free)
+__global__ void __launch_bounds__(KAB_WD_THREADS, 1)
+    kab_wide_ctc_free_kernel(const KabLattice *__restrict__ lats, int n_lat, KabParams p, unsigned char *wide_ws, int blank) {
+  kab_wide_body<true, true>(lats, n_lat, p, wide_ws, blank);
 }
