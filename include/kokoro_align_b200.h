@@ -253,6 +253,31 @@ int kab_plan_segment_stats_device(kab_plan *plan, const int32_t *d_best_path, co
                                   kab_segment_record *d_records, uint8_t *d_labels_u8, void *stream);
 
 /*
+ * Forward-backward posteriors of a CTC alignment (DESIGN.md 3.9f), a second device pass over a CTC plan's
+ * outputs.  For lattice b (ext = the blank-interleaved states, S = 2L + 1, move 2 into an odd v >= 3 iff
+ * ext[v] != ext[v-2]) and the plan's window [lo_t, hi_t) of frame t ([0, S) for kab_plan_create_ctc and
+ * kab_plan_create_ctc_long plans, kab_plan_create_ctc_band's band otherwise), in natural log:
+ *   alpha_0 = lp[0, blank] at state 0 and lp[0, ext[1]] at state 1; alpha_t(v) = logsumexp of alpha_{t-1} over
+ *   v, v-1 and v-2 where allowed, + lp[t, ext[v]]; beta_{T-1} = 0 at S-1 and S-2; beta_t(v) = logsumexp over
+ *   the successors v' of beta_{t+1}(v') + lp[t+1, ext[v']]; every state outside its frame's window is -inf.
+ *   d_log_likelihood[b] (double) = log Z = logsumexp(alpha_{T-1}(S-1), alpha_{T-1}(S-2)): -ctc_loss of an
+ *     unbanded lattice; for a banded one, the log of the probability of the paths inside the band.
+ *   d_posteriors[t] (float32, [sum T]) = exp(alpha_t(p_t) + beta_t(p_t) - log Z), clamped to [0, 1], for the
+ *     state path p = d_best_path (usually what kab_plan_run_device wrote; any path is accepted, a p_t outside
+ *     the window gives 0).
+ * A lattice whose d_status is not 0 gets posteriors 0 and log-likelihood NaN; log Z = -inf gives
+ * posteriors 0.  d_log_probs are the caller's [sum T, V] rows (16-byte aligned), read by label: any
+ * vocab_size works.  KAB_E_UNSUPPORTED for a plan that is not a CTC plan, a free-ends plan, or a lattice
+ * whose window min(beam_size, S) exceeds KAB_POSTERIOR_MAX_STATES (use kab_plan_create_ctc_band).  The
+ * first call builds and uploads what the pass needs (labels, lattice lists, 16 bytes per frame of
+ * values); kab_plan_get_info does not count it.  Asynchronous on `stream`; kab_plan_destroy waits for it.
+ */
+#define KAB_POSTERIOR_MAX_STATES 28000 /* the states of two float buffers in one CTA's shared memory */
+int kab_plan_ctc_posteriors_device(kab_plan *plan, const float *d_log_probs, const int32_t *d_best_path,
+                                   const int32_t *d_status, double *d_log_likelihood, float *d_posteriors,
+                                   void *stream);
+
+/*
  * kab_plan_run_host (is_logits = 0) / kab_plan_run_host_logits (is_logits != 0) that also -- or
  * only -- returns the segment records: h_best_path / h_best_labels / h_best_scores may be NULL
  * (all three), and then 24 bytes per segment come back instead of 12 bytes per frame;

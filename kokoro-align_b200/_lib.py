@@ -12,17 +12,18 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _ROOT = os.path.dirname(_HERE)
 SO_PATH = os.path.join(_HERE, "libkokoro_align_b200.so")
 SOURCES = [os.path.join(_HERE, "csrc", f) for f in
-           ("kab_api.cu", "kab_common.cuh", "kab_warp.cuh", "kab_band.cuh", "kab_bandp.cuh", "kab_bandq.cuh", "kab_bandr.cuh", "kab_btpar.cuh", "kab_wide.cuh", "kab_segstats.cuh", "kab_spans.cuh", "kab_compact.cuh", "kab_generic.cuh", "kab_softmax.cuh", "kab_pool.h", "kab_text.h", "kab_debug.h")]
+           ("kab_api.cu", "kab_common.cuh", "kab_warp.cuh", "kab_band.cuh", "kab_bandp.cuh", "kab_bandq.cuh", "kab_bandr.cuh", "kab_btpar.cuh", "kab_wide.cuh", "kab_segstats.cuh", "kab_posterior.cuh", "kab_spans.cuh", "kab_compact.cuh", "kab_generic.cuh", "kab_softmax.cuh", "kab_pool.h", "kab_text.h", "kab_debug.h")]
 HEADER = os.path.join(_ROOT, "include", "kokoro_align_b200.h")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
 
 KAB_OK, KAB_E_CUDA, KAB_E_BAD_ARG, KAB_E_NOMEM, KAB_E_UNSUPPORTED = 0, -1, -2, -3, -4
 ST_OK, ST_DEAD_BAND, ST_BAD_LABEL, ST_NONFINITE = 0, 1, 2, 3
+POSTERIOR_MAX_STATES = 28000  # KAB_POSTERIOR_MAX_STATES
 
 EXPORTS = ["kab_version", "kab_error_string", "kab_last_cuda_error", "kab_device_count",
            "kab_plan_create", "kab_plan_create_ctc", "kab_plan_create_ctc_long", "kab_plan_create_ctc_free", "kab_plan_create_ctc_band", "kab_plan_get_info", "kab_plan_destroy", "kab_plan_run_device",
-           "kab_plan_run_host", "kab_plan_run_host_logits", "kab_plan_run_host_segments", "kab_plan_segment_stats_device", "kab_log_softmax_device", "kab_log_softmax_pack_device", "kab_merge_tokens_device", "kab_word_spans_device", "kab_ctc_best_path", "kab_encode_transcript", "kab_merge_repeated", "kab_pool_trim", "kab_host_alloc", "kab_host_free"]
+           "kab_plan_run_host", "kab_plan_run_host_logits", "kab_plan_run_host_segments", "kab_plan_segment_stats_device", "kab_plan_ctc_posteriors_device", "kab_log_softmax_device", "kab_log_softmax_pack_device", "kab_merge_tokens_device", "kab_word_spans_device", "kab_ctc_best_path", "kab_encode_transcript", "kab_merge_repeated", "kab_pool_trim", "kab_host_alloc", "kab_host_free"]
 
 
 class PlanInfo(ctypes.Structure):
@@ -113,6 +114,7 @@ def lib():
     L.kab_log_softmax_device.argtypes = [vp, vp, i64, i32, vp]
     L.kab_log_softmax_pack_device.argtypes = [vp, i64, i64, i32, vp, vp, i64, vp]
     L.kab_plan_segment_stats_device.argtypes = [vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp]
+    L.kab_plan_ctc_posteriors_device.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     L.kab_plan_run_host_segments.argtypes = [vp, vp, i32, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.kab_merge_tokens_device.argtypes = [i64, vp, vp, vp, i32, vp, vp, vp]
     L.kab_word_spans_device.argtypes = [i64, vp, vp, vp, vp, vp, vp, vp, vp]

@@ -242,6 +242,28 @@ class AlignPlan:
                         final.data_ptr(), status.data_ptr(), s.cuda_stream)
         return path, labs, scores, final, status
 
+    def ctc_posteriors_torch(self, log_probs, best_path, status, stream=None):
+        """Forward-backward posteriors of a CTC plan's state paths (kab_plan_ctc_posteriors_device, DESIGN.md
+        3.9f), on the device: log_probs CUDA float32 [sum T, V] (the rows that were aligned), best_path int32
+        [sum T] (run_torch's state path, or any other state path), status int32 [B] (run_torch's).  Returns
+        (posteriors float32 [sum T], log_likelihood float64 [B]): posteriors[t] = exp(alpha_t(p_t) + beta_t(p_t) -
+        log Z), the probability that the lattice's paths pass through state p_t at frame t (0 where p_t is outside
+        the window), and log Z, the log of the total probability of the transcript (-ctc_loss; a banded plan: of
+        the paths inside the band).  A lattice whose status is not 0 gets 0 and NaN.  Asynchronous.  KabError for
+        a Kokoro or free-ends plan and for a window min(beam_size, S) above POSTERIOR_MAX_STATES."""
+        import torch
+        assert log_probs.is_cuda and log_probs.dtype == torch.float32 and log_probs.is_contiguous()
+        assert tuple(log_probs.shape) == (self.total_T, self.V), (tuple(log_probs.shape), self.total_T, self.V)
+        assert best_path.dtype == torch.int32 and best_path.is_contiguous() and best_path.numel() == self.total_T
+        assert status.dtype == torch.int32 and status.is_contiguous() and status.numel() == self.B
+        dev = log_probs.device
+        post = torch.empty(self.total_T, dtype=torch.float32, device=dev)
+        ll = torch.empty(self.B, dtype=torch.float64, device=dev)
+        s = torch.cuda.current_stream(dev) if stream is None else stream
+        _lib.check(_lib.lib().kab_plan_ctc_posteriors_device(
+            self._h, _vp(log_probs), _vp(best_path), _vp(status), _vp(ll), _vp(post), ctypes.c_void_p(s.cuda_stream)))
+        return post, ll
+
 
 def ctc_best_path(log_probs, labels, beam_size=1000, max_move=4, return_final_score=False):
     """Drop-in for kokoro_align.align.ctc_best_path (align.py:43-109).
@@ -327,12 +349,26 @@ def _check_free_ends(free_ends, beam_size):
                          "spans the whole recording")
 
 
+def _check_posteriors(free_ends, beam_size, S, where=lambda b: ""):
+    """posteriors=True: no free ends, and every item's window min(beam_size, S) within the posterior pass's limit.
+    S: int64 numpy [B] states per item."""
+    if free_ends:
+        raise ValueError("posteriors=True does not combine with free_ends=True")
+    w = S if beam_size is None else np.minimum(S, int(beam_size))
+    over = np.flatnonzero(w > _lib.POSTERIOR_MAX_STATES)
+    if over.size:
+        b = int(over[0])
+        raise ValueError(f"{where(b)}posteriors need at most {_lib.POSTERIOR_MAX_STATES} states per frame, the item has "
+                         f"S = {int(S[b])} (2 L + 1) states in a window of {int(w[b])}; pass beam_size <= "
+                         f"{_lib.POSTERIOR_MAX_STATES} for banded posteriors")
+
+
 def _band_lost(beam_size, where=""):
     return ValueError(f"{where}no CTC path stays within beam_size={beam_size}; widen the beam")
 
 
 def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, blank=0, *, long_form=False,
-                 beam_size=None, free_ends=False):
+                 beam_size=None, free_ends=False, posteriors=False):
     """Drop-in for torchaudio.functional.forced_align (same arguments, output shapes and dtypes,
     exception types): log_probs float32 [1, T, V], targets int32 / int64 [1, L] on the same device
     (CPU or CUDA).  Returns (paths [1, T] of the targets' dtype: the token id of every frame,
@@ -353,7 +389,13 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
     of it (speech before or after the transcript, a passage inside a longer recording; AlignPlan.ctc).
     Frames outside the window hold the blank and its log-prob, so merge_tokens gives the spans of the
     text.  For a gap in the middle of the transcript, append a zero log-prob column as a <star> token
-    (the MMS recipe) and put it in the targets.  Not combined with beam_size (ValueError)."""
+    (the MMS recipe) and put it in the targets.  Not combined with beam_size (ValueError).
+    posteriors=True: also returns the forward-backward posterior of the aligned state in every frame and the log
+    of the total probability of the targets (AlignPlan.ctc_posteriors_torch), computed on the device from the
+    same plan and rows: (paths, scores, posteriors float32 [1, T], log_likelihood float64 [1]).  The paths and
+    scores are those of posteriors=False; CPU tensors run on the current CUDA device.  exp(sum(scores) -
+    log_likelihood) is the posterior of the whole path, a confidence for the utterance.  ValueError with
+    free_ends=True and when the window min(beam_size, 2 L + 1) exceeds POSTERIOR_MAX_STATES (pass beam_size)."""
     import torch
     _check_beam(beam_size)
     _check_free_ends(free_ends, beam_size)
@@ -371,10 +413,20 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
     if T < L + R:
         raise RuntimeError(f"targets length is too long for CTC. Found log_probs length: {T}, targets length: {L}, "
                            f"and number of repeats: {R}")
+    if posteriors:
+        _check_posteriors(free_ends, beam_size, np.array([2 * L + 1]))
     dev = log_probs.device
     with AlignPlan.ctc([0, T], tg, [0, L], V, blank, device=dev.index if dev.type == "cuda" else _current_device(),
                        long_form=long_form, beam_size=beam_size, free_ends=free_ends) as plan:
-        if dev.type == "cuda":
+        if posteriors:
+            gdev = _span_device(log_probs)
+            with torch.cuda.device(gdev):
+                lp = log_probs[0].contiguous().to(gdev)
+                path, labs, scores, _, st = plan.run_torch(lp)
+                post, ll = plan.ctc_posteriors_torch(lp, path, st)
+                status = int(st[0])   # (synchronises: the plan is destroyed below)
+            labs, scores, post, ll = labs.to(dev), scores.to(dev), post.to(dev), ll.to(dev)
+        elif dev.type == "cuda":
             with torch.cuda.device(dev):
                 _, labs, scores, _, status = plan.run_torch(log_probs[0].contiguous())
                 status = int(status[0])   # (synchronises: the plan is destroyed below)
@@ -386,11 +438,13 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
     if status == ST_DEAD_BAND and beam_size is not None:
         raise _band_lost(beam_size)
     raise_for_status(status, V)
+    if posteriors:
+        return labs.to(targets.dtype).view(1, T), scores.view(1, T), post.view(1, T), ll
     return labs.to(targets.dtype).view(1, T), scores.view(1, T)
 
 
 def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=None, blank=0, *, long_form=False,
-                       beam_size=None, free_ends=False):
+                       beam_size=None, free_ends=False, posteriors=False):
     """forced_align for a padded batch, in one plan: log_probs float32 [B, T_max, V], targets
     int32 / int64 [B, L_max], input_lengths / target_lengths [B] (None: all full length).  Item b
     is aligned over its first input_lengths[b] frames and target_lengths[b] targets.  Returns
@@ -401,7 +455,10 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
     target ids run on the staged kernels and the others on the generic kernel (AlignPlan.ctc).
     beam_size: as in forced_align (each item's band follows its own T and S; the results are the best
     paths inside the bands); an item with no path inside its band raises ValueError naming it.
-    free_ends: as in forced_align, per item (each item's best window of its own frames)."""
+    free_ends: as in forced_align, per item (each item's best window of its own frames).
+    posteriors=True: as in forced_align, per item: (paths, scores, posteriors float32 [B, T_max] with 0 past an
+    item's length, log_likelihood float64 [B]); merge_tokens_batch(paths, posteriors, input_lengths) then gives
+    span scores that are mean posteriors.  ValueError naming the first item whose window is too wide."""
     import torch
     _check_beam(beam_size)
     _check_free_ends(free_ends, beam_size)
@@ -421,6 +478,8 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
         if tl[b] < ll[b] + R:
             raise RuntimeError(f"{where}targets length is too long for CTC. Found log_probs length: {tl[b]}, "
                                f"targets length: {ll[b]}, and number of repeats: {R}")
+    if posteriors:
+        _check_posteriors(free_ends, beam_size, 2 * ll + 1, lambda b: f"item {b}: ")
     t_off = np.concatenate([[0], np.cumsum(tl)]).astype(np.int64)
     l_off = np.concatenate([[0], np.cumsum(ll)]).astype(np.int64)
     labels = (np.concatenate([tg_all[b, :ll[b]] for b in range(B)]) if B else np.zeros(0, np.int64)).astype(np.int32)
@@ -428,11 +487,22 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
     valid = torch.arange(T_max, device=dev)[None, :] < torch.from_numpy(tl).to(dev)[:, None]   # [B, T_max]
     paths = torch.full((B, T_max), blank, dtype=targets.dtype, device=dev)
     scores = torch.zeros((B, T_max), dtype=torch.float32, device=dev)
+    if posteriors:
+        post_pad = torch.zeros((B, T_max), dtype=torch.float32, device=dev)
+        loglik = torch.zeros(B, dtype=torch.float64, device=dev)
     if B == 0:
-        return paths, scores
+        return (paths, scores, post_pad, loglik) if posteriors else (paths, scores)
     with AlignPlan.ctc(t_off, labels, l_off, V, blank, device=dev.index if dev.type == "cuda" else _current_device(),
                        long_form=long_form, beam_size=beam_size, free_ends=free_ends) as plan:
-        if dev.type == "cuda":
+        if posteriors:
+            gdev = _span_device(log_probs)
+            with torch.cuda.device(gdev):
+                lp = log_probs[valid].contiguous().to(gdev)   # rows packed on the input's device
+                path, labs, sc, _, st = plan.run_torch(lp)
+                post, loglik = plan.ctc_posteriors_torch(lp, path, st)
+                status = st.cpu().numpy()
+            labs, sc, post, loglik = labs.to(dev), sc.to(dev), post.to(dev), loglik.to(dev)
+        elif dev.type == "cuda":
             with torch.cuda.device(dev):
                 _, labs, sc, _, status = plan.run_torch(log_probs[valid].contiguous())   # rows packed on the device
                 status = status.cpu().numpy()
@@ -447,6 +517,9 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
         raise_for_status(int(status[b]), V)
     paths[valid] = labs.to(targets.dtype)
     scores[valid] = sc
+    if posteriors:
+        post_pad[valid] = post
+        return paths, scores, post_pad, loglik
     return paths, scores
 
 

@@ -30,6 +30,7 @@
 #include "kab_compact.cuh"
 #include "kab_debug.h"
 #include "kab_generic.cuh"
+#include "kab_posterior.cuh"
 #include "kab_softmax.cuh"
 #include "kab_segstats.cuh"
 #include "kab_spans.cuh"
@@ -247,6 +248,14 @@ struct kab_plan {
   KabSegmentRecord *d_seg_rec = nullptr;
   uint8_t *d_lab8 = nullptr;
   int64_t seg_cap = 0;
+  // CTC posteriors (kab_posterior.cuh), built at the first kab_plan_ctc_posteriors_device: a lattice list and
+  // launch per block size, the labels with their move-2 bits, the two [sum T] value rows
+  struct PostList { KabPostLat *d_lats = nullptr; int n = 0; Launch launch; int32_t bufcap = 0, e_words = 0; };
+  bool post_ready = false;
+  PostList post[3];
+  int32_t post_F = 0, post_p_words = 0;
+  int32_t *d_post_labs = nullptr;
+  double *d_post_scr = nullptr;
 };
 
 namespace {
@@ -298,6 +307,14 @@ void host_teardown(kab_plan *pl) {
   pl->host_ready = false;
 }
 
+// the posterior pass's device state (kab_plan_ctc_posteriors_device; also the undo of a failed set-up)
+void cleanup_post(kab_plan *pl) {
+  for (auto &l : pl->post) { pool_free(l.d_lats); l = kab_plan::PostList{}; }
+  pool_free(pl->d_post_labs); pool_free(pl->d_post_scr);
+  pl->d_post_labs = nullptr; pl->d_post_scr = nullptr;
+  pl->post_ready = false;
+}
+
 int plan_free(kab_plan *pl) {
   if (!pl) return KAB_OK;
   Trace tr("kab_plan_destroy");
@@ -322,6 +339,8 @@ int plan_free(kab_plan *pl) {
   for (int q = 0; q < N_QUEUES; ++q) pool_free(pl->d_lists[q]);
   pool_free(pl->d_col16); pool_free(pl->d_raw); pool_free(pl->d_bp); pool_free(pl->d_scratch);
   pool_free(pl->d_queue); pool_free(pl->d_status_init); pool_free(pl->d_wide_ws); pool_free(pl->d_band_fifo); pool_free(pl->d_bt_meta); pool_free(pl->d_bt_maps); pool_free(pl->d_bt_entry); pool_free(pl->d_end_state); pool_free(pl->d_gather); pool_free(pl->d_lpc); pool_free(pl->d_nonfinite); pool_free(pl->d_t_off); pool_free(pl->d_seg_scratch); pool_free(pl->d_started);
+
+  cleanup_post(pl);
   delete pl;
   tr.mark("free");
   return KAB_OK;
@@ -1188,6 +1207,112 @@ int kab_log_softmax_device(const float *d_logits, float *d_log_probs, int64_t n_
   }
   KAB_CUDA(cudaGetLastError());
   return KAB_OK;
+}
+
+namespace {
+// ---- CTC posteriors (kab_posterior.cuh): three block sizes, chosen per lattice by its pair slots per frame
+constexpr int POST_NT[3] = {64, 256, 1024};
+inline int post_class(int64_t np) { return np <= 128 ? 0 : np <= 1024 ? 1 : 2; }
+inline int64_t post_window(const kab_plan *pl, int64_t b) {
+  return std::min<int64_t>(pl->spec.W, 2 * (pl->h_l_off[b + 1] - pl->h_l_off[b]) + 1);
+}
+inline size_t post_smem(int32_t e_words, int32_t p_words, int32_t bufcap) {
+  return 8 * KAB_POST_NST + 16 + (size_t)KAB_POST_NST * (e_words + p_words) * 4 + (size_t)2 * bufcap * 4;
+}
+
+// The first kab_plan_ctc_posteriors_device of a plan: the labels with their move-2 bits, the lattice lists and
+// their launches, the value rows.  Emission rows are staged while the ring fits next to the state buffers.
+int post_setup(kab_plan *pl) {
+  const int64_t B = pl->B, V = pl->spec.V;
+  const std::vector<int64_t> &to = pl->h_t_off, &lo = pl->h_l_off;
+  const std::vector<int32_t> &lab = pl->h_labels;
+  std::vector<int32_t> labs((size_t)pl->total_L, 0);
+  for (int64_t b = 0; b < B; ++b)
+    for (int64_t l = lo[b]; l < lo[b + 1]; ++l) {
+      const bool in = l > lo[b] && lab[l] != lab[l - 1], out = l + 1 < lo[b + 1] && lab[l + 1] != lab[l];
+      labs[l] = (int32_t)((uint32_t)(lab[l] & 0xffff) | (uint32_t)in << 31 | (uint32_t)out << 30);
+    }
+  std::vector<KabPostLat> lists[3];
+  for (int64_t b = 0; b < B; ++b) {
+    const int64_t T = to[b + 1] - to[b], S = 2 * (lo[b + 1] - lo[b]) + 1;
+    const int64_t np = post_window(pl, b) / 2 + 2;
+    lists[post_class(np)].push_back(KabPostLat{to[b], lo[b], (int32_t)T, (int32_t)S, (int32_t)b, (int32_t)np,
+                                               unbanded(T, S, pl->spec.W) ? 0 : 1});
+  }
+  pl->post_F = (int32_t)std::max<int64_t>(1, std::min<int64_t>(16, 1024 / (4 * V)));
+  pl->post_p_words = (int32_t)(align_up(pl->post_F * 4, 16) + 32) / 4;
+  const int32_t e_words = (int32_t)((align_up(pl->post_F * V * 4, 16) + 32) / 4);
+  int rc;
+  for (int c = 0; c < 3; ++c) {
+    std::vector<KabPostLat> &v = lists[c];
+    kab_plan::PostList &pc = pl->post[c];
+    pc.n = (int)v.size();
+    if (v.empty()) continue;
+    std::sort(v.begin(), v.end(), [](const KabPostLat &x, const KabPostLat &y) {
+      return (int64_t)x.T * x.np > (int64_t)y.T * y.np;
+    });
+    int64_t np_max = 0;
+    for (const KabPostLat &x : v) np_max = std::max<int64_t>(np_max, x.np);
+    pc.bufcap = (int32_t)align_up(KAB_POST_PAD + 2 * np_max + KAB_POST_TAIL, 4);
+    pc.e_words = post_smem(e_words, pl->post_p_words, pc.bufcap) <= 227 * 1024 ? e_words : 0;
+    Launch &l = pc.launch;
+    l.fn = c == 0 ? (const void *)kab_ctc_posterior_kernel<POST_NT[0]>
+         : c == 1 ? (const void *)kab_ctc_posterior_kernel<POST_NT[1]> : (const void *)kab_ctc_posterior_kernel<POST_NT[2]>;
+    l.grid = dim3((unsigned)(2 * v.size()));
+    l.block = dim3(POST_NT[c]);
+    l.smem = post_smem(pc.e_words, pl->post_p_words, pc.bufcap);
+    cudaError_t e = ensure_dyn_smem(l.fn, pl->device, l.smem);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(posteriors)");
+    if ((rc = alloc((void **)&pc.d_lats, v.size() * sizeof(KabPostLat), "posterior lattices", v.data()))) return rc;
+  }
+  if ((rc = alloc((void **)&pl->d_post_labs, labs.size() * sizeof(int32_t), "posterior labels", labs.data()))) return rc;
+  if ((rc = alloc((void **)&pl->d_post_scr, (size_t)2 * std::max<int64_t>(pl->total_T, 1) * sizeof(double), "pool_malloc(posterior values)")))
+    return rc;
+  pl->post_ready = true;
+  return KAB_OK;
+}
+}  // namespace
+
+int kab_plan_ctc_posteriors_device(kab_plan *pl, const float *d_log_probs, const int32_t *d_best_path,
+                                   const int32_t *d_status, double *d_log_likelihood, float *d_posteriors,
+                                   void *stream_) {
+  if (!pl) return KAB_E_BAD_ARG;
+  if (!pl->spec.ctc || pl->spec.free_ends) return KAB_E_UNSUPPORTED;
+  for (int64_t b = 0; b < pl->B; ++b)
+    if (post_window(pl, b) > KAB_POSTERIOR_MAX_STATES) return KAB_E_UNSUPPORTED;
+  if (pl->B == 0) return KAB_OK;
+  if (!d_log_probs || !d_best_path || !d_status || !d_log_likelihood || !d_posteriors) return KAB_E_BAD_ARG;
+  if ((reinterpret_cast<uintptr_t>(d_log_probs) & 15) || (reinterpret_cast<uintptr_t>(d_best_path) & 3)) return KAB_E_BAD_ARG;
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  DeviceGuard guard;
+  KAB_CUDA(guard.enter(pl->device));
+  if (!pl->post_ready)
+    if (int rc = post_setup(pl)) { cleanup_post(pl); return rc; }
+  const uintptr_t pa = reinterpret_cast<uintptr_t>(d_best_path);
+  KabPostParams p{};
+  p.lp = d_log_probs; p.lp_bytes = pl->total_T * (int64_t)pl->spec.V * 4;
+  p.path_skew = (int32_t)((pa & 15) >> 2);
+  p.path = reinterpret_cast<const int32_t *>(pa & ~(uintptr_t)15);
+  p.path_bytes = (pl->total_T + p.path_skew) * 4;
+  p.labs = pl->d_post_labs; p.status = d_status;
+  p.fwd = pl->d_post_scr; p.bwd = pl->d_post_scr + std::max<int64_t>(pl->total_T, 1);
+  p.log_likelihood = d_log_likelihood;
+  p.W = pl->spec.W; p.V = pl->spec.V; p.blank = pl->spec.blank;
+  p.F = pl->post_F; p.p_words = pl->post_p_words;
+  for (const kab_plan::PostList &pc : pl->post) {
+    if (!pc.n) continue;
+    KabPostParams q = p;
+    q.e_words = pc.e_words; q.bufcap = pc.bufcap;
+    const KabPostLat *lats = pc.d_lats;
+    void *args[2] = {&lats, &q};
+    KAB_CUDA(cudaLaunchKernel(pc.launch.fn, pc.launch.grid, pc.launch.block, args, pc.launch.smem, stream));
+  }
+  const unsigned grid = (unsigned)std::min<int64_t>((pl->total_T + 255) / 256, (int64_t)pl->sm_count * 8);
+  if (grid > 0)
+    kab_ctc_posterior_combine_kernel<<<grid, 256, 0, stream>>>(pl->d_t_off, pl->B, pl->total_T, d_status, p.fwd, p.bwd,
+                                                               d_log_likelihood, d_posteriors);
+  KAB_CUDA(cudaGetLastError());
+  return record_run_event(pl, stream);
 }
 
 namespace {
