@@ -267,12 +267,19 @@ int kab_plan_segment_stats_device(kab_plan *plan, const int32_t *d_best_path, co
  *     the window gives 0).
  * A lattice whose d_status is not 0 gets posteriors 0 and log-likelihood NaN; log Z = -inf gives
  * posteriors 0.  d_log_probs are the caller's [sum T, V] rows (16-byte aligned), read by label: any
- * vocab_size works.  KAB_E_UNSUPPORTED for a plan that is not a CTC plan, a free-ends plan, or a lattice
- * whose window min(beam_size, S) exceeds KAB_POSTERIOR_MAX_STATES (use kab_plan_create_ctc_band).  The
- * first call builds and uploads what the pass needs (labels, lattice lists, 16 bytes per frame of
- * values); kab_plan_get_info does not count it.  Asynchronous on `stream`; kab_plan_destroy waits for it.
+ * vocab_size works.  A window of up to KAB_POSTERIOR_MAX_STATES states runs in one CTA.  The lattices of a
+ * kab_plan_create_ctc_long plan with more states (S up to KAB_POSTERIOR_LONG_MAX_STATES) run on a chain of
+ * warps over the whole GPU (DESIGN.md 3.9g), the same quantities with the same tolerances; such a plan's
+ * first call checks that the chain's grid can be resident.  KAB_E_UNSUPPORTED for a plan that is not a CTC
+ * plan, a free-ends plan, a lattice of a kab_plan_create_ctc or kab_plan_create_ctc_band plan whose window
+ * min(beam_size, S) exceeds KAB_POSTERIOR_MAX_STATES (use kab_plan_create_ctc_band or _long), a long-form
+ * lattice above KAB_POSTERIOR_LONG_MAX_STATES, or a chain grid the device cannot hold.  The first call
+ * builds and uploads what the pass needs (labels, lattice lists, 16 bytes per frame of values, and 8 KB per
+ * 256 states of a long-form lattice above the limit for the chain's FIFOs); kab_plan_get_info does not count
+ * it.  Asynchronous on `stream`; kab_plan_destroy waits for it.
  */
 #define KAB_POSTERIOR_MAX_STATES 28000 /* the states of two float buffers in one CTA's shared memory */
+#define KAB_POSTERIOR_LONG_MAX_STATES 324001 /* long-form plans: a three-hour lattice on a B200's resident warps */
 int kab_plan_ctc_posteriors_device(kab_plan *plan, const float *d_log_probs, const int32_t *d_best_path,
                                    const int32_t *d_status, double *d_log_likelihood, float *d_posteriors,
                                    void *stream);

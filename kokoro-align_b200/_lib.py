@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _ROOT = os.path.dirname(_HERE)
 SO_PATH = os.path.join(_HERE, "libkokoro_align_b200.so")
 SOURCES = [os.path.join(_HERE, "csrc", f) for f in
-           ("kab_api.cu", "kab_common.cuh", "kab_warp.cuh", "kab_band.cuh", "kab_bandp.cuh", "kab_bandq.cuh", "kab_bandr.cuh", "kab_btpar.cuh", "kab_wide.cuh", "kab_segstats.cuh", "kab_posterior.cuh", "kab_spans.cuh", "kab_compact.cuh", "kab_generic.cuh", "kab_softmax.cuh", "kab_pool.h", "kab_text.h", "kab_debug.h")]
+           ("kab_api.cu", "kab_common.cuh", "kab_warp.cuh", "kab_band.cuh", "kab_bandp.cuh", "kab_bandq.cuh", "kab_bandr.cuh", "kab_btpar.cuh", "kab_wide.cuh", "kab_segstats.cuh", "kab_posterior.cuh", "kab_posterior_chain.cuh", "kab_spans.cuh", "kab_compact.cuh", "kab_generic.cuh", "kab_softmax.cuh", "kab_pool.h", "kab_text.h", "kab_debug.h")]
 HEADER = os.path.join(_ROOT, "include", "kokoro_align_b200.h")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
@@ -20,6 +20,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 KAB_OK, KAB_E_CUDA, KAB_E_BAD_ARG, KAB_E_NOMEM, KAB_E_UNSUPPORTED = 0, -1, -2, -3, -4
 ST_OK, ST_DEAD_BAND, ST_BAD_LABEL, ST_NONFINITE = 0, 1, 2, 3
 POSTERIOR_MAX_STATES = 28000  # KAB_POSTERIOR_MAX_STATES
+POSTERIOR_LONG_MAX_STATES = 324001  # KAB_POSTERIOR_LONG_MAX_STATES
 
 EXPORTS = ["kab_version", "kab_error_string", "kab_last_cuda_error", "kab_device_count",
            "kab_plan_create", "kab_plan_create_ctc", "kab_plan_create_ctc_long", "kab_plan_create_ctc_free", "kab_plan_create_ctc_band", "kab_plan_get_info", "kab_plan_destroy", "kab_plan_run_device",

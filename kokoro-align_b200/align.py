@@ -250,7 +250,9 @@ class AlignPlan:
         log Z), the probability that the lattice's paths pass through state p_t at frame t (0 where p_t is outside
         the window), and log Z, the log of the total probability of the transcript (-ctc_loss; a banded plan: of
         the paths inside the band).  A lattice whose status is not 0 gets 0 and NaN.  Asynchronous.  KabError for
-        a Kokoro or free-ends plan and for a window min(beam_size, S) above POSTERIOR_MAX_STATES."""
+        a Kokoro or free-ends plan and for a window min(beam_size, S) above POSTERIOR_MAX_STATES, except in a
+        long_form plan without beam_size: there lattices up to POSTERIOR_LONG_MAX_STATES run on a chain of warps
+        over the whole GPU (DESIGN.md 3.9g)."""
         import torch
         assert log_probs.is_cuda and log_probs.dtype == torch.float32 and log_probs.is_contiguous()
         assert tuple(log_probs.shape) == (self.total_T, self.V), (tuple(log_probs.shape), self.total_T, self.V)
@@ -349,11 +351,20 @@ def _check_free_ends(free_ends, beam_size):
                          "spans the whole recording")
 
 
-def _check_posteriors(free_ends, beam_size, S, where=lambda b: ""):
-    """posteriors=True: no free ends, and every item's window min(beam_size, S) within the posterior pass's limit.
+def _check_posteriors(free_ends, beam_size, S, where=lambda b: "", long_form=False):
+    """posteriors=True: no free ends, and every item's window min(beam_size, S) within the posterior pass's limit
+    (long_form=True without beam_size: S within POSTERIOR_LONG_MAX_STATES, the chain pass of DESIGN.md 3.9g).
     S: int64 numpy [B] states per item."""
     if free_ends:
         raise ValueError("posteriors=True does not combine with free_ends=True")
+    if long_form and beam_size is None:
+        over = np.flatnonzero(S > _lib.POSTERIOR_LONG_MAX_STATES)
+        if over.size:
+            b = int(over[0])
+            raise ValueError(f"{where(b)}long-form posteriors need at most {_lib.POSTERIOR_LONG_MAX_STATES} states, the "
+                             f"item has S = {int(S[b])} (2 L + 1); pass beam_size <= {_lib.POSTERIOR_MAX_STATES} for "
+                             f"banded posteriors")
+        return
     w = S if beam_size is None else np.minimum(S, int(beam_size))
     over = np.flatnonzero(w > _lib.POSTERIOR_MAX_STATES)
     if over.size:
@@ -395,7 +406,10 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
     same plan and rows: (paths, scores, posteriors float32 [1, T], log_likelihood float64 [1]).  The paths and
     scores are those of posteriors=False; CPU tensors run on the current CUDA device.  exp(sum(scores) -
     log_likelihood) is the posterior of the whole path, a confidence for the utterance.  ValueError with
-    free_ends=True and when the window min(beam_size, 2 L + 1) exceeds POSTERIOR_MAX_STATES (pass beam_size)."""
+    free_ends=True and when the window min(beam_size, 2 L + 1) exceeds POSTERIOR_MAX_STATES (pass beam_size).
+    With long_form=True and no beam_size the limit is POSTERIOR_LONG_MAX_STATES (324 001 states, a three-hour
+    recording): lattices above POSTERIOR_MAX_STATES run on a chain of warps over the whole GPU (DESIGN.md 3.9g),
+    exact, unbanded, log_likelihood = -ctc_loss."""
     import torch
     _check_beam(beam_size)
     _check_free_ends(free_ends, beam_size)
@@ -414,7 +428,7 @@ def forced_align(log_probs, targets, input_lengths=None, target_lengths=None, bl
         raise RuntimeError(f"targets length is too long for CTC. Found log_probs length: {T}, targets length: {L}, "
                            f"and number of repeats: {R}")
     if posteriors:
-        _check_posteriors(free_ends, beam_size, np.array([2 * L + 1]))
+        _check_posteriors(free_ends, beam_size, np.array([2 * L + 1]), long_form=long_form)
     dev = log_probs.device
     with AlignPlan.ctc([0, T], tg, [0, L], V, blank, device=dev.index if dev.type == "cuda" else _current_device(),
                        long_form=long_form, beam_size=beam_size, free_ends=free_ends) as plan:
@@ -458,7 +472,8 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
     free_ends: as in forced_align, per item (each item's best window of its own frames).
     posteriors=True: as in forced_align, per item: (paths, scores, posteriors float32 [B, T_max] with 0 past an
     item's length, log_likelihood float64 [B]); merge_tokens_batch(paths, posteriors, input_lengths) then gives
-    span scores that are mean posteriors.  ValueError naming the first item whose window is too wide."""
+    span scores that are mean posteriors.  ValueError naming the first item whose window is too wide (long_form:
+    whose S exceeds POSTERIOR_LONG_MAX_STATES)."""
     import torch
     _check_beam(beam_size)
     _check_free_ends(free_ends, beam_size)
@@ -479,7 +494,7 @@ def forced_align_batch(log_probs, targets, input_lengths=None, target_lengths=No
             raise RuntimeError(f"{where}targets length is too long for CTC. Found log_probs length: {tl[b]}, "
                                f"targets length: {ll[b]}, and number of repeats: {R}")
     if posteriors:
-        _check_posteriors(free_ends, beam_size, 2 * ll + 1, lambda b: f"item {b}: ")
+        _check_posteriors(free_ends, beam_size, 2 * ll + 1, lambda b: f"item {b}: ", long_form)
     t_off = np.concatenate([[0], np.cumsum(tl)]).astype(np.int64)
     l_off = np.concatenate([[0], np.cumsum(ll)]).astype(np.int64)
     labels = (np.concatenate([tg_all[b, :ll[b]] for b in range(B)]) if B else np.zeros(0, np.int64)).astype(np.int32)

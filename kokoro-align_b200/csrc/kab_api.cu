@@ -31,6 +31,7 @@
 #include "kab_debug.h"
 #include "kab_generic.cuh"
 #include "kab_posterior.cuh"
+#include "kab_posterior_chain.cuh"
 #include "kab_softmax.cuh"
 #include "kab_segstats.cuh"
 #include "kab_spans.cuh"
@@ -256,6 +257,15 @@ struct kab_plan {
   int32_t post_F = 0, post_p_words = 0;
   int32_t *d_post_labs = nullptr;
   double *d_post_scr = nullptr;
+  // ... and the chain pass (kab_posterior_chain.cuh) of unbanded long-form lattices above
+  // KAB_POSTERIOR_MAX_STATES: its lattice list, launch (split: kab_ctc_posterior_chain_kernel's argument) and
+  // workspace (control words and FIFOs, zeroed before every call)
+  int64_t post_chain_min = KAB_POSTERIOR_MAX_STATES;  // lattices with more states take the chain pass
+  KabPostChainLat *d_post_chain = nullptr;
+  int post_chain_n = 0, post_chain_split = 0;
+  Launch post_chain;
+  unsigned char *d_post_chain_ws = nullptr;
+  int64_t post_chain_ws_bytes = 0;
 };
 
 namespace {
@@ -310,8 +320,9 @@ void host_teardown(kab_plan *pl) {
 // the posterior pass's device state (kab_plan_ctc_posteriors_device; also the undo of a failed set-up)
 void cleanup_post(kab_plan *pl) {
   for (auto &l : pl->post) { pool_free(l.d_lats); l = kab_plan::PostList{}; }
-  pool_free(pl->d_post_labs); pool_free(pl->d_post_scr);
-  pl->d_post_labs = nullptr; pl->d_post_scr = nullptr;
+  pool_free(pl->d_post_labs); pool_free(pl->d_post_scr); pool_free(pl->d_post_chain); pool_free(pl->d_post_chain_ws);
+  pl->d_post_labs = nullptr; pl->d_post_scr = nullptr; pl->d_post_chain = nullptr; pl->d_post_chain_ws = nullptr;
+  pl->post_chain_n = 0; pl->post_chain_split = 0; pl->post_chain = Launch{}; pl->post_chain_ws_bytes = 0;
   pl->post_ready = false;
 }
 
@@ -1216,6 +1227,11 @@ inline int post_class(int64_t np) { return np <= 128 ? 0 : np <= 1024 ? 1 : 2; }
 inline int64_t post_window(const kab_plan *pl, int64_t b) {
   return std::min<int64_t>(pl->spec.W, 2 * (pl->h_l_off[b + 1] - pl->h_l_off[b]) + 1);
 }
+// an unbanded lattice of a long-form plan (not free ends) above the single-CTA limit: the chain pass
+inline bool post_chained(const kab_plan *pl, int64_t b) {
+  const PlanSpec &s = pl->spec;
+  return s.ctc_long && !s.free_ends && s.W == CTC_W && 2 * (pl->h_l_off[b + 1] - pl->h_l_off[b]) + 1 > pl->post_chain_min;
+}
 inline size_t post_smem(int32_t e_words, int32_t p_words, int32_t bufcap) {
   return 8 * KAB_POST_NST + 16 + (size_t)KAB_POST_NST * (e_words + p_words) * 4 + (size_t)2 * bufcap * 4;
 }
@@ -1233,8 +1249,17 @@ int post_setup(kab_plan *pl) {
       labs[l] = (int32_t)((uint32_t)(lab[l] & 0xffff) | (uint32_t)in << 31 | (uint32_t)out << 30);
     }
   std::vector<KabPostLat> lists[3];
+  std::vector<KabPostChainLat> chain;
+  int nw_max = 0;
   for (int64_t b = 0; b < B; ++b) {
     const int64_t T = to[b + 1] - to[b], S = 2 * (lo[b + 1] - lo[b]) + 1;
+    if (post_chained(pl, b)) {
+      const int nw = (int)((S + 1) / 2 + KAB_PC_PAIRS - 1) / KAB_PC_PAIRS;
+      chain.push_back(KabPostChainLat{to[b], lo[b], pl->post_chain_ws_bytes, (int32_t)T, (int32_t)S, (int32_t)b, nw});
+      pl->post_chain_ws_bytes += (int64_t)align_up((int64_t)kab_pc_ws_bytes(nw), 256);
+      nw_max = std::max(nw_max, nw);
+      continue;
+    }
     const int64_t np = post_window(pl, b) / 2 + 2;
     lists[post_class(np)].push_back(KabPostLat{to[b], lo[b], (int32_t)T, (int32_t)S, (int32_t)b, (int32_t)np,
                                                unbanded(T, S, pl->spec.W) ? 0 : 1});
@@ -1265,6 +1290,28 @@ int post_setup(kab_plan *pl) {
     if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(posteriors)");
     if ((rc = alloc((void **)&pc.d_lats, v.size() * sizeof(KabPostLat), "posterior lattices", v.data()))) return rc;
   }
+  if (!chain.empty()) {
+    // every warp of the chain spins on its neighbours: the whole grid must be resident (a cooperative launch
+    // refuses rather than hangs); both directions side by side when they fit, else one after the other
+    Launch &l = pl->post_chain;
+    l.fn = (const void *)kab_ctc_posterior_chain_kernel;
+    l.block = dim3(KAB_PC_CW * 32);
+    l.cooperative = true;
+    int occ = 0;
+    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, l.fn, KAB_PC_CW * 32, 0);
+    if (e != cudaSuccess) return cuda_fail(e, "occupancy(posterior chain)");
+    const int64_t capacity = (int64_t)occ * pl->sm_count, ctas = (nw_max + KAB_PC_CW - 1) / KAB_PC_CW;
+    const bool serial = getenv("KAB_POSTERIOR_CHAIN_SERIAL") != nullptr;  // test knob: one direction at a time
+    if (ctas > capacity) return KAB_E_UNSUPPORTED;
+    const bool side = 2 * ctas <= capacity && !serial;
+    pl->post_chain_split = side ? (int)ctas * KAB_PC_CW : 0;
+    l.grid = dim3((unsigned)(side ? 2 * ctas : ctas));
+    pl->post_chain_n = (int)chain.size();
+    if ((rc = alloc((void **)&pl->d_post_chain, chain.size() * sizeof(KabPostChainLat), "posterior chain lattices", chain.data())))
+      return rc;
+    if ((rc = alloc((void **)&pl->d_post_chain_ws, (size_t)pl->post_chain_ws_bytes, "pool_malloc(posterior chain workspace)")))
+      return rc;
+  }
   if ((rc = alloc((void **)&pl->d_post_labs, labs.size() * sizeof(int32_t), "posterior labels", labs.data()))) return rc;
   if ((rc = alloc((void **)&pl->d_post_scr, (size_t)2 * std::max<int64_t>(pl->total_T, 1) * sizeof(double), "pool_malloc(posterior values)")))
     return rc;
@@ -1278,8 +1325,14 @@ int kab_plan_ctc_posteriors_device(kab_plan *pl, const float *d_log_probs, const
                                    void *stream_) {
   if (!pl) return KAB_E_BAD_ARG;
   if (!pl->spec.ctc || pl->spec.free_ends) return KAB_E_UNSUPPORTED;
+  if (!pl->post_ready) {  // test knob: move lattices with more states than this to the chain pass
+    const char *knob = getenv("KAB_POSTERIOR_CHAIN_MIN_STATES");
+    pl->post_chain_min = knob ? std::min<int64_t>(atoll(knob), KAB_POSTERIOR_MAX_STATES) : KAB_POSTERIOR_MAX_STATES;
+  }
   for (int64_t b = 0; b < pl->B; ++b)
-    if (post_window(pl, b) > KAB_POSTERIOR_MAX_STATES) return KAB_E_UNSUPPORTED;
+    if (post_chained(pl, b) ? 2 * (pl->h_l_off[b + 1] - pl->h_l_off[b]) + 1 > KAB_POSTERIOR_LONG_MAX_STATES
+                            : post_window(pl, b) > KAB_POSTERIOR_MAX_STATES)
+      return KAB_E_UNSUPPORTED;
   if (pl->B == 0) return KAB_OK;
   if (!d_log_probs || !d_best_path || !d_status || !d_log_likelihood || !d_posteriors) return KAB_E_BAD_ARG;
   if ((reinterpret_cast<uintptr_t>(d_log_probs) & 15) || (reinterpret_cast<uintptr_t>(d_best_path) & 3)) return KAB_E_BAD_ARG;
@@ -1306,6 +1359,16 @@ int kab_plan_ctc_posteriors_device(kab_plan *pl, const float *d_log_probs, const
     const KabPostLat *lats = pc.d_lats;
     void *args[2] = {&lats, &q};
     KAB_CUDA(cudaLaunchKernel(pc.launch.fn, pc.launch.grid, pc.launch.block, args, pc.launch.smem, stream));
+  }
+  if (pl->post_chain_n) {
+    KAB_CUDA(cudaMemsetAsync(pl->d_post_chain_ws, 0, (size_t)pl->post_chain_ws_bytes, stream));
+    const KabPostChainLat *lats = pl->d_post_chain;
+    int n = pl->post_chain_n, split = pl->post_chain_split;
+    unsigned char *ws = pl->d_post_chain_ws;
+    void *args[5] = {&lats, &n, &p, &ws, &split};
+    cudaLaunchAttribute at[1];
+    const cudaLaunchConfig_t cfg = launch_config(pl->post_chain, at, stream);
+    KAB_CUDA(cudaLaunchKernelExC(&cfg, pl->post_chain.fn, args));
   }
   const unsigned grid = (unsigned)std::min<int64_t>((pl->total_T + 255) / 256, (int64_t)pl->sm_count * 8);
   if (grid > 0)
